@@ -20,6 +20,9 @@ latencies (`e2e_python`).  `--workload cfg2|cfg3|cfg4` makes one of those the ma
            steps are also measured with two host threads / contexts (the copies of one step overlap the kernels of
            the other) and `e2e.value` is the better of the two, both are in the line
 
+`--dump-outputs DIR` writes what the last timed step returned (job_means.npy or scores.npy, float64) for comparing two
+builds output for output; the inputs depend only on the arguments (seeded generator).
+
 `--impl reference` times the CPU restatement of the reference algorithm (oracle/, all host threads; the Rust crate
 cannot be built in this image) on a bounded sample of the same workload.  That arm imports only `benchdata` and
 `oracle`: it never maps the CUDA library.
@@ -40,6 +43,7 @@ import numpy as np
 ROOT = Path(__file__).resolve().parent
 if str(ROOT) not in sys.path:
     sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (it may be read-only)
 
 
 
@@ -627,6 +631,26 @@ def python_api_latency(local_rank):
     return out
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, result, means_only, rank, world):
+    """--dump-outputs: what the last timed step handed to its caller (the per-structure-pair means, or the per-anchor
+    scores), float64, as OUT_DIR/<name>.npy; one file per rank when several run.  Above 64 MB in all, the values at a
+    fixed set of positions (seeded, sorted) are written instead, as <name>_sample.npy, so that two builds run with the
+    same arguments can still be compared value for value."""
+    name = ("job_means" if means_only else "scores") + (f"_rank{rank}" if world > 1 else "")
+    result = np.asarray(result, dtype=np.float64)
+    cap = DUMP_BYTES // (8 * world)
+    if len(result) > cap:
+        result = result[np.unique(np.random.default_rng(0).integers(0, len(result), size=cap))]
+        name += "_sample"
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / f"{name}.npy", result)
+    return out / f"{name}.npy"
+
+
 def run_gpu(args, rank, local_rank, world):
     stdout_fd = quiet_stdout()
     _ensure_built()
@@ -642,6 +666,8 @@ def run_gpu(args, rank, local_rank, world):
         wl.desc += f" [threshold overridden: {wl.threshold:g}]"
     ctx = _capi.Context(local_rank)
     m = measure(wl, ctx, local_rank, ranks, args.steps, args.warmup, args)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, m["check_scores"], m["means_only"], rank, world)
     if rank != 0:
         ctx.close()
         ranks.close()
@@ -824,7 +850,14 @@ def main():
     ap.add_argument("--score-cap", type=int, default=1 << 28,
                     help="above this many anchor pairs per GPU per step only the per-job means are copied out")
     ap.add_argument("--threshold", type=float, default=0.0, help="override the 10 A threshold (exploration only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the results of the last one to DIR/<name>.npy (float64, at most "
+                         "64 MB in all; a fixed seeded sample of larger results)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results; the reference arm has none")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     rank = int(os.environ.get("RANK", "0"))

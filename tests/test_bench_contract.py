@@ -1,11 +1,16 @@
 """bench.py's output contract as far as it can be checked without a GPU: the reference arm (`--impl reference`, the
 oracle port on the host cores) prints exactly one JSON line on stdout with the keys the driver reads, and under a
 multi-rank launch only rank 0 prints."""
+import argparse
+import importlib.util
 import json
 import os
 import subprocess
 import sys
 from pathlib import Path
+
+import numpy as np
+import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
 REQUIRED = {"impl", "metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
@@ -116,3 +121,48 @@ def test_other_workload_entry_is_built_from_a_measurement(monkeypatch):
     assert out["value"] == 1.0e8 and out["anchor_pairs_per_step"] == 2 * 300 and out["gpu_launches"] == 12
     assert out["kernel_ms_per_step"] == {"score": 1.2, "fill": 0.6} and abs(sum(out["kernel_share"].values()) - 1.0) < 1e-12
     assert out["env_size_mean"] == 150.0 and out["roofline_step_frac_fp64"] > 0
+
+
+def _load_bench(name):
+    spec = importlib.util.spec_from_file_location(name, ROOT / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    return bench
+
+
+def test_dump_outputs_writes_float64_within_the_cap(tmp_path):
+    """bench.dump_outputs (--dump-outputs): small results are written whole; above 64 MB in all the same seeded,
+    sorted positions are kept on every run, and each rank of a multi-rank launch gets its share of the cap."""
+    bench = _load_bench("_bench_mod3")
+    small = np.arange(10, dtype=np.float64)
+    p = bench.dump_outputs(tmp_path / "a", small, True, 0, 1)
+    assert p == tmp_path / "a" / "job_means.npy" and np.array_equal(np.load(p), small)
+    big = np.arange(bench.DUMP_BYTES // 8 + 1000, dtype=np.float64)   # value = position
+    p1 = bench.dump_outputs(tmp_path / "b", big, False, 0, 1)
+    p2 = bench.dump_outputs(tmp_path / "c", big, False, 0, 1)
+    v1 = np.load(p1)
+    assert p1.name == "scores_sample.npy" and v1.dtype == np.float64 and 0 < v1.nbytes <= bench.DUMP_BYTES
+    assert np.all(np.diff(v1) > 0) and v1[-1] < len(big) and np.array_equal(v1, np.load(p2))
+    p3 = bench.dump_outputs(tmp_path / "d", big, False, 1, 2)
+    assert p3.name == "scores_rank1_sample.npy" and np.load(p3).nbytes <= bench.DUMP_BYTES // 2
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dumps_the_last_steps_results(tmp_path, oracle_mod):
+    """--dump-outputs on a 4-member ensemble: job_means.npy holds the 6 structure-pair means of the last timed step,
+    which equal the oracle's within 1e-9."""
+    cmd = [sys.executable, str(ROOT / "bench.py"), "--steps", "2", "--warmup", "3", "--ensemble", "4",
+           "--no-cpu-baseline", "--no-extras", "--dump-outputs", str(tmp_path)]
+    res = subprocess.run(cmd, capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert res.returncode == 0, res.stderr[-2000:]
+    assert json.loads(res.stdout)["steps"] == 2
+    got = np.load(tmp_path / "job_means.npy")
+    bench = _load_bench("_bench_mod4")
+    wl = bench.make_workload("cfg5", 0, 1, argparse.Namespace(ensemble=4))
+    op = bench.oracle_params(oracle_mod, wl)
+    want = []
+    for j in range(len(wl.jobs)):
+        a, b, anchors = wl.job_arrays(j)
+        want.append(oracle_mod.from_primitives(op, a.xyz, a.cat, a.tag, b.xyz, b.cat, b.tag, anchors, wl.threshold).mean())
+    assert got.dtype == np.float64 and got.shape == (6,)
+    assert np.abs(got - np.array(want)).max() <= 1e-9

@@ -1,7 +1,7 @@
 """Runs the reference's OWN, unmodified unittest files (tests/test_wfs.py, test_tag_pairing_rule.py, test_locohd.py of
 fazekaszs/loco_hd) against this repository's drop-in `loco_hd` package.
 
-    python tools/run_reference_tests.py [DIR]      DIR defaults to /root/reference/tests
+    python tools/run_reference_tests.py [DIR]      DIR: tests/ of a reference checkout ($LOCOHD_REFERENCE_TESTS)
 
 The files are loaded by path (so that `import loco_hd` inside them resolves to this repository, not to the reference's
 pure-Python package directory next to them); nothing is copied.  Prints one JSON line: tests run, passed, skipped, and
@@ -13,6 +13,7 @@ host-side classes (weight functions, tag pairing rules, constructor validation) 
 import importlib.util
 import io
 import json
+import os
 import sys
 import unittest
 from pathlib import Path
@@ -41,7 +42,7 @@ def run(test_dir: Path) -> dict:
 
 
 if __name__ == "__main__":
-    d = Path(sys.argv[1]) if len(sys.argv) > 1 else Path("/root/reference/tests")
+    d = Path(sys.argv[1] if len(sys.argv) > 1 else os.environ["LOCOHD_REFERENCE_TESTS"])
     out = run(d)
     print(json.dumps(out))
     sys.exit(0 if not out["not_passed"] else 1)
