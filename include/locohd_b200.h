@@ -240,6 +240,15 @@ int locohd_plan_job_tiles(uint64_t n_jobs, const locohd_job* jobs, uint64_t* out
  * range. */
 int locohd_tile_unit(uint64_t n_tiles, uint64_t n_anchors, uint64_t slice, uint64_t unit, uint64_t* out_tile,
                      uint64_t* out_anchor);
+/* Planning query, no device needed: the launch geometry of the tile kernel for an instance of n_categories categories
+ * in the configuration the tile kernel requires (Hellinger-2, unit category weights, one weight function) and
+ * environment sets whose largest environments hold max_a / max_b members.  *teams = teams of four warps per CTA (0: the
+ * tile kernel does not apply; locohd_score_jobs[_stats] takes it only from 6 teams on), *cp = count rows per warp (8 for
+ * n_categories <= 8, else 16), *rep_n = head of the count-indexed tables replicated per bank pair (0: unreplicated),
+ * *table_n = entries per table.  LOCOHD_TILE_TEAMS / LOCOHD_TILE_REP in the environment lower teams / rep_n, as they do
+ * for a launch.  cp, rep_n and table_n may be NULL. */
+int locohd_tile_geometry(int n_categories, uint32_t max_a, uint32_t max_b, int* teams, int* cp, int* rep_n,
+                         int* table_n);
 /* from_anchors (locohd.rs:392-406): one pair of caller-ordered environments, walked in the reference's
  * exact three-way-merge order (the lists are NOT required to be sorted, as in the reference). */
 int locohd_score_anchor_lists(locohd_ctx* ctx, const uint16_t* seq_a, uint64_t len_a, const double* dists_a,

@@ -32,7 +32,7 @@ EXPORTED_SYMBOLS = [
     "locohd_envset_from_ragged_rows",
     "locohd_envset_from_coords", "locohd_envset_destroy", "locohd_envset_size", "locohd_envset_total_members",
     "locohd_envset_dump", "locohd_score_pairs", "locohd_score_jobs", "locohd_score_jobs_stats",
-    "locohd_score_anchor_lists", "locohd_plan_job_tiles", "locohd_tile_unit",
+    "locohd_score_anchor_lists", "locohd_plan_job_tiles", "locohd_tile_unit", "locohd_tile_geometry",
     "locohd_from_primitives", "locohd_wf_integral_points", "locohd_sd_run",
 ]
 
@@ -124,6 +124,8 @@ def load_library() -> C.CDLL:
         "locohd_score_anchor_lists": (C.c_int, [vp, vp, u64, vp, u64, vp, u64, vp, u64, u32, vp]),
         "locohd_plan_job_tiles": (C.c_int, [u64, vp, vp, vp, vp]),
         "locohd_tile_unit": (C.c_int, [u64, u64, u64, u64, C.POINTER(u64), C.POINTER(u64)]),
+        "locohd_tile_geometry": (C.c_int, [C.c_int, u32, u32, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                           C.POINTER(C.c_int)]),
         "locohd_from_primitives": (C.c_int, [vp, u64, vp, vp, vp, u64, vp, vp, vp, u64, vp, vp, dbl, vp]),
         "locohd_wf_integral_points": (C.c_int, [vp, C.POINTER(WeightFunctionC), u64, vp, vp]),
         "locohd_sd_run": (C.c_int, [vp, i32, vp, i32, u64, vp, vp, vp]),
@@ -170,6 +172,18 @@ def tile_unit(n_tiles: int, n_anchors: int, slice_: int, unit: int):
     if st:
         raise LocoHDError(st, "locohd_tile_unit")
     return int(t.value), int(p.value)
+
+
+def tile_geometry(n_categories: int, max_a: int, max_b: int) -> dict:
+    """Launch geometry of the tile kernel for environments of at most max_a / max_b members (locohd_tile_geometry;
+    host-side, no device).  Returns {"teams", "cp", "rep_n", "table_n"}; teams == 0: the tile kernel does not apply,
+    and jobs take it only from 6 teams on."""
+    teams, cp, rep_n, table_n = C.c_int(), C.c_int(), C.c_int(), C.c_int()
+    st = load_library().locohd_tile_geometry(n_categories, max_a, max_b, C.byref(teams), C.byref(cp), C.byref(rep_n),
+                                             C.byref(table_n))
+    if st:
+        raise LocoHDError(st, "locohd_tile_geometry")
+    return {"teams": teams.value, "cp": cp.value, "rep_n": rep_n.value, "table_n": table_n.value}
 
 
 def make_wf(name: str, params: Sequence[float]) -> WeightFunctionC:

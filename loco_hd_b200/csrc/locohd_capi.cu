@@ -1389,6 +1389,21 @@ int locohd_tile_unit(uint64_t n_tiles, uint64_t n_anchors, uint64_t slice, uint6
     return LOCOHD_OK;
 }
 
+int locohd_tile_geometry(int n_categories, uint32_t max_a, uint32_t max_b, int* teams, int* cp, int* rep_n,
+                         int* table_n) {
+    if (!teams) return LOCOHD_ERR_BAD_PARAM;
+    KParams p{};
+    p.C = n_categories;
+    p.hell2 = 1;
+    p.unit_w = 1;
+    const TileGeometry g = tile_geometry(p, max_a, max_b, 1);
+    *teams = g.teams;
+    if (cp) *cp = g.cp;
+    if (rep_n) *rep_n = g.rep_n;
+    if (table_n) *table_n = g.table_n;
+    return LOCOHD_OK;
+}
+
 int locohd_score_jobs(locohd_ctx* ctx, const locohd_envset* a, const locohd_envset* b, uint64_t n_jobs,
                       const locohd_job* jobs, const uint32_t* wf_idx, double* out_scores, double* out_job_means) {
     return locohd_score_jobs_stats(ctx, a, b, n_jobs, jobs, wf_idx, out_scores, out_job_means, nullptr, nullptr);

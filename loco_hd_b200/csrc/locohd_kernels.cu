@@ -2780,36 +2780,34 @@ static int launch_fast(const ScoreArgs& a, const KParams& p, bool check, int war
                  : launch_score_kernel(score_fast_kernel<CP, KEY_IS_W, false, false>, a, p, warps, per_warp, smem, st);
 }
 
-// Tile kernel geometry for environments of at most max_a / max_b members: teams per CTA (0: not applicable).
-static int tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, int* table_n_out,
-                         int* stage_keys_out, int* team_bytes_out, int* rep_n_out) {
-    if (!(p.hell2 && p.unit_w && p.C <= 16 && key_is_w)) return 0;   // the configuration of score_fast_kernel<CP, true, false, false>
-    if (max_a < 1 || max_b < 1 || max_a + max_b > 1024u) return 0;   // chunks of at most 128 events per lane
+TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w) {
+    TileGeometry g{};
+    if (!(p.hell2 && p.unit_w && p.C >= 1 && p.C <= 16 && key_is_w)) return g;   // the configuration of score_fast_kernel<CP, true, false, false>
+    if (max_a < 1 || max_b < 1 || max_a + max_b > 1024u) return g;   // chunks of at most 128 events per lane
     const unsigned need = (max_a > max_b ? max_a : max_b) + 2u;
-    const unsigned table_n = (need + 63u) & ~63u;
-    const int CP = p.C <= 8 ? 8 : 16;
-    const int stage_keys = kTileDim * (int)((max_a + 2u) & ~1u) + kTileDim * (int)((max_b + 2u) & ~1u);
-    const int team_bytes = tile_team_bytes(CP, stage_keys);
-    const int budget = 227 * 1024 - 3 * (int)table_n * 8;
-    int teams = budget / team_bytes;
+    g.table_n = (int)((need + 63u) & ~63u);
+    g.cp = p.C <= 8 ? 8 : 16;
+    g.stage_keys = kTileDim * (int)((max_a + 2u) & ~1u) + kTileDim * (int)((max_b + 2u) & ~1u);
+    g.team_bytes = tile_team_bytes(g.cp, g.stage_keys);
+    const int budget = 227 * 1024 - 3 * g.table_n * 8;
+    int teams = budget / g.team_bytes;
     if (teams > kTileMaxTeams) teams = kTileMaxTeams;
     if (const char* v = std::getenv("LOCOHD_TILE_TEAMS")) { const int t = std::atoi(v); if (t >= 1 && t < teams) teams = t; }   // occupancy sweeps
-    // what the teams leave over replicates the head of the two count-indexed tables (240 bytes per entry)
-    int rep_n = teams > 0 ? (budget - teams * team_bytes) / 240 : 0;
+    // what the teams leave over replicates the head of the two count-indexed tables (240 bytes per entry); only the
+    // 8-row instantiation has the replicated form
+    int rep_n = teams > 0 && g.cp == 8 ? (budget - teams * g.team_bytes) / 240 : 0;
     if (rep_n > kTileRepMax) rep_n = kTileRepMax;
     if (rep_n < 16) rep_n = 0;
     if (const char* v = std::getenv("LOCOHD_TILE_REP")) { const int r = std::atoi(v); if (r >= 0 && r < rep_n) rep_n = r; }   // A/B switch
-    if (table_n_out) *table_n_out = (int)table_n;
-    if (stage_keys_out) *stage_keys_out = stage_keys;
-    if (team_bytes_out) *team_bytes_out = team_bytes;
-    if (rep_n_out) *rep_n_out = rep_n;
-    return teams;
+    g.teams = teams;
+    g.rep_n = rep_n;
+    return g;
 }
 
 bool score_tiles_applicable(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w) {
     if (const char* v = std::getenv("LOCOHD_NO_TILES")) if (std::atoi(v)) return false;   // A/B switch
     // below 6 teams (24 warps) one pair per warp with a stage of its own is the better kernel
-    return tile_geometry(p, max_a, max_b, key_is_w, nullptr, nullptr, nullptr, nullptr) >= 6;
+    return tile_geometry(p, max_a, max_b, key_is_w).teams >= 6;
 }
 
 // Anchors per slice of the unit order (TileOrder): as many as keep the environments of one slice of every structure
@@ -2834,14 +2832,14 @@ static uint64_t tile_slice(const ScoreArgs& a, double mean_a, double mean_b) {
 static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a, double mean_b,
                         cudaStream_t st) {
     ScoreArgs a = args;
-    int table_n = 0, stage_keys = 0, team_bytes = 0, rep_n = 0;
-    const int teams = tile_geometry(p, max_a, max_b, a.a.key_is_w, &table_n, &stage_keys, &team_bytes, &rep_n);
+    const TileGeometry g = tile_geometry(p, max_a, max_b, a.a.key_is_w);
+    const int teams = g.teams, team_bytes = g.team_bytes;
     if (teams < 1) return -1;
-    a.table_n = table_n;
-    a.stage_cap = stage_keys;
-    a.rep_n = p.C <= 8 ? rep_n : 0;
+    a.table_n = g.table_n;
+    a.stage_cap = g.stage_keys;
+    a.rep_n = g.rep_n;
     const bool rep = a.rep_n > 0;
-    const int smem = (table_n + 2 * (15 * a.rep_n + table_n)) * 8 + teams * team_bytes;
+    const int smem = (g.table_n + 2 * (15 * a.rep_n + g.table_n)) * 8 + teams * team_bytes;
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -2858,7 +2856,7 @@ static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a,
         cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         kernel<<<grid, teams * kTeamThreads, smem, st>>>(a, p, teams, team_bytes);
     };
-    if (p.C <= 8) { if (rep) go(score_tile_kernel<8, true>); else go(score_tile_kernel<8, false>); }
+    if (g.cp == 8) { if (rep) go(score_tile_kernel<8, true>); else go(score_tile_kernel<8, false>); }
     else go(score_tile_kernel<16, false>);
     return 1;
 }

@@ -244,6 +244,18 @@ int launch_score(const ScoreArgs& args, const KParams& p, unsigned max_a, unsign
                  cudaStream_t st);
 // true when a job list grouped into ScoreTiles can be scored by score_tile_kernel for environments of these sizes
 bool score_tiles_applicable(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w);
+// Launch geometry of score_tile_kernel for environments of at most max_a / max_b members (teams = 0: the kernel does
+// not apply).  The one place that decides it: launch_tiles, score_tiles_applicable and locohd_tile_geometry read it.
+struct TileGeometry {
+    int teams;        // teams of four warps per CTA (LOCOHD_TILE_TEAMS lowers it)
+    int cp;           // count rows per warp: 8 (C <= 8) or 16 (C <= 16), the instantiation score_tile_kernel<cp, ...>
+    int rep_n;        // replicated head of the count-indexed tables, 0 = unreplicated (always 0 for cp 16;
+                      // LOCOHD_TILE_REP lowers it)
+    int table_n;      // entries of each table
+    int stage_keys;   // keys a team stages per unit
+    int team_bytes;   // shared memory per team
+};
+TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w);
 int launch_job_means(const double* scores, const uint64_t* job_pair_off, uint64_t n_jobs, double* means,
                      cudaStream_t st);
 int launch_widen_xyz(const float* in, double* out, uint64_t n3, cudaStream_t st);
