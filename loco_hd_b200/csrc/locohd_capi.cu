@@ -3,7 +3,6 @@
 // ordering and the launch sequence K0 -> K1 -> scan -> K1' -> K2.  No CPU fallback exists: every entry point
 // needs a CUDA device.
 #include <algorithm>
-#include <chrono>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -23,6 +22,12 @@ using namespace locohd;
 namespace {
 std::mutex g_err_mutex;
 std::string g_global_err;
+
+// A job list grouped into tiles (plan_job_tiles) and whether score_tile_kernel pays for that grouping (tiles_pay)
+struct TilePlan {
+    std::vector<ScoreTile> tiles;
+    bool pays = false;
+};
 }
 
 struct locohd_ctx {
@@ -31,9 +36,9 @@ struct locohd_ctx {
     std::string err;
     uint64_t launches = 0;
     uint64_t tile_launches = 0;
-    // grouping of the last job list into tiles (a benchmark step, the next block of frames: the same list again)
+    // tile plan of the last job list (a benchmark step, the next block of frames: the same list again)
     std::vector<locohd_job> tile_cache_jobs;
-    std::vector<ScoreTile> tile_cache_tiles;
+    TilePlan tile_cache_plan;
     bool has_params = false;
     KParams kp{};
     int n_categories = 0;
@@ -56,7 +61,6 @@ struct locohd_ctx {
     // pinned staging area of the one-call entry point (small calls: all inputs travel in one copy)
     unsigned char* h_stage = nullptr;
     size_t h_stage_bytes = 0;
-    int legacy_gather = 0;         // LOCOHD_LEGACY_GATHER=1: always use the multi-kernel gather (A/B runs)
     int fused_cap_hint = kFusedCap;  // members per environment the fused gather starts with (512 or 1024)
     uint64_t hist_n_anchors = 0, hist_capacity = 0;   // store size that worked for the last call of this shape (0: none)
     double hist_threshold = 0.0;
@@ -73,18 +77,6 @@ struct locohd_ctx {
 };
 
 namespace {
-// LOCOHD_TRACE=1: host wall-clock of the phases of an environment build on stderr (development aid)
-struct Trace {
-    bool on;
-    std::chrono::steady_clock::time_point t0;
-    Trace() : on(false) { const char* v = std::getenv("LOCOHD_TRACE"); on = v && v[0] && v[0] != '0'; t0 = std::chrono::steady_clock::now(); }
-    void mark(const char* what) {
-        if (!on) return;
-        const auto t1 = std::chrono::steady_clock::now();
-        std::fprintf(stderr, "[locohd trace] %-28s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(t1 - t0).count());
-        t0 = t1;
-    }
-};
 // Brackets the launches issued in its scope with a pair of events when profiling is enabled.
 struct ProfScope {
     locohd_ctx* ctx;
@@ -439,11 +431,11 @@ void destroy_envset(locohd_envset* e) {
 //   -> K1b exact gather into the store -> K1c per-environment sort + CDF + key packing.
 // One host synchronisation (the store size) per call.
 int build_envset(locohd_ctx* ctx, locohd_structs* s, uint64_t n_anchors, const uint32_t* d_anchor_struct,
-                 const uint32_t* d_anchor_prim, double threshold, int keep_indices, locohd_envset** out) {
+                 const uint32_t* d_anchor_prim, double threshold, int keep_indices, const LaunchOverrides& ov,
+                 locohd_envset** out) {
     if (!(threshold > 0.0))  // NaN included: nothing passes `d2 < r*r`, the reference then panics on dists[0]
         return fail(ctx, LOCOHD_ERR_EMPTY_ENV, "threshold_distance must be positive (got %g): every environment would be empty", threshold);
     if (n_anchors > 0xFFFFFFF0ull) return fail(ctx, LOCOHD_ERR_UNSUPPORTED, "more than 2^32 anchors in one call");
-    Trace tr;
     TRY_ST(ensure_cells(s, threshold));
     locohd_envset* e = new locohd_envset();
     e->ctx = ctx;
@@ -477,10 +469,9 @@ int build_envset(locohd_ctx* ctx, locohd_structs* s, uint64_t n_anchors, const u
         ctx->launches += launch_anchor_order(sv, ctx->kp, n_anchors, d_anchor_struct, d_anchor_prim, n_prims, d_slot_cnt,
                                              d_slot_off, d_scratch, ctx->d_scan, d_order, d_order_rec, ctx->stream);
     }
-    tr.mark("cells + order launched");
     // ---- fused path: sample the sizes (every anchor for small calls), reserve the store, one kernel does the rest
     // the fused kernel works with r^2 in the f32 exponent range (fixed-point sort keys, f32-seeded square roots)
-    if (!ctx->legacy_gather && threshold * threshold < 1.0e30) {
+    if (!ov.legacy_gather && threshold * threshold < 1.0e30) {
         // Store sizing.  Small calls (one structure pair is the typical call of the reference API) take the bound
         // kFusedCap per environment and skip the sizing pass and its synchronisation; large batches sample the FP32
         // upper-bound sizes of every 16th anchor.
@@ -504,7 +495,6 @@ int build_envset(locohd_ctx* ctx, locohd_structs* s, uint64_t n_anchors, const u
                 return bail(fail(ctx, LOCOHD_ERR_CUDA, "copy of the gather statistics failed"));
             if ((st = sync_and_check(ctx))) return bail(st);
             fs = ctx->h_fstats[0];
-            tr.mark("sample + sync");
         }
         // Members per environment the kernel is instantiated for: 512, and 1024 once a call has reported larger
         // environments (the hint stays with the context until a 1024 run sees only small ones again).
@@ -522,14 +512,10 @@ int build_envset(locohd_ctx* ctx, locohd_structs* s, uint64_t n_anchors, const u
             for (uint64_t step = 1ull << 62; step >= 32; step >>= 1)
                 if (capacity & step) { step >>= 4; capacity = (capacity + step - 1) & ~(step - 1); break; }
             if (by_history) capacity = ctx->hist_capacity;
-            tr.mark("grid + capacity");
-            if (tr.on) std::fprintf(stderr, "[locohd trace] cap %d, capacity %llu entries, grid %u, cached blocks %zu\n", cap,
-                                    (unsigned long long)capacity, grid, ctx->big_free.size());
             if ((st = dev_alloc(ctx, &e->d_key, capacity))) return bail(st);
             if (keep_indices) {
                 if ((st = dev_alloc(ctx, &e->d_idx, capacity)) || (st = dev_alloc(ctx, &e->d_dist, capacity))) return bail(st);
             }
-            tr.mark("store allocation");
             EnvBuild b{};
             b.n_env = n_anchors; b.order = d_order; b.order_rec = d_order_rec; b.ub = nullptr; b.off = nullptr; b.off_out = e->d_off;
             b.count = e->d_count;
@@ -548,7 +534,6 @@ int build_envset(locohd_ctx* ctx, locohd_structs* s, uint64_t n_anchors, const u
                 return bail(fail(ctx, LOCOHD_ERR_CUDA, "copy of the gather statistics failed"));
             if ((st = sync_and_check(ctx))) return bail(st);
             const FusedStats fr = ctx->h_fstats[1];
-            tr.mark("fused kernel + sync");
             if (!fr.overflow) {
                 // remember the size for the next call of this shape unless it was a tight fit
                 ctx->hist_n_anchors = n_anchors; ctx->hist_threshold = threshold; ctx->hist_cap = cap;
@@ -683,17 +668,38 @@ std::vector<ScoreTile> group_job_tiles_sorted(const std::vector<locohd_job>& job
 // A row of a tile is one warp, four pairs wide; full tiles run 1.5 x the pair kernel's rate (profiles/r6a).  The tile
 // kernel pays when the rows are mostly filled and a team mostly has work for its four warps (one-against-many lists -
 // trajectory frames against frame 0 - give tiles of a single row: three of four warps would idle).
-bool tiles_pay(const std::vector<ScoreTile>& tiles, uint64_t n_jobs) {
+uint64_t tile_rows(const std::vector<ScoreTile>& tiles) {
     uint64_t rows = 0;
     for (const ScoreTile& t : tiles)
         for (int r = 0; r < kTileDim; ++r) rows += t.a_first[r] != kTileNone ? 1 : 0;
+    return rows;
+}
+
+bool tiles_pay(const std::vector<ScoreTile>& tiles, uint64_t n_jobs) {
+    const uint64_t rows = tile_rows(tiles);
     return !tiles.empty() && n_jobs * 10 >= rows * kTileDim * 6 && rows >= 3 * tiles.size();
+}
+
+// The list order itself (batch.py::blocked_pairs) when its tiles pay, else the sorted grouping (any other order).
+// Lists of fewer than 4 jobs, of unequal jobs or of empty jobs get no tiles.
+TilePlan plan_job_tiles(const std::vector<locohd_job>& jobs, const std::vector<uint64_t>& joff) {
+    TilePlan plan;
+    if (jobs.size() < 4 || jobs[0].n == 0) return plan;
+    for (const locohd_job& j : jobs)
+        if (j.n != jobs[0].n) return plan;
+    plan.tiles = group_job_tiles(jobs, joff);
+    plan.pays = tiles_pay(plan.tiles, jobs.size());
+    if (!plan.pays) {
+        plan.tiles = group_job_tiles_sorted(jobs, joff);
+        plan.pays = tiles_pay(plan.tiles, jobs.size());
+    }
+    return plan;
 }
 
 int run_score(locohd_ctx* ctx, const locohd_envset* a, const locohd_envset* b, uint64_t n_pairs,
               const uint32_t* d_pairs, const locohd_job* d_jobs, const uint64_t* d_job_off, uint64_t n_jobs,
-              uint64_t uniform_n, const uint32_t* d_wf_idx, double* d_out, const ScoreTile* d_tiles = nullptr,
-              uint64_t n_tiles = 0) {
+              uint64_t uniform_n, const uint32_t* d_wf_idx, double* d_out, const LaunchOverrides& ov,
+              const ScoreTile* d_tiles = nullptr, uint64_t n_tiles = 0) {
     ScoreArgs sa{};
     sa.tiles = d_tiles; sa.n_tiles = n_tiles;
     sa.a = a->view(); sa.b = b->view();
@@ -705,7 +711,7 @@ int run_score(locohd_ctx* ctx, const locohd_envset* a, const locohd_envset* b, u
     const double mean_a = a->n_env ? (double)a->total / (double)a->n_env : 0.0;
     const double mean_b = b->n_env ? (double)b->total / (double)b->n_env : 0.0;
     { ProfScope ps(ctx, LOCOHD_PROF_SCORE);
-      n = launch_score(sa, ctx->kp, a->max_count, b->max_count, mean_a, mean_b, ctx->stream); }
+      n = launch_score(sa, ctx->kp, a->max_count, b->max_count, mean_a, mean_b, ov, ctx->stream); }
     if (n < 0) return fail(ctx, LOCOHD_ERR_UNSUPPORTED, "shared memory budget exceeded for %d categories", ctx->kp.C);
     ctx->launches += n;
     if (d_tiles) ctx->tile_launches += n;
@@ -794,10 +800,6 @@ int locohd_ctx_create(int device, locohd_ctx** out) {
     if ((ce = cudaHostAlloc((void**)&ctx->h_err, sizeof(int), cudaHostAllocDefault)) != cudaSuccess) return bail(ce);
     if ((ce = cudaHostAlloc((void**)&ctx->h_fstats, 2 * sizeof(FusedStats), cudaHostAllocDefault)) != cudaSuccess) return bail(ce);
     *ctx->h_err = 0;
-    {
-        const char* lg = std::getenv("LOCOHD_LEGACY_GATHER");
-        ctx->legacy_gather = (lg && lg[0] && lg[0] != '0') ? 1 : 0;
-    }
     if ((ce = cudaMalloc(&ctx->d_sqrt_tbl, kSqrtTableSize * sizeof(double))) != cudaSuccess) return bail(ce);
     if ((ce = cudaMalloc(&ctx->d_rsqrt_tbl, kSqrtTableSize * sizeof(double))) != cudaSuccess) return bail(ce);
     std::vector<double> t(kSqrtTableSize), r(kSqrtTableSize);
@@ -1124,7 +1126,7 @@ int locohd_envset_build(locohd_ctx* ctx, locohd_structs* s, uint64_t n_anchors, 
     InBuf<uint32_t> as, ap;
     TRY_ST(as.load(ctx, anchor_struct, n_anchors));
     TRY_ST(ap.load(ctx, anchor_prim, n_anchors));
-    TRY_ST(build_envset(ctx, s, n_anchors, as.ptr, ap.ptr, threshold, keep_indices, out));
+    TRY_ST(build_envset(ctx, s, n_anchors, as.ptr, ap.ptr, threshold, keep_indices, read_launch_overrides(), out));
     // the anchor arrays may be temporaries that are released (stream-ordered) when this scope ends
     return 0;
     API_END()
@@ -1343,7 +1345,7 @@ int locohd_score_pairs(locohd_ctx* ctx, const locohd_envset* a, const locohd_env
     TRY_ST(wf.load(ctx, wf_idx, n_pairs));
     OutBuf<double> out;
     TRY_ST(out.prepare(ctx, out_scores, n_pairs));
-    TRY_ST(run_score(ctx, a, b, n_pairs, pr.ptr, nullptr, nullptr, 0, 0, wf.ptr, out.ptr));
+    TRY_ST(run_score(ctx, a, b, n_pairs, pr.ptr, nullptr, nullptr, 0, 0, wf.ptr, out.ptr, read_launch_overrides()));
     TRY_ST(out.commit());
     return sync_and_check(ctx);
     API_END()
@@ -1354,21 +1356,11 @@ int locohd_plan_job_tiles(uint64_t n_jobs, const locohd_job* jobs, uint64_t* out
     try {
         std::vector<locohd_job> hj(jobs, jobs + n_jobs);   // host memory only: this is a host-side query
         std::vector<uint64_t> joff(n_jobs + 1, 0);
-        bool uniform = n_jobs > 0;
-        for (uint64_t j = 0; j < n_jobs; ++j) { joff[j + 1] = joff[j] + hj[j].n; uniform = uniform && hj[j].n == hj[0].n; }
-        std::vector<ScoreTile> tiles;
-        bool pays = false;
-        if (uniform && hj[0].n && n_jobs >= 4) {
-            tiles = group_job_tiles(hj, joff);
-            if (!tiles_pay(tiles, n_jobs)) tiles = group_job_tiles_sorted(hj, joff);
-            pays = tiles_pay(tiles, n_jobs);
-        }
-        uint64_t rows = 0;
-        for (const ScoreTile& t : tiles)
-            for (int r = 0; r < kTileDim; ++r) rows += t.a_first[r] != kTileNone ? 1 : 0;
-        if (out_tiles) *out_tiles = tiles.size();
-        if (out_rows) *out_rows = rows;
-        if (out_pays) *out_pays = pays ? 1 : 0;
+        for (uint64_t j = 0; j < n_jobs; ++j) joff[j + 1] = joff[j] + hj[j].n;
+        const TilePlan plan = plan_job_tiles(hj, joff);
+        if (out_tiles) *out_tiles = plan.tiles.size();
+        if (out_rows) *out_rows = tile_rows(plan.tiles);
+        if (out_pays) *out_pays = plan.pays ? 1 : 0;
         return LOCOHD_OK;
     } catch (const std::exception&) {
         return LOCOHD_ERR_CUDA;
@@ -1396,7 +1388,7 @@ int locohd_tile_geometry(int n_categories, uint32_t max_a, uint32_t max_b, int* 
     p.C = n_categories;
     p.hell2 = 1;
     p.unit_w = 1;
-    const TileGeometry g = tile_geometry(p, max_a, max_b, 1);
+    const TileGeometry g = tile_geometry(p, max_a, max_b, 1, read_launch_overrides());
     *teams = g.teams;
     if (cp) *cp = g.cp;
     if (rep_n) *rep_n = g.rep_n;
@@ -1454,28 +1446,28 @@ int locohd_score_jobs_stats(locohd_ctx* ctx, const locohd_envset* a, const locoh
         return cleanup(st);
     if (anchor_stats && (st = dev_alloc(ctx, &d_stat, 2 * n_per_job))) return cleanup(st);
     // Jobs that share runs of environments (an all-vs-all ensemble in 4 x 4 blocks) go to the tile kernel, which
-    // stages every environment once per tile instead of once per pair.  It pays when the tiles are mostly full.
+    // stages every environment once per tile instead of once per pair.  It pays when the tiles are mostly full and
+    // at least 6 teams fit an SM: below that, one pair per warp with a stage of its own is the better kernel.
+    const LaunchOverrides ov = read_launch_overrides();
     InBuf<ScoreTile> dtiles;
-    std::vector<ScoreTile> tiles;   // alive until the call's final synchronisation
-    uint64_t n_tiles = 0;
-    if (uniform && n_per_job && n_jobs >= 4 && !wf_idx && a->key_is_w && b->key_is_w &&
-        score_tiles_applicable(ctx->kp, a->max_count, b->max_count, 1)) {
-        if (ctx->tile_cache_jobs.size() == hj.size() &&
+    TilePlan plan;   // alive until the call's final synchronisation
+    if (!wf_idx && a->key_is_w && b->key_is_w && !ov.no_tiles &&
+        tile_geometry(ctx->kp, a->max_count, b->max_count, 1, ov).teams >= 6) {
+        if (!ctx->tile_cache_plan.tiles.empty() && ctx->tile_cache_jobs.size() == hj.size() &&
             std::memcmp(ctx->tile_cache_jobs.data(), hj.data(), hj.size() * sizeof(locohd_job)) == 0) {
-            tiles = ctx->tile_cache_tiles;   // the list of the previous call: 2 ms instead of 25 for 500 000 jobs
+            plan = ctx->tile_cache_plan;   // the list of the previous call: 2 ms instead of 25 for 500 000 jobs
         } else {
-            tiles = group_job_tiles(hj, joff);                                      // the list order itself (blocked_pairs)
-            if (!tiles_pay(tiles, n_jobs)) tiles = group_job_tiles_sorted(hj, joff);   // any other order
-            ctx->tile_cache_jobs = hj;
-            ctx->tile_cache_tiles = tiles;
+            plan = plan_job_tiles(hj, joff);
+            if (!plan.tiles.empty()) {   // a list without tiles is planned at once and does not evict the cached one
+                ctx->tile_cache_jobs = hj;
+                ctx->tile_cache_plan = plan;
+            }
         }
-        if (tiles_pay(tiles, n_jobs)) {
-            n_tiles = tiles.size();
-            if ((st = dtiles.load(ctx, tiles.data(), n_tiles))) return cleanup(st);
-        }
+        if (plan.pays && (st = dtiles.load(ctx, plan.tiles.data(), plan.tiles.size()))) return cleanup(st);
     }
+    const uint64_t n_tiles = plan.pays ? plan.tiles.size() : 0;
     st = run_score(ctx, a, b, n_pairs, nullptr, dj.ptr, djoff.ptr, n_jobs, (uniform && hj[0].n) ? hj[0].n : 0,
-                   wf.ptr, d_scores, n_tiles ? dtiles.ptr : nullptr, n_tiles);
+                   wf.ptr, d_scores, ov, n_tiles ? dtiles.ptr : nullptr, n_tiles);
     if (!st && (means.ptr || anchor_stats)) {
         ProfScope ps(ctx, LOCOHD_PROF_OTHER);
         if (means.ptr) ctx->launches += launch_job_means(d_scores, djoff.ptr, n_jobs, means.ptr, ctx->stream);
@@ -1535,6 +1527,7 @@ int locohd_from_primitives(locohd_ctx* ctx, uint64_t n_a, const double* xyz_a, c
     if (!(threshold > 0.0))
         return fail(ctx, LOCOHD_ERR_EMPTY_ENV, "threshold_distance must be positive (got %g): every environment would be empty", threshold);
     TRY_ST(check_wf_indices(ctx, wf_idx, n_pairs));
+    const LaunchOverrides ov = read_launch_overrides();
     const uint64_t n = n_a + n_b;
     {
         // Small calls with host inputs (the typical call of the reference API: one structure pair) travel in ONE
@@ -1614,12 +1607,12 @@ int locohd_from_primitives(locohd_ctx* ctx, uint64_t n_a, const double* xyz_a, c
                 ctx->launches += launch_convert_categories(reinterpret_cast<const uint16_t*>(d + o_cat16), s->d_cat, n, ctx->kp.C, ctx->stream);
                 ctx->launches += launch_validate_xyz(s->d_xyz, 3 * n, ctx->d_err, ctx->stream);
                 int st = build_envset(ctx, s, 2 * n_pairs, reinterpret_cast<const uint32_t*>(d + o_as),
-                                      reinterpret_cast<const uint32_t*>(d + o_ap), threshold, 0, &env);
+                                      reinterpret_cast<const uint32_t*>(d + o_ap), threshold, 0, ov, &env);
                 if (st) return done(st);
                 OutBuf<double> out;
                 if ((st = out.prepare(ctx, out_scores, n_pairs))) return done(st);
                 st = run_score(ctx, env, env, n_pairs, nullptr, reinterpret_cast<const locohd_job*>(d + o_job), nullptr, 1, n_pairs,
-                               wf_idx ? reinterpret_cast<const uint32_t*>(d + o_wf) : nullptr, out.ptr);
+                               wf_idx ? reinterpret_cast<const uint32_t*>(d + o_wf) : nullptr, out.ptr, ov);
                 if (!st) st = out.commit();
                 const int st2 = sync_and_check(ctx);
                 return done(st ? st : st2);
@@ -1681,14 +1674,14 @@ int locohd_from_primitives(locohd_ctx* ctx, uint64_t n_a, const double* xyz_a, c
     ce = cudaMemcpyAsync(d_as, h_as.data(), 2 * n_pairs * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream);
     if (ce == cudaSuccess) ce = cudaMemcpyAsync(d_ap, h_ap.data(), 2 * n_pairs * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream);
     if (ce != cudaSuccess) return cleanup(fail(ctx, LOCOHD_ERR_CUDA, "upload failed: %s", cudaGetErrorString(ce)));
-    if ((st = build_envset(ctx, s, 2 * n_pairs, d_as, d_ap, threshold, 0, &env))) return cleanup(st);
+    if ((st = build_envset(ctx, s, 2 * n_pairs, d_as, d_ap, threshold, 0, ov, &env))) return cleanup(st);
     const locohd_job job{0, n_pairs, n_pairs};
     InBuf<locohd_job> dj;
     InBuf<uint32_t> wf;
     OutBuf<double> out;
     if ((st = dj.load(ctx, &job, 1)) || (st = wf.load(ctx, wf_idx, n_pairs)) || (st = out.prepare(ctx, out_scores, n_pairs)))
         return cleanup(st);
-    st = run_score(ctx, env, env, n_pairs, nullptr, dj.ptr, nullptr, 1, n_pairs, wf.ptr, out.ptr);
+    st = run_score(ctx, env, env, n_pairs, nullptr, dj.ptr, nullptr, 1, n_pairs, wf.ptr, out.ptr, ov);
     if (!st) st = out.commit();
     const int st2 = sync_and_check(ctx);
     return cleanup(st ? st : st2);

@@ -59,9 +59,6 @@ __global__ void validate_xyz_kernel(const double* __restrict__ xyz, uint64_t n3,
 // ------------------------------------------------------------------------------------------------
 // Exclusive scan of u32 values into u64 offsets (three kernels: tile sums, scan of the sums, apply).
 // ------------------------------------------------------------------------------------------------
-#ifndef LOCOHD_CELL_THREADS
-#define LOCOHD_CELL_THREADS 512
-#endif
 constexpr int kScanThreads = 256;
 constexpr int kScanPer = 8;
 constexpr int kScanTile = kScanThreads * kScanPer;
@@ -150,7 +147,7 @@ __global__ void __launch_bounds__(kScanThreads) scan_apply_kernel(const uint32_t
 // K0: cell list.  One CTA (256 threads) per structure; cell edge = half the radius (search +-2 cells), enlarged
 // when the structure would need more than max(2 N, 8) cells.
 // ------------------------------------------------------------------------------------------------
-constexpr int kCellThreads = LOCOHD_CELL_THREADS;   // latency-bound passes over one structure: more threads, more loads in flight
+constexpr int kCellThreads = 512;   // latency-bound passes over one structure: more threads, more loads in flight
 constexpr int kMaxCellsAxis = 1024;
 
 __device__ __forceinline__ int cell_coord(double rel, double inv_cell, int n) {
@@ -601,7 +598,6 @@ template <int CAP> struct FusedKey {
     static constexpr int SB = CAP == 512 ? 9 : 10;
     static constexpr uint32_t kSlotMask = (1u << SB) - 1u;
     static constexpr double kScale = (double)((1u << (32 - SB)) - 16u);   // d2 < r2 -> fixed point < 2^(32-SB) - 15
-    static constexpr uint32_t kInfKey = (1u << (32 - SB)) - 8u;           // non-finite squared distance
 };
 
 // ascending compare-exchange of two registers of one lane
@@ -1330,7 +1326,6 @@ constexpr int kScoreMaxWarps = 8;
 // fast kernel: one large CTA per SM shares a single copy of the tables.  The W-keyed instantiations need 50 registers
 // (32 warps fit the register file); the distance-keyed ones (several weight functions) and the ones with table
 // bound checks need up to 72: 28 warps.
-constexpr int kScoreFastMaxWarps = 32;
 __host__ __device__ constexpr int score_fast_max_warps(bool key_is_w, bool check, bool weighted = false) { return weighted ? 24 : ((key_is_w && !check) ? 32 : 28); }
 constexpr uint64_t kWMask = ~kCatMask;
 
@@ -2601,7 +2596,6 @@ static unsigned fused_grid_t(uint64_t n_env) {
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, env_fused_kernel<WFK, DEBUG, CAP, LIST>, fused_warps(CAP, DEBUG) * 32, smem);
     if (occ < 1) occ = 1;
-    if (const char* v = std::getenv("LOCOHD_FUSED_CTAS")) { const int c = std::atoi(v); if (c >= 1 && c < occ) occ = c; }
     const uint64_t need = (n_env + fused_warps(CAP, DEBUG) - 1) / fused_warps(CAP, DEBUG);
     const uint64_t cap = (uint64_t)sms * occ;
     return (unsigned)(need < cap ? need : cap);
@@ -2780,7 +2774,20 @@ static int launch_fast(const ScoreArgs& a, const KParams& p, bool check, int war
                  : launch_score_kernel(score_fast_kernel<CP, KEY_IS_W, false, false>, a, p, warps, per_warp, smem, st);
 }
 
-TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w) {
+LaunchOverrides read_launch_overrides() {
+    const auto env = [](const char* name) { return std::getenv(name); };
+    LaunchOverrides o;
+    if (const char* v = env("LOCOHD_NO_TILES")) o.no_tiles = std::atoi(v) != 0;
+    if (const char* v = env("LOCOHD_TILE_TEAMS")) o.tile_teams = std::atoi(v);
+    if (const char* v = env("LOCOHD_TILE_REP")) o.tile_rep = std::atoi(v);
+    if (const char* v = env("LOCOHD_TILE_RUN")) { const int r = std::atoi(v); if (r >= 1 && r <= 4096) o.tile_run = (unsigned)r; }
+    if (const char* v = env("LOCOHD_TILE_SLICE")) { const long long s = std::atoll(v); o.tile_slice = s < 0 ? 0 : s; }
+    if (const char* v = env("LOCOHD_TILE_SLICE_MB")) { const double mb = std::atof(v); if (mb > 0.0) o.tile_slice_mb = mb; }
+    if (const char* v = env("LOCOHD_LEGACY_GATHER")) o.legacy_gather = v[0] && v[0] != '0';
+    return o;
+}
+
+TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, const LaunchOverrides& ov) {
     TileGeometry g{};
     if (!(p.hell2 && p.unit_w && p.C >= 1 && p.C <= 16 && key_is_w)) return g;   // the configuration of score_fast_kernel<CP, true, false, false>
     if (max_a < 1 || max_b < 1 || max_a + max_b > 1024u) return g;   // chunks of at most 128 events per lane
@@ -2792,33 +2799,26 @@ TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int
     const int budget = 227 * 1024 - 3 * g.table_n * 8;
     int teams = budget / g.team_bytes;
     if (teams > kTileMaxTeams) teams = kTileMaxTeams;
-    if (const char* v = std::getenv("LOCOHD_TILE_TEAMS")) { const int t = std::atoi(v); if (t >= 1 && t < teams) teams = t; }   // occupancy sweeps
+    if (ov.tile_teams >= 1 && ov.tile_teams < teams) teams = ov.tile_teams;
     // what the teams leave over replicates the head of the two count-indexed tables (240 bytes per entry); only the
     // 8-row instantiation has the replicated form
     int rep_n = teams > 0 && g.cp == 8 ? (budget - teams * g.team_bytes) / 240 : 0;
     if (rep_n > kTileRepMax) rep_n = kTileRepMax;
     if (rep_n < 16) rep_n = 0;
-    if (const char* v = std::getenv("LOCOHD_TILE_REP")) { const int r = std::atoi(v); if (r >= 0 && r < rep_n) rep_n = r; }   // A/B switch
+    if (ov.tile_rep >= 0 && ov.tile_rep < rep_n) rep_n = ov.tile_rep;
     g.teams = teams;
     g.rep_n = rep_n;
     return g;
 }
 
-bool score_tiles_applicable(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w) {
-    if (const char* v = std::getenv("LOCOHD_NO_TILES")) if (std::atoi(v)) return false;   // A/B switch
-    // below 6 teams (24 warps) one pair per warp with a stage of its own is the better kernel
-    return tile_geometry(p, max_a, max_b, key_is_w).teams >= 6;
-}
-
 // Anchors per slice of the unit order (TileOrder): as many as keep the environments of one slice of every structure
 // inside a budget of L2 (126 MB on a B200, in two halves; 32 MB leaves room for the scores written and for the tile
 // descriptors), a multiple of the run length so that a claimed run stays inside one tile.  0 = tile-major order
-// (the whole store fits the budget, or LOCOHD_TILE_SLICE=0).  LOCOHD_TILE_SLICE=<anchors> / LOCOHD_TILE_SLICE_MB=<MB>: sweeps.
-static uint64_t tile_slice(const ScoreArgs& a, double mean_a, double mean_b) {
+// (the whole store fits the budget, or LaunchOverrides::tile_slice = 0).
+static uint64_t tile_slice(const ScoreArgs& a, double mean_a, double mean_b, const LaunchOverrides& ov) {
     const uint64_t n = a.uniform_n;
-    if (const char* v = std::getenv("LOCOHD_TILE_SLICE")) { const long long s = std::atoll(v); return s <= 0 || (uint64_t)s >= n ? 0 : (uint64_t)s; }
-    double budget = 32.0 * 1048576.0;
-    if (const char* v = std::getenv("LOCOHD_TILE_SLICE_MB")) { const double mb = std::atof(v); if (mb > 0.0) budget = mb * 1048576.0; }
+    if (ov.tile_slice >= 0) return (uint64_t)ov.tile_slice >= n ? 0 : (uint64_t)ov.tile_slice;
+    const double budget = (ov.tile_slice_mb > 0.0 ? ov.tile_slice_mb : 32.0) * 1048576.0;
     const bool same = a.a.key == a.b.key && a.a.off == a.b.off;
     const double store = 8.0 * ((double)a.a.n_env * (mean_a + 1.0) + (same ? 0.0 : (double)a.b.n_env * (mean_b + 1.0)));
     if (n == 0 || store <= budget) return 0;
@@ -2830,9 +2830,9 @@ static uint64_t tile_slice(const ScoreArgs& a, double mean_a, double mean_b) {
 }
 
 static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a, double mean_b,
-                        cudaStream_t st) {
+                        const LaunchOverrides& ov, cudaStream_t st) {
     ScoreArgs a = args;
-    const TileGeometry g = tile_geometry(p, max_a, max_b, a.a.key_is_w);
+    const TileGeometry g = tile_geometry(p, max_a, max_b, a.a.key_is_w, ov);
     const int teams = g.teams, team_bytes = g.team_bytes;
     if (teams < 1) return -1;
     a.table_n = g.table_n;
@@ -2848,10 +2848,9 @@ static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a,
     const unsigned grid = (unsigned)(need < (uint64_t)sms ? need : (uint64_t)sms);   // persistent: teams claim units from the cursor
     cudaMemsetAsync(a.cursor, 0, sizeof(unsigned long long), st);
     const uint64_t per_team = units / ((uint64_t)grid * teams * 4);   // short launches: shorter runs even out the tail
-    uint64_t max_run = kTileRun;
-    if (const char* v = std::getenv("LOCOHD_TILE_RUN")) { const int r = std::atoi(v); if (r >= 1 && r <= 4096) max_run = (uint64_t)r; }   // sweeps
+    const uint64_t max_run = ov.tile_run ? ov.tile_run : kTileRun;
     a.run = (unsigned)(per_team < 1 ? 1 : (per_team > max_run ? max_run : per_team));
-    a.order = make_tile_order(a.n_tiles, a.uniform_n, tile_slice(a, mean_a, mean_b));
+    a.order = make_tile_order(a.n_tiles, a.uniform_n, tile_slice(a, mean_a, mean_b, ov));
     auto go = [&](auto kernel) {
         cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         kernel<<<grid, teams * kTeamThreads, smem, st>>>(a, p, teams, team_bytes);
@@ -2862,9 +2861,9 @@ static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a,
 }
 
 int launch_score(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a, double mean_b,
-                 cudaStream_t st) {
+                 const LaunchOverrides& ov, cudaStream_t st) {
     if (!args.n_pairs) return 0;
-    if (args.tiles) return launch_tiles(args, p, max_a, max_b, mean_a, mean_b, st);
+    if (args.tiles) return launch_tiles(args, p, max_a, max_b, mean_a, mean_b, ov, st);
     const unsigned pad_max = ((max_a + 1) & ~1u) + ((max_b + 1) & ~1u);
     const bool key_is_w = args.a.key_is_w != 0;
     const bool fast = p.hell2 && p.C <= 16;   // Hellinger-2 with or without category weights
@@ -2895,7 +2894,6 @@ int launch_score(const ScoreArgs& args, const KParams& p, unsigned max_a, unsign
     const int budget = 220 * 1024;  // one CTA per SM: the tables are staged once, the rest goes to the warps' stages
     int warps = (budget - tables) / per_warp;
     if (warps > score_fast_max_warps(key_is_w, check, !p.unit_w)) warps = score_fast_max_warps(key_is_w, check, !p.unit_w);
-    if (const char* v = std::getenv("LOCOHD_SCORE_WARPS")) { const int w = std::atoi(v); if (w >= 1 && w < warps) warps = w; }   // occupancy sweeps
     if (warps < 1) warps = 1;
     const int smem = tables + per_warp * warps;
     if (CP == 8) n += key_is_w ? launch_fast<8, true>(a, p, check, warps, per_warp, smem, st)

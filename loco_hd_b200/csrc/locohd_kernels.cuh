@@ -95,11 +95,8 @@ struct ScanStats {  // written by the scan kernels, read back by the host
 // warps per CTA (one anchor per warp at a time): one CTA per SM for the 512-member instantiation - the warps of a CTA
 // work on consecutive anchors of the cell order and share their candidate rows in L1; measured 24.6 / 23.6 / 22.6 ms
 // at 4 / 8 / 16 warps per CTA with the same 32 warps per SM
-#ifndef LOCOHD_FUSED_WARPS
-#define LOCOHD_FUSED_WARPS 32   // build-time knob for register / occupancy experiments (24 warps leave 85 registers per thread)
-#endif
-__host__ __device__ constexpr int fused_warps(int cap, bool debug) { return cap == 512 ? (debug ? 16 : LOCOHD_FUSED_WARPS) : 8; }  // debug: the parity arrays need more shared memory per warp
-constexpr int kFusedWarps = 32;     // largest warps-per-CTA (store sizing)
+constexpr int kFusedWarps = 32;     // the 512-member instantiation, and the largest warps-per-CTA (store sizing)
+__host__ __device__ constexpr int fused_warps(int cap, bool debug) { return cap == 512 ? (debug ? 16 : kFusedWarps) : 8; }  // debug: the parity arrays need more shared memory per warp
 constexpr int kFusedCap = 512;      // members per environment (default instantiation)
 constexpr int kFusedCapBig = 1024;  // second instantiation, used when the first reports larger environments
 constexpr int kFusedChunk = 2048;   // store entries a warp reserves with one atomicAdd
@@ -240,22 +237,36 @@ int launch_rows_copy(const double* dmx, const uint8_t* cat, uint64_t n_rows, uin
 int launch_ragged_rows_copy(const double* values, const uint8_t* cat, uint64_t n_rows, uint64_t max_len,
                             const uint64_t* in_off, const uint64_t* out_off, uint64_t* off, uint32_t* count,
                             const EnvBuild& b, cudaStream_t st);
+// Test and A/B hooks that override launch decisions of the library, read from the process environment by
+// read_launch_overrides() once per API call, so that a process can change them between calls.  The defaults leave
+// every decision to the library.  No other code of the library reads the environment.
+struct LaunchOverrides {
+    bool no_tiles = false;        // LOCOHD_NO_TILES (non-zero integer): job lists never take score_tile_kernel
+    int tile_teams = 0;           // LOCOHD_TILE_TEAMS: lowers TileGeometry::teams when in [1, teams)
+    int tile_rep = -1;            // LOCOHD_TILE_REP: lowers TileGeometry::rep_n when in [0, rep_n)
+    unsigned tile_run = 0;        // LOCOHD_TILE_RUN (1 ... 4096): longest run of units a team claims (0: kTileRun)
+    long long tile_slice = -1;    // LOCOHD_TILE_SLICE: anchors per slice of a tile launch, 0 = tile-major order (a
+                                  // value <= 0); -1: not set, the slice follows from the L2 budget
+    double tile_slice_mb = 0.0;   // LOCOHD_TILE_SLICE_MB (> 0): that L2 budget in MB (0: the default)
+    bool legacy_gather = false;   // LOCOHD_LEGACY_GATHER (any value not starting with '0'): environments are built
+                                  // with the multi-kernel gather
+};
+LaunchOverrides read_launch_overrides();
 int launch_score(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a, double mean_b,
-                 cudaStream_t st);
-// true when a job list grouped into ScoreTiles can be scored by score_tile_kernel for environments of these sizes
-bool score_tiles_applicable(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w);
+                 const LaunchOverrides& ov, cudaStream_t st);
 // Launch geometry of score_tile_kernel for environments of at most max_a / max_b members (teams = 0: the kernel does
-// not apply).  The one place that decides it: launch_tiles, score_tiles_applicable and locohd_tile_geometry read it.
+// not apply; below 6 teams the pair kernel is the better one and job lists are not tiled).  The one place that decides
+// it: launch_tiles, the tile eligibility of locohd_score_jobs_stats and locohd_tile_geometry read it.
 struct TileGeometry {
-    int teams;        // teams of four warps per CTA (LOCOHD_TILE_TEAMS lowers it)
+    int teams;        // teams of four warps per CTA (LaunchOverrides::tile_teams lowers it)
     int cp;           // count rows per warp: 8 (C <= 8) or 16 (C <= 16), the instantiation score_tile_kernel<cp, ...>
     int rep_n;        // replicated head of the count-indexed tables, 0 = unreplicated (always 0 for cp 16;
-                      // LOCOHD_TILE_REP lowers it)
+                      // LaunchOverrides::tile_rep lowers it)
     int table_n;      // entries of each table
     int stage_keys;   // keys a team stages per unit
     int team_bytes;   // shared memory per team
 };
-TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w);
+TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, const LaunchOverrides& ov);
 int launch_job_means(const double* scores, const uint64_t* job_pair_off, uint64_t n_jobs, double* means,
                      cudaStream_t st);
 int launch_widen_xyz(const float* in, double* out, uint64_t n3, cudaStream_t st);

@@ -167,3 +167,7 @@ def test_job_lists_group_into_tiles_on_the_host():
     uneven["n"][5] = n - 1
     assert not _capi.plan_job_tiles(uneven)["pays"]
     assert _capi.plan_job_tiles(jobs_of([]))["tiles"] == 0
+    # nor are lists of fewer than 4 equal jobs
+    for k in (1, 2, 3):
+        few = _capi.plan_job_tiles(jobs_of(blocked[:k]))
+        assert not few["pays"] and few["tiles"] == 0 and few["rows"] == 0

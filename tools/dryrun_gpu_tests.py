@@ -50,7 +50,7 @@ class OracleCtx:
                    statistical_distance=("Hellinger", (2.0,)), tag_rule=None):
         self.p = oracle.Params(n_categories, [(n, list(q)) for n, q in weight_functions], category_weights,
                                (statistical_distance[0], list(statistical_distance[1])), tag_rule)
-        # what decides whether score_jobs_stats may take the tile kernel (locohd_capi.cu, score_tiles_applicable)
+        # what decides whether score_jobs_stats may take the tile kernel (locohd_capi.cu, locohd_score_jobs_stats)
         self.tile_config = (len(weight_functions) == 1 and statistical_distance[0] == "Hellinger" and
                             list(statistical_distance[1]) == [2.0] and
                             (category_weights is None or all(w == 1.0 for w in category_weights)))
