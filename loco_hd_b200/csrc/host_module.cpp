@@ -559,11 +559,6 @@ struct LoCoHD {
             for (size_t r = 0; r + 1 < off.size(); ++r) m = std::max<size_t>(m, off[r + 1] - off[r]);
             return m;
         }
-        bool rectangular() const {
-            for (size_t r = 1; r + 1 < off.size(); ++r)
-                if (off[r + 1] - off[r] != off[1] - off[0]) return false;
-            return true;
-        }
     };
     static Rows to_rows(const py::object& m, const char* what) {
         Rows rows;
@@ -607,7 +602,6 @@ struct LoCoHD {
                 if (m->off[r + 1] == m->off[r]) throw py::value_error("Empty distance matrix rows!");
         const auto d = ensure_ctx();
         auto build = [&](locohd_ctx* c, const Rows& m, const std::vector<uint16_t>& cats, locohd_envset** e) {
-            if (m.rectangular()) return locohd_envset_from_rows(c, m.n(), m.off[1], m.val.data(), cats.data(), e);
             return locohd_envset_from_ragged_rows(c, m.n(), m.off.data(), m.val.data(), cats.data(), cats.size(), e);
         };
         return score_rows(d, rows_a, wf, [&](locohd_ctx* c, locohd_envset** ea, locohd_envset** eb) {

@@ -112,7 +112,7 @@ struct locohd_structs {
     uint32_t* d_cell_fill = nullptr;
     bool cells_valid = false;
     double cell_threshold = 0.0;
-    void* blob = nullptr;            // one-call entry point: all arrays above are views into this single device block
+    unsigned char* block = nullptr;  // the one device block the arrays above are views into (structs_layout)
     StructsView view() const {
         StructsView v;
         v.n_structs = n_structs; v.prim_off = d_prim_off; v.xyz = d_xyz; v.cat = d_cat; v.tag = d_tag;
@@ -979,6 +979,67 @@ int locohd_ctx_set_params(locohd_ctx* ctx, const locohd_params* params) {
 }
 
 // ---------------------------------------------------------------------------------------------- structures
+// Places arrays one after another in one device block, each at a multiple of 256 bytes: the alignment the kernels
+// would get from a cudaMallocAsync block of its own.
+struct BlockCursor {
+    size_t end = 0;
+    size_t take(size_t bytes) {
+        const size_t at = (end + 255) & ~(size_t)255;
+        end = at + bytes;
+        return at;
+    }
+};
+
+// Byte offsets of the arrays of a structure set in its device block.  The block starts with `head` bytes that the
+// caller uses for arrays of its own (locohd_from_primitives: those of the call).  The arrays that come from the host
+// follow, so that the head and they form one range [0, upload_end) that one copy can fill.
+struct StructsLayout {
+    size_t prim_off, xyz, tag, upload_end, cat, meta, pf, pd, porig, sorted_pos, cell_start, cell_fill, bytes;
+};
+
+static StructsLayout structs_layout(uint64_t n_structs, uint64_t n_prims, size_t head) {
+    BlockCursor c{head};
+    StructsLayout l;
+    l.prim_off = c.take((n_structs + 1) * sizeof(uint64_t));
+    l.xyz = c.take(3 * n_prims * sizeof(double));
+    l.tag = c.take(n_prims * sizeof(uint32_t));
+    l.upload_end = c.end;
+    l.cat = c.take(n_prims);
+    l.meta = c.take(n_structs * sizeof(StructMeta));
+    l.pf = c.take(n_prims * sizeof(float4));
+    l.pd = c.take(n_prims * sizeof(PrimRec));
+    l.porig = c.take(n_prims * sizeof(uint32_t));
+    l.sorted_pos = c.take(n_prims * sizeof(uint32_t));
+    l.cell_start = c.take(cell_entries(n_prims, n_structs) * sizeof(uint32_t));
+    l.cell_fill = c.take(cell_entries(n_prims, n_structs) * sizeof(uint32_t));
+    l.bytes = c.end;
+    return l;
+}
+
+// A structure set whose arrays are views into one new device block laid out by `l`; offs: host copy of the
+// n_structs + 1 primitive offsets.  The contents of the arrays are the caller's to upload.
+static int structs_alloc(locohd_ctx* ctx, uint64_t n_structs, const uint64_t* offs, const StructsLayout& l,
+                         locohd_structs** out) {
+    locohd_structs* s = new locohd_structs();
+    unsigned char* d = nullptr;
+    if (int st = dev_alloc(ctx, &d, l.bytes)) { delete s; return st; }
+    s->ctx = ctx; s->n_structs = n_structs; s->n_prims = offs[n_structs]; s->block = d;
+    for (uint64_t k = 0; k < n_structs; ++k) s->max_prims = std::max<uint64_t>(s->max_prims, offs[k + 1] - offs[k]);
+    s->d_prim_off = reinterpret_cast<uint64_t*>(d + l.prim_off);
+    s->d_xyz = reinterpret_cast<double*>(d + l.xyz);
+    s->d_tag = reinterpret_cast<uint32_t*>(d + l.tag);
+    s->d_cat = d + l.cat;
+    s->d_meta = reinterpret_cast<StructMeta*>(d + l.meta);
+    s->d_pf = reinterpret_cast<float4*>(d + l.pf);
+    s->d_pd = reinterpret_cast<PrimRec*>(d + l.pd);
+    s->d_porig = reinterpret_cast<uint32_t*>(d + l.porig);
+    s->d_sorted_pos = reinterpret_cast<uint32_t*>(d + l.sorted_pos);
+    s->d_cell_start = reinterpret_cast<uint32_t*>(d + l.cell_start);
+    s->d_cell_fill = reinterpret_cast<uint32_t*>(d + l.cell_fill);
+    *out = s;
+    return 0;
+}
+
 // Coordinates arrive as f64 (24 B per primitive) or as f32 (12 B, widened on the device: exact).
 static int upload_xyz(locohd_ctx* ctx, double* d_xyz, const void* xyz, bool f32, uint64_t n3) {
     if (!n3) return 0;
@@ -1013,19 +1074,10 @@ static int structs_create_impl(locohd_ctx* ctx, uint64_t n_structs, const uint64
     }
     const uint64_t n = offs[n_structs];
     if (n && (!xyz || !category || !tag)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null primitive arrays");
-    locohd_structs* s = new locohd_structs();
-    s->ctx = ctx; s->n_structs = n_structs; s->n_prims = n;
-    for (uint64_t k = 0; k < n_structs; ++k) s->max_prims = std::max<uint64_t>(s->max_prims, offs[k + 1] - offs[k]);
+    locohd_structs* s = nullptr;
+    TRY_ST(structs_alloc(ctx, n_structs, offs.data(), structs_layout(n_structs, n, 0), &s));
     auto bail = [&](int st) { locohd_structs_destroy(s); return st; };
     int st;
-    if ((st = dev_alloc(ctx, &s->d_prim_off, n_structs + 1)) || (st = dev_alloc(ctx, &s->d_xyz, 3 * n)) ||
-        (st = dev_alloc(ctx, &s->d_cat, n)) || (st = dev_alloc(ctx, &s->d_tag, n)) ||
-        (st = dev_alloc(ctx, &s->d_meta, n_structs)) || (st = dev_alloc(ctx, &s->d_pf, n)) ||
-        (st = dev_alloc(ctx, &s->d_pd, n)) || (st = dev_alloc(ctx, &s->d_porig, n)) ||
-        (st = dev_alloc(ctx, &s->d_sorted_pos, n)) ||
-        (st = dev_alloc(ctx, &s->d_cell_start, cell_entries(n, n_structs))) ||
-        (st = dev_alloc(ctx, &s->d_cell_fill, cell_entries(n, n_structs))))
-        return bail(st);
     cudaError_t ce = cudaMemcpyAsync(s->d_prim_off, offs.data(), offs.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream);
     if (ce == cudaSuccess && n) ce = cudaMemcpyAsync(s->d_tag, tag, n * sizeof(uint32_t), cudaMemcpyDefault, ctx->stream);
     if (ce != cudaSuccess) return bail(fail(ctx, LOCOHD_ERR_CUDA, "upload failed: %s", cudaGetErrorString(ce)));
@@ -1057,11 +1109,7 @@ void locohd_structs_destroy(locohd_structs* s) {
     if (!s) return;
     locohd_ctx* ctx = s->ctx;
     DeviceGuard g(ctx->device);
-    if (s->blob) { dev_free_bytes(ctx, s->blob); delete s; return; }
-    dev_free(ctx, s->d_prim_off); dev_free(ctx, s->d_xyz); dev_free(ctx, s->d_cat); dev_free(ctx, s->d_tag);
-    dev_free(ctx, s->d_meta); dev_free(ctx, s->d_pf); dev_free(ctx, s->d_pd); dev_free(ctx, s->d_porig);
-    dev_free(ctx, s->d_sorted_pos);
-    dev_free(ctx, s->d_cell_start); dev_free(ctx, s->d_cell_fill);
+    dev_free_bytes(ctx, s->block);
     delete s;
 }
 
@@ -1132,40 +1180,55 @@ int locohd_envset_build(locohd_ctx* ctx, locohd_structs* s, uint64_t n_anchors, 
     API_END()
 }
 
-static int rows_envset(locohd_ctx* ctx, uint64_t n_rows, uint64_t row_len, const double* dmx, const double* xyz,
-                       const uint16_t* category, locohd_envset** out) {
-    TRY_ST(need_params(ctx));
-    if (!out || (!dmx && !xyz) || (row_len && !category)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
+// Rows as environments (from_dmxs / from_coords, locohd.rs:410-476): row r becomes environment r, copied unsorted into
+// the store and sorted there.  With host offsets `row_off` (ragged input, checked by the caller) row r is
+// values[row_off[r], row_off[r + 1]) and row_len is the longest row; without them every row has row_len entries: row r
+// is values[r * row_len, (r + 1) * row_len) or the distances of point r to the row_len points `xyz`.  Row r is
+// co-sorted with the first categories (utils.rs:25-39).
+static int rows_envset(locohd_ctx* ctx, uint64_t n_rows, const uint64_t* row_off, uint64_t row_len,
+                       const double* values, const double* xyz, const uint16_t* category, locohd_envset** out) {
+    if (!out || (row_len && !category)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
     *out = nullptr;
     if (row_len > 0xFFFFFFFFull) return fail(ctx, LOCOHD_ERR_UNSUPPORTED, "rows longer than 2^32");
+    // every row starts at an even entry of the store
+    uint64_t n_in = xyz ? 3 * row_len : n_rows * row_len, total = n_rows * ((row_len + 1) & ~1ull);
+    std::vector<uint64_t> store_off;
+    if (row_off) {
+        store_off.assign(n_rows + 1, 0);
+        for (uint64_t r = 0; r < n_rows; ++r) store_off[r + 1] = store_off[r] + ((row_off[r + 1] - row_off[r] + 1) & ~1ull);
+        n_in = row_off[n_rows];
+        total = store_off[n_rows];
+    }
     InBuf<double> in;
-    if (dmx) TRY_ST(in.load(ctx, dmx, n_rows * row_len));
-    else TRY_ST(in.load(ctx, xyz, 3 * row_len));
     InBuf<uint16_t> cat16;
+    InBuf<uint64_t> d_row_off, d_store_off;
+    TRY_ST(in.load(ctx, xyz ? xyz : values, n_in));
     TRY_ST(cat16.load(ctx, category, row_len));
-    uint8_t* d_cat8 = nullptr;
-    TRY_ST(dev_alloc(ctx, &d_cat8, row_len));
-    ctx->launches += launch_convert_categories(cat16.ptr, d_cat8, row_len, ctx->kp.C, ctx->stream);
-    if (xyz) ctx->launches += launch_validate_xyz(in.ptr, 3 * row_len, ctx->d_err, ctx->stream);
+    if (row_off) {
+        TRY_ST(d_row_off.load(ctx, row_off, n_rows + 1));
+        TRY_ST(d_store_off.load(ctx, store_off.data(), n_rows + 1));
+    }
     locohd_envset* e = new locohd_envset();
-    const uint64_t row_stride = (row_len + 1) & ~1ull;
-    e->ctx = ctx; e->n_env = n_rows; e->total = n_rows * row_stride; e->capacity = e->total + 2;
+    e->ctx = ctx; e->n_env = n_rows; e->total = total; e->capacity = total + 2;
     e->max_count = (unsigned)row_len;
     e->key_is_w = ctx->kp.n_wf == 1;
-    uint8_t* d_cat = nullptr;
+    uint8_t *d_cat8 = nullptr, *d_cat = nullptr;
     auto bail = [&](int st) { dev_free(ctx, d_cat8); dev_free(ctx, d_cat); destroy_envset(e); return st; };
     int st;
-    if ((st = dev_alloc(ctx, &e->d_count, n_rows)) || (st = dev_alloc(ctx, &e->d_off, n_rows + 1)) ||
-        (st = dev_alloc(ctx, &e->d_key, e->capacity)) || (st = dev_alloc(ctx, &d_cat, e->capacity)) ||
-        (st = dev_alloc(ctx, &e->d_idx, e->capacity)) || (st = dev_alloc(ctx, &e->d_dist, e->capacity)))
+    if ((st = dev_alloc(ctx, &d_cat8, row_len)) || (st = dev_alloc(ctx, &e->d_count, n_rows)) ||
+        (st = dev_alloc(ctx, &e->d_off, n_rows + 1)) || (st = dev_alloc(ctx, &e->d_key, e->capacity)) ||
+        (st = dev_alloc(ctx, &d_cat, e->capacity)) || (st = dev_alloc(ctx, &e->d_idx, e->capacity)) ||
+        (st = dev_alloc(ctx, &e->d_dist, e->capacity)))
         return bail(st);
+    ctx->launches += launch_convert_categories(cat16.ptr, d_cat8, row_len, ctx->kp.C, ctx->stream);
+    if (xyz) ctx->launches += launch_validate_xyz(in.ptr, 3 * row_len, ctx->d_err, ctx->stream);
     EnvBuild b{};
     b.n_env = n_rows; b.off = e->d_off; b.count = e->d_count; b.key = e->d_key; b.cat = d_cat; b.idx = e->d_idx;
     b.dist = e->d_dist; b.key_is_w = e->key_is_w ? 1 : 0; b.key_is_sq = 0; b.check_first_zero = 1;
     {
         ProfScope ps(ctx, LOCOHD_PROF_OTHER);
-        ctx->launches += launch_rows_copy(dmx ? in.ptr : nullptr, d_cat8, n_rows, row_len, xyz ? in.ptr : nullptr,
-                                          ctx->kp, e->d_off, e->d_count, b, ctx->stream);
+        ctx->launches += launch_rows_copy(xyz ? nullptr : in.ptr, xyz ? in.ptr : nullptr, d_cat8, n_rows, row_len,
+                                          d_row_off.ptr, d_store_off.ptr, e->d_off, e->d_count, b, ctx->stream);
     }
     {
         ProfScope ps(ctx, LOCOHD_PROF_SORT);
@@ -1173,7 +1236,7 @@ static int rows_envset(locohd_ctx* ctx, uint64_t n_rows, uint64_t row_len, const
     }
     cudaError_t ce = cudaGetLastError();
     if (ce != cudaSuccess) return bail(fail(ctx, LOCOHD_ERR_CUDA, "launch failed: %s", cudaGetErrorString(ce)));
-    if ((st = sync_and_check(ctx))) return bail(st);
+    if ((st = sync_and_check(ctx))) return bail(st);   // also keeps store_off alive until its copy is done
     dev_free(ctx, d_cat8); dev_free(ctx, d_cat);
     *out = e;
     return 0;
@@ -1182,16 +1245,18 @@ static int rows_envset(locohd_ctx* ctx, uint64_t n_rows, uint64_t row_len, const
 int locohd_envset_from_rows(locohd_ctx* ctx, uint64_t n_rows, uint64_t row_len, const double* dmx,
                             const uint16_t* category, locohd_envset** out) {
     API_BEGIN(ctx)
-    if (!dmx && n_rows * row_len) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null distance matrix");
-    return rows_envset(ctx, n_rows, row_len, dmx, nullptr, category, out);
+    TRY_ST(need_params(ctx));
+    if (!dmx) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null distance matrix");
+    return rows_envset(ctx, n_rows, nullptr, row_len, dmx, nullptr, category, out);
     API_END()
 }
 
 int locohd_envset_from_coords(locohd_ctx* ctx, uint64_t n_points, const double* xyz, const uint16_t* category,
                               locohd_envset** out) {
     API_BEGIN(ctx)
-    if (!xyz && n_points) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null coordinates");
-    return rows_envset(ctx, n_points, n_points, nullptr, xyz, category, out);
+    TRY_ST(need_params(ctx));
+    if (!xyz) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null coordinates");
+    return rows_envset(ctx, n_points, nullptr, n_points, nullptr, xyz, category, out);
     API_END()
 }
 
@@ -1201,7 +1266,7 @@ int locohd_envset_from_ragged_rows(locohd_ctx* ctx, uint64_t n_rows, const uint6
     TRY_ST(need_params(ctx));
     if (!out || !row_offsets) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
     *out = nullptr;
-    std::vector<uint64_t> in_off(n_rows + 1), out_off(n_rows + 1, 0);
+    std::vector<uint64_t> in_off(n_rows + 1);
     if (is_device_ptr(ctx, row_offsets)) CU(ctx, cudaMemcpy(in_off.data(), row_offsets, in_off.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost));
     else std::memcpy(in_off.data(), row_offsets, in_off.size() * sizeof(uint64_t));
     uint64_t max_len = 0;
@@ -1214,48 +1279,9 @@ int locohd_envset_from_ragged_rows(locohd_ctx* ctx, uint64_t n_rows, const uint6
             return fail(ctx, LOCOHD_ERR_LEN_MISMATCH, "row %llu has %llu distances but only %llu categories were given",
                         (unsigned long long)r, (unsigned long long)len, (unsigned long long)n_categories_given);
         max_len = std::max(max_len, len);
-        out_off[r + 1] = out_off[r] + ((len + 1) & ~1ull);
     }
-    const uint64_t total_in = in_off[n_rows];
-    if (total_in && (!values || !category)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
-    InBuf<double> vals;
-    InBuf<uint16_t> cat16;
-    InBuf<uint64_t> d_in, d_out;
-    TRY_ST(vals.load(ctx, values, total_in));
-    TRY_ST(cat16.load(ctx, category, max_len));
-    TRY_ST(d_in.load(ctx, in_off.data(), n_rows + 1));
-    TRY_ST(d_out.load(ctx, out_off.data(), n_rows + 1));
-    uint8_t *d_cat8 = nullptr, *d_cat = nullptr;
-    locohd_envset* e = new locohd_envset();
-    e->ctx = ctx; e->n_env = n_rows; e->total = out_off[n_rows]; e->capacity = e->total + 2;
-    e->max_count = (unsigned)max_len;
-    e->key_is_w = ctx->kp.n_wf == 1;
-    auto bail = [&](int st) { dev_free(ctx, d_cat8); dev_free(ctx, d_cat); destroy_envset(e); return st; };
-    int st;
-    if ((st = dev_alloc(ctx, &d_cat8, max_len)) || (st = dev_alloc(ctx, &e->d_count, n_rows)) ||
-        (st = dev_alloc(ctx, &e->d_off, n_rows + 1)) || (st = dev_alloc(ctx, &e->d_key, e->capacity)) ||
-        (st = dev_alloc(ctx, &d_cat, e->capacity)) || (st = dev_alloc(ctx, &e->d_idx, e->capacity)) ||
-        (st = dev_alloc(ctx, &e->d_dist, e->capacity)))
-        return bail(st);
-    ctx->launches += launch_convert_categories(cat16.ptr, d_cat8, max_len, ctx->kp.C, ctx->stream);
-    EnvBuild b{};
-    b.n_env = n_rows; b.off = e->d_off; b.count = e->d_count; b.key = e->d_key; b.cat = d_cat; b.idx = e->d_idx;
-    b.dist = e->d_dist; b.key_is_w = e->key_is_w ? 1 : 0; b.key_is_sq = 0; b.check_first_zero = 1;
-    {
-        ProfScope ps(ctx, LOCOHD_PROF_OTHER);
-        ctx->launches += launch_ragged_rows_copy(vals.ptr, d_cat8, n_rows, max_len, d_in.ptr, d_out.ptr, e->d_off, e->d_count,
-                                                 b, ctx->stream);
-    }
-    {
-        ProfScope ps(ctx, LOCOHD_PROF_SORT);
-        ctx->launches += launch_env_sort(ctx->kp, b, e->max_count, 0.0, ctx->stream);
-    }
-    cudaError_t ce = cudaGetLastError();
-    if (ce != cudaSuccess) return bail(fail(ctx, LOCOHD_ERR_CUDA, "launch failed: %s", cudaGetErrorString(ce)));
-    if ((st = sync_and_check(ctx))) return bail(st);   // also keeps the host offset vectors alive until their copies are done
-    dev_free(ctx, d_cat8); dev_free(ctx, d_cat);
-    *out = e;
-    return 0;
+    if (in_off[n_rows] && (!values || !category)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
+    return rows_envset(ctx, n_rows, in_off.data(), max_len, values, nullptr, category, out);
     API_END()
 }
 
@@ -1529,162 +1555,89 @@ int locohd_from_primitives(locohd_ctx* ctx, uint64_t n_a, const double* xyz_a, c
     TRY_ST(check_wf_indices(ctx, wf_idx, n_pairs));
     const LaunchOverrides ov = read_launch_overrides();
     const uint64_t n = n_a + n_b;
-    {
-        // Small calls with host inputs (the typical call of the reference API: one structure pair) travel in ONE
-        // pinned staging buffer and one host-to-device copy, and all device arrays of the call are views into one
-        // device block: a dozen pageable copies and allocations of ~10 us each otherwise dominate such a call.
-        const bool host_in = !is_device_ptr(ctx, xyz_a) && !is_device_ptr(ctx, xyz_b) && !is_device_ptr(ctx, cat_a) &&
-                             !is_device_ptr(ctx, cat_b) && !is_device_ptr(ctx, tag_a) && !is_device_ptr(ctx, tag_b) &&
-                             !is_device_ptr(ctx, anchors) && !(wf_idx && is_device_ptr(ctx, wf_idx));
-        auto up = [](size_t v, size_t a) { return (v + a - 1) / a * a; };
-        size_t o = 0;
-        const size_t o_prim = o; o = up(o + 3 * sizeof(uint64_t), 32);
-        const size_t o_job = o; o = up(o + sizeof(locohd_job), 32);
-        const size_t o_xyz = o; o = up(o + 3 * n * sizeof(double), 32);
-        const size_t o_tag = o; o = up(o + n * sizeof(uint32_t), 32);
-        const size_t o_as = o; o = up(o + 2 * n_pairs * sizeof(uint32_t), 32);
-        const size_t o_ap = o; o = up(o + 2 * n_pairs * sizeof(uint32_t), 32);
-        const size_t o_cat16 = o; o = up(o + n * sizeof(uint16_t), 32);
-        const size_t o_wf = o; o = up(o + (wf_idx ? n_pairs * sizeof(uint32_t) : 0), 32);
-        const size_t upload_bytes = o;
-        if (host_in && upload_bytes <= (8u << 20)) {
-            // device-only part of the block
-            const size_t o_cat8 = o; o = up(o + n, 32);
-            const size_t o_meta = o; o = up(o + 2 * sizeof(StructMeta), 32);
-            const size_t o_pf = o; o = up(o + n * sizeof(float4), 32);
-            const size_t o_pd = o; o = up(o + n * sizeof(PrimRec), 32);
-            const size_t o_porig = o; o = up(o + n * sizeof(uint32_t), 32);
-            const size_t o_spos = o; o = up(o + n * sizeof(uint32_t), 32);
-            const size_t o_cs = o; o = up(o + cell_entries(n, 2) * sizeof(uint32_t), 32);
-            const size_t o_cf = o; o = up(o + cell_entries(n, 2) * sizeof(uint32_t), 32);
-            const size_t total_bytes = o;
-            if (ctx->h_stage_bytes < upload_bytes) {
-                if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
-                ctx->h_stage = nullptr; ctx->h_stage_bytes = 0;
-                const size_t want = std::max<size_t>(upload_bytes * 2, 1u << 20);
-                if (cudaHostAlloc((void**)&ctx->h_stage, want, cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); ctx->h_stage = nullptr; }
-                else ctx->h_stage_bytes = want;
-            }
-            if (ctx->h_stage) {
-                unsigned char* h = ctx->h_stage;
-                const uint64_t offs[3] = {0, n_a, n};
-                std::memcpy(h + o_prim, offs, sizeof offs);
-                const locohd_job job{0, n_pairs, n_pairs};
-                std::memcpy(h + o_job, &job, sizeof job);
-                std::memcpy(h + o_xyz, xyz_a, 3 * n_a * sizeof(double));
-                std::memcpy(h + o_xyz + 3 * n_a * sizeof(double), xyz_b, 3 * n_b * sizeof(double));
-                std::memcpy(h + o_tag, tag_a, n_a * sizeof(uint32_t));
-                std::memcpy(h + o_tag + n_a * sizeof(uint32_t), tag_b, n_b * sizeof(uint32_t));
-                std::memcpy(h + o_cat16, cat_a, n_a * sizeof(uint16_t));
-                std::memcpy(h + o_cat16 + n_a * sizeof(uint16_t), cat_b, n_b * sizeof(uint16_t));
-                uint32_t* has = reinterpret_cast<uint32_t*>(h + o_as);
-                uint32_t* hap = reinterpret_cast<uint32_t*>(h + o_ap);
-                for (uint64_t i = 0; i < n_pairs; ++i) {   // environments [0, P) belong to A, [P, 2P) to B
-                    has[i] = 0; hap[i] = anchors[2 * i];
-                    has[n_pairs + i] = 1; hap[n_pairs + i] = anchors[2 * i + 1];
-                }
-                if (wf_idx) std::memcpy(h + o_wf, wf_idx, n_pairs * sizeof(uint32_t));
-                unsigned char* d = nullptr;
-                TRY_ST(dev_alloc(ctx, &d, total_bytes));
-                locohd_structs* s = new locohd_structs();
-                s->ctx = ctx; s->n_structs = 2; s->n_prims = n; s->max_prims = std::max<uint64_t>(n_a, n_b);
-                s->blob = d;
-                s->d_prim_off = reinterpret_cast<uint64_t*>(d + o_prim);
-                s->d_xyz = reinterpret_cast<double*>(d + o_xyz);
-                s->d_tag = reinterpret_cast<uint32_t*>(d + o_tag);
-                s->d_cat = d + o_cat8;
-                s->d_meta = reinterpret_cast<StructMeta*>(d + o_meta);
-                s->d_pf = reinterpret_cast<float4*>(d + o_pf);
-                s->d_pd = reinterpret_cast<PrimRec*>(d + o_pd);
-                s->d_porig = reinterpret_cast<uint32_t*>(d + o_porig);
-                s->d_sorted_pos = reinterpret_cast<uint32_t*>(d + o_spos);
-                s->d_cell_start = reinterpret_cast<uint32_t*>(d + o_cs);
-                s->d_cell_fill = reinterpret_cast<uint32_t*>(d + o_cf);
-                locohd_envset* env = nullptr;
-                auto done = [&](int st) { if (env) destroy_envset(env); locohd_structs_destroy(s); return st; };
-                if (cudaMemcpyAsync(d, h, upload_bytes, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess)
-                    return done(fail(ctx, LOCOHD_ERR_CUDA, "upload failed: %s", cudaGetErrorString(cudaGetLastError())));
-                ctx->launches += launch_convert_categories(reinterpret_cast<const uint16_t*>(d + o_cat16), s->d_cat, n, ctx->kp.C, ctx->stream);
-                ctx->launches += launch_validate_xyz(s->d_xyz, 3 * n, ctx->d_err, ctx->stream);
-                int st = build_envset(ctx, s, 2 * n_pairs, reinterpret_cast<const uint32_t*>(d + o_as),
-                                      reinterpret_cast<const uint32_t*>(d + o_ap), threshold, 0, ov, &env);
-                if (st) return done(st);
-                OutBuf<double> out;
-                if ((st = out.prepare(ctx, out_scores, n_pairs))) return done(st);
-                st = run_score(ctx, env, env, n_pairs, nullptr, reinterpret_cast<const locohd_job*>(d + o_job), nullptr, 1, n_pairs,
-                               wf_idx ? reinterpret_cast<const uint32_t*>(d + o_wf) : nullptr, out.ptr, ov);
-                if (!st) st = out.commit();
-                const int st2 = sync_and_check(ctx);
-                return done(st ? st : st2);
-            }
+    // One structure set holding A then B.  Its device block starts with the arrays of the call: the job, the anchors
+    // of the 2 P environments ([0, P) belong to A, [P, 2 P) to B), the categories as given and the per-pair weight
+    // function indices.  Everything the host sends lands in the range [0, upload_end) of the block.
+    BlockCursor head;
+    const size_t o_job = head.take(sizeof(locohd_job));
+    const size_t o_as = head.take(2 * n_pairs * sizeof(uint32_t));
+    const size_t o_ap = head.take(2 * n_pairs * sizeof(uint32_t));
+    const size_t o_cat16 = head.take(n * sizeof(uint16_t));
+    const size_t o_wf = head.take(wf_idx ? n_pairs * sizeof(uint32_t) : 0);
+    const StructsLayout l = structs_layout(2, n, head.end);
+    // Small calls with host inputs (the typical call of the reference API: one structure pair) are packed into one
+    // pinned staging buffer and sent with one copy: a dozen pageable copies of ~10 us each otherwise dominate such a
+    // call.  Any other call copies every input into its place in the block.
+    const bool host_in = !is_device_ptr(ctx, xyz_a) && !is_device_ptr(ctx, xyz_b) && !is_device_ptr(ctx, cat_a) &&
+                         !is_device_ptr(ctx, cat_b) && !is_device_ptr(ctx, tag_a) && !is_device_ptr(ctx, tag_b) &&
+                         !is_device_ptr(ctx, anchors) && !(wf_idx && is_device_ptr(ctx, wf_idx));
+    unsigned char* h = nullptr;
+    if (host_in && l.upload_end <= (8u << 20)) {
+        if (ctx->h_stage_bytes < l.upload_end) {
+            if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
+            ctx->h_stage = nullptr; ctx->h_stage_bytes = 0;
+            const size_t want = std::max<size_t>(l.upload_end * 2, 1u << 20);
+            if (cudaHostAlloc((void**)&ctx->h_stage, want, cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); ctx->h_stage = nullptr; }
+            else ctx->h_stage_bytes = want;
         }
+        h = ctx->h_stage;
     }
-    // one structure set holding A then B
-    locohd_structs* s = new locohd_structs();
-    s->ctx = ctx; s->n_structs = 2; s->n_prims = n;
-    s->max_prims = std::max<uint64_t>(n_a, n_b);
-    locohd_envset* env = nullptr;
-    uint32_t *d_as = nullptr, *d_ap = nullptr;
-    auto cleanup = [&](int st) {
-        dev_free(ctx, d_as); dev_free(ctx, d_ap);
-        if (env) destroy_envset(env);
-        locohd_structs_destroy(s);
-        return st;
-    };
-    int st;
-    if ((st = dev_alloc(ctx, &s->d_prim_off, 3)) || (st = dev_alloc(ctx, &s->d_xyz, 3 * n)) ||
-        (st = dev_alloc(ctx, &s->d_cat, n)) || (st = dev_alloc(ctx, &s->d_tag, n)) ||
-        (st = dev_alloc(ctx, &s->d_meta, 2)) || (st = dev_alloc(ctx, &s->d_pf, n)) ||
-        (st = dev_alloc(ctx, &s->d_pd, n)) || (st = dev_alloc(ctx, &s->d_porig, n)) ||
-        (st = dev_alloc(ctx, &s->d_sorted_pos, n)) ||
-        (st = dev_alloc(ctx, &s->d_cell_start, cell_entries(n, 2))) ||
-        (st = dev_alloc(ctx, &s->d_cell_fill, cell_entries(n, 2))))
-        return cleanup(st);
+    // the A/B split of the anchors is built on the host (device anchors are copied back first)
+    std::vector<uint32_t> h_anchor, h_split;
+    const uint32_t* an = anchors;
+    if (is_device_ptr(ctx, anchors)) {
+        h_anchor.resize(2 * n_pairs);
+        CU(ctx, cudaMemcpy(h_anchor.data(), anchors, 2 * n_pairs * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+        an = h_anchor.data();
+    }
+    if (!h) h_split.resize(4 * n_pairs);
+    uint32_t* has = h ? reinterpret_cast<uint32_t*>(h + o_as) : h_split.data();
+    uint32_t* hap = h ? reinterpret_cast<uint32_t*>(h + o_ap) : h_split.data() + 2 * n_pairs;
+    for (uint64_t i = 0; i < n_pairs; ++i) {
+        has[i] = 0; hap[i] = an[2 * i];
+        has[n_pairs + i] = 1; hap[n_pairs + i] = an[2 * i + 1];
+    }
     const uint64_t offs[3] = {0, n_a, n};
-    cudaError_t ce = cudaMemcpyAsync(s->d_prim_off, offs, sizeof offs, cudaMemcpyHostToDevice, ctx->stream);
-    if (ce == cudaSuccess && n_a) ce = cudaMemcpyAsync(s->d_xyz, xyz_a, 3 * n_a * sizeof(double), cudaMemcpyDefault, ctx->stream);
-    if (ce == cudaSuccess && n_b) ce = cudaMemcpyAsync(s->d_xyz + 3 * n_a, xyz_b, 3 * n_b * sizeof(double), cudaMemcpyDefault, ctx->stream);
-    if (ce == cudaSuccess && n_a) ce = cudaMemcpyAsync(s->d_tag, tag_a, n_a * sizeof(uint32_t), cudaMemcpyDefault, ctx->stream);
-    if (ce == cudaSuccess && n_b) ce = cudaMemcpyAsync(s->d_tag + n_a, tag_b, n_b * sizeof(uint32_t), cudaMemcpyDefault, ctx->stream);
-    if (ce != cudaSuccess) return cleanup(fail(ctx, LOCOHD_ERR_CUDA, "upload failed: %s", cudaGetErrorString(ce)));
-    {
-        InBuf<uint16_t> ca, cb;
-        if ((st = ca.load(ctx, cat_a, n_a)) || (st = cb.load(ctx, cat_b, n_b))) return cleanup(st);
-        ctx->launches += launch_convert_categories(ca.ptr, s->d_cat, n_a, ctx->kp.C, ctx->stream);
-        ctx->launches += launch_convert_categories(cb.ptr, s->d_cat + n_a, n_b, ctx->kp.C, ctx->stream);
-    }
-    ctx->launches += launch_validate_xyz(s->d_xyz, 3 * n, ctx->d_err, ctx->stream);
-    // anchors: environments [0, P) belong to A, [P, 2P) to B
-    std::vector<uint32_t> h_as(2 * n_pairs), h_ap(2 * n_pairs);
-    {
-        std::vector<uint32_t> h_anchor;
-        const uint32_t* an = anchors;
-        if (is_device_ptr(ctx, anchors)) {
-            h_anchor.resize(2 * n_pairs);
-            ce = cudaMemcpy(h_anchor.data(), anchors, 2 * n_pairs * sizeof(uint32_t), cudaMemcpyDeviceToHost);
-            if (ce != cudaSuccess) return cleanup(fail(ctx, LOCOHD_ERR_CUDA, "anchor download failed: %s", cudaGetErrorString(ce)));
-            an = h_anchor.data();
-        }
-        for (uint64_t i = 0; i < n_pairs; ++i) {
-            h_as[i] = 0; h_ap[i] = an[2 * i];
-            h_as[n_pairs + i] = 1; h_ap[n_pairs + i] = an[2 * i + 1];
-        }
-    }
-    if ((st = dev_alloc(ctx, &d_as, 2 * n_pairs)) || (st = dev_alloc(ctx, &d_ap, 2 * n_pairs))) return cleanup(st);
-    ce = cudaMemcpyAsync(d_as, h_as.data(), 2 * n_pairs * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream);
-    if (ce == cudaSuccess) ce = cudaMemcpyAsync(d_ap, h_ap.data(), 2 * n_pairs * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream);
-    if (ce != cudaSuccess) return cleanup(fail(ctx, LOCOHD_ERR_CUDA, "upload failed: %s", cudaGetErrorString(ce)));
-    if ((st = build_envset(ctx, s, 2 * n_pairs, d_as, d_ap, threshold, 0, ov, &env))) return cleanup(st);
+    locohd_structs* s = nullptr;
+    TRY_ST(structs_alloc(ctx, 2, offs, l, &s));
+    unsigned char* d = s->block;
+    locohd_envset* env = nullptr;
+    auto done = [&](int st) { if (env) destroy_envset(env); locohd_structs_destroy(s); return st; };
+    cudaError_t ce = cudaSuccess;
+    auto put = [&](size_t at, const void* src, size_t bytes) {
+        if (!bytes || ce != cudaSuccess) return;
+        if (h) std::memcpy(h + at, src, bytes);
+        else ce = cudaMemcpyAsync(d + at, src, bytes, cudaMemcpyDefault, ctx->stream);
+    };
     const locohd_job job{0, n_pairs, n_pairs};
-    InBuf<locohd_job> dj;
-    InBuf<uint32_t> wf;
+    put(o_job, &job, sizeof job);
+    put(l.prim_off, offs, sizeof offs);
+    put(l.xyz, xyz_a, 3 * n_a * sizeof(double));
+    put(l.xyz + 3 * n_a * sizeof(double), xyz_b, 3 * n_b * sizeof(double));
+    put(l.tag, tag_a, n_a * sizeof(uint32_t));
+    put(l.tag + n_a * sizeof(uint32_t), tag_b, n_b * sizeof(uint32_t));
+    put(o_cat16, cat_a, n_a * sizeof(uint16_t));
+    put(o_cat16 + n_a * sizeof(uint16_t), cat_b, n_b * sizeof(uint16_t));
+    if (wf_idx) put(o_wf, wf_idx, n_pairs * sizeof(uint32_t));
+    if (h) {
+        ce = cudaMemcpyAsync(d, h, l.upload_end, cudaMemcpyHostToDevice, ctx->stream);
+    } else {
+        put(o_as, has, 2 * n_pairs * sizeof(uint32_t));
+        put(o_ap, hap, 2 * n_pairs * sizeof(uint32_t));
+    }
+    if (ce != cudaSuccess) return done(fail(ctx, LOCOHD_ERR_CUDA, "upload failed: %s", cudaGetErrorString(ce)));
+    ctx->launches += launch_convert_categories(reinterpret_cast<const uint16_t*>(d + o_cat16), s->d_cat, n, ctx->kp.C, ctx->stream);
+    ctx->launches += launch_validate_xyz(s->d_xyz, 3 * n, ctx->d_err, ctx->stream);
+    int st = build_envset(ctx, s, 2 * n_pairs, reinterpret_cast<const uint32_t*>(d + o_as),
+                          reinterpret_cast<const uint32_t*>(d + o_ap), threshold, 0, ov, &env);
+    if (st) return done(st);
     OutBuf<double> out;
-    if ((st = dj.load(ctx, &job, 1)) || (st = wf.load(ctx, wf_idx, n_pairs)) || (st = out.prepare(ctx, out_scores, n_pairs)))
-        return cleanup(st);
-    st = run_score(ctx, env, env, n_pairs, nullptr, dj.ptr, nullptr, 1, n_pairs, wf.ptr, out.ptr, ov);
+    if ((st = out.prepare(ctx, out_scores, n_pairs))) return done(st);
+    st = run_score(ctx, env, env, n_pairs, nullptr, reinterpret_cast<const locohd_job*>(d + o_job), nullptr, 1, n_pairs,
+                   wf_idx ? reinterpret_cast<const uint32_t*>(d + o_wf) : nullptr, out.ptr, ov);
     if (!st) st = out.commit();
-    const int st2 = sync_and_check(ctx);
-    return cleanup(st ? st : st2);
+    const int st2 = sync_and_check(ctx);   // also keeps the host arrays of the upload alive until it is done
+    return done(st ? st : st2);
     API_END()
 }
 

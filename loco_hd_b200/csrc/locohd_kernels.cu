@@ -1259,31 +1259,22 @@ __device__ __forceinline__ double row_distance(const double* xyz, uint64_t i, ui
     return sqrt(__dadd_rn(__dadd_rn(__dmul_rn(ex, ex), __dmul_rn(ey, ey)), __dmul_rn(ez, ez)));
 }
 
-__global__ void rows_copy_kernel(const double* __restrict__ dmx, const uint8_t* __restrict__ cat, uint64_t n_rows,
-                                 uint64_t row_len, uint64_t row_stride, const double* __restrict__ xyz,
+// Row r starts at in_off[r] of the input and at out_off[r] of the store (ragged rows, utils.rs:25-39: row r is
+// co-sorted with the first len_r categories), or, without offsets, holds row_len entries and starts at r * row_len of
+// the input and at r * row_stride of the store.  With xyz the entries are the distances of point r to the points.
+__global__ void rows_copy_kernel(const double* __restrict__ values, const double* __restrict__ xyz,
+                                 const uint8_t* __restrict__ cat, uint64_t n_rows, uint64_t row_len,
+                                 const uint64_t* __restrict__ in_off, const uint64_t* __restrict__ out_off,
                                  uint64_t* off, uint32_t* count, EnvBuild b) {
+    const uint64_t row_stride = (row_len + 1) & ~1ull;
     for (uint64_t row = blockIdx.y; row < n_rows; row += gridDim.y) {
-        if (blockIdx.x == 0 && threadIdx.x == 0) { off[row] = row * row_stride; count[row] = (uint32_t)row_len; }
-        for (uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; j < row_len;
-             j += (uint64_t)gridDim.x * blockDim.x) {
-            const double d = xyz ? row_distance(xyz, row, j) : dmx[row * row_len + j];
-            b.key[row * row_stride + j] = (uint64_t)__double_as_longlong(d);
-            b.cat[row * row_stride + j] = cat[j];
-            if (b.idx) b.idx[row * row_stride + j] = (uint32_t)j;
-        }
-    }
-}
-
-// Ragged rows (from_dmxs with rows of different lengths, utils.rs:25-39: row r is co-sorted with the first len_r
-// categories): in_off / out_off are the offsets of the rows in the input and in the store.
-__global__ void ragged_rows_copy_kernel(const double* __restrict__ values, const uint8_t* __restrict__ cat,
-                                        uint64_t n_rows, const uint64_t* __restrict__ in_off,
-                                        const uint64_t* __restrict__ out_off, uint64_t* off, uint32_t* count, EnvBuild b) {
-    for (uint64_t row = blockIdx.y; row < n_rows; row += gridDim.y) {
-        const uint64_t i0 = in_off[row], len = in_off[row + 1] - i0, o0 = out_off[row];
+        const uint64_t i0 = in_off ? in_off[row] : row * row_len;
+        const uint64_t len = in_off ? in_off[row + 1] - i0 : row_len;
+        const uint64_t o0 = out_off ? out_off[row] : row * row_stride;
         if (blockIdx.x == 0 && threadIdx.x == 0) { off[row] = o0; count[row] = (uint32_t)len; }
         for (uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; j < len; j += (uint64_t)gridDim.x * blockDim.x) {
-            b.key[o0 + j] = (uint64_t)__double_as_longlong(values[i0 + j]);
+            const double d = xyz ? row_distance(xyz, row, j) : values[i0 + j];
+            b.key[o0 + j] = (uint64_t)__double_as_longlong(d);
             b.cat[o0 + j] = cat[j];
             if (b.idx) b.idx[o0 + j] = (uint32_t)j;
         }
@@ -2692,25 +2683,13 @@ int launch_env_sort(const KParams& p, const EnvBuild& b, unsigned max_count, dou
     return b.idx ? launch_env_sort_t<true>(p, b, max_count, scale, st) : launch_env_sort_t<false>(p, b, max_count, scale, st);
 }
 
-int launch_rows_copy(const double* dmx, const uint8_t* cat, uint64_t n_rows, uint64_t row_len, const double* xyz,
-                     const KParams& p, uint64_t* off, uint32_t* count, const EnvBuild& b, cudaStream_t st) {
-    (void)p;
+int launch_rows_copy(const double* values, const double* xyz, const uint8_t* cat, uint64_t n_rows, uint64_t row_len,
+                     const uint64_t* in_off, const uint64_t* out_off, uint64_t* off, uint32_t* count, const EnvBuild& b,
+                     cudaStream_t st) {
     if (!n_rows || !row_len) return 0;
-    const uint64_t row_stride = (row_len + 1) & ~1ull;
     dim3 grid((unsigned)((row_len + 255) / 256), (unsigned)(n_rows > 32768 ? 32768 : n_rows));
     if (grid.x > 64) grid.x = 64;
-    rows_copy_kernel<<<grid, 256, 0, st>>>(dmx, cat, n_rows, row_len, row_stride, xyz, off, count, b);
-    return 1;
-}
-
-int launch_ragged_rows_copy(const double* values, const uint8_t* cat, uint64_t n_rows, uint64_t max_len,
-                            const uint64_t* in_off, const uint64_t* out_off, uint64_t* off, uint32_t* count,
-                            const EnvBuild& b, cudaStream_t st) {
-    if (!n_rows) return 0;
-    dim3 grid((unsigned)((max_len + 255) / 256), (unsigned)(n_rows > 32768 ? 32768 : n_rows));
-    if (grid.x > 64) grid.x = 64;
-    if (grid.x < 1) grid.x = 1;
-    ragged_rows_copy_kernel<<<grid, 256, 0, st>>>(values, cat, n_rows, in_off, out_off, off, count, b);
+    rows_copy_kernel<<<grid, 256, 0, st>>>(values, xyz, cat, n_rows, row_len, in_off, out_off, off, count, b);
     return 1;
 }
 

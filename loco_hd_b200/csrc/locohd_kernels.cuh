@@ -232,11 +232,11 @@ int launch_env_fill(const StructsView& s, const KParams& p, const uint32_t* anch
                     double threshold, const EnvBuild& b, cudaStream_t st);
 // sorts every environment of the store in place and packs the keys; max_count bounds the environment sizes
 int launch_env_sort(const KParams& p, const EnvBuild& b, unsigned max_count, double threshold, cudaStream_t st);
-int launch_rows_copy(const double* dmx, const uint8_t* cat, uint64_t n_rows, uint64_t row_len, const double* xyz,
-                     const KParams& p, uint64_t* off, uint32_t* count, const EnvBuild& b, cudaStream_t st);
-int launch_ragged_rows_copy(const double* values, const uint8_t* cat, uint64_t n_rows, uint64_t max_len,
-                            const uint64_t* in_off, const uint64_t* out_off, uint64_t* off, uint32_t* count,
-                            const EnvBuild& b, cudaStream_t st);
+// rows into the store, unsorted: values (or the distances among the row_len points xyz) of rows of row_len entries,
+// or, with in_off / out_off, of ragged rows (row_len: the longest row) at those offsets of the input and the store
+int launch_rows_copy(const double* values, const double* xyz, const uint8_t* cat, uint64_t n_rows, uint64_t row_len,
+                     const uint64_t* in_off, const uint64_t* out_off, uint64_t* off, uint32_t* count, const EnvBuild& b,
+                     cudaStream_t st);
 // Test and A/B hooks that override launch decisions of the library, read from the process environment by
 // read_launch_overrides() once per API call, so that a process can change them between calls.  The defaults leave
 // every decision to the library.  No other code of the library reads the environment.

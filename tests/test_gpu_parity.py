@@ -165,6 +165,53 @@ def test_per_anchor_weight_functions(gpu_ctx, oracle_mod):
     check_from_primitives(gpu_ctx, oracle_mod, op, A, B, anchors, 11.0, wf_idx=wf_idx, check_envs=False)
 
 
+# ------------------------------------------------------------------ one-call upload routes (staged / copied per input)
+def test_from_primitives_device_inputs(gpu_ctx, oracle_mod):
+    """Every input of a one-call score already on the device (torch CUDA tensors passed as raw pointers): the inputs
+    are copied one by one into the call's device block instead of travelling in the pinned staging buffer.  Same
+    scores, bit for bit, as the same call with numpy inputs."""
+    import torch
+
+    a, b = synth.config1()
+    op = set_both(gpu_ctx, oracle_mod, 7, [("uniform", (3.0, 10.0)), ("kumaraswamy", (3.0, 10.0, 2.0, 5.0))],
+                  tag_rule={"accept_same": False})
+    rng = np.random.default_rng(19)
+    anchors = np.stack([rng.permutation(a.n)[:200], rng.permutation(b.n)[:200]], axis=1).astype(np.uint32)
+    wf_idx = rng.integers(0, 2, len(anchors)).astype(np.uint32)
+    host = gpu_ctx.from_primitives(a.xyz, a.cat, a.tag, b.xyz, b.cat, b.tag, anchors, 10.0, wf_idx=wf_idx)
+    # unsigned arrays travel as signed torch tensors of the same bits
+    arrays = (a.xyz, a.cat.view(np.int16), a.tag.view(np.int32), b.xyz, b.cat.view(np.int16), b.tag.view(np.int32),
+              anchors.view(np.int32), wf_idx.view(np.int32))
+    dev = [torch.from_numpy(np.ascontiguousarray(x)).cuda() for x in arrays]
+    torch.cuda.synchronize()
+    ptr = [t.data_ptr() for t in dev]
+    got = gpu_ctx.from_primitives(*ptr[:7], 10.0, wf_idx=ptr[7], n_a=a.n, n_b=b.n, n_pairs=len(anchors))
+    assert np.array_equal(got, host)
+    ref = oracle_mod.from_primitives(op, a.xyz, a.cat, a.tag, b.xyz, b.cat, b.tag, anchors, 10.0, wf_idx=wf_idx)
+    assert_scores_close(got, ref)
+    # the indices matter: weight function 0 for every pair gives other scores
+    assert not np.array_equal(got, gpu_ctx.from_primitives(a.xyz, a.cat, a.tag, b.xyz, b.cat, b.tag, anchors, 10.0))
+
+
+def test_from_primitives_above_the_staging_limit(gpu_ctx, oracle_mod):
+    """A host call whose upload exceeds the 8 MB staging buffer (525 000 anchor pairs of 16 B) copies its inputs one
+    by one into the call's device block.  Every pair fits the scoring stage and its arithmetic does not depend on the
+    other pairs of the launch, so the scores equal, bit for bit, those of the same pairs in two staged calls."""
+    a = synth.gen(41, 625, 8, 7)   # 5 000 primitives each
+    b = synth.partner(a, 1.0, 42)
+    A, B = (a.xyz, a.cat, a.tag), (b.xyz, b.cat, b.tag)
+    op = set_both(gpu_ctx, oracle_mod, 7, [("kumaraswamy", (3.0, 10.0, 2.0, 5.0))], tag_rule={"accept_same": False})
+    rng = np.random.default_rng(43)
+    anchors = rng.integers(0, a.n, size=(525_000, 2)).astype(np.uint32)
+    whole = gpu_ctx.from_primitives(*A, *B, anchors, 10.0)
+    half = len(anchors) // 2
+    parts = np.concatenate([gpu_ctx.from_primitives(*A, *B, anchors[:half], 10.0),
+                            gpu_ctx.from_primitives(*A, *B, anchors[half:], 10.0)])
+    assert np.array_equal(whole, parts)
+    sample = np.sort(rng.choice(len(anchors), 2000, replace=False))
+    assert_scores_close(whole[sample], oracle_mod.from_primitives(op, *A, *B, anchors[sample], 10.0))
+
+
 # --------------------------------------------------------------------------------------------------- edge cases
 def test_ties_duplicates_and_lattice(gpu_ctx, oracle_mod):
     # cubic lattice: many exactly equal distances inside and across environments; plus coincident points
@@ -300,6 +347,14 @@ def test_from_coords_and_dmxs(gpu_ctx, oracle_mod, n):
         got = gpu_ctx.score_pairs(ea2, eb2, pairs)
         ref = oracle_mod.from_dmxs(op, ca, cb, ma, mb)
         assert np.abs(got - ref).max() <= SCORE_TOL
+        # the same matrices as ragged rows of equal length (the path of the Python API's from_dmxs): same store
+        ea3 = gpu_ctx.envset_from_ragged_rows(ma, ca)
+        eb3 = gpu_ctx.envset_from_ragged_rows(mb, cb)
+        assert np.array_equal(gpu_ctx.score_pairs(ea3, eb3, pairs), got)
+        for rect, ragged in ((ea2, ea3), (eb2, eb3)):
+            for x, y in zip(rect.dump(), ragged.dump()):
+                assert np.array_equal(x, y)
+            rect.close(); ragged.close()
 
 
 # ------------------------------------------------------------------------------------------------- leaf math
