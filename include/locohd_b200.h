@@ -262,11 +262,25 @@ int locohd_from_primitives(locohd_ctx* ctx, uint64_t n_a, const double* xyz_a, c
                            const uint32_t* tag_a, uint64_t n_b, const double* xyz_b, const uint16_t* cat_b,
                            const uint32_t* tag_b, uint64_t n_pairs, const uint32_t* anchors,
                            const uint32_t* wf_idx, double threshold, double* out_scores);
+/* The same call with the coordinate gradients of the scores (an extension: the reference has none).
+ * out_grad_a [n_a][3] and out_grad_b [n_b][3] are overwritten with sum_p g_p dS_p/dxyz, g_p = pair_weights[p]
+ * (NULL: all 1).  out_scores [n_pairs] may be NULL.  The gradient is the one-sided derivative in the walk's order
+ * (distance, then A before B, then store order) where distances tie; membership changes at the threshold are not
+ * differentiated.  Scores are deterministic; gradients are summed with FP64 atomics and may differ in the last bits
+ * from call to call.  Any argument may be host or device memory. */
+int locohd_from_primitives_grad(locohd_ctx* ctx, uint64_t n_a, const double* xyz_a, const uint16_t* cat_a,
+                                const uint32_t* tag_a, uint64_t n_b, const double* xyz_b, const uint16_t* cat_b,
+                                const uint32_t* tag_b, uint64_t n_pairs, const uint32_t* anchors,
+                                const uint32_t* wf_idx, double threshold, const double* pair_weights,
+                                double* out_scores, double* out_grad_a, double* out_grad_b);
 
 /* ---- leaf math on the device (parity checks of the FP64 device functions) --------------- */
 /* WeightFunction::integral_point over n points (weight_function.rs:95-116). */
 int locohd_wf_integral_points(locohd_ctx* ctx, const locohd_weight_function* wf, uint64_t n, const double* x,
                               double* out);
+/* The density w(x) = dW/dx of the weight function over n points (the derivative of integral_point). */
+int locohd_wf_density_points(locohd_ctx* ctx, const locohd_weight_function* wf, uint64_t n, const double* x,
+                             double* out);
 /* StatisticalDistance::run on n pairs of already-normalised vectors [n][n_categories]
  * (statistical_distances.rs:123-142); uses sd_kind/sd_params given here, not the context's. */
 int locohd_sd_run(locohd_ctx* ctx, int32_t sd_kind, const double* sd_params, int32_t n_categories, uint64_t n,

@@ -33,7 +33,8 @@ EXPORTED_SYMBOLS = [
     "locohd_envset_from_coords", "locohd_envset_destroy", "locohd_envset_size", "locohd_envset_total_members",
     "locohd_envset_dump", "locohd_score_pairs", "locohd_score_jobs", "locohd_score_jobs_stats",
     "locohd_score_anchor_lists", "locohd_plan_job_tiles", "locohd_tile_unit", "locohd_tile_geometry",
-    "locohd_from_primitives", "locohd_wf_integral_points", "locohd_sd_run",
+    "locohd_from_primitives", "locohd_from_primitives_grad", "locohd_wf_integral_points", "locohd_wf_density_points",
+    "locohd_sd_run",
 ]
 
 
@@ -127,7 +128,10 @@ def load_library() -> C.CDLL:
         "locohd_tile_geometry": (C.c_int, [C.c_int, u32, u32, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int),
                                            C.POINTER(C.c_int)]),
         "locohd_from_primitives": (C.c_int, [vp, u64, vp, vp, vp, u64, vp, vp, vp, u64, vp, vp, dbl, vp]),
+        "locohd_from_primitives_grad": (C.c_int, [vp, u64, vp, vp, vp, u64, vp, vp, vp, u64, vp, vp, dbl, vp, vp, vp,
+                                                  vp]),
         "locohd_wf_integral_points": (C.c_int, [vp, C.POINTER(WeightFunctionC), u64, vp, vp]),
+        "locohd_wf_density_points": (C.c_int, [vp, C.POINTER(WeightFunctionC), u64, vp, vp]),
         "locohd_sd_run": (C.c_int, [vp, i32, vp, i32, u64, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
@@ -435,12 +439,41 @@ class Context:
                                                     float(threshold), _p(res)))
         return res
 
+    def from_primitives_grad(self, xyz_a, cat_a, tag_a, xyz_b, cat_b, tag_b, anchors, threshold: float, wf_idx=None,
+                             pair_weights=None, out=None, grad_a=None, grad_b=None, n_a=None, n_b=None, n_pairs=None):
+        """Scores and their coordinate gradients: returns (scores [P], grad_a [n_a, 3], grad_b [n_b, 3]) with
+        grad = sum_p pair_weights[p] dS_p/dxyz (pair_weights None: all 1).  Every array may be a numpy array or a raw
+        device pointer, as in from_primitives."""
+        xyz_a, xyz_b = _arr(xyz_a, np.float64), _arr(xyz_b, np.float64)
+        cat_a, cat_b = _arr(cat_a, np.uint16), _arr(cat_b, np.uint16)
+        tag_a, tag_b = _arr(tag_a, np.uint32), _arr(tag_b, np.uint32)
+        anchors, wf_idx = _arr(anchors, np.uint32), _arr(wf_idx, np.uint32)
+        pair_weights = _arr(pair_weights, np.float64)
+        na = int(n_a) if n_a is not None else len(cat_a)
+        nb = int(n_b) if n_b is not None else len(cat_b)
+        P = int(n_pairs) if n_pairs is not None else len(anchors.reshape(-1, 2))
+        res = np.empty(P, np.float64) if out is None else out
+        ga = np.empty((na, 3), np.float64) if grad_a is None else grad_a
+        gb = np.empty((nb, 3), np.float64) if grad_b is None else grad_b
+        self._check(self.lib.locohd_from_primitives_grad(self.h, na, _p(xyz_a), _p(cat_a), _p(tag_a), nb, _p(xyz_b),
+                                                         _p(cat_b), _p(tag_b), P, _p(anchors), _p(wf_idx),
+                                                         float(threshold), _p(pair_weights), _p(res), _p(ga), _p(gb)))
+        return res, ga, gb
+
     # ---- leaf math --------------------------------------------------------------------------------
     def wf_integral_points(self, name: str, params, x):
         w = make_wf(name, params)
         x = np.ascontiguousarray(x, dtype=np.float64)
         out = np.empty(len(x), np.float64)
         self._check(self.lib.locohd_wf_integral_points(self.h, C.byref(w), len(x), _p(x), _p(out)))
+        return out
+
+    def wf_density_points(self, name: str, params, x):
+        """The weight function's density dW/dx at the points x."""
+        w = make_wf(name, params)
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        out = np.empty(len(x), np.float64)
+        self._check(self.lib.locohd_wf_density_points(self.h, C.byref(w), len(x), _p(x), _p(out)))
         return out
 
     def sd_run(self, name: str, params, p1, p2):

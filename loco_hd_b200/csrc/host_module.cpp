@@ -804,13 +804,19 @@ struct LoCoHD {
         return out;
     }
 
-    py::array_t<double> from_arrays(F64Array xyz_a, U16Array cat_a, U32Array tag_a, F64Array xyz_b, U16Array cat_b,
-                                    U32Array tag_b, U32Array anchors, double threshold, const py::object& wf_idx) {
+    static size_t check_arrays(const F64Array& xyz_a, const U16Array& cat_a, const U32Array& tag_a, const F64Array& xyz_b,
+                               const U16Array& cat_b, const U32Array& tag_b, const U32Array& anchors) {
         const size_t na = cat_a.size(), nb = cat_b.size();
         if ((size_t)xyz_a.size() != 3 * na || (size_t)tag_a.size() != na || (size_t)xyz_b.size() != 3 * nb || (size_t)tag_b.size() != nb)
             throw py::value_error("xyz must be [n, 3], category and tag [n]");
         if (anchors.size() % 2) throw py::value_error("anchors must be [n_pairs, 2]");
-        const size_t P = anchors.size() / 2;
+        return anchors.size() / 2;
+    }
+
+    py::array_t<double> from_arrays(F64Array xyz_a, U16Array cat_a, U32Array tag_a, F64Array xyz_b, U16Array cat_b,
+                                    U32Array tag_b, U32Array anchors, double threshold, const py::object& wf_idx) {
+        const size_t na = cat_a.size(), nb = cat_b.size();
+        const size_t P = check_arrays(xyz_a, cat_a, tag_a, xyz_b, cat_b, tag_b, anchors);
         const auto wf = wf_indices(wf_idx, P);
         py::array_t<double> out(P);
         const auto d = ensure_ctx();
@@ -820,6 +826,30 @@ struct LoCoHD {
                                           tag_b.data(), P, anchors.data(), wf.empty() ? nullptr : wf.data(), threshold, o);
         });
         return out;
+    }
+
+    // from_arrays with the coordinate gradients of the scores: (scores [P], grad_a [n_a, 3], grad_b [n_b, 3]),
+    // grad = sum_p pair_weights[p] dS_p/dxyz (pair_weights None: all 1)
+    py::tuple from_arrays_grad(F64Array xyz_a, U16Array cat_a, U32Array tag_a, F64Array xyz_b, U16Array cat_b,
+                               U32Array tag_b, U32Array anchors, double threshold, const py::object& wf_idx,
+                               const py::object& pair_weights) {
+        const size_t na = cat_a.size(), nb = cat_b.size();
+        const size_t P = check_arrays(xyz_a, cat_a, tag_a, xyz_b, cat_b, tag_b, anchors);
+        const auto wf = wf_indices(wf_idx, P);
+        F64Array pw;
+        if (!pair_weights.is_none()) {
+            pw = pair_weights.cast<F64Array>();
+            if ((size_t)pw.size() != P) throw py::value_error("pair_weights must have one entry per anchor pair");
+        }
+        py::array_t<double> out(P), ga({(py::ssize_t)na, (py::ssize_t)3}), gb({(py::ssize_t)nb, (py::ssize_t)3});
+        const auto d = ensure_ctx();
+        double *o = out.mutable_data(), *pga = ga.mutable_data(), *pgb = gb.mutable_data();
+        device_call(d, [&](locohd_ctx* c) {
+            return locohd_from_primitives_grad(c, na, xyz_a.data(), cat_a.data(), tag_a.data(), nb, xyz_b.data(),
+                                               cat_b.data(), tag_b.data(), P, anchors.data(), wf.empty() ? nullptr : wf.data(),
+                                               threshold, pair_weights.is_none() ? nullptr : pw.data(), o, pga, pgb);
+        });
+        return py::make_tuple(out, ga, gb);
     }
 
     // ---- resident batches (SURVEY.md §8(f) N1 / N4): what the callers loop over upstream - one reference against
@@ -984,6 +1014,12 @@ PYBIND11_MODULE(loco_hd, m) {
              "Array form of from_primitives: integer category ids (index into `categories`, 0xFFFF = unknown; see "
              "category_ids), integer tag ids (opaque for a rule without a tag list, from intern_tags otherwise), "
              "[n, 3] float64 coordinates, [n_pairs, 2] anchor indices.  Returns a float64 array.")
+        .def("from_arrays_grad", &LoCoHD::from_arrays_grad, py::arg("xyz_a"), py::arg("cat_a"), py::arg("tag_a"),
+             py::arg("xyz_b"), py::arg("cat_b"), py::arg("tag_b"), py::arg("anchors"), py::arg("threshold_distance"),
+             py::arg("wf_idx") = py::none(), py::arg("pair_weights") = py::none(),
+             "from_arrays with the coordinate gradients of the scores (an extension): returns (scores [n_pairs], "
+             "grad_a [n_a, 3], grad_b [n_b, 3]) with grad = sum_p pair_weights[p] dS_p/dxyz (None: all 1).  At tied "
+             "distances the gradient is one-sided; threshold crossings are not differentiated.")
         .def("intern_tags", &LoCoHD::intern_tags, py::arg("tags"),
              "Tag strings -> the uint32 ids this instance uses for them (the ids of a WithList rule's tag pairs included).")
         .def("to_arrays", &LoCoHD::to_arrays, py::arg("primitives"),

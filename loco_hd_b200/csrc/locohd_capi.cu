@@ -1540,30 +1540,42 @@ int locohd_score_anchor_lists(locohd_ctx* ctx, const uint16_t* seq_a, uint64_t l
     API_END()
 }
 
-int locohd_from_primitives(locohd_ctx* ctx, uint64_t n_a, const double* xyz_a, const uint16_t* cat_a,
+// The shared head of locohd_from_primitives and locohd_from_primitives_grad: one structure set holding A then B, its
+// inputs uploaded, categories converted, coordinates validated and the 2 P environments built.  The members release
+// the set and the environments, and keep the host arrays of the upload alive until the caller has synchronised.
+struct PrimCall {
+    locohd_structs* s = nullptr;
+    locohd_envset* env = nullptr;
+    size_t o_job = 0, o_as = 0, o_ap = 0, o_wf = 0;   // the call's arrays at the start of the block of `s`
+    uint64_t offs[3] = {0, 0, 0};
+    std::vector<uint32_t> h_anchor, h_split;
+    ~PrimCall() { if (env) destroy_envset(env); if (s) locohd_structs_destroy(s); }
+    const unsigned char* at(size_t o) const { return s->block + o; }
+};
+
+// Validates the arguments; with n_pairs = 0 it returns 0 and builds nothing (pc.s stays null).
+static int prim_call_build(locohd_ctx* ctx, uint64_t n_a, const double* xyz_a, const uint16_t* cat_a,
                            const uint32_t* tag_a, uint64_t n_b, const double* xyz_b, const uint16_t* cat_b,
-                           const uint32_t* tag_b, uint64_t n_pairs, const uint32_t* anchors,
-                           const uint32_t* wf_idx, double threshold, double* out_scores) {
-    API_BEGIN(ctx)
+                           const uint32_t* tag_b, uint64_t n_pairs, const uint32_t* anchors, const uint32_t* wf_idx,
+                           double threshold, bool has_out, int keep_indices, const LaunchOverrides& ov, PrimCall& pc) {
     TRY_ST(need_params(ctx));
-    if (n_pairs && (!anchors || !out_scores)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
+    if (n_pairs && (!anchors || !has_out)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
     if ((n_a && (!xyz_a || !cat_a || !tag_a)) || (n_b && (!xyz_b || !cat_b || !tag_b)))
         return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null primitive arrays");
     if (n_pairs == 0) return 0;
     if (!(threshold > 0.0))
         return fail(ctx, LOCOHD_ERR_EMPTY_ENV, "threshold_distance must be positive (got %g): every environment would be empty", threshold);
     TRY_ST(check_wf_indices(ctx, wf_idx, n_pairs));
-    const LaunchOverrides ov = read_launch_overrides();
     const uint64_t n = n_a + n_b;
-    // One structure set holding A then B.  Its device block starts with the arrays of the call: the job, the anchors
-    // of the 2 P environments ([0, P) belong to A, [P, 2 P) to B), the categories as given and the per-pair weight
-    // function indices.  Everything the host sends lands in the range [0, upload_end) of the block.
+    // Its device block starts with the arrays of the call: the job, the anchors of the 2 P environments ([0, P) belong
+    // to A, [P, 2 P) to B), the categories as given and the per-pair weight function indices.  Everything the host
+    // sends lands in the range [0, upload_end) of the block.
     BlockCursor head;
-    const size_t o_job = head.take(sizeof(locohd_job));
-    const size_t o_as = head.take(2 * n_pairs * sizeof(uint32_t));
-    const size_t o_ap = head.take(2 * n_pairs * sizeof(uint32_t));
+    pc.o_job = head.take(sizeof(locohd_job));
+    pc.o_as = head.take(2 * n_pairs * sizeof(uint32_t));
+    pc.o_ap = head.take(2 * n_pairs * sizeof(uint32_t));
     const size_t o_cat16 = head.take(n * sizeof(uint16_t));
-    const size_t o_wf = head.take(wf_idx ? n_pairs * sizeof(uint32_t) : 0);
+    pc.o_wf = head.take(wf_idx ? n_pairs * sizeof(uint32_t) : 0);
     const StructsLayout l = structs_layout(2, n, head.end);
     // Small calls with host inputs (the typical call of the reference API: one structure pair) are packed into one
     // pinned staging buffer and sent with one copy: a dozen pageable copies of ~10 us each otherwise dominate such a
@@ -1583,26 +1595,22 @@ int locohd_from_primitives(locohd_ctx* ctx, uint64_t n_a, const double* xyz_a, c
         h = ctx->h_stage;
     }
     // the A/B split of the anchors is built on the host (device anchors are copied back first)
-    std::vector<uint32_t> h_anchor, h_split;
     const uint32_t* an = anchors;
     if (is_device_ptr(ctx, anchors)) {
-        h_anchor.resize(2 * n_pairs);
-        CU(ctx, cudaMemcpy(h_anchor.data(), anchors, 2 * n_pairs * sizeof(uint32_t), cudaMemcpyDeviceToHost));
-        an = h_anchor.data();
+        pc.h_anchor.resize(2 * n_pairs);
+        CU(ctx, cudaMemcpy(pc.h_anchor.data(), anchors, 2 * n_pairs * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+        an = pc.h_anchor.data();
     }
-    if (!h) h_split.resize(4 * n_pairs);
-    uint32_t* has = h ? reinterpret_cast<uint32_t*>(h + o_as) : h_split.data();
-    uint32_t* hap = h ? reinterpret_cast<uint32_t*>(h + o_ap) : h_split.data() + 2 * n_pairs;
+    if (!h) pc.h_split.resize(4 * n_pairs);
+    uint32_t* has = h ? reinterpret_cast<uint32_t*>(h + pc.o_as) : pc.h_split.data();
+    uint32_t* hap = h ? reinterpret_cast<uint32_t*>(h + pc.o_ap) : pc.h_split.data() + 2 * n_pairs;
     for (uint64_t i = 0; i < n_pairs; ++i) {
         has[i] = 0; hap[i] = an[2 * i];
         has[n_pairs + i] = 1; hap[n_pairs + i] = an[2 * i + 1];
     }
-    const uint64_t offs[3] = {0, n_a, n};
-    locohd_structs* s = nullptr;
-    TRY_ST(structs_alloc(ctx, 2, offs, l, &s));
-    unsigned char* d = s->block;
-    locohd_envset* env = nullptr;
-    auto done = [&](int st) { if (env) destroy_envset(env); locohd_structs_destroy(s); return st; };
+    pc.offs[1] = n_a; pc.offs[2] = n;
+    TRY_ST(structs_alloc(ctx, 2, pc.offs, l, &pc.s));
+    unsigned char* d = pc.s->block;
     cudaError_t ce = cudaSuccess;
     auto put = [&](size_t at, const void* src, size_t bytes) {
         if (!bytes || ce != cudaSuccess) return;
@@ -1610,41 +1618,104 @@ int locohd_from_primitives(locohd_ctx* ctx, uint64_t n_a, const double* xyz_a, c
         else ce = cudaMemcpyAsync(d + at, src, bytes, cudaMemcpyDefault, ctx->stream);
     };
     const locohd_job job{0, n_pairs, n_pairs};
-    put(o_job, &job, sizeof job);
-    put(l.prim_off, offs, sizeof offs);
+    put(pc.o_job, &job, sizeof job);
+    put(l.prim_off, pc.offs, sizeof pc.offs);
     put(l.xyz, xyz_a, 3 * n_a * sizeof(double));
     put(l.xyz + 3 * n_a * sizeof(double), xyz_b, 3 * n_b * sizeof(double));
     put(l.tag, tag_a, n_a * sizeof(uint32_t));
     put(l.tag + n_a * sizeof(uint32_t), tag_b, n_b * sizeof(uint32_t));
     put(o_cat16, cat_a, n_a * sizeof(uint16_t));
     put(o_cat16 + n_a * sizeof(uint16_t), cat_b, n_b * sizeof(uint16_t));
-    if (wf_idx) put(o_wf, wf_idx, n_pairs * sizeof(uint32_t));
+    if (wf_idx) put(pc.o_wf, wf_idx, n_pairs * sizeof(uint32_t));
     if (h) {
         ce = cudaMemcpyAsync(d, h, l.upload_end, cudaMemcpyHostToDevice, ctx->stream);
     } else {
-        put(o_as, has, 2 * n_pairs * sizeof(uint32_t));
-        put(o_ap, hap, 2 * n_pairs * sizeof(uint32_t));
+        put(pc.o_as, has, 2 * n_pairs * sizeof(uint32_t));
+        put(pc.o_ap, hap, 2 * n_pairs * sizeof(uint32_t));
     }
-    if (ce != cudaSuccess) return done(fail(ctx, LOCOHD_ERR_CUDA, "upload failed: %s", cudaGetErrorString(ce)));
-    ctx->launches += launch_convert_categories(reinterpret_cast<const uint16_t*>(d + o_cat16), s->d_cat, n, ctx->kp.C, ctx->stream);
-    ctx->launches += launch_validate_xyz(s->d_xyz, 3 * n, ctx->d_err, ctx->stream);
-    int st = build_envset(ctx, s, 2 * n_pairs, reinterpret_cast<const uint32_t*>(d + o_as),
-                          reinterpret_cast<const uint32_t*>(d + o_ap), threshold, 0, ov, &env);
-    if (st) return done(st);
+    if (ce != cudaSuccess) return fail(ctx, LOCOHD_ERR_CUDA, "upload failed: %s", cudaGetErrorString(ce));
+    ctx->launches += launch_convert_categories(reinterpret_cast<const uint16_t*>(d + o_cat16), pc.s->d_cat, n, ctx->kp.C, ctx->stream);
+    ctx->launches += launch_validate_xyz(pc.s->d_xyz, 3 * n, ctx->d_err, ctx->stream);
+    return build_envset(ctx, pc.s, 2 * n_pairs, reinterpret_cast<const uint32_t*>(d + pc.o_as),
+                        reinterpret_cast<const uint32_t*>(d + pc.o_ap), threshold, keep_indices, ov, &pc.env);
+}
+
+int locohd_from_primitives(locohd_ctx* ctx, uint64_t n_a, const double* xyz_a, const uint16_t* cat_a,
+                           const uint32_t* tag_a, uint64_t n_b, const double* xyz_b, const uint16_t* cat_b,
+                           const uint32_t* tag_b, uint64_t n_pairs, const uint32_t* anchors,
+                           const uint32_t* wf_idx, double threshold, double* out_scores) {
+    API_BEGIN(ctx)
+    const LaunchOverrides ov = read_launch_overrides();
+    PrimCall pc;
+    TRY_ST(prim_call_build(ctx, n_a, xyz_a, cat_a, tag_a, n_b, xyz_b, cat_b, tag_b, n_pairs, anchors, wf_idx,
+                           threshold, out_scores != nullptr, 0, ov, pc));
+    if (!pc.s) return 0;
     OutBuf<double> out;
-    if ((st = out.prepare(ctx, out_scores, n_pairs))) return done(st);
-    st = run_score(ctx, env, env, n_pairs, nullptr, reinterpret_cast<const locohd_job*>(d + o_job), nullptr, 1, n_pairs,
-                   wf_idx ? reinterpret_cast<const uint32_t*>(d + o_wf) : nullptr, out.ptr, ov);
+    int st = out.prepare(ctx, out_scores, n_pairs);
+    if (!st) st = run_score(ctx, pc.env, pc.env, n_pairs, nullptr, reinterpret_cast<const locohd_job*>(pc.at(pc.o_job)),
+                            nullptr, 1, n_pairs, wf_idx ? reinterpret_cast<const uint32_t*>(pc.at(pc.o_wf)) : nullptr,
+                            out.ptr, ov);
     if (!st) st = out.commit();
     const int st2 = sync_and_check(ctx);   // also keeps the host arrays of the upload alive until it is done
-    return done(st ? st : st2);
+    return st ? st : st2;
+    API_END()
+}
+
+int locohd_from_primitives_grad(locohd_ctx* ctx, uint64_t n_a, const double* xyz_a, const uint16_t* cat_a,
+                                const uint32_t* tag_a, uint64_t n_b, const double* xyz_b, const uint16_t* cat_b,
+                                const uint32_t* tag_b, uint64_t n_pairs, const uint32_t* anchors,
+                                const uint32_t* wf_idx, double threshold, const double* pair_weights,
+                                double* out_scores, double* out_grad_a, double* out_grad_b) {
+    API_BEGIN(ctx)
+    if ((n_a && !out_grad_a) || (n_b && !out_grad_b)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null gradient array");
+    const LaunchOverrides ov = read_launch_overrides();
+    PrimCall pc;
+    TRY_ST(prim_call_build(ctx, n_a, xyz_a, cat_a, tag_a, n_b, xyz_b, cat_b, tag_b, n_pairs, anchors, wf_idx,
+                           threshold, true, 1, ov, pc));
+    OutBuf<double> ga, gb, out;
+    TRY_ST(ga.prepare(ctx, out_grad_a, 3 * n_a));
+    TRY_ST(gb.prepare(ctx, out_grad_b, 3 * n_b));
+    if (n_a) CU(ctx, cudaMemsetAsync(ga.ptr, 0, 3 * n_a * sizeof(double), ctx->stream));
+    if (n_b) CU(ctx, cudaMemsetAsync(gb.ptr, 0, 3 * n_b * sizeof(double), ctx->stream));
+    int st = 0;
+    if (pc.s) {
+        InBuf<double> pw;
+        double* d_scores = nullptr;   // scores are always computed; a caller without `out_scores` gets them dropped
+        if (!(st = pw.load(ctx, pair_weights, n_pairs)))
+            st = out_scores ? out.prepare(ctx, out_scores, n_pairs) : dev_alloc(ctx, &d_scores, n_pairs);
+        if (!st) {
+            GradArgs g{};
+            g.env = pc.env->view();
+            g.dist = pc.env->d_dist; g.idx = pc.env->d_idx;
+            g.xyz = pc.s->d_xyz; g.prim_off = pc.s->d_prim_off; g.n_structs = 2;
+            g.anchor_struct = reinterpret_cast<const uint32_t*>(pc.at(pc.o_as));
+            g.anchor_prim = reinterpret_cast<const uint32_t*>(pc.at(pc.o_ap));
+            g.n_pairs = n_pairs;
+            g.wf_idx = wf_idx ? reinterpret_cast<const uint32_t*>(pc.at(pc.o_wf)) : nullptr;
+            g.pair_weights = pw.ptr;
+            g.out = out_scores ? out.ptr : d_scores;
+            g.grad[0] = ga.ptr; g.grad[1] = gb.ptr;
+            int nl;
+            { ProfScope ps(ctx, LOCOHD_PROF_SCORE); nl = launch_score_grad(g, ctx->kp, ctx->stream); }
+            if (nl < 0) st = fail(ctx, LOCOHD_ERR_UNSUPPORTED, "shared memory budget exceeded for %d categories", ctx->kp.C);
+            else ctx->launches += nl;
+            if (!st && cudaPeekAtLastError() != cudaSuccess)
+                st = fail(ctx, LOCOHD_ERR_CUDA, "launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        }
+        if (!st) st = out.commit();
+        dev_free(ctx, d_scores);
+    }
+    if (!st) st = ga.commit();
+    if (!st) st = gb.commit();
+    const int st2 = sync_and_check(ctx);
+    return st ? st : st2;
     API_END()
 }
 
 // ----------------------------------------------------------------------------------------------- leaf math
-int locohd_wf_integral_points(locohd_ctx* ctx, const locohd_weight_function* wf, uint64_t n, const double* x,
-                              double* out) {
-    API_BEGIN(ctx)
+// W(x) (density = false) or w(x) = W'(x) at n points
+static int wf_points(locohd_ctx* ctx, const locohd_weight_function* wf, uint64_t n, const double* x, double* out,
+                     bool density) {
     if (!wf || (n && (!x || !out))) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
     WfDev w;
     TRY_ST(make_wf(ctx, *wf, &w));
@@ -1659,12 +1730,26 @@ int locohd_wf_integral_points(locohd_ctx* ctx, const locohd_weight_function* wf,
     int st = in.load(ctx, x, n);
     if (!st) st = o.prepare(ctx, out, n);
     if (!st) {
-        ctx->launches += launch_wf_points(d_w, n, in.ptr, o.ptr, ctx->d_err, ctx->stream);
+        ctx->launches += density ? launch_wf_density(d_w, n, in.ptr, o.ptr, ctx->d_err, ctx->stream)
+                                 : launch_wf_points(d_w, n, in.ptr, o.ptr, ctx->d_err, ctx->stream);
         st = o.commit();
     }
     const int st2 = sync_and_check(ctx);
     dev_free(ctx, d_w);
     return st ? st : st2;
+}
+
+int locohd_wf_integral_points(locohd_ctx* ctx, const locohd_weight_function* wf, uint64_t n, const double* x,
+                              double* out) {
+    API_BEGIN(ctx)
+    return wf_points(ctx, wf, n, x, out, false);
+    API_END()
+}
+
+int locohd_wf_density_points(locohd_ctx* ctx, const locohd_weight_function* wf, uint64_t n, const double* x,
+                             double* out) {
+    API_BEGIN(ctx)
+    return wf_points(ctx, wf, n, x, out, true);
     API_END()
 }
 

@@ -1574,6 +1574,194 @@ __global__ void __launch_bounds__(kScoreMaxWarps * 32) score_kernel(ScoreArgs a,
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Coordinate gradients (locohd_from_primitives_grad).  With the non-anchor members of both environments in merged
+// order at distances t_1 <= ... <= t_K and H_k the statistical distance after event k,
+//     S = sum_k (W(t_k) - W(t_{k-1})) H_{k-1} + (W(inf) - W(t_K)) H_K,   dS/dt_k = w(t_k) (H_{k-1} - H_k),
+// so the walk of score_kernel yields the gradient without a derivative of H.  Events are merged by the exact
+// distances of the keep_indices store (A before B on ties), W and w are evaluated there, and dt/dx_member =
+// (x_member - x_anchor) / t = -dt/dx_anchor.  Membership changes at the threshold are not differentiated.
+// ------------------------------------------------------------------------------------------------
+__host__ __device__ inline int grad_state_bytes(int C) { return ((2 * C * 32 * 8 + 2 * C * 32 * 4) + 15) & ~15; }
+
+// merge-path split of score_kernel on exact distances
+__device__ __forceinline__ uint32_t merge_path_dist(const double* dA, const double* dB, uint32_t na, uint32_t nb,
+                                                    uint32_t diag) {
+    uint32_t lo = diag > nb ? diag - nb : 0, hi = min(diag, na);
+    while (lo < hi) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (dA[mid] <= dB[diag - 1 - mid]) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
+__global__ void __launch_bounds__(kScoreMaxWarps * 32) score_grad_kernel(GradArgs g, KParams P, int warps_per_block) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    if (wib >= warps_per_block) return;
+    const int C = P.C;
+    unsigned char* mine = smem_raw + (size_t)wib * grad_state_bytes(C);
+    double* val = reinterpret_cast<double*>(mine);                         // [2C][32]
+    uint32_t* cnt = reinterpret_cast<uint32_t*>(mine + 2 * C * 32 * 8);    // [2C][32]
+
+    for (uint64_t pair = (uint64_t)blockIdx.x * warps_per_block + wib; pair < g.n_pairs;
+         pair += (uint64_t)gridDim.x * warps_per_block) {
+        __syncwarp();
+        const uint64_t env[2] = {pair, g.n_pairs + pair};
+        uint32_t M[2];
+        uint64_t off[2], sid[2], base[2], nprim[2];
+        double xa[2][3];
+        bool bad = false;
+        for (int s = 0; s < 2; ++s) {
+            off[s] = g.env.off[env[s]];
+            M[s] = g.env.count[env[s]];
+            sid[s] = g.anchor_struct[env[s]];
+            const uint32_t ap = g.anchor_prim[env[s]];
+            bad |= sid[s] >= g.n_structs;
+            if (bad) break;
+            base[s] = g.prim_off[sid[s]];
+            nprim[s] = g.prim_off[sid[s] + 1] - base[s];
+            bad |= ap >= nprim[s];
+            if (bad) break;
+            for (int k = 0; k < 3; ++k) xa[s][k] = g.xyz[3 * (base[s] + ap) + k];
+        }
+        if (bad) { raise(P.err, LOCOHD_ERR_INDEX); continue; }
+        if (M[0] == 0 || M[1] == 0) { raise(P.err, LOCOHD_ERR_EMPTY_ENV); continue; }
+        const uint64_t* kA = g.env.key + off[0] + 1;   // events = members after the anchor
+        const uint64_t* kB = g.env.key + off[1] + 1;
+        const double* dA = g.dist + off[0] + 1;
+        const double* dB = g.dist + off[1] + 1;
+        const uint32_t* xA = g.idx + off[0] + 1;
+        const uint32_t* xB = g.idx + off[1] + 1;
+        const uint32_t catA0 = (uint32_t)(g.env.key[off[0]] & kCatMask), catB0 = (uint32_t)(g.env.key[off[1]] & kCatMask);
+        const double t0 = fmax(g.dist[off[0]], g.dist[off[1]]);
+        const uint32_t na = M[0] - 1, nb = M[1] - 1;
+        const uint32_t E = na + nb;
+        const uint32_t Q = (E + 31) / 32;
+
+        // ---- merge-path split: lane l owns merged events [l*Q, (l+1)*Q)
+        const uint32_t diag = min(E, (uint32_t)lane * Q);
+        uint32_t i = merge_path_dist(dA, dB, na, nb, diag), j = diag - i;
+        uint32_t i1 = __shfl_down_sync(kFull, i, 1), j1 = __shfl_down_sync(kFull, j, 1);
+        if (lane == 31) { i1 = na; j1 = nb; }
+
+        // ---- category counts before my chunk (as in score_kernel)
+        for (int r = 0; r < 2 * C; ++r) cnt[r * 32 + lane] = 0;
+        bool unknown = (catA0 >= (uint32_t)C) || (catB0 >= (uint32_t)C);
+        bool bad_idx = false;
+        for (uint32_t x = i; x < i1; ++x) {
+            const uint32_t c = (uint32_t)(kA[x] & kCatMask);
+            if (c < (uint32_t)C) cnt[c * 32 + lane] += 1; else unknown = true;
+            bad_idx |= xA[x] >= nprim[0];
+        }
+        for (uint32_t x = j; x < j1; ++x) {
+            const uint32_t c = (uint32_t)(kB[x] & kCatMask);
+            if (c < (uint32_t)C) cnt[(C + c) * 32 + lane] += 1; else unknown = true;
+            bad_idx |= xB[x] >= nprim[1];
+        }
+        if (__any_sync(kFull, unknown)) { raise(P.err, LOCOHD_ERR_UNKNOWN_CATEGORY); continue; }
+        if (__any_sync(kFull, bad_idx)) { raise(P.err, LOCOHD_ERR_INDEX); continue; }
+        for (int r = 0; r < 2 * C; ++r) {
+            const uint32_t v = cnt[r * 32 + lane];
+            uint32_t incl = v;
+            for (int o = 1; o < 32; o <<= 1) {
+                const uint32_t u = __shfl_up_sync(kFull, incl, o);
+                if (lane >= o) incl += u;
+            }
+            uint32_t ex = incl - v;
+            if (r == (int)catA0 || r == C + (int)catB0) ex += 1;   // anchors
+            cnt[r * 32 + lane] = ex;
+        }
+
+        // ---- state: the Hellinger distance keeps (weighted count)^(1/e) for any exponent, the others the weighted
+        //      count (score_kernel's generic branches)
+        const bool hell = P.sd_kind == LOCOHD_SD_HELLINGER;
+        const double inv_e = hell ? 1.0 / P.sd_p0 : 0.0;
+        auto root_e = [&](double x) -> double { return x > 0.0 ? exp(inv_e * log(x)) : 0.0; };
+        auto side_scale = [&](double norm) -> double { return hell ? exp(-inv_e * log(norm)) : 1.0 / norm; };
+        double norm[2] = {0.0, 0.0};
+        for (int r = 0; r < C; ++r) {
+            const uint32_t ka = cnt[r * 32 + lane], kb = cnt[(C + r) * 32 + lane];
+            const double w = P.cat_w[r];
+            norm[0] += (double)ka * w; norm[1] += (double)kb * w;
+            val[r * 32 + lane] = hell ? root_e((double)ka * w) : (double)ka * w;
+            val[(C + r) * 32 + lane] = hell ? root_e((double)kb * w) : (double)kb * w;
+        }
+        double iA = side_scale(norm[0]), iB = side_scale(norm[1]);
+        auto stat_dist = [&]() -> double {
+            if (hell) {
+                double dist = 0.0;
+                for (int r = 0; r < C; ++r) {
+                    const double t = fabs(__dmul_rn(val[r * 32 + lane], iA) - __dmul_rn(val[(C + r) * 32 + lane], iB));
+                    if (t > 0.0) dist += exp(P.sd_p0 * log(t));
+                }
+                return dist > 0.0 ? exp(inv_e * log(0.5 * dist)) : 0.0;
+            }
+            auto va = [&](int r) { return val[r * 32 + lane]; };
+            auto vb = [&](int r) { return val[(C + r) * 32 + lane]; };
+            return sd_scaled(P.sd_kind, P.sd_p0, P.sd_p1, C, va, vb, iA, iB);
+        };
+
+        const WfDev& wf = P.wfs[g.wf_idx ? min(g.wf_idx[pair], (uint32_t)(P.n_wf - 1)) : 0u];   // range checked on entry
+        const double gp = g.pair_weights ? g.pair_weights[pair] : 1.0;
+        double tprev = t0;
+        if (i > 0) tprev = dA[i - 1];
+        if (j > 0) tprev = fmax(tprev, dB[j - 1]);
+        double wprev = wf_cdf(wf, tprev);
+        double h = stat_dist();
+        double acc = 0.0;
+        double ganc[2][3] = {{0.0, 0.0, 0.0}, {0.0, 0.0, 0.0}};   // the anchors' shares
+
+        // ---- walk my chunk
+        while (i < i1 || j < j1) {
+            const bool takeA = (i < i1) && (!(j < j1) || dA[i] <= dB[j]);
+            const int s = takeA ? 0 : 1;
+            const uint32_t x = takeA ? i : j;
+            const double t = takeA ? dA[x] : dB[x];
+            const uint32_t c = (uint32_t)((takeA ? kA[x] : kB[x]) & kCatMask);
+            const uint32_t m = takeA ? xA[x] : xB[x];
+            const double w = wf_cdf(wf, t);
+            acc = fma(w - wprev, h, acc);
+            wprev = w;
+            const int row = s * C + (int)c;
+            const uint32_t k = cnt[row * 32 + lane] + 1;
+            cnt[row * 32 + lane] = k;
+            const double wc = P.cat_w[c];
+            val[row * 32 + lane] = hell ? root_e((double)k * wc) : (double)k * wc;
+            norm[s] += wc;
+            if (takeA) { iA = side_scale(norm[0]); ++i; } else { iB = side_scale(norm[1]); ++j; }
+            const double hn = stat_dist();
+            if (gp != 0.0 && t > 0.0) {   // a member on top of its anchor has no direction: it contributes 0
+                const double coef = gp * wf_pdf(wf, t) * (h - hn) / t;
+                double* gm = g.grad[sid[s]] + 3 * (uint64_t)m;
+                const double* xm = g.xyz + 3 * (base[s] + m);
+                for (int q = 0; q < 3; ++q) {
+                    const double v = coef * (xm[q] - xa[s][q]);
+                    atomicAdd(gm + q, v);
+                    ganc[s][q] -= v;
+                }
+            }
+            h = hn;
+        }
+        // ---- tail to infinity: owned by the last lane, whose state is final
+        if (lane == 31) acc = fma(wf.w_inf - wprev, h, acc);
+        for (int o = 16; o; o >>= 1) {
+            acc += __shfl_xor_sync(kFull, acc, o);
+            for (int s = 0; s < 2; ++s)
+                for (int q = 0; q < 3; ++q) ganc[s][q] += __shfl_xor_sync(kFull, ganc[s][q], o);
+        }
+        if (lane == 0) {
+            g.out[pair] = acc;
+            if (gp != 0.0) {
+                for (int s = 0; s < 2; ++s) {
+                    const uint32_t ap = g.anchor_prim[env[s]];
+                    for (int q = 0; q < 3; ++q) atomicAdd(g.grad[sid[s]] + 3 * (uint64_t)ap + q, ganc[s][q]);
+                }
+            }
+        }
+    }
+}
+
 // Fast kernel: Hellinger-2, unit category weights, C <= CP (8 or 16), both environments staged in shared memory.
 //
 // With unit weights the compositions are count_r / n, so
@@ -2465,6 +2653,15 @@ __global__ void wf_points_kernel(const WfDev* wf, uint64_t n, const double* __re
     out[i] = wf_cdf(*wf, v);
 }
 
+__global__ void wf_density_kernel(const WfDev* wf, uint64_t n, const double* __restrict__ x, double* __restrict__ out,
+                                  int* err) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const double v = x[i];
+    if (v < 0.0) { raise(err, LOCOHD_ERR_NEGATIVE_POINT); return; }
+    out[i] = wf_pdf(*wf, v);
+}
+
 __global__ void sd_run_kernel(int kind, double q0, double q1, int C, uint64_t n, const double* __restrict__ p1,
                               const double* __restrict__ p2, double* __restrict__ out) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -2945,6 +3142,26 @@ int launch_anchor_lists(const KParams& p, const uint8_t* seq_a, uint64_t len_a, 
 int launch_wf_points(const WfDev* wf, uint64_t n, const double* x, double* out, int* err, cudaStream_t st) {
     if (!n) return 0;
     wf_points_kernel<<<blocks_for(n, 256), 256, 0, st>>>(wf, n, x, out, err);
+    return 1;
+}
+
+int launch_wf_density(const WfDev* wf, uint64_t n, const double* x, double* out, int* err, cudaStream_t st) {
+    if (!n) return 0;
+    wf_density_kernel<<<blocks_for(n, 256), 256, 0, st>>>(wf, n, x, out, err);
+    return 1;
+}
+
+int launch_score_grad(const GradArgs& g, const KParams& p, cudaStream_t st) {
+    if (!g.n_pairs) return 0;
+    const int per_warp = grad_state_bytes(p.C);
+    if (per_warp > 220 * 1024) return -1;
+    int warps = (100 * 1024) / per_warp;
+    if (warps > kScoreMaxWarps) warps = kScoreMaxWarps;
+    if (warps < 1) warps = 1;
+    const int smem = per_warp * warps;
+    cudaFuncSetAttribute(score_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    const unsigned grid = persistent_grid(score_grad_kernel, warps * 32, smem, g.n_pairs, warps);
+    score_grad_kernel<<<grid, warps * 32, smem, st>>>(g, p, warps);
     return 1;
 }
 

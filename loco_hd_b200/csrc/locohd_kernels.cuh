@@ -267,6 +267,27 @@ struct TileGeometry {
     int team_bytes;   // shared memory per team
 };
 TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, const LaunchOverrides& ov);
+// Coordinate gradients of the scores of one from_primitives call (score_grad_kernel).  The environment set was built
+// with keep_indices: environment p is the A side of pair p, environment n_pairs + p its B side, and `dist` / `idx`
+// hold the exact distances and the members' indices inside their structure.
+struct GradArgs {
+    EnvView env;
+    const double* dist;
+    const uint32_t* idx;
+    const double* xyz;              // raw [n_prims][3] of the structure set
+    const uint64_t* prim_off;       // [n_structs + 1]
+    uint64_t n_structs;
+    const uint32_t* anchor_struct;  // [2 n_pairs]
+    const uint32_t* anchor_prim;    // [2 n_pairs]
+    uint64_t n_pairs;
+    const uint32_t* wf_idx;         // per pair or nullptr
+    const double* pair_weights;     // upstream gradient g_p per pair or nullptr (all 1)
+    double* out;                    // [n_pairs] scores
+    double* grad[2];                // [n_prims of structure s][3], zeroed by the caller: sum_p g_p dS_p / dxyz
+};
+// returns the number of launches, or -1 when the per-warp state of C categories does not fit shared memory
+int launch_score_grad(const GradArgs& g, const KParams& p, cudaStream_t st);
+int launch_wf_density(const WfDev* wf, uint64_t n, const double* x, double* out, int* err, cudaStream_t st);
 int launch_job_means(const double* scores, const uint64_t* job_pair_off, uint64_t n_jobs, double* means,
                      cudaStream_t st);
 int launch_widen_xyz(const float* in, double* out, uint64_t n3, cudaStream_t st);

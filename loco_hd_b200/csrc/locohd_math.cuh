@@ -79,6 +79,45 @@ __device__ __forceinline__ double wf_cdf(const WfDev& w, double x) {
     }
 }
 
+// Density w(x) = W'(x) for x >= 0, branch by branch the derivative of wf_cdf (the same comparisons at the kinks of
+// uniform and kumaraswamy: x < x_min -> 0, x > x_max -> 0).
+__device__ __forceinline__ double wf_pdf(const WfDev& w, double x) {
+    switch (w.kind) {
+        case LOCOHD_WF_UNIFORM: {
+            if (x < w.p[0] || x > w.p[1]) return 0.0;
+            return w.inv_range;
+        }
+        case LOCOHD_WF_KUMARASWAMY: {
+            if (x < w.p[0] || x > w.p[1]) return 0.0;
+            const double a = w.p[2], b = w.p[3];
+            const double z = (x - w.p[0]) * w.inv_range;
+            const double za1 = (w.int_a >= 1) ? powi_small(z, w.int_a - 1) : pow(z, a - 1.0);   // z^(a-1)
+            const double u = 1.0 - ((w.int_a >= 0) ? powi_small(z, w.int_a) : pow(z, a));
+            const double ub1 = (w.int_b >= 1) ? powi_small(u, w.int_b - 1) : pow(u, b - 1.0);   // (1 - z^a)^(b-1)
+            return a * b * za1 * ub1 * w.inv_range;
+        }
+        case LOCOHD_WF_DAGUM: {
+            // W = (1 + u)^-p with u = (x/b)^-a:  w = (a p / x) u (1 + u)^-(p+1), all in one exponent so that neither
+            // u, (1 + u) nor a p / x overflows for small x (inf * 0 would give NaN)
+            const double a = w.p[0], b = w.p[1], p = w.p[2];
+            if (!(x > 0.0)) {   // limit x -> 0 of (a p / x) (x/b)^(a p): 0, a p / b^(a p) or +inf
+                const double ap = a * p;
+                return ap > 1.0 ? 0.0 : (ap == 1.0 ? ap / b : INFINITY);
+            }
+            const double lx = log(x);
+            const double lu = -a * (lx - log(b));   // log u (x / b would underflow for the smallest x)
+            const double l = lu > 0.0 ? -p * lu - (p + 1.0) * log1p(exp(-lu)) : lu - (p + 1.0) * log1p(exp(lu));
+            return exp(l + log(a * p) - lx);
+        }
+        default: {  // LOCOHD_WF_HYPER_EXP
+            const int half = w.n >> 1;
+            double sum = 0.0;
+            for (int i = 0; i < half; ++i) sum += w.p[i] * w.p[half + i] * exp(-w.p[half + i] * x);
+            return sum * w.inv_norm;
+        }
+    }
+}
+
 // ---- statistical distances on normalised compositions --------------------------------------------
 // P1(i) / P2(i) are callables returning the i-th normalised probability.
 

@@ -59,6 +59,27 @@ class OracleCtx:
     def from_primitives(self, xa, ca, ta, xb, cb, tb, anchors, thr, wf_idx=None):
         return oracle.from_primitives(self.p, xa, ca, ta, xb, cb, tb, anchors, thr, wf_idx=wf_idx)
 
+    def from_primitives_grad(self, xa, ca, ta, xb, cb, tb, anchors, thr, wf_idx=None, pair_weights=None, out=None,
+                             grad_a=None, grad_b=None):
+        import grad_reference
+        from loco_hd_b200 import _capi
+        try:
+            s, ga, gb = grad_reference.from_primitives_grad(oracle, self.p, xa, ca, ta, xb, cb, tb, anchors, thr,
+                                                            wf_idx=wf_idx, pair_weights=pair_weights)
+        except oracle.OracleError as e:
+            raise _capi.LocoHDError(e.status, str(e))
+        for dst, src in ((grad_a, ga), (grad_b, gb)):
+            if dst is not None:
+                dst[...] = src
+        return s, ga if grad_a is None else grad_a, gb if grad_b is None else grad_b
+
+    def wf_integral_points(self, name, params, x):
+        return np.array([oracle.wf_integral_point(name, list(params), float(v)) for v in x])
+
+    def wf_density_points(self, name, params, x):
+        import grad_reference
+        return np.array([grad_reference.wf_density(name, params, float(v)) for v in x])
+
     def structs_create(self, offs, xyz, cat, tag):
         return _H(off=np.asarray(offs, dtype=np.int64), xyz=np.asarray(xyz, dtype=np.float64), cat=np.asarray(cat), tag=np.asarray(tag))
 
@@ -146,6 +167,23 @@ if __name__ == "__main__":
         hp.test_cuda_path_against_exact_values(ctx)
         hp.test_cuda_batch_path_against_exact_values(ctx)
         print("ok  test_highprec.py::test_cuda_path_against_exact_values / test_cuda_batch_path_against_exact_values (test logic only)")
+
+    import test_gpu_grad as tg
+    grad_cases = [(f"test_gradients_match_the_reference[{sd}-{wf}]", tg.test_gradients_match_the_reference, (wf, sd))
+                  for wf in sorted(tg.WFS) for sd in sorted(tg.SDS)]
+    grad_cases += [(f"test_weight_function_densities[{n}-{p}]",
+                    lambda c, o, n, p: tg.test_weight_function_densities(c, n, p), (n, p)) for n, p in tg.DENSITY_WFS]
+    grad_cases += [("test_gradients_integer_kumaraswamy", tg.test_gradients_integer_kumaraswamy, ()),
+                   ("test_gradients_per_pair_weight_functions", tg.test_gradients_per_pair_weight_functions, ()),
+                   ("test_renyi_zero_on_disjoint_compositions", tg.test_renyi_zero_on_disjoint_compositions, ()),
+                   ("test_no_pairs_leaves_zero_gradients", tg.test_no_pairs_leaves_zero_gradients, ())]
+    grad_cases += [(f"test_directional_derivative_matches_finite_differences[{wf}]",
+                    tg.test_directional_derivative_matches_finite_differences, (wf,)) for wf in sorted(tg.WFS)]
+    for name, fn, args in grad_cases:
+        if only and not any(o in name for o in only):
+            continue
+        fn(ctx, oracle, *args)
+        print(f"ok  test_gpu_grad.py::{name} (test logic only)")
 
     import test_gpu_tile_matrix as tm
     tm._env_offsets = lambda env: env.offsets()   # the stand-in has no C-ABI handle to dump
