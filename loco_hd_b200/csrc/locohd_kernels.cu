@@ -1315,9 +1315,8 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) {
 constexpr uint64_t kSentinel = ~0ull;   // staged behind either list of the fast kernel: above every key
 constexpr int kScoreMaxWarps = 8;
 // fast kernel: one large CTA per SM shares a single copy of the tables.  The W-keyed instantiations need 50 registers
-// (32 warps fit the register file); the distance-keyed ones (several weight functions) and the ones with table
-// bound checks need up to 72: 28 warps.
-__host__ __device__ constexpr int score_fast_max_warps(bool key_is_w, bool check, bool weighted = false) { return weighted ? 24 : ((key_is_w && !check) ? 32 : 28); }
+// (32 warps fit the register file); the distance-keyed ones (several weight functions) need up to 72: 28 warps.
+__host__ __device__ constexpr int score_fast_max_warps(bool key_is_w, bool weighted) { return weighted ? 24 : (key_is_w ? 32 : 28); }
 constexpr uint64_t kWMask = ~kCatMask;
 
 // per-lane values and counts of the generic kernel + the warp's mbarrier (16 bytes at the end)
@@ -1834,22 +1833,22 @@ __device__ __forceinline__ void sts_u32_rmw(uint32_t addr, uint32_t v) {
 //     H^2 = 1 - D / sqrt(NA NB),   D = sum_r w_r sqrt(a_r) sqrt(b_r),
 // so the incremental update only gains a factor w_c, and 1 / sqrt(NA) comes from rsqrt() instead of a table indexed by
 // an integer total.  (Weighted counts enter as count * w; upstream adds w repeatedly: <= 1e-13, documented deviation.)
-template <int CP, bool KEY_IS_W, bool CHECK, bool WEIGHTED>
-__global__ void __launch_bounds__(score_fast_max_warps(KEY_IS_W, CHECK, WEIGHTED) * 32) score_fast_kernel(ScoreArgs a, KParams P, int warps_per_block,
-                                                                         int per_warp_bytes) {
+template <int CP, bool KEY_IS_W, bool WEIGHTED>
+__global__ void __launch_bounds__(score_fast_max_warps(KEY_IS_W, WEIGHTED) * 32) score_fast_kernel(ScoreArgs a, KParams P, int warps_per_block,
+                                                                  int per_warp_bytes) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int table_n = a.table_n;
     double* s_sqrt = reinterpret_cast<double*>(smem_raw);   // sqrt(k)
     double* s_dsq = s_sqrt + table_n;                       // sqrt(k + 1) - sqrt(k)   (exact: Sterbenz)
-    double* s_rsqrt = s_dsq + table_n;                      // CHECK: 1 / sqrt(k); else sqrt(k / (k + 1)), the factor
-                                                            // that takes 1 / sqrt(k) to 1 / sqrt(k + 1)
+    double* s_rsqrt = s_dsq + table_n;                      // sqrt(k / (k + 1)), the factor that takes 1 / sqrt(k)
+                                                            // to 1 / sqrt(k + 1)
     double* s_w = s_rsqrt + table_n;                        // [16] category weights (WEIGHTED)
     for (int k = threadIdx.x; k < table_n; k += blockDim.x) {
         const double s0 = P.sqrt_tbl[k], s1 = P.sqrt_tbl[k + 1];
         s_sqrt[k] = s0;
         s_dsq[k] = s1 - s0;
-        s_rsqrt[k] = CHECK ? P.rsqrt_tbl[k] : sqrt((double)k / (double)(k + 1));
+        s_rsqrt[k] = sqrt((double)k / (double)(k + 1));
     }
     if (threadIdx.x < 16) s_w[threadIdx.x] = (WEIGHTED && (int)threadIdx.x < P.C) ? P.cat_w[threadIdx.x] : 1.0;
     __syncthreads();
@@ -1868,19 +1867,8 @@ __global__ void __launch_bounds__(score_fast_max_warps(KEY_IS_W, CHECK, WEIGHTED
     const uint32_t dsq_base = __shfl_sync(kFull, smem_u32(s_dsq), lane);
     const uint32_t ratio_base = __shfl_sync(kFull, smem_u32(s_rsqrt), lane);
     const uint32_t cnt_lane = __shfl_sync(kFull, smem_u32(cnt + lane), lane);
-    auto sqrt_of = [&](uint32_t k) -> double {
-        if (CHECK && k >= (uint32_t)table_n) return sqrt((double)k);
-        return s_sqrt[k];
-    };
-    auto dsq_of = [&](uint32_t k) -> double {   // sqrt(k + 1) - sqrt(k)
-        if (CHECK && k >= (uint32_t)table_n) return sqrt((double)k + 1.0) - sqrt((double)k);
-        return s_dsq[k];
-    };
-    auto rsqrt_of = [&](uint32_t k) -> double {
-        if (CHECK && k >= (uint32_t)table_n) return 1.0 / sqrt((double)k);
-        if (!CHECK) return __ldg(P.rsqrt_tbl + k);   // chunk start and the small-H^2 path only
-        return s_rsqrt[k];
-    };
+    auto sqrt_of = [&](uint32_t k) -> double { return s_sqrt[k]; };
+    auto rsqrt_of = [&](uint32_t k) -> double { return __ldg(P.rsqrt_tbl + k); };   // chunk start and the small-H^2 path only
 
     // Work distribution: warps claim runs of kScoreRun consecutive pairs from a global cursor.  All resident warps
     // then work at one moving frontier of the pair list, so consecutive jobs that share a structure find its
@@ -2028,94 +2016,57 @@ __global__ void __launch_bounds__(score_fast_max_warps(KEY_IS_W, CHECK, WEIGHTED
         // The first nev events of the merge that starts at (i, j) are exactly my chunk (same comparison as the
         // merge-path split: A before B on ties); the sentinels end the lists.
         const uint32_t nev = (i1 - i) + (j1 - j);
-        if constexpr (!CHECK) {
-            // Tables cover every count.  Per-lane state: shared-space addresses of the next key of either list
-            // (pa, pb); the index into the ratio table advances in step with them, so it is a constant offset
-            // (dA, dB) from the key address; R = rA * rB is carried as a product and updated by one table factor
-            // (<= 64 events per chunk: <= 64 roundings, ~1e-14 relative - H >= 1e-4 here, bar 1e-9).
-            uint32_t pa = smem_u32(kA + i), pb = smem_u32(kB + j);
-            const uint32_t dA = ratio_base + 8u * totA - pa, dB = ratio_base + 8u * totB - pb;
-            double R = __dmul_rn(rA, rB);
-            uint64_t ra = lds_u64(pa), rb = lds_u64(pb);
-            for (uint32_t it = 0; it < nev; ++it) {   // (unrolled by 2: 5.58 -> 5.60 ms on config 2, profiles/r6z - this kernel sits on the shared-memory pipe)
-                const bool takeA = ra <= (rb | kCatMask);   // == (ra & kWMask) <= (rb & kWMask)
-                const uint64_t raw = takeA ? ra : rb;
-                const double w = weight(raw);
-                acc = fma(w - wprev, h, acc);
-                wprev = w;
-                uint32_t ca;   // cnt_lane + category * 128 (one IMAD; the compiler's shift + mask + add are three)
-                asm("mad.lo.u32 %0, %1, 128, %2;" : "=r"(ca) : "r"((uint32_t)raw & 0xFFu), "r"(cnt_lane));
-                const uint32_t word = lds_u32_rmw(ca);
-                const uint32_t ka = word & 0xffffu, kb = word >> 16;
-                const uint32_t mine_k = takeA ? ka : kb, other_k = takeA ? kb : ka;
-                sts_u32_rmw(ca, word + (takeA ? 1u : 0x10000u));
-                mism += (mine_k == other_k ? 1 : 0) - (mine_k + 1u == other_k ? 1 : 0);
-                const uint32_t pk = takeA ? pa : pb;
-                if (WEIGHTED) {
-                    const double wc = s_w[(uint32_t)raw & 0xFFu];
-                    D = fma(wc * lds_f64(dsq_base + 8u * mine_k), lds_f64(sq_base + 8u * other_k), D);
-                    NA += takeA ? wc : 0.0;
-                    NB += takeA ? 0.0 : wc;
-                    const double rnew = rsqrt_pos(takeA ? NA : NB);
-                    rA = takeA ? rnew : rA;
-                    rB = takeA ? rB : rnew;
-                    R = rA * rB;
-                } else {
-                    D = fma(lds_f64(dsq_base + 8u * mine_k), lds_f64(sq_base + 8u * other_k), D);
-                    R *= lds_f64(pk + (takeA ? dA : dB));
-                }
-                const uint64_t nxt = lds_u64(pk + 8u);
-                pa = takeA ? pk + 8u : pa;
-                pb = takeA ? pb : pk + 8u;
-                ra = takeA ? nxt : ra;
-                rb = takeA ? rb : nxt;
-                const double h2 = fma(-R, D, 1.0);
-                // (measured and dropped, profiles/r4d: sum |a_r - b_r| instead of the mismatch count and an integer test
-                //  of h2's high word - fewer instructions, 1-2 % slower: the kernel is bound by the shared-memory pipe)
-                h = (mism == 0) ? 0.0 : sqrt_unit(h2);       // identical counts: exactly 0
-                if (mism != 0 && h2 < kSmallH2) {            // rare: difference form from the counts
-                    if (!WEIGHTED) {
-                        rA = rsqrt_of((pa + dA - ratio_base) >> 3);
-                        rB = rsqrt_of((pb + dB - ratio_base) >> 3);
-                    }
-                    h = sqrt(exact_h2());
-                }
-            }
-            if (lane == 31) acc = fma(wf.w_inf - wprev, h, acc);
-            for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(kFull, acc, o);
-            if (lane == 0) a.out[pair] = acc;
-            continue;
-        }
-        uint64_t ra = kA[i], rb = kB[j];
-        for (uint32_t it = 0; it < nev; ++it) {
-            const bool takeA = (ra & kWMask) <= (rb & kWMask);
+        // The tables cover every count (launch_score sizes them to the stage).  Per-lane state: shared-space addresses
+        // of the next key of either list (pa, pb); the index into the ratio table advances in step with them, so it is
+        // a constant offset (dA, dB) from the key address; R = rA * rB is carried as a product and updated by one table
+        // factor (<= 64 events per chunk: <= 64 roundings, ~1e-14 relative - H >= 1e-4 here, bar 1e-9).
+        uint32_t pa = smem_u32(kA + i), pb = smem_u32(kB + j);
+        const uint32_t dA = ratio_base + 8u * totA - pa, dB = ratio_base + 8u * totB - pb;
+        double R = __dmul_rn(rA, rB);
+        uint64_t ra = lds_u64(pa), rb = lds_u64(pb);
+        for (uint32_t it = 0; it < nev; ++it) {   // (unrolled by 2: 5.58 -> 5.60 ms on config 2, profiles/r6z - this kernel sits on the shared-memory pipe)
+            const bool takeA = ra <= (rb | kCatMask);   // == (ra & kWMask) <= (rb & kWMask)
             const uint64_t raw = takeA ? ra : rb;
-            const uint32_t c = (uint32_t)(raw & kCatMask);
             const double w = weight(raw);
             acc = fma(w - wprev, h, acc);
             wprev = w;
-            const uint32_t word = cnt[c * 32 + lane];
+            uint32_t ca;   // cnt_lane + category * 128 (one IMAD; the compiler's shift + mask + add are three)
+            asm("mad.lo.u32 %0, %1, 128, %2;" : "=r"(ca) : "r"((uint32_t)raw & 0xFFu), "r"(cnt_lane));
+            const uint32_t word = lds_u32_rmw(ca);
             const uint32_t ka = word & 0xffffu, kb = word >> 16;
             const uint32_t mine_k = takeA ? ka : kb, other_k = takeA ? kb : ka;
-            cnt[c * 32 + lane] = word + (takeA ? 1u : 0x10000u);
+            sts_u32_rmw(ca, word + (takeA ? 1u : 0x10000u));
             mism += (mine_k == other_k ? 1 : 0) - (mine_k + 1u == other_k ? 1 : 0);
-            const double wc = WEIGHTED ? s_w[c] : 1.0;
-            D = WEIGHTED ? fma(wc * dsq_of(mine_k), sqrt_of(other_k), D) : fma(dsq_of(mine_k), sqrt_of(other_k), D);
-            {   // one table read and one key read per event, whichever side moved (two predicated reads of each
-                // kind cost twice the shared-memory wavefronts: ncu, profiles/r1t)
-                totA += takeA ? 1u : 0u;
-                totB += takeA ? 0u : 1u;
-                if (WEIGHTED) { NA += takeA ? wc : 0.0; NB += takeA ? 0.0 : wc; }
-                const double rnew = WEIGHTED ? rsqrt_pos(takeA ? NA : NB) : rsqrt_of(takeA ? totA : totB);
+            const uint32_t pk = takeA ? pa : pb;
+            if (WEIGHTED) {
+                const double wc = s_w[(uint32_t)raw & 0xFFu];
+                D = fma(wc * lds_f64(dsq_base + 8u * mine_k), lds_f64(sq_base + 8u * other_k), D);
+                NA += takeA ? wc : 0.0;
+                NB += takeA ? 0.0 : wc;
+                const double rnew = rsqrt_pos(takeA ? NA : NB);
                 rA = takeA ? rnew : rA;
                 rB = takeA ? rB : rnew;
-                i += takeA ? 1u : 0u;
-                j += takeA ? 0u : 1u;
-                const uint64_t nxt = *(takeA ? (kA + i) : (kB + j));
-                ra = takeA ? nxt : ra;
-                rb = takeA ? rb : nxt;
+                R = rA * rB;
+            } else {
+                D = fma(lds_f64(dsq_base + 8u * mine_k), lds_f64(sq_base + 8u * other_k), D);
+                R *= lds_f64(pk + (takeA ? dA : dB));
             }
-            h = stat_dist();
+            const uint64_t nxt = lds_u64(pk + 8u);
+            pa = takeA ? pk + 8u : pa;
+            pb = takeA ? pb : pk + 8u;
+            ra = takeA ? nxt : ra;
+            rb = takeA ? rb : nxt;
+            const double h2 = fma(-R, D, 1.0);
+            // (measured and dropped, profiles/r4d: sum |a_r - b_r| instead of the mismatch count and an integer test
+            //  of h2's high word - fewer instructions, 1-2 % slower: the kernel is bound by the shared-memory pipe)
+            h = (mism == 0) ? 0.0 : sqrt_unit(h2);       // identical counts: exactly 0
+            if (mism != 0 && h2 < kSmallH2) {            // rare: difference form from the counts
+                if (!WEIGHTED) {
+                    rA = rsqrt_of((pa + dA - ratio_base) >> 3);
+                    rB = rsqrt_of((pb + dB - ratio_base) >> 3);
+                }
+                h = sqrt(exact_h2());
+            }
         }
         if (lane == 31) acc = fma(wf.w_inf - wprev, h, acc);
         for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(kFull, acc, o);
@@ -2133,7 +2084,7 @@ __global__ void __launch_bounds__(score_fast_max_warps(KEY_IS_W, CHECK, WEIGHTED
 //   * the straight-line set-up of a pair (merge-path split, prefix scans, D from the counts, reduction: ~1 000 of the
 //     1 860 warp instructions of score_fast_kernel) is issued once for four pairs; prefix scans and the reduction
 //     take 3 shuffle steps instead of 5.
-// The arithmetic per event is that of score_fast_kernel<CP, true, false, false> (same tables, same expanded form, same
+// The arithmetic per event is that of score_fast_kernel<CP, true, false> (same tables, same expanded form, same
 // small-H^2 fallback); a lane's chunk is E / 8 events instead of E / 32 (the host caps E at 1024: <= 128 roundings of
 // R and D per chunk, ~3e-14 relative).  One CTA per SM (tables staged once), teams synchronise on named barriers.
 // ncu (profiles/r6b): 1 214 warp instructions and 375 shared-memory wavefronts per pair (1 949 / 523 for one pair per
@@ -2941,13 +2892,9 @@ static int launch_generic(const ScoreArgs& args, const KParams& p, unsigned stag
 }
 
 template <int CP, bool KEY_IS_W>
-static int launch_fast(const ScoreArgs& a, const KParams& p, bool check, int warps, int per_warp, int smem,
-                       cudaStream_t st) {
-    if (!p.unit_w)
-        return check ? launch_score_kernel(score_fast_kernel<CP, KEY_IS_W, true, true>, a, p, warps, per_warp, smem, st)
-                     : launch_score_kernel(score_fast_kernel<CP, KEY_IS_W, false, true>, a, p, warps, per_warp, smem, st);
-    return check ? launch_score_kernel(score_fast_kernel<CP, KEY_IS_W, true, false>, a, p, warps, per_warp, smem, st)
-                 : launch_score_kernel(score_fast_kernel<CP, KEY_IS_W, false, false>, a, p, warps, per_warp, smem, st);
+static int launch_fast(const ScoreArgs& a, const KParams& p, int warps, int per_warp, int smem, cudaStream_t st) {
+    return p.unit_w ? launch_score_kernel(score_fast_kernel<CP, KEY_IS_W, false>, a, p, warps, per_warp, smem, st)
+                    : launch_score_kernel(score_fast_kernel<CP, KEY_IS_W, true>, a, p, warps, per_warp, smem, st);
 }
 
 LaunchOverrides read_launch_overrides() {
@@ -2965,7 +2912,7 @@ LaunchOverrides read_launch_overrides() {
 
 TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, const LaunchOverrides& ov) {
     TileGeometry g{};
-    if (!(p.hell2 && p.unit_w && p.C >= 1 && p.C <= 16 && key_is_w)) return g;   // the configuration of score_fast_kernel<CP, true, false, false>
+    if (!(p.hell2 && p.unit_w && p.C >= 1 && p.C <= 16 && key_is_w)) return g;   // the configuration of score_fast_kernel<CP, true, false>
     if (max_a < 1 || max_b < 1 || max_a + max_b > 1024u) return g;   // chunks of at most 128 events per lane
     const unsigned need = (max_a > max_b ? max_a : max_b) + 2u;
     g.table_n = (int)((need + 63u) & ~63u);
@@ -3057,11 +3004,10 @@ int launch_score(const ScoreArgs& args, const KParams& p, unsigned max_a, unsign
         if (stage > pad_max) stage = pad_max;
     }
     int n = 0;
-    // tables: counts never exceed the environment sizes
-    unsigned need = (max_a > max_b ? max_a : max_b) + 2u;
-    bool check = false;
-    unsigned table_n = (need + 63u) & ~63u;
-    if (table_n > 1024u) { table_n = 1024u; check = true; }
+    // tables: counts never exceed the environment sizes, and a staged pair's counts and totals are below stage - 1
+    static_assert(2048 + 1 < kSqrtTableSize, "the table fill reads sqrt_tbl[k + 1] for k < the largest stage");
+    const unsigned need = (max_a > max_b ? max_a : max_b) + 2u;
+    const unsigned table_n = ((need < stage ? need : stage) + 63u) & ~63u;
     a.table_n = (int)table_n;
     a.stage_cap = (int)stage;
     a.only_unstaged = 0;
@@ -3069,13 +3015,13 @@ int launch_score(const ScoreArgs& args, const KParams& p, unsigned max_a, unsign
     const int per_warp = fast_state_bytes(CP) + ((int)stage + 4) * 8;   // + the two sentinels and their padding
     const int budget = 220 * 1024;  // one CTA per SM: the tables are staged once, the rest goes to the warps' stages
     int warps = (budget - tables) / per_warp;
-    if (warps > score_fast_max_warps(key_is_w, check, !p.unit_w)) warps = score_fast_max_warps(key_is_w, check, !p.unit_w);
+    if (warps > score_fast_max_warps(key_is_w, !p.unit_w)) warps = score_fast_max_warps(key_is_w, !p.unit_w);
     if (warps < 1) warps = 1;
     const int smem = tables + per_warp * warps;
-    if (CP == 8) n += key_is_w ? launch_fast<8, true>(a, p, check, warps, per_warp, smem, st)
-                               : launch_fast<8, false>(a, p, check, warps, per_warp, smem, st);
-    else n += key_is_w ? launch_fast<16, true>(a, p, check, warps, per_warp, smem, st)
-                       : launch_fast<16, false>(a, p, check, warps, per_warp, smem, st);
+    if (CP == 8) n += key_is_w ? launch_fast<8, true>(a, p, warps, per_warp, smem, st)
+                               : launch_fast<8, false>(a, p, warps, per_warp, smem, st);
+    else n += key_is_w ? launch_fast<16, true>(a, p, warps, per_warp, smem, st)
+                       : launch_fast<16, false>(a, p, warps, per_warp, smem, st);
     if (pad_max > stage) {
         const int m = launch_generic(args, p, 0, (int)stage, st);
         if (m < 0) return m;

@@ -248,6 +248,30 @@ def test_large_environments(gpu_ctx, oracle_mod, n, thr):
     check_from_primitives(gpu_ctx, oracle_mod, op, A, B, anchors, thr)
 
 
+def test_category_counts_above_1024_in_the_fast_kernel(gpu_ctx, oracle_mod):
+    """Hellinger-2 pairs whose environments fit the fast kernel's stage together (Ma + Mb <= 2 046) while one category
+    of A holds more than 1 024 members: the kernel's sqrt and ratio tables must reach every such count and total.  A is
+    a dense ball (environments of 1 300-1 600 members around its centre), B a sparse one (~300), both 90 % category 0;
+    A + B hold 2 040 points, so no pair can exceed the bound."""
+    rng = np.random.default_rng(1024)
+
+    def ball(n):   # n points uniform in a ball of radius 10 around the origin, 90 % of them category 0
+        d = rng.normal(size=(n, 3))
+        d /= np.linalg.norm(d, axis=1, keepdims=True)
+        xyz = d * (10.0 * rng.random(n) ** (1.0 / 3.0))[:, None]
+        return xyz, (rng.random(n) < 0.1).astype(np.uint16), np.zeros(n, np.uint32)
+
+    A, B = ball(1650), ball(390)
+    core_a = np.flatnonzero(np.linalg.norm(A[0], axis=1) < 2.5)
+    core_b = np.flatnonzero(np.linalg.norm(B[0], axis=1) < 4.0)
+    anchors = np.stack([core_a, core_b[np.arange(len(core_a)) % len(core_b)]], axis=1)
+    op = set_both(gpu_ctx, oracle_mod, 2, [("uniform", (0.0, 10.0))])
+    _, ref = check_from_primitives(gpu_ctx, oracle_mod, op, A, B, anchors, 10.0)
+    sizes = ref["env_sizes"]
+    assert sizes[:, 0].max() > 1100 and sizes.sum(axis=1).max() <= 2046
+    assert ref["counts"][:, 0, 0].max() > 1024
+
+
 def test_empty_anchor_list(gpu_ctx, oracle_mod):
     rng = np.random.default_rng(12)
     A = random_cloud(rng, 30, 3)
