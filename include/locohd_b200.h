@@ -98,9 +98,11 @@ typedef struct locohd_params {
 
 typedef enum locohd_prof_group {
     LOCOHD_PROF_CELLS = 0,   /* K0 build_cells_kernel */
-    LOCOHD_PROF_COUNT = 1,   /* K1a env_tile_kernel<false>: upper-bound sizes (fused gather: of a 1/16 sample) */
+    LOCOHD_PROF_COUNT = 1,   /* K1a env_tile_kernel<false>: upper-bound sizes (fused gather: of a 1/16 sample, only
+                                for calls above 32 768 anchors without a remembered store size) */
     LOCOHD_PROF_SCAN = 2,    /* scan of the environment sizes (multi-kernel fallback only) */
-    LOCOHD_PROF_FILL = 3,    /* K1 env_fused_kernel: gather + sort + packing (fallback: K1b env_tile_kernel<true>) */
+    LOCOHD_PROF_FILL = 3,    /* K1 env_fused_kernel, once per attempt: gather + sort + packing (fallback: K1b
+                                env_tile_kernel<true>) */
     LOCOHD_PROF_SCORE = 4,   /* K2 score_fast_kernel / score_kernel */
     LOCOHD_PROF_OTHER = 5,   /* anchor ordering, conversions, validation, means, row copies, ... */
     LOCOHD_PROF_SORT = 6,    /* K1c env_sort_kernel (multi-kernel fallback only): per-environment sort, CDF, packing */

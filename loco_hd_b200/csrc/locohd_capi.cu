@@ -61,10 +61,12 @@ struct locohd_ctx {
     // pinned staging area of the one-call entry point (small calls: all inputs travel in one copy)
     unsigned char* h_stage = nullptr;
     size_t h_stage_bytes = 0;
-    int fused_cap_hint = kFusedCap;  // members per environment the fused gather starts with (512 or 1024)
-    uint64_t hist_n_anchors = 0, hist_capacity = 0;   // store size that worked for the last call of this shape (0: none)
-    double hist_threshold = 0.0;
-    int hist_cap = 0;
+    struct {   // sizing state of the fused gather, carried from call to call (fused_gather alone reads and writes it)
+        int cap_hint = kFusedCap;               // members per environment the fused gather starts with (512 or 1024)
+        uint64_t n_anchors = 0, capacity = 0;   // store size that worked for the last call of this shape (0: none)
+        double threshold = 0.0;
+        int cap = 0;
+    } store_hist;
     // Large device buffers (environment stores, scratch) are recycled per context: the stream-ordered pool of the
     // driver splits and re-merges multi-GB blocks unpredictably, which shows up as 30-60 ms stalls per call.
     std::mutex cache_mu;
@@ -417,6 +419,14 @@ int read_scan_stats(locohd_ctx* ctx, int slot, ScanStats* host) {
     return sync_and_check(ctx);
 }
 
+int read_fused_stats(locohd_ctx* ctx, int slot, FusedStats* host) {
+    if (cudaMemcpyAsync(&ctx->h_fstats[slot], ctx->d_fstats, sizeof(FusedStats), cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess)
+        return fail(ctx, LOCOHD_ERR_CUDA, "copy of the gather statistics failed");
+    TRY_ST(sync_and_check(ctx));
+    *host = ctx->h_fstats[slot];
+    return 0;
+}
+
 void destroy_envset(locohd_envset* e) {
     if (!e) return;
     locohd_ctx* ctx = e->ctx;
@@ -426,10 +436,115 @@ void destroy_envset(locohd_envset* e) {
     delete e;
 }
 
-// kd-tree build + env_from_idx for a list of anchors (locohd.rs:504-542):
-//   K0 cells (cached per threshold) -> anchors into cell order -> K1a upper-bound sizes -> scan -> store allocation
-//   -> K1b exact gather into the store -> K1c per-environment sort + CDF + key packing.
-// One host synchronisation (the store size) per call.
+constexpr uint64_t kBoundAnchors = 32768;
+constexpr uint32_t kSampleStride = 16;
+
+// Store entries of the fused gather for n_anchors environments of at most `cap` members gathered by `grid` blocks:
+// the `history` size when not 0 (the store size that worked for the last call of this shape), else for calls of up to
+// kBoundAnchors anchors (one structure pair is the typical call of the reference API) the bound `cap` per environment,
+// else the sum `sample` of the FP32 upper-bound sizes of every kSampleStride-th anchor.
+uint64_t fused_store_capacity(uint64_t n_anchors, int cap, unsigned grid, uint64_t sample, uint64_t history) {
+    if (history) return history;
+    // sampled sizes are FP32 upper bounds; even-rounding adds at most one entry per environment, every warp can leave
+    // most of a chunk unused at every refill and at the end
+    const double est = n_anchors <= kBoundAnchors ? (double)n_anchors * (double)cap
+                                                  : (double)sample * (double)kSampleStride * 1.03 + 65536.0;
+    const double waste = 1.0 + (double)cap / (double)kFusedChunk;
+    const uint64_t capacity = (uint64_t)((est + (double)n_anchors) * waste) + (uint64_t)grid * kFusedWarps * kFusedChunk + 2 * kFusedChunk;
+    // The sample differs a little from call to call (cell order depends on atomics): round the size up to 4
+    // significant bits so that repeated calls ask the block cache for the same size (a fresh multi-GB
+    // cudaMallocAsync costs 0.5-2 s).
+    for (uint64_t step = 1ull << 62; step >= 32; step >>= 1)
+        if (capacity & step) { step >>= 4; return (capacity + step - 1) & ~(step - 1); }
+    return capacity;
+}
+
+// The fused gather: env_fused_kernel gathers, sorts and packs every environment in one launch.  It runs the 512-member
+// instantiation, or the 1024-member one once a call has reported larger environments (the hint stays with the context
+// until a 1024 run sees none above 384 members).  *built stays false, with no store allocated, when an environment has
+// more than 1024 members or the store overflows for another reason than the cap.
+int fused_gather(locohd_ctx* ctx, const StructsView& sv, locohd_envset* e, const uint32_t* d_anchor_struct,
+                 const uint32_t* d_anchor_prim, double threshold, int keep_indices, const uint32_t* d_order,
+                 const uint2* d_order_rec, bool* built) {
+    const uint64_t n_anchors = e->n_env;
+    const bool by_bound = n_anchors <= kBoundAnchors;
+    auto& h = ctx->store_hist;
+    // A call of the same shape as the last one (a benchmark step, the next block of trajectory frames) takes the store
+    // size that worked then and skips the sizing pass and its synchronisation.  If that store turns out too small, the
+    // history is dropped and the call is redone once, sized by a sample like a first call.
+    for (int attempt = 0; attempt < 2; ++attempt) {
+        const uint64_t history = !by_bound && h.n_anchors == n_anchors && h.threshold == threshold && h.cap == h.cap_hint ? h.capacity : 0;
+        cudaMemsetAsync(ctx->d_fstats, 0, sizeof(FusedStats), ctx->stream);
+        FusedStats fs{};
+        if (!by_bound && !history) {
+            { ProfScope ps(ctx, LOCOHD_PROF_COUNT);
+              ctx->launches += launch_env_sample(sv, ctx->kp, n_anchors, d_order, d_anchor_struct, d_anchor_prim, threshold,
+                                                 kSampleStride, &ctx->d_fstats->sample, ctx->stream); }
+            TRY_ST(read_fused_stats(ctx, 0, &fs));
+        }
+        for (int cap = h.cap_hint; cap <= kFusedCapBig; cap *= 2) {
+            const unsigned grid = fused_grid(ctx->kp, &ctx->h_wf0, e->key_is_w ? 1 : 0, keep_indices != 0, cap, n_anchors);
+            const uint64_t capacity = fused_store_capacity(n_anchors, cap, grid, fs.sample, history);
+            TRY_ST(dev_alloc(ctx, &e->d_key, capacity));
+            if (keep_indices) { TRY_ST(dev_alloc(ctx, &e->d_idx, capacity)); TRY_ST(dev_alloc(ctx, &e->d_dist, capacity)); }
+            EnvBuild b{};   // ub, off and cat stay null: the fused kernel needs neither sizes nor scratch
+            b.n_env = n_anchors; b.order = d_order; b.order_rec = d_order_rec; b.off_out = e->d_off; b.count = e->d_count;
+            b.key = e->d_key; b.idx = e->d_idx; b.dist = e->d_dist; b.key_is_w = e->key_is_w ? 1 : 0; b.key_is_sq = 1;
+            cudaMemsetAsync(&ctx->d_fstats->cursor, 0, sizeof(unsigned long long), ctx->stream);
+            cudaMemsetAsync(&ctx->d_fstats->max_count, 0, 2 * sizeof(unsigned int), ctx->stream);
+            { ProfScope ps(ctx, LOCOHD_PROF_FILL);
+              ctx->launches += launch_env_fused(sv, ctx->kp, &ctx->h_wf0, d_anchor_struct, d_anchor_prim, threshold, b, cap,
+                                                ctx->d_fstats, capacity, grid, ctx->stream); }
+            CU(ctx, cudaGetLastError());
+            FusedStats fr{}; TRY_ST(read_fused_stats(ctx, 1, &fr));
+            if (!fr.overflow) {
+                // remember the size for the next call of this shape unless it was a tight fit
+                h.n_anchors = n_anchors; h.threshold = threshold; h.cap = cap;
+                h.capacity = (!by_bound && (double)fr.cursor <= 0.94 * (double)capacity) ? capacity : 0;
+                if (cap == kFusedCapBig && fr.max_count <= (unsigned)(kFusedCap * 3 / 4)) h.cap_hint = kFusedCap;
+                e->capacity = capacity; e->total = fr.cursor < capacity ? fr.cursor : capacity; e->max_count = fr.max_count;
+                *built = true;
+                return 0;
+            }
+            dev_free(ctx, e->d_key); dev_free(ctx, e->d_idx); dev_free(ctx, e->d_dist);
+            if (fr.overflow == 8u) h.cap_hint = kFusedCapBig;   // only "more members than cap": on with 1024 members
+            if (history) { h.capacity = 0; break; }           // the history-sized store was too small: sample
+            if (fr.overflow != 8u) return 0;                  // the larger instantiation will not help
+        }
+        if (!history) return 0;                               // an environment has more than 1024 members
+    }
+    return 0;
+}
+
+// The multi-kernel gather, for every environment size and threshold: K1a upper-bound sizes -> scan -> store
+// allocation -> K1b exact gather into the store -> K1c per-environment sort + CDF + key packing.  One host
+// synchronisation (the store size).  *d_cat is allocated here; the caller releases it with its own scratch.
+int multi_kernel_gather(locohd_ctx* ctx, const StructsView& sv, locohd_envset* e, const uint32_t* d_anchor_struct,
+                        const uint32_t* d_anchor_prim, double threshold, int keep_indices, const uint32_t* d_order,
+                        uint32_t* d_ub, uint64_t* d_scratch, uint8_t** d_cat) {
+    { ProfScope ps(ctx, LOCOHD_PROF_COUNT);
+      ctx->launches += launch_env_count(sv, ctx->kp, e->n_env, d_order, d_anchor_struct, d_anchor_prim, threshold, d_ub, ctx->stream); }
+    { ProfScope ps(ctx, LOCOHD_PROF_SCAN); ctx->launches += launch_scan(d_ub, e->n_env, 1, e->d_off, d_scratch, ctx->d_scan + 1, ctx->stream); }
+    ScanStats ss{};
+    TRY_ST(read_scan_stats(ctx, 1, &ss));
+    e->capacity = ss.total + 2;
+    e->max_count = ss.max_value;   // upper bound of every environment size
+    TRY_ST(dev_alloc(ctx, &e->d_key, e->capacity)); TRY_ST(dev_alloc(ctx, d_cat, e->capacity));
+    if (keep_indices) { TRY_ST(dev_alloc(ctx, &e->d_idx, e->capacity)); TRY_ST(dev_alloc(ctx, &e->d_dist, e->capacity)); }
+    EnvBuild b{};
+    b.n_env = e->n_env; b.order = d_order; b.ub = d_ub; b.off = e->d_off; b.count = e->d_count; b.key = e->d_key;
+    b.cat = *d_cat; b.idx = e->d_idx; b.dist = e->d_dist; b.key_is_w = e->key_is_w ? 1 : 0; b.key_is_sq = 1;
+    { ProfScope ps(ctx, LOCOHD_PROF_FILL); ctx->launches += launch_env_fill(sv, ctx->kp, d_anchor_struct, d_anchor_prim, threshold, b, ctx->stream); }
+    { ProfScope ps(ctx, LOCOHD_PROF_SORT); ctx->launches += launch_env_sort(ctx->kp, b, e->max_count, threshold, ctx->stream); }
+    CU(ctx, cudaGetLastError());
+    e->total = ss.total;  // stored entries (upper bound of the member count; exact sizes are in d_count)
+    return 0;
+}
+
+// Environments of a list of anchors (kd-tree build + env_from_idx, locohd.rs:504-542): K0 cells (cached per
+// threshold), the anchors in cell order, then the fused gather, or the multi-kernel gather when the fused one does not
+// apply or falls back.  The fused kernel works with r^2 in the f32 exponent range (fixed-point sort keys, f32-seeded
+// square roots); LOCOHD_LEGACY_GATHER takes the multi-kernel gather for every call.
 int build_envset(locohd_ctx* ctx, locohd_structs* s, uint64_t n_anchors, const uint32_t* d_anchor_struct,
                  const uint32_t* d_anchor_prim, double threshold, int keep_indices, const LaunchOverrides& ov,
                  locohd_envset** out) {
@@ -445,7 +560,7 @@ int build_envset(locohd_ctx* ctx, locohd_structs* s, uint64_t n_anchors, const u
     uint2* d_order_rec = nullptr;
     uint64_t *d_slot_off = nullptr, *d_scratch = nullptr;
     uint8_t* d_cat = nullptr;
-    auto release = [&]() {
+    auto release = [&]() {  // stream-ordered: freed after the kernels of this call have run
         dev_free(ctx, d_order); dev_free(ctx, d_order_rec); dev_free(ctx, d_slot_cnt); dev_free(ctx, d_ub); dev_free(ctx, d_slot_off);
         dev_free(ctx, d_scratch); dev_free(ctx, d_cat);
     };
@@ -453,138 +568,23 @@ int build_envset(locohd_ctx* ctx, locohd_structs* s, uint64_t n_anchors, const u
     int st;
     if ((st = dev_alloc(ctx, &e->d_count, n_anchors)) || (st = dev_alloc(ctx, &e->d_off, n_anchors + 1))) return bail(st);
     const StructsView sv = s->view();
-    if (n_anchors == 0) {
-        cudaMemsetAsync(e->d_off, 0, sizeof(uint64_t), ctx->stream);
-        *out = e;
-        return 0;
-    }
+    if (n_anchors == 0) { cudaMemsetAsync(e->d_off, 0, sizeof(uint64_t), ctx->stream); *out = e; return 0; }
     const uint64_t n_prims = s->n_prims;
     const uint64_t scratch_n = std::max(scan_scratch_entries(n_prims + 1), scan_scratch_entries(n_anchors));
     if ((st = dev_alloc(ctx, &d_order, n_anchors)) || (st = dev_alloc(ctx, &d_order_rec, n_anchors)) || (st = dev_alloc(ctx, &d_slot_cnt, n_prims + 1)) ||
         (st = dev_alloc(ctx, &d_slot_off, n_prims + 2)) || (st = dev_alloc(ctx, &d_scratch, scratch_n)) ||
         (st = dev_alloc(ctx, &d_ub, n_anchors)))
         return bail(st);
-    {
-        ProfScope ps(ctx, LOCOHD_PROF_OTHER);
-        ctx->launches += launch_anchor_order(sv, ctx->kp, n_anchors, d_anchor_struct, d_anchor_prim, n_prims, d_slot_cnt,
-                                             d_slot_off, d_scratch, ctx->d_scan, d_order, d_order_rec, ctx->stream);
-    }
-    // ---- fused path: sample the sizes (every anchor for small calls), reserve the store, one kernel does the rest
-    // the fused kernel works with r^2 in the f32 exponent range (fixed-point sort keys, f32-seeded square roots)
-    if (!ov.legacy_gather && threshold * threshold < 1.0e30) {
-        // Store sizing.  Small calls (one structure pair is the typical call of the reference API) take the bound
-        // kFusedCap per environment and skip the sizing pass and its synchronisation; large batches sample the FP32
-        // upper-bound sizes of every 16th anchor.
-        const bool sized_by_bound = n_anchors <= 32768;
-        const uint32_t stride = 16u;
-    resize:
-        // A call of the same shape as the last one (a benchmark step, the next block of trajectory frames) takes the
-        // store size that worked then and skips the sizing pass and its synchronisation; if the store turns out too
-        // small after all, the history is dropped and the call is sized by a sample like a first call.
-        const bool by_history = !sized_by_bound && ctx->hist_capacity && ctx->hist_n_anchors == n_anchors &&
-                                ctx->hist_threshold == threshold && ctx->hist_cap == ctx->fused_cap_hint;
-        cudaMemsetAsync(ctx->d_fstats, 0, sizeof(FusedStats), ctx->stream);
-        FusedStats fs{};
-        if (!sized_by_bound && !by_history) {
-            {
-                ProfScope ps(ctx, LOCOHD_PROF_COUNT);
-                ctx->launches += launch_env_sample(sv, ctx->kp, n_anchors, d_order, d_anchor_struct, d_anchor_prim,
-                                                   threshold, stride, &ctx->d_fstats->sample, ctx->stream);
-            }
-            if (cudaMemcpyAsync(&ctx->h_fstats[0], ctx->d_fstats, sizeof fs, cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess)
-                return bail(fail(ctx, LOCOHD_ERR_CUDA, "copy of the gather statistics failed"));
-            if ((st = sync_and_check(ctx))) return bail(st);
-            fs = ctx->h_fstats[0];
-        }
-        // Members per environment the kernel is instantiated for: 512, and 1024 once a call has reported larger
-        // environments (the hint stays with the context until a 1024 run sees only small ones again).
-        for (int cap = ctx->fused_cap_hint; cap <= kFusedCapBig; cap *= 2) {
-            const unsigned grid = fused_grid(ctx->kp, &ctx->h_wf0, e->key_is_w ? 1 : 0, keep_indices != 0, cap, n_anchors);
-            // sampled sizes are FP32 upper bounds; even-rounding adds at most one entry per environment, every warp
-            // can leave most of a chunk unused at every refill and at the end
-            const double est = sized_by_bound ? (double)n_anchors * (double)cap
-                                              : (double)fs.sample * (double)stride * 1.03 + 65536.0;
-            const double waste = 1.0 + (double)cap / (double)kFusedChunk;
-            uint64_t capacity = (uint64_t)((est + (double)n_anchors) * waste) + (uint64_t)grid * kFusedWarps * kFusedChunk + 2 * kFusedChunk;
-            // The sample differs a little from call to call (cell order depends on atomics): round the size up to 4
-            // significant bits so that repeated calls ask the block cache for the same size (a fresh multi-GB
-            // cudaMallocAsync costs 0.5-2 s).
-            for (uint64_t step = 1ull << 62; step >= 32; step >>= 1)
-                if (capacity & step) { step >>= 4; capacity = (capacity + step - 1) & ~(step - 1); break; }
-            if (by_history) capacity = ctx->hist_capacity;
-            if ((st = dev_alloc(ctx, &e->d_key, capacity))) return bail(st);
-            if (keep_indices) {
-                if ((st = dev_alloc(ctx, &e->d_idx, capacity)) || (st = dev_alloc(ctx, &e->d_dist, capacity))) return bail(st);
-            }
-            EnvBuild b{};
-            b.n_env = n_anchors; b.order = d_order; b.order_rec = d_order_rec; b.ub = nullptr; b.off = nullptr; b.off_out = e->d_off;
-            b.count = e->d_count;
-            b.key = e->d_key; b.cat = nullptr; b.idx = e->d_idx; b.dist = e->d_dist; b.key_is_w = e->key_is_w ? 1 : 0;
-            b.key_is_sq = 1; b.check_first_zero = 0;
-            cudaMemsetAsync(&ctx->d_fstats->cursor, 0, sizeof(unsigned long long), ctx->stream);
-            cudaMemsetAsync(&ctx->d_fstats->max_count, 0, 2 * sizeof(unsigned int), ctx->stream);
-            {
-                ProfScope ps(ctx, LOCOHD_PROF_FILL);
-                ctx->launches += launch_env_fused(sv, ctx->kp, &ctx->h_wf0, d_anchor_struct, d_anchor_prim, threshold, b, cap,
-                                                  ctx->d_fstats, capacity, grid, ctx->stream);
-            }
-            cudaError_t ce = cudaGetLastError();
-            if (ce != cudaSuccess) return bail(fail(ctx, LOCOHD_ERR_CUDA, "launch failed: %s", cudaGetErrorString(ce)));
-            if (cudaMemcpyAsync(&ctx->h_fstats[1], ctx->d_fstats, sizeof(FusedStats), cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess)
-                return bail(fail(ctx, LOCOHD_ERR_CUDA, "copy of the gather statistics failed"));
-            if ((st = sync_and_check(ctx))) return bail(st);
-            const FusedStats fr = ctx->h_fstats[1];
-            if (!fr.overflow) {
-                // remember the size for the next call of this shape unless it was a tight fit
-                ctx->hist_n_anchors = n_anchors; ctx->hist_threshold = threshold; ctx->hist_cap = cap;
-                ctx->hist_capacity = (!sized_by_bound && (double)fr.cursor <= 0.94 * (double)capacity) ? capacity : 0;
-                if (cap == kFusedCapBig && fr.max_count <= (unsigned)(kFusedCap * 3 / 4)) ctx->fused_cap_hint = kFusedCap;
-                e->capacity = capacity;
-                e->total = fr.cursor < capacity ? fr.cursor : capacity;
-                e->max_count = fr.max_count;
-                release();
-                *out = e;
-                return 0;
-            }
-            dev_free(ctx, e->d_key); dev_free(ctx, e->d_idx); dev_free(ctx, e->d_dist);
-            if (by_history) { ctx->hist_capacity = 0; if (fr.overflow == 8u) ctx->fused_cap_hint = kFusedCapBig; goto resize; }
-            if (fr.overflow != 8u) break;          // not (only) "more members than cap": the larger kernel will not help
-            ctx->fused_cap_hint = kFusedCapBig;     // environments beyond 512 members: go on with the 1024 instantiation
-        }
-        // some environment did not fit the fused kernel: rebuild everything with the exact multi-kernel path
-    }
-    {
-        ProfScope ps(ctx, LOCOHD_PROF_COUNT);
-        ctx->launches += launch_env_count(sv, ctx->kp, n_anchors, d_order, d_anchor_struct, d_anchor_prim, threshold,
-                                          d_ub, ctx->stream);
-    }
-    {
-        ProfScope ps(ctx, LOCOHD_PROF_SCAN);
-        ctx->launches += launch_scan(d_ub, n_anchors, 1, e->d_off, d_scratch, ctx->d_scan + 1, ctx->stream);
-    }
-    ScanStats ss{};
-    if ((st = read_scan_stats(ctx, 1, &ss))) return bail(st);
-    e->capacity = ss.total + 2;
-    e->max_count = ss.max_value;   // upper bound of every environment size
-    if ((st = dev_alloc(ctx, &e->d_key, e->capacity)) || (st = dev_alloc(ctx, &d_cat, e->capacity))) return bail(st);
-    if (keep_indices) {
-        if ((st = dev_alloc(ctx, &e->d_idx, e->capacity)) || (st = dev_alloc(ctx, &e->d_dist, e->capacity))) return bail(st);
-    }
-    EnvBuild b{};
-    b.n_env = n_anchors; b.order = d_order; b.ub = d_ub; b.off = e->d_off; b.count = e->d_count; b.key = e->d_key;
-    b.cat = d_cat; b.idx = e->d_idx; b.dist = e->d_dist; b.key_is_w = e->key_is_w ? 1 : 0; b.key_is_sq = 1; b.check_first_zero = 0;
-    {
-        ProfScope ps(ctx, LOCOHD_PROF_FILL);
-        ctx->launches += launch_env_fill(sv, ctx->kp, d_anchor_struct, d_anchor_prim, threshold, b, ctx->stream);
-    }
-    {
-        ProfScope ps(ctx, LOCOHD_PROF_SORT);
-        ctx->launches += launch_env_sort(ctx->kp, b, e->max_count, threshold, ctx->stream);
-    }
-    cudaError_t ce = cudaGetLastError();
-    if (ce != cudaSuccess) return bail(fail(ctx, LOCOHD_ERR_CUDA, "launch failed: %s", cudaGetErrorString(ce)));
-    e->total = ss.total;  // stored entries (upper bound of the member count; exact sizes are in d_count)
-    release();            // stream-ordered: freed after the kernels above have run
+    { ProfScope ps(ctx, LOCOHD_PROF_OTHER);
+      ctx->launches += launch_anchor_order(sv, ctx->kp, n_anchors, d_anchor_struct, d_anchor_prim, n_prims, d_slot_cnt,
+                                           d_slot_off, d_scratch, ctx->d_scan, d_order, d_order_rec, ctx->stream); }
+    bool built = false;
+    if (!ov.legacy_gather && threshold * threshold < 1.0e30)
+        st = fused_gather(ctx, sv, e, d_anchor_struct, d_anchor_prim, threshold, keep_indices, d_order, d_order_rec, &built);
+    if (!st && !built)
+        st = multi_kernel_gather(ctx, sv, e, d_anchor_struct, d_anchor_prim, threshold, keep_indices, d_order, d_ub, d_scratch, &d_cat);
+    if (st) return bail(st);
+    release();
     *out = e;
     return 0;
 }
