@@ -1781,8 +1781,7 @@ __global__ void __launch_bounds__(kScoreMaxWarps * 32) score_grad_kernel(GradArg
 //  needs ~6 cycles per instruction (fixed-latency and shared-memory dependencies): issue slots 63 % busy instead of
 //  82 %, 12.3 ms against 11.6 ms.)
 constexpr double kSmallH2 = 1e-8;
-constexpr int kSmallH2Hi = 0x3E45798E;   // high word of 1e-8 (0x3E45798E E2308C3A): hi(h2) < this  <=>  h2 < 1e-8 up to the low
-                                         // word (1e-8 - 2^-59 relative) or h2 negative - a signed integer compare, no FP64 constant
+constexpr float kSmallH2f = 1e-8f;   // the same bound, tested on (float)h2 - the seed's input (tile kernel)
 
 // sqrt of a double in [1e-8, ~1]: MUFU.RSQ (f32) seed + one coupled Newton step in FP64, relative error
 // 1.5 * 2^-44 = 8.5e-14.  Used for H itself (nothing amplifies the error; bar 1e-9 on the score); IEEE sqrt costs
@@ -1792,6 +1791,14 @@ __device__ __forceinline__ double sqrt_unit(double v) {
     const double s0 = v * g;
     const double r = fma(-s0, 0.5 * g, 0.5);
     return fma(s0, r, s0);
+}
+
+// 2 sqrt(v) for v in [1e-8, ~1]: the seed and Newton step of sqrt_unit with the factor 1/2 left out,
+// s0 (3 - g s0) = 2 sqrt(v) (1 - 1.5 e^2 + ...) for a seed g of relative error e - the same error bound, one DMUL fewer.
+__device__ __forceinline__ double twice_sqrt_unit(double v) {
+    const double g = (double)rsqrt_approx((float)v);
+    const double s0 = v * g;
+    return s0 * fma(-s0, g, 3.0);
 }
 
 // 1 / sqrt(x) for a positive, normal double: MUFU.RSQ64H seed (rsqrt.approx.f64, 2^-22 relative) and two Newton steps
@@ -2085,8 +2092,12 @@ __global__ void __launch_bounds__(score_fast_max_warps(KEY_IS_W, WEIGHTED) * 32)
 //     1 860 warp instructions of score_fast_kernel) is issued once for four pairs; prefix scans and the reduction
 //     take 3 shuffle steps instead of 5.
 // The arithmetic per event is that of score_fast_kernel<CP, true, false> (same tables, same expanded form, same
-// small-H^2 fallback); a lane's chunk is E / 8 events instead of E / 32 (the host caps E at 1024: <= 128 roundings of
-// R and D per chunk, ~3e-14 relative).  One CTA per SM (tables staged once), teams synchronise on named barriers.
+// small-H^2 fallback, exact 0 for identical counts); a lane's chunk is E / 8 events instead of E / 32 (the host caps
+// E at 1024: <= 128 roundings of R and D per chunk, ~3e-14 relative).  One CTA per SM (tables staged once), teams
+// synchronise on named barriers.  The walk is bound by its instruction count (profiles/r6w, r6x, r7a), so its event is
+// kept short (49 SASS instructions in <8, true>, profiles/r11a_tile_walk.md): count words hold 8 count (the table
+// offset, one add-min per look-up), identical compositions are found from sum |a_r - b_r| inside the small-H^2 branch
+// only, and the walk carries 2 H (twice_sqrt_unit).
 // ncu (profiles/r6b): 1 214 warp instructions and 375 shared-memory wavefronts per pair (1 949 / 523 for one pair per
 // warp); the shared-memory data pipe is 92 % busy and is the wall - 245 of the 375 wavefronts are the four scattered
 // 8-byte reads of the walk (next key 73, ratio table 70, the two sqrt tables 51 each; a half-warp of 14 active lanes
@@ -2151,7 +2162,8 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
     if (team >= teams) return;
     const int C = P.C;
     unsigned char* mine = smem_raw + (size_t)(table_n + 2 * mix_n) * 8 + (size_t)team * team_bytes;
-    uint32_t* cnt = reinterpret_cast<uint32_t*>(mine) + row * CP * 32;            // [CP][32] per warp: A | B << 16
+    uint32_t* cnt = reinterpret_cast<uint32_t*>(mine) + row * CP * 32;   // [CP][32] per warp: 8 A | 8 B << 16 (8 count:
+                                                                         // the byte offset of the count's table entry)
     TileCtrl* ctrl = reinterpret_cast<TileCtrl*>(mine + CP * kTeamThreads * 4);
     uint64_t* stage = reinterpret_cast<uint64_t*>(mine + CP * kTeamThreads * 4 + kTileCtrlBytes);
     const bool loader = row == 0;
@@ -2161,13 +2173,14 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
     const uint32_t dsq_base = __shfl_sync(kFull, smem_u32(s_dsq), lane);
     const uint32_t ratio_base = __shfl_sync(kFull, smem_u32(s_ratio), lane);
     const uint32_t cnt_lane = __shfl_sync(kFull, smem_u32(cnt + lane), lane);
-    // shared-space address of entry e of a count-indexed table: base + 8 e + min(120 e + 8 copy, 120 rep_n); the base is
-    // folded into both arguments of the min, which leaves one IMAD, one min and one shift-add per look-up
+    // shared-space address of entry e of a count-indexed table, from e8 = 8 e (the count words hold 8 count):
+    // base + 8 e + min(120 e + 8 copy, 120 rep_n) = min(16 e8 + base + 8 copy, e8 + base + 120 rep_n) - one shift-add
+    // and one add-min (VIADDMNMX) per look-up
     const uint32_t copy8 = 8u * (lane & 15), cap8 = 120u * (uint32_t)rep_n;
     const uint32_t sq_copy = __shfl_sync(kFull, sq_base + copy8, lane), sq_cap = __shfl_sync(kFull, sq_base + cap8, lane);
     const uint32_t dsq_copy = __shfl_sync(kFull, dsq_base + copy8, lane), dsq_cap = __shfl_sync(kFull, dsq_base + cap8, lane);
-    auto sq_addr = [&](uint32_t e) -> uint32_t { return REP ? 8u * e + min(120u * e + sq_copy, sq_cap) : sq_base + 8u * e; };
-    auto dsq_addr = [&](uint32_t e) -> uint32_t { return REP ? 8u * e + min(120u * e + dsq_copy, dsq_cap) : dsq_base + 8u * e; };
+    auto sq_addr = [&](uint32_t e8) -> uint32_t { return REP ? min(16u * e8 + sq_copy, e8 + sq_cap) : sq_base + e8; };
+    auto dsq_addr = [&](uint32_t e8) -> uint32_t { return REP ? min(16u * e8 + dsq_copy, e8 + dsq_cap) : dsq_base + e8; };
     // warp = row of the tile, 8 lanes per column.  (Measured and dropped, profiles/r6p: warp w scoring the pairs
     // (r, (r + w) mod 4) - a Latin square, equal event totals for the four warps, where ncu shows 19.6 % of the warp time
     // in the team barrier waiting for the row with the largest A_r - 134.9 -> 139.5 ms: the 32 lanes of a row share
@@ -2289,7 +2302,7 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
         if (sub == kTileLanes - 1) { i1 = na; j1 = nb; }
 
         // per-lane histogram of my chunk (8-bit fields: a chunk has at most 128 events), exclusive prefix over the 8
-        // lanes of the pair, anchors added; D and the mismatch count are built from the prefixes while they are in
+        // lanes of the pair, anchors added; D and sum_r |a_r - b_r| are built from the prefixes while they are in
         // registers
         constexpr int HW = CP / 8;
         unsigned long long hA[HW], hB[HW];
@@ -2328,7 +2341,7 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
             }
         }
         if (__any_sync(kFull, unknown)) { raise(P.err, LOCOHD_ERR_UNKNOWN_CATEGORY); continue; }  // pmf.rs:38-42
-        int mism = 0;
+        uint32_t l1 = 0;   // sum_r |a_r - b_r|: 0 <=> identical compositions
         double D = 0.0;
 #pragma unroll
         for (int r = 0; r < CP; ++r) {
@@ -2343,14 +2356,15 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
             uint32_t ex = incl - v;
             if (r == (int)catA0) ex += 1u;          // anchors (locohd.rs:82-84)
             if (r == (int)catB0) ex += 0x10000u;
-            cnt[r * 32 + lane] = ex;
+            cnt[r * 32 + lane] = 8u * ex;   // <= 1024 members a side (tile_geometry): 8 count fits 16 bits
             const uint32_t ka = ex & 0xffffu, kb = ex >> 16;
-            mism += (ka != kb) ? 1 : 0;
-            D = fma(lds_f64(sq_addr(ka)), lds_f64(sq_addr(kb)), D);
+            l1 += ka > kb ? ka - kb : kb - ka;
+            D = fma(lds_f64(sq_addr(8u * ka)), lds_f64(sq_addr(8u * kb)), D);
         }
         const uint32_t totA = i + 1u, totB = j + 1u;   // members of either side before my chunk, anchors included
         double rA = __ldg(P.rsqrt_tbl + totA), rB = __ldg(P.rsqrt_tbl + totB);
-        auto exact_h2 = [&]() -> double {   // difference form from the counts (small H^2 only)
+        // 4 H^2 in the difference form from the counts (small H^2 only)
+        auto exact_4h2 = [&]() -> double {
             double s = 0.0;
 #pragma unroll
             for (int r = 0; r < CP; ++r) {
@@ -2358,27 +2372,37 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
                 const double u = __dmul_rn(lds_f64(sq_addr(word & 0xffffu)), rA) - __dmul_rn(lds_f64(sq_addr(word >> 16)), rB);
                 s = fma(u, u, s);
             }
-            return 0.5 * s;
+            return 2.0 * s;
         };
         uint64_t kprev = key0;
         if (i > 0) kprev = kA[i - 1] & kWMask;
         if (j > 0) kprev = max(kprev, kB[j - 1] & kWMask);
         double wprev = key_value(kprev);
         double R = __dmul_rn(rA, rB);
+        // The walk carries h = 2 H (twice_sqrt_unit saves a multiply per event) and halves the sum at the end: scaling
+        // by 2 is exact, the sum is the one of H itself.
         double h;
         {
             const double h2 = fma(-R, D, 1.0);
-            h = (mism == 0) ? 0.0 : (h2 < kSmallH2 ? sqrt(exact_h2()) : sqrt_unit(h2));
+            h = (l1 == 0) ? 0.0 : (h2 < kSmallH2 ? sqrt(exact_4h2()) : twice_sqrt_unit(h2));
         }
         double acc = 0.0;
         const uint32_t nev = (i1 - i) + (j1 - j);
         uint32_t pa = smem_u32(kA + i), pb = smem_u32(kB + j);
         const uint32_t dA = ratio_base + 8u * totA - pa, dB = ratio_base + 8u * totB - pb;
         uint64_t ra = lds_u64(pa), rb = lds_u64(pb);
+        // Identical compositions: an event moves sum_r |a_r - b_r| by +1 (my count of the category was >= the other
+        // side's) or -1, so after k events the sum is l1 - k + 2 #{events with mine >= other}.  The walk keeps
+        // m = l1 - 1 + 2 #{...} (one predicated add per event) and compares only where H^2 is tiny: there, after the
+        // event taken with `left` events to go (k = nev - left + 1), m + left == nev <=> identical <=> H = 0 exactly.
+        // Identical compositions are frequent in ensembles of near-copies; their h2 is a rounding residue below 1e-8,
+        // so they take the branch of the small-H^2 case instead of a test and a select on every event (6 -> 2
+        // instructions of bookkeeping per event against the count of differing categories).
+        uint32_t m = l1 - 1u;
         // unrolled by 2: no register rotation of the carried key / weight and half the loop overhead, 130.8 -> 126.9 ms
         // on the 200-structure ensemble (profiles/r6x); by 4: 128.7 ms (profiles/r6y)
 #pragma unroll 2
-        for (uint32_t it = 0; it < nev; ++it) {
+        for (uint32_t left = nev; left != 0; --left) {
             const bool takeA = ra <= (rb | kCatMask);   // == (ra & kWMask) <= (rb & kWMask)
             const uint64_t raw = takeA ? ra : rb;
             const double w = key_value(raw);
@@ -2389,11 +2413,9 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
             const uint32_t word = lds_u32_rmw(ca);
             const uint32_t ka = word & 0xffffu, kb = word >> 16;
             const uint32_t mine_k = takeA ? ka : kb, other_k = takeA ? kb : ka;
-            sts_u32_rmw(ca, word + (takeA ? 1u : 0x10000u));
-            {   // the category's counts were equal before (d == 0: one more mismatch) or are equal now (d == -1: one less)
-                const uint32_t t = mine_k - other_k + 1u;
-                if (t < 2u) mism += 2 * (int)t - 1;
-            }
+            sts_u32_rmw(ca, word + (takeA ? 8u : 0x80000u));
+            // a predicated add in place (left to itself, ptxas adds into a new register and selects: two instructions)
+            asm("{\n\t.reg .pred p;\n\tsetp.ge.u32 p, %1, %2;\n\t@p add.u32 %0, %0, 2;\n\t}" : "+r"(m) : "r"(mine_k), "r"(other_k));
             const uint32_t pk = takeA ? pa : pb;
             D = fma(lds_f64(dsq_addr(mine_k)), lds_f64(sq_addr(other_k)), D);
             R *= lds_f64(pk + (takeA ? dA : dB));
@@ -2403,17 +2425,21 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
             ra = takeA ? nxt : ra;
             rb = takeA ? rb : nxt;
             const double h2 = fma(-R, D, 1.0);
-            h = (mism == 0) ? 0.0 : sqrt_unit(h2);       // identical counts: exactly 0
-            if (mism != 0 && __double2hiint(h2) < kSmallH2Hi) {   // h2 < 1e-8 (or negative): rare, difference form from the counts
-                rA = __ldg(P.rsqrt_tbl + ((pa + dA - ratio_base) >> 3));
-                rB = __ldg(P.rsqrt_tbl + ((pb + dB - ratio_base) >> 3));
-                h = sqrt(exact_h2());
+            h = twice_sqrt_unit(h2);
+            if ((float)h2 < kSmallH2f) {   // h2 < 1e-8 (or negative): identical counts (exactly 0) or rare (difference form)
+                if (m + left == nev) {
+                    h = 0.0;
+                } else {
+                    rA = __ldg(P.rsqrt_tbl + ((pa + dA - ratio_base) >> 3));
+                    rB = __ldg(P.rsqrt_tbl + ((pb + dB - ratio_base) >> 3));
+                    h = sqrt(exact_4h2());
+                }
             }
         }
         if (sub == kTileLanes - 1) acc = fma(wf.w_inf - wprev, h, acc);   // tail to infinity: the last chunk's state is final
 #pragma unroll
         for (int o = kTileLanes / 2; o; o >>= 1) acc += __shfl_xor_sync(kFull, acc, o * lstep);
-        if (sub == 0 && valid) a.out[out_first + p] = acc;
+        if (sub == 0 && valid) a.out[out_first + p] = 0.5 * acc;
     }
 }
 
