@@ -275,6 +275,31 @@ int locohd_from_primitives_grad(locohd_ctx* ctx, uint64_t n_a, const double* xyz
                                 const uint32_t* tag_b, uint64_t n_pairs, const uint32_t* anchors,
                                 const uint32_t* wf_idx, double threshold, const double* pair_weights,
                                 double* out_scores, double* out_grad_a, double* out_grad_b);
+/* from_dmxs (ragged rows, as locohd_envset_from_ragged_rows, per side) with the gradient of the scores with respect to
+ * every entry: out_grad_s has row_offsets_s[n_rows] entries in the layout of values_s (an extension: the reference has
+ * none).  Row r of A is scored against row r of B; entry (r, c) of side s receives g_r dS_r/d values_s[r][c],
+ * g_r = pair_weights[r] (NULL: all 1).  Each row is sorted stably; its first entry is the anchor (distance 0) and
+ * the others are events in merged order (distance, then A before B, then store order); an event's entry receives
+ * g_r w(t) (H_{k-1} - H_k), w = dW/dt.  The anchor's entry, entries at t = 0 and non-finite entries (+inf bans) get
+ * exactly 0; where distances tie the result is the one-sided derivative in that order.  Every entry is written by
+ * one plain store, so scores and gradients are deterministic.  Validation and errors are those of from_dmxs
+ * (locohd_envset_from_ragged_rows per side, the weight-function indices of locohd_score_jobs).  out_scores [n_rows]
+ * may be NULL; any argument may be host or device memory. */
+int locohd_from_rows_grad(locohd_ctx* ctx, uint64_t n_rows,
+                          const uint64_t* row_offsets_a, const double* values_a, const uint16_t* category_a, uint64_t n_categories_a,
+                          const uint64_t* row_offsets_b, const double* values_b, const uint16_t* category_b, uint64_t n_categories_b,
+                          const uint32_t* wf_idx, const double* pair_weights,
+                          double* out_scores, double* out_grad_a, double* out_grad_b);
+/* from_coords with coordinate gradients: out_grad_s is [n_points][3], overwritten with sum_r g_r dS_r/dxyz_s.  The
+ * entry gradients G_s[i][j] of locohd_from_rows_grad on the Euclidean rows t_ij = |x_j - x_i| give
+ * grad_i = sum_j (G_s[i][j] + G_s[j][i]) (x_i - x_j) / t_ij, summed in a fixed order: deterministic.  Every point is in
+ * every environment, so no member crosses a cutoff and the score is continuous in the coordinates (kinks: ties and
+ * the weight function's own).  Memory: besides the 20 n^2 bytes per side of the row environments that from_coords
+ * builds, 8 n^2 bytes per side of scratch for G.  Validation and errors are those of locohd_envset_from_coords; any
+ * argument may be host or device memory. */
+int locohd_from_coords_grad(locohd_ctx* ctx, uint64_t n_points, const double* xyz_a, const uint16_t* cat_a,
+                            const double* xyz_b, const uint16_t* cat_b, const uint32_t* wf_idx,
+                            const double* pair_weights, double* out_scores, double* out_grad_a, double* out_grad_b);
 
 /* ---- leaf math on the device (parity checks of the FP64 device functions) --------------- */
 /* WeightFunction::integral_point over n points (weight_function.rs:95-116). */

@@ -33,8 +33,8 @@ EXPORTED_SYMBOLS = [
     "locohd_envset_from_coords", "locohd_envset_destroy", "locohd_envset_size", "locohd_envset_total_members",
     "locohd_envset_dump", "locohd_score_pairs", "locohd_score_jobs", "locohd_score_jobs_stats",
     "locohd_score_anchor_lists", "locohd_plan_job_tiles", "locohd_tile_unit", "locohd_tile_geometry",
-    "locohd_from_primitives", "locohd_from_primitives_grad", "locohd_wf_integral_points", "locohd_wf_density_points",
-    "locohd_sd_run",
+    "locohd_from_primitives", "locohd_from_primitives_grad", "locohd_from_rows_grad", "locohd_from_coords_grad",
+    "locohd_wf_integral_points", "locohd_wf_density_points", "locohd_sd_run",
 ]
 
 
@@ -130,6 +130,8 @@ def load_library() -> C.CDLL:
         "locohd_from_primitives": (C.c_int, [vp, u64, vp, vp, vp, u64, vp, vp, vp, u64, vp, vp, dbl, vp]),
         "locohd_from_primitives_grad": (C.c_int, [vp, u64, vp, vp, vp, u64, vp, vp, vp, u64, vp, vp, dbl, vp, vp, vp,
                                                   vp]),
+        "locohd_from_rows_grad": (C.c_int, [vp, u64, vp, vp, vp, u64, vp, vp, vp, u64, vp, vp, vp, vp, vp]),
+        "locohd_from_coords_grad": (C.c_int, [vp, u64, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
         "locohd_wf_integral_points": (C.c_int, [vp, C.POINTER(WeightFunctionC), u64, vp, vp]),
         "locohd_wf_density_points": (C.c_int, [vp, C.POINTER(WeightFunctionC), u64, vp, vp]),
         "locohd_sd_run": (C.c_int, [vp, i32, vp, i32, u64, vp, vp, vp]),
@@ -458,6 +460,61 @@ class Context:
         self._check(self.lib.locohd_from_primitives_grad(self.h, na, _p(xyz_a), _p(cat_a), _p(tag_a), nb, _p(xyz_b),
                                                          _p(cat_b), _p(tag_b), P, _p(anchors), _p(wf_idx),
                                                          float(threshold), _p(pair_weights), _p(res), _p(ga), _p(gb)))
+        return res, ga, gb
+
+    def from_rows_grad(self, rows_a, cat_a, rows_b, cat_b, wf_idx=None, pair_weights=None, out=None, grad_a=None,
+                       grad_b=None, offsets_a=None, offsets_b=None, n_rows=None):
+        """from_dmxs scores with the gradient of row r's score with respect to every entry of row r of either side:
+        returns (scores [n_rows], grad_a, grad_b), grad = pair_weights[r] dS_r / d entry (pair_weights None: all 1).
+        rows_s is a 2-D array (grads come back [n_rows, row_len]) or a list of 1-D rows (grads come back as a list of
+        1-D arrays).  With offsets_s given, rows_s is the flat values (numpy or a raw device pointer) of ragged rows
+        at those offsets and grad_s comes back flat in the same layout.  wf_idx, pair_weights, out, grad_a and grad_b
+        may be raw device pointers."""
+        def flat(rows, offsets):
+            if offsets is not None:
+                offsets = _arr(offsets, np.uint64)
+                return _arr(rows, np.float64), offsets, lambda g: g
+            if not isinstance(rows, np.ndarray):
+                try:
+                    rows = np.asarray(rows, dtype=np.float64)
+                except ValueError:   # ragged
+                    rows = [np.ascontiguousarray(r, dtype=np.float64).ravel() for r in rows]
+                    offs = np.cumsum([0] + [len(r) for r in rows]).astype(np.uint64)
+                    vals = np.concatenate(rows) if rows else np.zeros(0)
+                    return vals, offs, lambda g: np.split(g, offs[1:-1]) if len(rows) else []
+            rows = np.ascontiguousarray(rows, dtype=np.float64)
+            if rows.ndim != 2:
+                rows = rows.reshape(len(rows), -1)
+            offs = (np.arange(rows.shape[0] + 1) * rows.shape[1]).astype(np.uint64)
+            return rows.ravel(), offs, lambda g: g.reshape(rows.shape)
+
+        va, oa, shape_a = flat(rows_a, offsets_a)
+        vb, ob, shape_b = flat(rows_b, offsets_b)
+        n = int(n_rows) if n_rows is not None else len(oa) - 1
+        cat_a, cat_b = _arr(cat_a, np.uint16), _arr(cat_b, np.uint16)
+        wf_idx, pair_weights = _arr(wf_idx, np.uint32), _arr(pair_weights, np.float64)
+        res = np.empty(n, np.float64) if out is None else out
+        ga = np.empty(int(oa[n]), np.float64) if grad_a is None else grad_a
+        gb = np.empty(int(ob[n]), np.float64) if grad_b is None else grad_b
+        self._check(self.lib.locohd_from_rows_grad(self.h, n, _p(oa), _p(va), _p(cat_a), len(cat_a), _p(ob), _p(vb),
+                                                   _p(cat_b), len(cat_b), _p(wf_idx), _p(pair_weights), _p(res),
+                                                   _p(ga), _p(gb)))
+        return (res, shape_a(ga) if grad_a is None else ga, shape_b(gb) if grad_b is None else gb)
+
+    def from_coords_grad(self, xyz_a, cat_a, xyz_b, cat_b, wf_idx=None, pair_weights=None, out=None, grad_a=None,
+                         grad_b=None, n_points=None):
+        """from_coords scores and their coordinate gradients: (scores [n], grad_a [n, 3], grad_b [n, 3]) with
+        grad = sum_r pair_weights[r] dS_r/dxyz (pair_weights None: all 1).  Every array may be a numpy array or a
+        raw device pointer (then n_points is needed)."""
+        xyz_a, xyz_b = _arr(xyz_a, np.float64), _arr(xyz_b, np.float64)
+        cat_a, cat_b = _arr(cat_a, np.uint16), _arr(cat_b, np.uint16)
+        wf_idx, pair_weights = _arr(wf_idx, np.uint32), _arr(pair_weights, np.float64)
+        n = int(n_points) if n_points is not None else len(xyz_a.reshape(-1, 3))
+        res = np.empty(n, np.float64) if out is None else out
+        ga = np.empty((n, 3), np.float64) if grad_a is None else grad_a
+        gb = np.empty((n, 3), np.float64) if grad_b is None else grad_b
+        self._check(self.lib.locohd_from_coords_grad(self.h, n, _p(xyz_a), _p(cat_a), _p(xyz_b), _p(cat_b),
+                                                     _p(wf_idx), _p(pair_weights), _p(res), _p(ga), _p(gb)))
         return res, ga, gb
 
     # ---- leaf math --------------------------------------------------------------------------------

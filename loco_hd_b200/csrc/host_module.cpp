@@ -553,6 +553,8 @@ struct LoCoHD {
     struct Rows {
         std::vector<uint64_t> off{0};
         std::vector<double> val;
+        size_t cols = 0;      // row length of rectangular input (a 2-D array or equally long nested lists)
+        bool rect = false;
         size_t n() const { return off.size() - 1; }
         size_t max_len() const {
             size_t m = 0;
@@ -567,6 +569,8 @@ struct LoCoHD {
             const size_t nr = a.shape(0), nc = a.shape(1);
             rows.val.assign(a.data(), a.data() + nr * nc);
             for (size_t r = 0; r < nr; ++r) rows.off.push_back((r + 1) * nc);
+            rows.rect = true;
+            rows.cols = nc;
             return rows;
         }
         PyErr_Clear();
@@ -584,39 +588,110 @@ struct LoCoHD {
         return rows;
     }
 
-    std::vector<double> from_dmxs(const py::object& seq_a, const py::object& seq_b, const py::object& dmx_a,
-                                  const py::object& dmx_b, const std::optional<std::vector<std::string>>& keys) {
-        auto sa = cat_ids(to_strings(seq_a, "seq_a")), sb = cat_ids(to_strings(seq_b, "seq_b"));
-        const Rows ma = to_rows(dmx_a, "dmx_a"), mb = to_rows(dmx_b, "dmx_b");
-        const size_t rows_a = ma.n(), rows_b = mb.n();
+    // The arguments of from_dmxs / from_dmxs_grad, converted and checked as the reference does.
+    struct DmxCall {
+        std::vector<uint16_t> sa, sb;
+        Rows ma, mb;
+        std::vector<uint32_t> wf;
+        size_t n_rows() const { return ma.n(); }
+    };
+    DmxCall dmx_call(const py::object& seq_a, const py::object& seq_b, const py::object& dmx_a, const py::object& dmx_b,
+                     const std::optional<std::vector<std::string>>& keys) const {
+        DmxCall a;
+        a.sa = cat_ids(to_strings(seq_a, "seq_a"));
+        a.sb = cat_ids(to_strings(seq_b, "seq_b"));
+        a.ma = to_rows(dmx_a, "dmx_a");
+        a.mb = to_rows(dmx_b, "dmx_b");
+        const size_t rows_a = a.ma.n(), rows_b = a.mb.n();
         if (rows_a != rows_b)  // locohd.rs:420-428
             throw py::value_error("Expected matrices with the same length, got lengths " + std::to_string(rows_a) + " and " +
                                   std::to_string(rows_b) + "!");
-        const auto wf = resolve_keys(keys, rows_a);
-        if (rows_a == 0) return {};
+        a.wf = resolve_keys(keys, rows_a);
+        if (rows_a == 0) return a;
         // sort_together indexes seq by the row's indices (utils.rs:33-36): a short seq panics upstream, a long one is cut
-        if (sa.size() < ma.max_len() || sb.size() < mb.max_len())
+        if (a.sa.size() < a.ma.max_len() || a.sb.size() < a.mb.max_len())
             throw py::value_error("The category sequences are shorter than the distance matrix rows!");
-        for (const Rows* m : {&ma, &mb})
+        for (const Rows* m : {&a.ma, &a.mb})
             for (size_t r = 0; r < m->n(); ++r)
                 if (m->off[r + 1] == m->off[r]) throw py::value_error("Empty distance matrix rows!");
+        return a;
+    }
+
+    std::vector<double> from_dmxs(const py::object& seq_a, const py::object& seq_b, const py::object& dmx_a,
+                                  const py::object& dmx_b, const std::optional<std::vector<std::string>>& keys) {
+        const DmxCall a = dmx_call(seq_a, seq_b, dmx_a, dmx_b, keys);
+        if (a.n_rows() == 0) return {};
         const auto d = ensure_ctx();
         auto build = [&](locohd_ctx* c, const Rows& m, const std::vector<uint16_t>& cats, locohd_envset** e) {
             return locohd_envset_from_ragged_rows(c, m.n(), m.off.data(), m.val.data(), cats.data(), cats.size(), e);
         };
-        return score_rows(d, rows_a, wf, [&](locohd_ctx* c, locohd_envset** ea, locohd_envset** eb) {
-            int st = build(c, ma, sa, ea);
-            if (!st) st = build(c, mb, sb, eb);
+        return score_rows(d, a.n_rows(), a.wf, [&](locohd_ctx* c, locohd_envset** ea, locohd_envset** eb) {
+            int st = build(c, a.ma, a.sa, ea);
+            if (!st) st = build(c, a.mb, a.sb, eb);
             return st;
         });
     }
 
+    static const double* weights_of(const py::object& pair_weights, size_t n, F64Array& keep) {
+        if (pair_weights.is_none()) return nullptr;
+        keep = pair_weights.cast<F64Array>();
+        if ((size_t)keep.size() != n) throw py::value_error("pair_weights must have one entry per row");
+        return keep.data();
+    }
+
+    // from_dmxs with the gradients of the scores with respect to every matrix entry: (scores, grad_dmx_a, grad_dmx_b),
+    // grad = pair_weights[r] dS_r / d dmx[r][c] (pair_weights None: all 1); [n_rows, row_len] arrays for rectangular
+    // input, lists of 1-D arrays for ragged rows
+    py::tuple from_dmxs_grad(const py::object& seq_a, const py::object& seq_b, const py::object& dmx_a,
+                             const py::object& dmx_b, const std::optional<std::vector<std::string>>& keys,
+                             const py::object& pair_weights) {
+        const DmxCall a = dmx_call(seq_a, seq_b, dmx_a, dmx_b, keys);
+        const size_t n = a.n_rows();
+        F64Array pw;
+        const double* w = weights_of(pair_weights, n, pw);
+        py::array_t<double> out(n);
+        std::vector<double> ga(a.ma.val.size()), gb(a.mb.val.size());
+        if (n) {
+            const auto d = ensure_ctx();
+            double* o = out.mutable_data();
+            device_call(d, [&](locohd_ctx* c) {
+                return locohd_from_rows_grad(c, n, a.ma.off.data(), a.ma.val.data(), a.sa.data(), a.sa.size(),
+                                             a.mb.off.data(), a.mb.val.data(), a.sb.data(), a.sb.size(),
+                                             a.wf.empty() ? nullptr : a.wf.data(), w, o, ga.data(), gb.data());
+            });
+        }
+        auto shape = [](const Rows& m, const std::vector<double>& g) -> py::object {
+            if (m.rect) {
+                py::array_t<double> r({(py::ssize_t)m.n(), (py::ssize_t)m.cols});
+                std::copy(g.begin(), g.end(), r.mutable_data());
+                return r;
+            }
+            py::list l;
+            for (size_t r = 0; r < m.n(); ++r) {
+                py::array_t<double> row((py::ssize_t)(m.off[r + 1] - m.off[r]));
+                std::copy(g.begin() + m.off[r], g.begin() + m.off[r + 1], row.mutable_data());
+                l.append(row);
+            }
+            return l;
+        };
+        return py::make_tuple(out, shape(a.ma, ga), shape(a.mb, gb));
+    }
+
     // ---- from_coords (locohd.rs:463-476)
-    std::vector<double> from_coords(const py::object& seq_a, const py::object& seq_b, const py::object& coords_a,
-                                    const py::object& coords_b, const std::optional<std::vector<std::string>>& keys) {
-        auto sa = cat_ids(to_strings(seq_a, "seq_a")), sb = cat_ids(to_strings(seq_b, "seq_b"));
+    // The arguments of from_coords / from_coords_grad, converted and checked as the reference does.
+    struct CoordsCall {
+        std::vector<uint16_t> sa, sb;
+        F64Array xa, xb;
+        size_t n = 0;
+        std::vector<uint32_t> wf;
+    };
+    CoordsCall coords_call(const py::object& seq_a, const py::object& seq_b, const py::object& coords_a,
+                           const py::object& coords_b, const std::optional<std::vector<std::string>>& keys) const {
+        CoordsCall a;
+        a.sa = cat_ids(to_strings(seq_a, "seq_a"));
+        a.sb = cat_ids(to_strings(seq_b, "seq_b"));
         auto to_xyz = [](const py::object& m, const char* what) {
-            auto a = py::array_t<double, py::array::c_style | py::array::forcecast>::ensure(m);
+            auto a = F64Array::ensure(m);
             if (!a) { PyErr_Clear(); throw py::type_error(std::string(what) + " must be a sequence of 3-vectors"); }
             if (a.ndim() == 1 && a.shape(0) == 0) return std::make_pair(a, (size_t)0);
             if (a.ndim() != 2 || a.shape(1) != 3) throw py::type_error(std::string(what) + " must be a sequence of 3-vectors");
@@ -626,17 +701,46 @@ struct LoCoHD {
         auto [xb, nb] = to_xyz(coords_b, "coords_b");
         if (na != nb)
             throw py::value_error("Expected matrices with the same length, got lengths " + std::to_string(na) + " and " + std::to_string(nb) + "!");
-        const auto wf = resolve_keys(keys, na);
-        if (na == 0) return {};
-        if (sa.size() < na || sb.size() < nb) throw py::value_error("The category sequences are shorter than the coordinate lists!");
+        a.wf = resolve_keys(keys, na);
+        a.xa = xa; a.xb = xb; a.n = na;
+        if (na == 0) return a;
+        if (a.sa.size() < na || a.sb.size() < nb) throw py::value_error("The category sequences are shorter than the coordinate lists!");
+        return a;
+    }
+
+    std::vector<double> from_coords(const py::object& seq_a, const py::object& seq_b, const py::object& coords_a,
+                                    const py::object& coords_b, const std::optional<std::vector<std::string>>& keys) {
+        const CoordsCall a = coords_call(seq_a, seq_b, coords_a, coords_b, keys);
+        if (a.n == 0) return {};
         const auto d = ensure_ctx();
-        const size_t n_pts = na;
-        const double *pa = xa.data(), *pb = xb.data();
-        return score_rows(d, n_pts, wf, [&](locohd_ctx* c, locohd_envset** ea, locohd_envset** eb) {
-            int st = locohd_envset_from_coords(c, n_pts, pa, sa.data(), ea);
-            if (!st) st = locohd_envset_from_coords(c, n_pts, pb, sb.data(), eb);
+        const size_t n_pts = a.n;
+        const double *pa = a.xa.data(), *pb = a.xb.data();
+        return score_rows(d, n_pts, a.wf, [&](locohd_ctx* c, locohd_envset** ea, locohd_envset** eb) {
+            int st = locohd_envset_from_coords(c, n_pts, pa, a.sa.data(), ea);
+            if (!st) st = locohd_envset_from_coords(c, n_pts, pb, a.sb.data(), eb);
             return st;
         });
+    }
+
+    // from_coords with the coordinate gradients of the scores: (scores [n], grad_a [n, 3], grad_b [n, 3]),
+    // grad = sum_r pair_weights[r] dS_r/dxyz (pair_weights None: all 1)
+    py::tuple from_coords_grad(const py::object& seq_a, const py::object& seq_b, const py::object& coords_a,
+                               const py::object& coords_b, const std::optional<std::vector<std::string>>& keys,
+                               const py::object& pair_weights) {
+        const CoordsCall a = coords_call(seq_a, seq_b, coords_a, coords_b, keys);
+        const size_t n = a.n;
+        F64Array pw;
+        const double* w = weights_of(pair_weights, n, pw);
+        py::array_t<double> out(n), ga({(py::ssize_t)n, (py::ssize_t)3}), gb({(py::ssize_t)n, (py::ssize_t)3});
+        if (n) {
+            const auto d = ensure_ctx();
+            double *o = out.mutable_data(), *pga = ga.mutable_data(), *pgb = gb.mutable_data();
+            device_call(d, [&](locohd_ctx* c) {
+                return locohd_from_coords_grad(c, n, a.xa.data(), a.sa.data(), a.xb.data(), a.sb.data(),
+                                               a.wf.empty() ? nullptr : a.wf.data(), w, o, pga, pgb);
+            });
+        }
+        return py::make_tuple(out, ga, gb);
     }
 
     // ---- from_primitives (locohd.rs:479-567)
@@ -1006,6 +1110,12 @@ PYBIND11_MODULE(loco_hd, m) {
              py::arg("w_func_keys") = py::none())
         .def("from_coords", &LoCoHD::from_coords, py::arg("seq_a"), py::arg("seq_b"), py::arg("coords_a"),
              py::arg("coords_b"), py::arg("w_func_keys") = py::none())
+        .def("from_dmxs_grad", &LoCoHD::from_dmxs_grad, py::arg("seq_a"), py::arg("seq_b"), py::arg("dmx_a"),
+             py::arg("dmx_b"), py::arg("w_func_keys") = py::none(), py::arg("pair_weights") = py::none(),
+             "from_dmxs with the gradients of the scores with respect to every matrix entry (an extension)")
+        .def("from_coords_grad", &LoCoHD::from_coords_grad, py::arg("seq_a"), py::arg("seq_b"), py::arg("coords_a"),
+             py::arg("coords_b"), py::arg("w_func_keys") = py::none(), py::arg("pair_weights") = py::none(),
+             "from_coords with the coordinate gradients of the scores (an extension)")
         .def("from_primitives", &LoCoHD::from_primitives, py::arg("prim_a"), py::arg("prim_b"), py::arg("anchor_pairs"),
              py::arg("threshold_distance"))
         .def("from_arrays", &LoCoHD::from_arrays, py::arg("xyz_a"), py::arg("cat_a"), py::arg("tag_a"), py::arg("xyz_b"),

@@ -1260,16 +1260,16 @@ int locohd_envset_from_coords(locohd_ctx* ctx, uint64_t n_points, const double* 
     API_END()
 }
 
-int locohd_envset_from_ragged_rows(locohd_ctx* ctx, uint64_t n_rows, const uint64_t* row_offsets, const double* values,
-                                   const uint16_t* category, uint64_t n_categories_given, locohd_envset** out) {
-    API_BEGIN(ctx)
-    TRY_ST(need_params(ctx));
-    if (!out || !row_offsets) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
-    *out = nullptr;
-    std::vector<uint64_t> in_off(n_rows + 1);
+// Host checks of ragged rows (locohd_envset_from_ragged_rows, locohd_from_rows_grad): copies the offsets (host or
+// device memory) to in_off and sets *max_len to the longest row.
+static int ragged_rows_check(locohd_ctx* ctx, uint64_t n_rows, const uint64_t* row_offsets, const double* values,
+                             const uint16_t* category, uint64_t n_categories_given, std::vector<uint64_t>& in_off,
+                             uint64_t* max_len) {
+    if (!row_offsets) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
+    in_off.assign(n_rows + 1, 0);
     if (is_device_ptr(ctx, row_offsets)) CU(ctx, cudaMemcpy(in_off.data(), row_offsets, in_off.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost));
     else std::memcpy(in_off.data(), row_offsets, in_off.size() * sizeof(uint64_t));
-    uint64_t max_len = 0;
+    *max_len = 0;
     for (uint64_t r = 0; r < n_rows; ++r) {
         if (in_off[r + 1] < in_off[r]) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "row_offsets must be non-decreasing");
         const uint64_t len = in_off[r + 1] - in_off[r];
@@ -1278,9 +1278,21 @@ int locohd_envset_from_ragged_rows(locohd_ctx* ctx, uint64_t n_rows, const uint6
         if (len > n_categories_given)   // sort_together indexes the categories by the row's indices (utils.rs:33-36)
             return fail(ctx, LOCOHD_ERR_LEN_MISMATCH, "row %llu has %llu distances but only %llu categories were given",
                         (unsigned long long)r, (unsigned long long)len, (unsigned long long)n_categories_given);
-        max_len = std::max(max_len, len);
+        *max_len = std::max(*max_len, len);
     }
     if (in_off[n_rows] && (!values || !category)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
+    return 0;
+}
+
+int locohd_envset_from_ragged_rows(locohd_ctx* ctx, uint64_t n_rows, const uint64_t* row_offsets, const double* values,
+                                   const uint16_t* category, uint64_t n_categories_given, locohd_envset** out) {
+    API_BEGIN(ctx)
+    TRY_ST(need_params(ctx));
+    if (!out) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
+    *out = nullptr;
+    std::vector<uint64_t> in_off;
+    uint64_t max_len = 0;
+    TRY_ST(ragged_rows_check(ctx, n_rows, row_offsets, values, category, n_categories_given, in_off, &max_len));
     return rows_envset(ctx, n_rows, in_off.data(), max_len, values, nullptr, category, out);
     API_END()
 }
@@ -1685,8 +1697,8 @@ int locohd_from_primitives_grad(locohd_ctx* ctx, uint64_t n_a, const double* xyz
             st = out_scores ? out.prepare(ctx, out_scores, n_pairs) : dev_alloc(ctx, &d_scores, n_pairs);
         if (!st) {
             GradArgs g{};
-            g.env = pc.env->view();
-            g.dist = pc.env->d_dist; g.idx = pc.env->d_idx;
+            for (int side = 0; side < 2; ++side)
+                g.side[side] = {pc.env->view(), pc.env->d_dist, pc.env->d_idx, side ? n_pairs : 0};
             g.xyz = pc.s->d_xyz; g.prim_off = pc.s->d_prim_off; g.n_structs = 2;
             g.anchor_struct = reinterpret_cast<const uint32_t*>(pc.at(pc.o_as));
             g.anchor_prim = reinterpret_cast<const uint32_t*>(pc.at(pc.o_ap));
@@ -1696,7 +1708,7 @@ int locohd_from_primitives_grad(locohd_ctx* ctx, uint64_t n_a, const double* xyz
             g.out = out_scores ? out.ptr : d_scores;
             g.grad[0] = ga.ptr; g.grad[1] = gb.ptr;
             int nl;
-            { ProfScope ps(ctx, LOCOHD_PROF_SCORE); nl = launch_score_grad(g, ctx->kp, ctx->stream); }
+            { ProfScope ps(ctx, LOCOHD_PROF_SCORE); nl = launch_score_grad(g, ctx->kp, GradTarget::kCoords, ctx->stream); }
             if (nl < 0) st = fail(ctx, LOCOHD_ERR_UNSUPPORTED, "shared memory budget exceeded for %d categories", ctx->kp.C);
             else ctx->launches += nl;
             if (!st && cudaPeekAtLastError() != cudaSuccess)
@@ -1709,6 +1721,134 @@ int locohd_from_primitives_grad(locohd_ctx* ctx, uint64_t n_a, const double* xyz
     if (!st) st = gb.commit();
     const int st2 = sync_and_check(ctx);
     return st ? st : st2;
+    API_END()
+}
+
+// --------------------------------------------------------------------- gradients of from_dmxs / from_coords
+// The two row sets of one gradient call, released with it (stream-ordered).
+struct RowSets {
+    locohd_envset* e[2] = {nullptr, nullptr};
+    ~RowSets() { destroy_envset(e[0]); destroy_envset(e[1]); }
+};
+
+// Scores of the row pairs p of two row sets and g_p dS_p/dt of every entry (score_grad_kernel<kEntries>): entry c of row
+// p of side s goes to d_grad[s][d_entry_off[s][p] + c].  wf_idx, pair_weights and out_scores may be host or device
+// memory; the caller synchronises.
+static int rows_grad(locohd_ctx* ctx, const RowSets& rs, uint64_t n_rows, const uint32_t* wf_idx,
+                     const double* pair_weights, double* out_scores, const uint64_t* const d_entry_off[2],
+                     double* const d_grad[2]) {
+    InBuf<uint32_t> wf;
+    InBuf<double> pw;
+    OutBuf<double> out;
+    double* d_scores = nullptr;   // scores are always computed; a caller without `out_scores` gets them dropped
+    int st = wf.load(ctx, wf_idx, n_rows);
+    if (!st) st = pw.load(ctx, pair_weights, n_rows);
+    if (!st) st = out_scores ? out.prepare(ctx, out_scores, n_rows) : dev_alloc(ctx, &d_scores, n_rows);
+    if (!st) {
+        GradArgs g{};
+        for (int side = 0; side < 2; ++side) {
+            g.side[side] = {rs.e[side]->view(), rs.e[side]->d_dist, rs.e[side]->d_idx, 0};
+            g.entry_off[side] = d_entry_off[side];
+            g.entry_grad[side] = d_grad[side];
+        }
+        g.n_pairs = n_rows;
+        g.wf_idx = wf.ptr;
+        g.pair_weights = pw.ptr;
+        g.out = out_scores ? out.ptr : d_scores;
+        int nl;
+        { ProfScope ps(ctx, LOCOHD_PROF_SCORE); nl = launch_score_grad(g, ctx->kp, GradTarget::kEntries, ctx->stream); }
+        if (nl < 0) st = fail(ctx, LOCOHD_ERR_UNSUPPORTED, "shared memory budget exceeded for %d categories", ctx->kp.C);
+        else ctx->launches += nl;
+        if (!st && cudaPeekAtLastError() != cudaSuccess)
+            st = fail(ctx, LOCOHD_ERR_CUDA, "launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    }
+    if (!st) st = out.commit();
+    dev_free(ctx, d_scores);
+    return st;
+}
+
+int locohd_from_rows_grad(locohd_ctx* ctx, uint64_t n_rows,
+                          const uint64_t* row_offsets_a, const double* values_a, const uint16_t* category_a,
+                          uint64_t n_categories_a,
+                          const uint64_t* row_offsets_b, const double* values_b, const uint16_t* category_b,
+                          uint64_t n_categories_b,
+                          const uint32_t* wf_idx, const double* pair_weights,
+                          double* out_scores, double* out_grad_a, double* out_grad_b) {
+    API_BEGIN(ctx)
+    TRY_ST(need_params(ctx));
+    const uint64_t* offsets[2] = {row_offsets_a, row_offsets_b};
+    const double* values[2] = {values_a, values_b};
+    const uint16_t* cats[2] = {category_a, category_b};
+    const uint64_t n_cats[2] = {n_categories_a, n_categories_b};
+    double* grads[2] = {out_grad_a, out_grad_b};
+    std::vector<uint64_t> in_off[2];
+    uint64_t max_len[2];
+    for (int s = 0; s < 2; ++s) {
+        TRY_ST(ragged_rows_check(ctx, n_rows, offsets[s], values[s], cats[s], n_cats[s], in_off[s], &max_len[s]));
+        if (in_off[s][n_rows] && !grads[s]) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null gradient array");
+    }
+    TRY_ST(check_wf_indices(ctx, wf_idx, n_rows));
+    if (n_rows == 0) return 0;
+    RowSets rs;
+    InBuf<uint64_t> d_off[2];
+    OutBuf<double> g[2];
+    for (int s = 0; s < 2; ++s) {
+        TRY_ST(rows_envset(ctx, n_rows, in_off[s].data(), max_len[s], values[s], nullptr, cats[s], &rs.e[s]));
+        TRY_ST(d_off[s].load(ctx, in_off[s].data(), n_rows));
+        TRY_ST(g[s].prepare(ctx, grads[s], in_off[s][n_rows]));
+    }
+    const uint64_t* entry_off[2] = {d_off[0].ptr, d_off[1].ptr};
+    double* entry_grad[2] = {g[0].ptr, g[1].ptr};
+    int st = rows_grad(ctx, rs, n_rows, wf_idx, pair_weights, out_scores, entry_off, entry_grad);
+    if (!st) st = g[0].commit();
+    if (!st) st = g[1].commit();
+    const int st2 = sync_and_check(ctx);   // also keeps in_off alive until its copies are done
+    return st ? st : st2;
+    API_END()
+}
+
+int locohd_from_coords_grad(locohd_ctx* ctx, uint64_t n_points, const double* xyz_a, const uint16_t* cat_a,
+                            const double* xyz_b, const uint16_t* cat_b, const uint32_t* wf_idx,
+                            const double* pair_weights, double* out_scores, double* out_grad_a, double* out_grad_b) {
+    API_BEGIN(ctx)
+    TRY_ST(need_params(ctx));
+    if (n_points && (!xyz_a || !xyz_b)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null coordinates");
+    if (n_points && (!out_grad_a || !out_grad_b)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null gradient array");
+    TRY_ST(check_wf_indices(ctx, wf_idx, n_points));
+    if (n_points == 0) return 0;
+    const double* xyz[2] = {xyz_a, xyz_b};
+    const uint16_t* cats[2] = {cat_a, cat_b};
+    double* grads[2] = {out_grad_a, out_grad_b};
+    RowSets rs;
+    InBuf<double> x[2];
+    OutBuf<double> g[2];
+    double* G[2] = {nullptr, nullptr};   // dense [n][n] per side: entry (i, j) of row i at i n + j
+    auto release = [&](int st) { dev_free(ctx, G[0]); dev_free(ctx, G[1]); return st; };
+    int st = 0;
+    for (int s = 0; s < 2 && !st; ++s) {
+        st = rows_envset(ctx, n_points, nullptr, n_points, nullptr, xyz[s], cats[s], &rs.e[s]);
+        if (!st) st = x[s].load(ctx, xyz[s], 3 * n_points);
+        if (!st) st = g[s].prepare(ctx, grads[s], 3 * n_points);
+        if (!st) st = dev_alloc(ctx, &G[s], n_points * n_points);
+    }
+    std::vector<uint64_t> row_off(n_points);
+    for (uint64_t r = 0; r < n_points; ++r) row_off[r] = r * n_points;
+    InBuf<uint64_t> d_off;
+    if (!st) st = d_off.load(ctx, row_off.data(), n_points);
+    if (!st) {
+        const uint64_t* entry_off[2] = {d_off.ptr, d_off.ptr};
+        st = rows_grad(ctx, rs, n_points, wf_idx, pair_weights, out_scores, entry_off, G);
+    }
+    if (!st) {
+        ProfScope ps(ctx, LOCOHD_PROF_OTHER);
+        for (int s = 0; s < 2; ++s) ctx->launches += launch_coords_chain(x[s].ptr, G[s], n_points, g[s].ptr, ctx->stream);
+        if (cudaPeekAtLastError() != cudaSuccess)
+            st = fail(ctx, LOCOHD_ERR_CUDA, "launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    }
+    if (!st) st = g[0].commit();
+    if (!st) st = g[1].commit();
+    const int st2 = sync_and_check(ctx);   // also keeps row_off alive until its copy is done
+    return release(st ? st : st2);
     API_END()
 }
 

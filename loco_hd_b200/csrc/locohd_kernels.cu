@@ -1594,7 +1594,15 @@ __device__ __forceinline__ uint32_t merge_path_dist(const double* dA, const doub
     return lo;
 }
 
+// The walk is the same for both targets; GradTarget decides where an event's dS/dt goes and what bounds the members'
+// indices (the structure's primitives, or the row's length).
+template <GradTarget T>
 __global__ void __launch_bounds__(kScoreMaxWarps * 32) score_grad_kernel(GradArgs g, KParams P, int warps_per_block) {
+    constexpr bool kEntries = T == GradTarget::kEntries;
+    // The store that holds the B sides: the coordinate target scores the pairs of one environment set, which
+    // from_primitives_grad passes as both sides, and reading it through side[0] alone keeps one set of store pointers
+    // live (that instantiation's registers and spills are those of the single-set kernel it replaced).
+    constexpr int kStoreB = kEntries ? 1 : 0;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     if (wib >= warps_per_block) return;
@@ -1606,16 +1614,23 @@ __global__ void __launch_bounds__(kScoreMaxWarps * 32) score_grad_kernel(GradArg
     for (uint64_t pair = (uint64_t)blockIdx.x * warps_per_block + wib; pair < g.n_pairs;
          pair += (uint64_t)gridDim.x * warps_per_block) {
         __syncwarp();
-        const uint64_t env[2] = {pair, g.n_pairs + pair};
+        const uint64_t env[2] = {g.side[0].first + pair, g.side[1].first + pair};
         uint32_t M[2];
-        uint64_t off[2], sid[2], base[2], nprim[2];
+        uint64_t off[2], sid[2], base[2], nprim[2];   // kEntries: nprim = the row's length
+        uint32_t anchor[2];
         double xa[2][3];
         bool bad = false;
         for (int s = 0; s < 2; ++s) {
-            off[s] = g.env.off[env[s]];
-            M[s] = g.env.count[env[s]];
+            off[s] = g.side[s * kStoreB].env.off[env[s]];
+            M[s] = g.side[s * kStoreB].env.count[env[s]];
+            if (kEntries) {
+                nprim[s] = M[s];
+                bad |= M[s] > 0 && g.side[s].idx[off[s]] >= M[s];
+                continue;
+            }
             sid[s] = g.anchor_struct[env[s]];
             const uint32_t ap = g.anchor_prim[env[s]];
+            anchor[s] = ap;
             bad |= sid[s] >= g.n_structs;
             if (bad) break;
             base[s] = g.prim_off[sid[s]];
@@ -1626,14 +1641,15 @@ __global__ void __launch_bounds__(kScoreMaxWarps * 32) score_grad_kernel(GradArg
         }
         if (bad) { raise(P.err, LOCOHD_ERR_INDEX); continue; }
         if (M[0] == 0 || M[1] == 0) { raise(P.err, LOCOHD_ERR_EMPTY_ENV); continue; }
-        const uint64_t* kA = g.env.key + off[0] + 1;   // events = members after the anchor
-        const uint64_t* kB = g.env.key + off[1] + 1;
-        const double* dA = g.dist + off[0] + 1;
-        const double* dB = g.dist + off[1] + 1;
-        const uint32_t* xA = g.idx + off[0] + 1;
-        const uint32_t* xB = g.idx + off[1] + 1;
-        const uint32_t catA0 = (uint32_t)(g.env.key[off[0]] & kCatMask), catB0 = (uint32_t)(g.env.key[off[1]] & kCatMask);
-        const double t0 = fmax(g.dist[off[0]], g.dist[off[1]]);
+        const uint64_t* kA = g.side[0].env.key + off[0] + 1;   // events = members after the anchor
+        const uint64_t* kB = g.side[kStoreB].env.key + off[1] + 1;
+        const double* dA = g.side[0].dist + off[0] + 1;
+        const double* dB = g.side[kStoreB].dist + off[1] + 1;
+        const uint32_t* xA = g.side[0].idx + off[0] + 1;
+        const uint32_t* xB = g.side[kStoreB].idx + off[1] + 1;
+        const uint32_t catA0 = (uint32_t)(g.side[0].env.key[off[0]] & kCatMask);
+        const uint32_t catB0 = (uint32_t)(g.side[kStoreB].env.key[off[1]] & kCatMask);
+        const double t0 = fmax(g.side[0].dist[off[0]], g.side[kStoreB].dist[off[1]]);
         const uint32_t na = M[0] - 1, nb = M[1] - 1;
         const uint32_t E = na + nb;
         const uint32_t Q = (E + 31) / 32;
@@ -1730,7 +1746,11 @@ __global__ void __launch_bounds__(kScoreMaxWarps * 32) score_grad_kernel(GradArg
             norm[s] += wc;
             if (takeA) { iA = side_scale(norm[0]); ++i; } else { iB = side_scale(norm[1]); ++j; }
             const double hn = stat_dist();
-            if (gp != 0.0 && t > 0.0) {   // a member on top of its anchor has no direction: it contributes 0
+            if (kEntries) {
+                // every entry is written: the anchor's, t = 0 and non-finite t (+inf bans) give exactly 0
+                const bool live = gp != 0.0 && t > 0.0 && isfinite(t);
+                g.entry_grad[s][g.entry_off[s][pair] + m] = live ? gp * wf_pdf(wf, t) * (h - hn) : 0.0;
+            } else if (gp != 0.0 && t > 0.0) {   // a member on top of its anchor has no direction: it contributes 0
                 const double coef = gp * wf_pdf(wf, t) * (h - hn) / t;
                 double* gm = g.grad[sid[s]] + 3 * (uint64_t)m;
                 const double* xm = g.xyz + 3 * (base[s] + m);
@@ -1751,13 +1771,43 @@ __global__ void __launch_bounds__(kScoreMaxWarps * 32) score_grad_kernel(GradArg
         }
         if (lane == 0) {
             g.out[pair] = acc;
-            if (gp != 0.0) {
+            if (kEntries) {
+                for (int s = 0; s < 2; ++s) g.entry_grad[s][g.entry_off[s][pair] + g.side[s].idx[off[s]]] = 0.0;
+            } else if (gp != 0.0) {
                 for (int s = 0; s < 2; ++s) {
-                    const uint32_t ap = g.anchor_prim[env[s]];
-                    for (int q = 0; q < 3; ++q) atomicAdd(g.grad[sid[s]] + 3 * (uint64_t)ap + q, ganc[s][q]);
+                    for (int q = 0; q < 3; ++q) atomicAdd(g.grad[sid[s]] + 3 * (uint64_t)anchor[s] + q, ganc[s][q]);
                 }
             }
         }
+    }
+}
+
+// Chain rule of from_coords_grad: G[i][j] = g_i dS_i/dt_ij of row i (score_grad_kernel<kEntries>), and t_ij enters
+// row i and row j, so grad_i = sum_j (G[i][j] + G[j][i]) (x_i - x_j) / t_ij.  One warp per point; lane l takes
+// j = l, l + 32, ... and a fixed shuffle tree sums the lanes, so the result does not depend on scheduling.  t_ij is
+// recomputed as in rows_copy_kernel (row_distance(i, j) and row_distance(j, i) are bitwise equal); t = 0 contributes 0,
+// as do its G entries.
+__global__ void __launch_bounds__(256) coords_chain_kernel(const double* __restrict__ xyz, const double* __restrict__ G,
+                                                           uint64_t n, double* __restrict__ grad) {
+    const int lane = threadIdx.x & 31;
+    for (uint64_t i = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n;
+         i += ((uint64_t)gridDim.x * blockDim.x) >> 5) {
+        const double xi = xyz[3 * i], yi = xyz[3 * i + 1], zi = xyz[3 * i + 2];
+        double gx = 0.0, gy = 0.0, gz = 0.0;
+        for (uint64_t j = lane; j < n; j += 32) {
+            const double t = row_distance(xyz, i, j);
+            if (!(t > 0.0)) continue;
+            const double c = (G[i * n + j] + G[j * n + i]) / t;
+            gx = fma(c, xi - xyz[3 * j], gx);
+            gy = fma(c, yi - xyz[3 * j + 1], gy);
+            gz = fma(c, zi - xyz[3 * j + 2], gz);
+        }
+        for (int o = 16; o; o >>= 1) {
+            gx += __shfl_xor_sync(kFull, gx, o);
+            gy += __shfl_xor_sync(kFull, gy, o);
+            gz += __shfl_xor_sync(kFull, gz, o);
+        }
+        if (lane == 0) { grad[3 * i] = gx; grad[3 * i + 1] = gy; grad[3 * i + 2] = gz; }
     }
 }
 
@@ -3123,17 +3173,29 @@ int launch_wf_density(const WfDev* wf, uint64_t n, const double* x, double* out,
     return 1;
 }
 
-int launch_score_grad(const GradArgs& g, const KParams& p, cudaStream_t st) {
-    if (!g.n_pairs) return 0;
+template <GradTarget T>
+static int launch_score_grad_t(const GradArgs& g, const KParams& p, cudaStream_t st) {
     const int per_warp = grad_state_bytes(p.C);
     if (per_warp > 220 * 1024) return -1;
     int warps = (100 * 1024) / per_warp;
     if (warps > kScoreMaxWarps) warps = kScoreMaxWarps;
     if (warps < 1) warps = 1;
     const int smem = per_warp * warps;
-    cudaFuncSetAttribute(score_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    const unsigned grid = persistent_grid(score_grad_kernel, warps * 32, smem, g.n_pairs, warps);
-    score_grad_kernel<<<grid, warps * 32, smem, st>>>(g, p, warps);
+    cudaFuncSetAttribute(score_grad_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    const unsigned grid = persistent_grid(score_grad_kernel<T>, warps * 32, smem, g.n_pairs, warps);
+    score_grad_kernel<T><<<grid, warps * 32, smem, st>>>(g, p, warps);
+    return 1;
+}
+
+int launch_score_grad(const GradArgs& g, const KParams& p, GradTarget target, cudaStream_t st) {
+    if (!g.n_pairs) return 0;
+    return target == GradTarget::kEntries ? launch_score_grad_t<GradTarget::kEntries>(g, p, st)
+                                          : launch_score_grad_t<GradTarget::kCoords>(g, p, st);
+}
+
+int launch_coords_chain(const double* xyz, const double* G, uint64_t n, double* grad, cudaStream_t st) {
+    if (!n) return 0;
+    coords_chain_kernel<<<(unsigned)((n + 7) / 8), 256, 0, st>>>(xyz, G, n, grad);   // one warp per point
     return 1;
 }
 

@@ -267,26 +267,42 @@ struct TileGeometry {
     int team_bytes;   // shared memory per team
 };
 TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, const LaunchOverrides& ov);
-// Coordinate gradients of the scores of one from_primitives call (score_grad_kernel).  The environment set was built
-// with keep_indices: environment p is the A side of pair p, environment n_pairs + p its B side, and `dist` / `idx`
-// hold the exact distances and the members' indices inside their structure.
-struct GradArgs {
+// One side of the pairs of a gradient call: environment `first` + p of `env` is that side of pair p.  The set was built
+// with keep_indices or from rows, so `dist` / `idx` hold the exact distances and the members' indices (inside their
+// structure, or the column inside their row).
+struct GradSide {
     EnvView env;
     const double* dist;
     const uint32_t* idx;
+    uint64_t first;
+};
+// Gradients of the scores of n_pairs pairs (score_grad_kernel).  Where each event's dS/dt goes is the kernel's
+// GradTarget: the coordinates of a from_primitives call (one set passed as both sides, side[s].first = {0, n_pairs};
+// the kernel reads that set through side[0]) or the entries of two row sets (from_dmxs / from_coords,
+// side[s].first = 0).
+struct GradArgs {
+    GradSide side[2];
+    uint64_t n_pairs;
+    const uint32_t* wf_idx;         // per pair or nullptr
+    const double* pair_weights;     // upstream gradient g_p per pair or nullptr (all 1)
+    double* out;                    // [n_pairs] scores
+    // GradTarget::kCoords
     const double* xyz;              // raw [n_prims][3] of the structure set
     const uint64_t* prim_off;       // [n_structs + 1]
     uint64_t n_structs;
     const uint32_t* anchor_struct;  // [2 n_pairs]
     const uint32_t* anchor_prim;    // [2 n_pairs]
-    uint64_t n_pairs;
-    const uint32_t* wf_idx;         // per pair or nullptr
-    const double* pair_weights;     // upstream gradient g_p per pair or nullptr (all 1)
-    double* out;                    // [n_pairs] scores
     double* grad[2];                // [n_prims of structure s][3], zeroed by the caller: sum_p g_p dS_p / dxyz
+    // GradTarget::kEntries: g_p dS_p / dt of entry (row p, column c) of side s at entry_grad[s][entry_off[s][p] + c];
+    // every entry of every row is written (0 for the anchor, t = 0 and non-finite t)
+    const uint64_t* entry_off[2];   // [n_pairs]
+    double* entry_grad[2];
 };
+enum class GradTarget { kCoords, kEntries };
 // returns the number of launches, or -1 when the per-warp state of C categories does not fit shared memory
-int launch_score_grad(const GradArgs& g, const KParams& p, cudaStream_t st);
+int launch_score_grad(const GradArgs& g, const KParams& p, GradTarget target, cudaStream_t st);
+// grad[i] = sum_j (G[i][j] + G[j][i]) (x_i - x_j) / t_ij over the n points xyz, G dense [n][n] (from_coords_grad)
+int launch_coords_chain(const double* xyz, const double* G, uint64_t n, double* grad, cudaStream_t st);
 int launch_wf_density(const WfDev* wf, uint64_t n, const double* x, double* out, int* err, cudaStream_t st);
 int launch_job_means(const double* scores, const uint64_t* job_pair_off, uint64_t n_jobs, double* means,
                      cudaStream_t st);
