@@ -227,6 +227,28 @@ int locohd_score_jobs(locohd_ctx* ctx, const locohd_envset* a, const locohd_envs
 int locohd_score_jobs_stats(locohd_ctx* ctx, const locohd_envset* a, const locohd_envset* b, uint64_t n_jobs,
                             const locohd_job* jobs, const uint32_t* wf_idx, double* out_scores, double* out_job_means,
                             double* out_anchor_means, double* out_anchor_stds);
+/* Every environment of a range of A against every environment of a range of B (an extension: the reference scores
+ * listed pairs only; kras_scan.py:47-52 lists one anchor against every anchor, clustering and nearest-site searches
+ * need the whole matrix).  Row i = environment a_first + i of A (i < n_a), column j = environment b_first + j of B
+ * (j < n_b), all with weight function wf_idx: M[i][j] is the score locohd_score_pairs gives for the pair
+ * (a_first + i, b_first + j).
+ *   out_scores      [n_a][n_b] M, row-major, or NULL.
+ *   k               0: no k-nearest output; 1 .. 32: per row the k smallest M[i][j] in ascending order - equal scores
+ *                   by smaller j, NaN after +inf (a deterministic function of M) - into out_knn_scores [n_a][k] and
+ *                   out_knn_index [n_a][k] (u32 column j, relative to b_first); either may be NULL, not both.
+ *   skip_self       leaves out the column of the row's own environment (a_first + i == b_first + j); needs a == b.
+ * Rows are scored in chunks of whole rows whose scores fit a fixed scratch budget (256 MB; LOCOHD_CROSS_ROWS in the
+ * environment lowers the rows per chunk), so with out_scores == NULL the matrix never leaves the device and device
+ * memory stays bounded whatever n_a is.  The tile kernel scores the matrix when locohd_score_jobs_stats would tile a
+ * job list of these sets (one weight function, Hellinger-2, unit category weights, at most 16 categories, >= 6 teams
+ * at the sets' largest environments, LOCOHD_NO_TILES unset; counted by locohd_ctx_tile_launches); otherwise the pair
+ * kernel scores explicit pairs.  Errors: a range outside its set LOCOHD_ERR_INDEX; no output, k out of range (above
+ * 32, above the columns a row has left, 0 with a k-nearest output or non-zero without one), skip_self with two sets
+ * LOCOHD_ERR_BAD_PARAM; a bad wf_idx as in locohd_score_pairs; unknown categories and empty environments as in
+ * locohd_score_jobs.  Outputs may be host or device memory. */
+int locohd_score_cross(locohd_ctx* ctx, const locohd_envset* a, uint64_t a_first, uint64_t n_a, const locohd_envset* b,
+                       uint64_t b_first, uint64_t n_b, uint32_t wf_idx, int skip_self, double* out_scores, uint32_t k,
+                       double* out_knn_scores, uint32_t* out_knn_index);
 /* Planning query, no device needed: how locohd_score_jobs[_stats] would group this job list for the tile kernel (jobs
  * that share runs of environments are scored tile by tile: up to 4 runs of A against up to 4 runs of B staged once per
  * anchor).  *out_tiles = tiles the list groups into (in list order if that tiles well, else regrouped by the ranks of

@@ -31,7 +31,7 @@ EXPORTED_SYMBOLS = [
     "locohd_structs_update_from_atoms", "locohd_structs_drop_cells", "locohd_envset_build", "locohd_envset_from_rows",
     "locohd_envset_from_ragged_rows",
     "locohd_envset_from_coords", "locohd_envset_destroy", "locohd_envset_size", "locohd_envset_total_members",
-    "locohd_envset_dump", "locohd_score_pairs", "locohd_score_jobs", "locohd_score_jobs_stats",
+    "locohd_envset_dump", "locohd_score_pairs", "locohd_score_jobs", "locohd_score_jobs_stats", "locohd_score_cross",
     "locohd_score_anchor_lists", "locohd_plan_job_tiles", "locohd_tile_unit", "locohd_tile_geometry",
     "locohd_from_primitives", "locohd_from_primitives_grad", "locohd_from_rows_grad", "locohd_from_coords_grad",
     "locohd_wf_integral_points", "locohd_wf_density_points", "locohd_sd_run",
@@ -122,6 +122,7 @@ def load_library() -> C.CDLL:
         "locohd_score_pairs": (C.c_int, [vp, vp, vp, u64, vp, vp, vp]),
         "locohd_score_jobs": (C.c_int, [vp, vp, vp, u64, vp, vp, vp, vp]),
         "locohd_score_jobs_stats": (C.c_int, [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp]),
+        "locohd_score_cross": (C.c_int, [vp, vp, u64, u64, vp, u64, u64, u32, C.c_int, vp, u32, vp, vp]),
         "locohd_score_anchor_lists": (C.c_int, [vp, vp, u64, vp, u64, vp, u64, vp, u64, u32, vp]),
         "locohd_plan_job_tiles": (C.c_int, [u64, vp, vp, vp, vp]),
         "locohd_tile_unit": (C.c_int, [u64, u64, u64, u64, C.POINTER(u64), C.POINTER(u64)]),
@@ -400,6 +401,27 @@ class Context:
                                                      _p(res["scores"]), _p(res["job_means"]), _p(res["anchor_means"]),
                                                      _p(res["anchor_stds"])))
         return {k: v for k, v in res.items() if v is not None}
+
+    def score_cross(self, a: "EnvSet", b: "EnvSet", a_first: int = 0, n_a: Optional[int] = None, b_first: int = 0,
+                    n_b: Optional[int] = None, wf_idx: int = 0, skip_self: bool = False, scores=True, k: int = 0,
+                    knn_scores=None, knn_index=None):
+        """locohd_score_cross: every environment a_first + i (i < n_a) of `a` against every environment b_first + j
+        (j < n_b) of `b`.  Returns (M [n_a, n_b] or None, knn_scores [n_a, k] or None, knn_index [n_a, k] uint32 or
+        None); n_a / n_b default to the rest of the set.  `scores` False: no matrix; True: a new host array; or an
+        output array / raw device pointer.  k > 0 asks for the k nearest columns of every row (knn_scores / knn_index:
+        output arrays or raw device pointers, None = new host arrays)."""
+        na = len(a) - a_first if n_a is None else int(n_a)
+        nb = len(b) - b_first if n_b is None else int(n_b)
+        if scores is True:
+            scores = np.empty((max(na, 0), max(nb, 0)), np.float64)
+        elif scores is False:
+            scores = None
+        if k:
+            knn_scores = np.empty((max(na, 0), k), np.float64) if knn_scores is None else knn_scores
+            knn_index = np.empty((max(na, 0), k), np.uint32) if knn_index is None else knn_index
+        self._check(self.lib.locohd_score_cross(self.h, a.h, a_first, na, b.h, b_first, nb, wf_idx, int(skip_self),
+                                                _p(scores), k, _p(knn_scores), _p(knn_index)))
+        return scores, knn_scores, knn_index
 
     def score_jobs(self, a: "EnvSet", b: "EnvSet", jobs, wf_idx=None, out=None, want_scores=True, want_means=False,
                    means_out=None):

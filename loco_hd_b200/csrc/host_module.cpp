@@ -1054,6 +1054,85 @@ struct LoCoHD {
         if (want_as) out["anchor_std"] = as;
         return out;
     }
+
+    // ---- pairwise scores between environment sets: explicit pairs, the whole matrix of two ranges, its k nearest
+    static void check_pair(const std::shared_ptr<Environments>& ea, const std::shared_ptr<Environments>& eb) {
+        if (!ea || !eb || !ea->h || !eb->h) throw py::value_error("environments are None or closed");
+        if (ea->dev != eb->dev) throw py::value_error("the two environment sets live in different contexts");
+    }
+    // range: None (the whole set) or (start, stop) with 0 <= start <= stop <= len -> (first, count)
+    static std::pair<uint64_t, uint64_t> env_range(const py::object& range, uint64_t n_env, const char* what) {
+        if (range.is_none()) return {0, n_env};
+        const auto r = range.cast<std::pair<int64_t, int64_t>>();
+        if (r.first < 0 || r.second < r.first || (uint64_t)r.second > n_env)
+            throw py::value_error(std::string(what) + " = (" + std::to_string(r.first) + ", " + std::to_string(r.second) +
+                                  ") is not a range (start, stop) inside the " + std::to_string(n_env) + " environments");
+        return {(uint64_t)r.first, (uint64_t)(r.second - r.first)};
+    }
+    uint32_t wf_position(int64_t wf_idx) const {
+        if (wf_idx < 0 || (uint64_t)wf_idx >= wfs.size()) throw py::value_error("wf_idx out of range");
+        return (uint32_t)wf_idx;
+    }
+
+    py::array_t<double> score_pairs(const std::shared_ptr<Environments>& ea, const std::shared_ptr<Environments>& eb,
+                                    const py::array_t<int64_t, py::array::c_style | py::array::forcecast>& pairs,
+                                    const py::object& wf_idx) {
+        check_pair(ea, eb);
+        if (!(pairs.ndim() == 2 && pairs.shape(1) == 2) && !(pairs.ndim() == 1 && pairs.size() == 0))
+            throw py::value_error("pairs must be [n_pairs, 2]: (environment of env_a, environment of env_b)");
+        const uint64_t n = (uint64_t)pairs.size() / 2;
+        std::vector<uint32_t> pr(2 * n);
+        for (uint64_t i = 0; i < n; ++i)
+            for (int s = 0; s < 2; ++s) {
+                const int64_t e = pairs.data()[2 * i + s];
+                if (e < 0 || (uint64_t)e >= (s ? eb->n_env : ea->n_env))
+                    throw py::value_error("pair " + std::to_string(i) + " addresses environment " + std::to_string(e) +
+                                          " beyond env_" + (s ? "b" : "a"));
+                pr[2 * i + s] = (uint32_t)e;
+            }
+        const auto wf = wf_indices(wf_idx, n);
+        py::array_t<double> out(n);
+        double* o = out.mutable_data();
+        if (n)
+            device_call(ea->dev, [&](locohd_ctx* c) {
+                return locohd_score_pairs(c, ea->h, eb->h, n, pr.data(), wf.empty() ? nullptr : wf.data(), o);
+            });
+        return out;
+    }
+
+    py::array_t<double> score_matrix(const std::shared_ptr<Environments>& ea, const std::shared_ptr<Environments>& eb,
+                                     const py::object& a_range, const py::object& b_range, int64_t wf_idx) {
+        check_pair(ea, eb);
+        const auto ra = env_range(a_range, ea->n_env, "a_range"), rb = env_range(b_range, eb->n_env, "b_range");
+        const uint32_t wf = wf_position(wf_idx);
+        py::array_t<double> out({(py::ssize_t)ra.second, (py::ssize_t)rb.second});
+        double* o = out.mutable_data();
+        if (ra.second && rb.second)
+            device_call(ea->dev, [&](locohd_ctx* c) {
+                return locohd_score_cross(c, ea->h, ra.first, ra.second, eb->h, rb.first, rb.second, wf, 0, o, 0, nullptr,
+                                          nullptr);
+            });
+        return out;
+    }
+
+    py::tuple nearest_environments(const std::shared_ptr<Environments>& ea, const std::shared_ptr<Environments>& eb,
+                                   int64_t k, const py::object& a_range, const py::object& b_range, bool exclude_self,
+                                   int64_t wf_idx) {
+        check_pair(ea, eb);
+        const auto ra = env_range(a_range, ea->n_env, "a_range"), rb = env_range(b_range, eb->n_env, "b_range");
+        const uint32_t wf = wf_position(wf_idx);
+        if (k < 1 || k > 32) throw py::value_error("k must be in 1 ... 32");
+        if (exclude_self && ea != eb) throw py::value_error("exclude_self needs env_b to be env_a");
+        py::array_t<double> sc({(py::ssize_t)ra.second, (py::ssize_t)k});
+        py::array_t<uint32_t> ix({(py::ssize_t)ra.second, (py::ssize_t)k});
+        double* ps = sc.mutable_data();
+        uint32_t* pi = ix.mutable_data();
+        device_call(ea->dev, [&](locohd_ctx* c) {
+            return locohd_score_cross(c, ea->h, ra.first, ra.second, eb->h, rb.first, rb.second, wf, exclude_self ? 1 : 0,
+                                      nullptr, (uint32_t)k, ps, pi);
+        });
+        return py::make_tuple(sc, ix);
+    }
 };
 
 }  // namespace
@@ -1146,7 +1225,22 @@ PYBIND11_MODULE(loco_hd, m) {
              py::arg("reduce") = py::none(), py::arg("wf_idx") = py::none(),
              "Score runs of identity-paired environments: jobs is [n_jobs, 3] (a_first, b_first, n).  reduce=None returns "
              "the per-anchor scores; \"job_mean\", \"anchor_mean\", \"anchor_std\" (or a list of them, optionally with "
-             "\"scores\") are reduced on the device and returned in a dict.");
+             "\"scores\") are reduced on the device and returned in a dict.")
+        .def("score_pairs", &LoCoHD::score_pairs, py::arg("env_a"), py::arg("env_b"), py::arg("pairs"),
+             py::arg("wf_idx") = py::none(),
+             "Scores of explicit pairs: pairs is [n_pairs, 2] (environment of env_a, environment of env_b), wf_idx one "
+             "weight-function index per pair (None: function 0).")
+        .def("score_matrix", &LoCoHD::score_matrix, py::arg("env_a"), py::arg("env_b"), py::arg("a_range") = py::none(),
+             py::arg("b_range") = py::none(), py::arg("wf_idx") = 0,
+             "Every environment of a_range of env_a against every environment of b_range of env_b (ranges are "
+             "(start, stop), None = the whole set): a float64 array [n_a, n_b].")
+        .def("nearest_environments", &LoCoHD::nearest_environments, py::arg("env_a"), py::arg("env_b"), py::arg("k"),
+             py::arg("a_range") = py::none(), py::arg("b_range") = py::none(), py::arg("exclude_self") = false,
+             py::arg("wf_idx") = 0,
+             "The k (1 ... 32) environments of b_range closest to every environment of a_range: (scores [n_a, k] "
+             "ascending, columns [n_a, k] uint32 relative to the start of b_range).  Equal scores are ordered by column, "
+             "NaN after inf.  exclude_self (env_b is env_a) leaves out each environment itself.  The score matrix "
+             "stays on the device.");
 
     py::class_<Structures, std::shared_ptr<Structures>>(m, "Structures")
         .def_readonly("n_structures", &Structures::n_structs)

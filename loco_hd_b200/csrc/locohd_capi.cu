@@ -1522,6 +1522,107 @@ int locohd_score_jobs_stats(locohd_ctx* ctx, const locohd_envset* a, const locoh
     API_END()
 }
 
+// Scratch of one cross-matrix chunk: its scores (unless they go straight to a device output) and, on the pair-kernel
+// route, its explicit pairs.  256 MB: a chunk of a 10^5-column matrix still has ~300 rows (3 x 10^7 pairs, far more
+// than one launch needs to fill the GPU), and the rows of a chunk stay in L2 while the column blocks pass.
+constexpr uint64_t kCrossScratchBytes = 256ull << 20;
+
+int locohd_score_cross(locohd_ctx* ctx, const locohd_envset* a, uint64_t a_first, uint64_t n_a, const locohd_envset* b,
+                       uint64_t b_first, uint64_t n_b, uint32_t wf_idx, int skip_self, double* out_scores, uint32_t k,
+                       double* out_knn_scores, uint32_t* out_knn_index) {
+    API_BEGIN(ctx)
+    TRY_ST(need_params(ctx));
+    if (!a || !b) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
+    if (a_first > a->n_env || n_a > a->n_env - a_first || b_first > b->n_env || n_b > b->n_env - b_first)
+        return fail(ctx, LOCOHD_ERR_INDEX, "cross range beyond the env-set: A [%llu, +%llu) of %llu, B [%llu, +%llu) of %llu",
+                    (unsigned long long)a_first, (unsigned long long)n_a, (unsigned long long)a->n_env,
+                    (unsigned long long)b_first, (unsigned long long)n_b, (unsigned long long)b->n_env);
+    const bool knn = out_knn_scores || out_knn_index;
+    if (!out_scores && !knn) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "no output requested");
+    if (knn != (k != 0) || k > 32) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "k = %u: k-nearest outputs need 1 <= k <= 32", k);
+    if (skip_self && a != b) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "skip_self needs the same env-set on both sides");
+    if (n_b > 0xFFFFFFFEull) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "more than 2^32 - 2 columns");
+    // rows whose own environment lies inside the column range have one column fewer
+    const bool self_in_range = skip_self && a_first < b_first + n_b && b_first < a_first + n_a;
+    if (knn && (uint64_t)k > n_b - (self_in_range ? 1 : 0))
+        return fail(ctx, LOCOHD_ERR_BAD_PARAM, "k = %u exceeds the %llu eligible columns", k,
+                    (unsigned long long)(n_b - (self_in_range ? 1 : 0)));
+    TRY_ST(check_wf_indices(ctx, &wf_idx, 1));
+    if (a->key_is_w != b->key_is_w) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "environment sets were built with different weight-function modes");
+    if (!n_a || !n_b) return 0;
+
+    // Route: the tile kernel under the condition of locohd_score_jobs_stats (W-keyed sets - one weight function, so
+    // wf_idx is 0 -, Hellinger-2 with unit weights, C <= 16, >= 6 teams); else explicit pairs on the pair kernel, with
+    // the chosen weight function as the kernels' function 0.
+    const LaunchOverrides ov = read_launch_overrides();
+    const bool tiles = a->key_is_w && b->key_is_w && !ov.no_tiles &&
+                       tile_geometry(ctx->kp, a->max_count, b->max_count, 1, ov).teams >= 6;
+    KParams kp = ctx->kp;
+    kp.wfs = ctx->d_wfs + wf_idx;
+    kp.n_wf = 1;
+    // Chunks of R whole rows (R a multiple of 4): a chunk of the dense output is one contiguous block, and the k nearest
+    // of a row are found in one pass over it.
+    const bool direct = out_scores && is_device_ptr(ctx, out_scores);   // scores go straight to the caller's matrix
+    const uint64_t per_entry = (direct ? 0 : 8) + (tiles ? 0 : 8);
+    uint64_t R = per_entry ? kCrossScratchBytes / (per_entry * n_b) : n_a;
+    if (ov.cross_rows && ov.cross_rows < R) R = ov.cross_rows;
+    R = std::max<uint64_t>(R / 4 * 4, 4);
+    R = std::min<uint64_t>(R, (n_a + 3) / 4 * 4);
+    OutBuf<double> kscores;
+    OutBuf<uint32_t> kindex;
+    TRY_ST(kscores.prepare(ctx, out_knn_scores, knn ? n_a * k : 0));
+    TRY_ST(kindex.prepare(ctx, out_knn_index, knn ? n_a * k : 0));
+    double* d_chunk = nullptr;
+    uint32_t* d_pairs = nullptr;
+    auto cleanup = [&](int st) { dev_free(ctx, d_chunk); dev_free(ctx, d_pairs); return st; };
+    int st = 0;
+    if (!direct && (st = dev_alloc(ctx, &d_chunk, R * n_b))) return cleanup(st);
+    if (!tiles && (st = dev_alloc(ctx, &d_pairs, 2 * R * n_b))) return cleanup(st);
+    const int64_t self_off = skip_self ? (int64_t)a_first - (int64_t)b_first : INT64_MIN;
+    for (uint64_t row0 = 0; row0 < n_a && !st; row0 += R) {
+        const uint64_t rows = std::min(R, n_a - row0);
+        double* scores = direct ? out_scores + row0 * n_b : d_chunk;
+        int n = 0;
+        {
+            ProfScope ps(ctx, LOCOHD_PROF_SCORE);
+            ScoreArgs sa{};
+            sa.a = a->view(); sa.b = b->view();
+            sa.out = scores;
+            sa.cursor = ctx->d_score_cursor; sa.run = 1;
+            if (tiles) {
+                sa.n_pairs = rows * n_b;
+                sa.cross = CrossGrid{a_first + row0, b_first, rows, n_b};
+                n = launch_score_cross(sa, kp, a->max_count, b->max_count, ov, ctx->stream);
+            } else {
+                ctx->launches += launch_cross_pairs(a_first + row0, b_first, rows, n_b, d_pairs, ctx->stream);
+                sa.n_pairs = rows * n_b; sa.pairs = d_pairs;
+                const double mean_a = a->n_env ? (double)a->total / (double)a->n_env : 0.0;
+                const double mean_b = b->n_env ? (double)b->total / (double)b->n_env : 0.0;
+                n = launch_score(sa, kp, a->max_count, b->max_count, mean_a, mean_b, ov, ctx->stream);
+            }
+        }
+        if (n < 0) { st = fail(ctx, LOCOHD_ERR_UNSUPPORTED, "shared memory budget exceeded for %d categories", ctx->kp.C); break; }
+        ctx->launches += n;
+        if (tiles) ctx->tile_launches += n;
+        if (knn) {
+            ProfScope ps(ctx, LOCOHD_PROF_OTHER);
+            ctx->launches += launch_row_topk(scores, rows, n_b, (int)k, skip_self ? self_off + (int64_t)row0 : INT64_MIN,
+                                             kscores.ptr ? kscores.ptr + row0 * k : nullptr,
+                                             kindex.ptr ? kindex.ptr + row0 * k : nullptr, ctx->stream);
+        }
+        if (cudaGetLastError() != cudaSuccess) { st = fail(ctx, LOCOHD_ERR_CUDA, "cross-matrix launch failed"); break; }
+        if (out_scores && !direct &&
+            cudaMemcpyAsync(out_scores + row0 * n_b, d_chunk, rows * n_b * sizeof(double), cudaMemcpyDeviceToHost,
+                            ctx->stream) != cudaSuccess)
+            st = fail(ctx, LOCOHD_ERR_CUDA, "copy of a cross-matrix chunk failed");
+    }
+    if (!st) st = kscores.commit();
+    if (!st) st = kindex.commit();
+    const int st2 = sync_and_check(ctx);
+    return cleanup(st ? st : st2);
+    API_END()
+}
+
 int locohd_score_anchor_lists(locohd_ctx* ctx, const uint16_t* seq_a, uint64_t len_a, const double* dists_a,
                               uint64_t dlen_a, const uint16_t* seq_b, uint64_t len_b, const double* dists_b,
                               uint64_t dlen_b, uint32_t wf_idx, double* out_score) {

@@ -2184,7 +2184,9 @@ __device__ __forceinline__ void team_barrier(int team) {
     asm volatile("bar.sync %0, %1;" ::"r"(team + 1), "r"(kTeamThreads) : "memory");
 }
 
-template <int CP, bool REP>
+// CROSS: the cross matrix a.cross (CrossGrid) instead of a job list in tiles - the loader derives the rows and
+// columns of a unit from its index, a unit has one anchor, and rows / columns past the matrix are absent.
+template <int CP, bool REP, bool CROSS = false>
 __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_kernel(ScoreArgs a, KParams P, int teams,
                                                                                       int team_bytes) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -2241,7 +2243,7 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
     constexpr int lstep = kTileDim;   // lane distance between consecutive chunks of a pair
     const int sub = lane >> 2;
     const int prow = row, pcol = lane & (kTileDim - 1);
-    const uint64_t n = a.uniform_n, n_units = a.n_tiles * n;
+    const uint64_t n = a.uniform_n, n_units = CROSS ? cross_units(a.cross) : a.n_tiles * n;
     const WfDev& wf = P.wfs[0];
 
     // Loader lanes 0..7 of warp 0 hold the descriptor of the NEXT unit: it is fetched one iteration ahead, right
@@ -2264,7 +2266,27 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
         const uint64_t u = run_pos;
         if (run_pos < run_end) ++run_pos;
         nx_unit = u; nx_off = 0; nx_M = 0; nx_last = 0; nx_present = false;
-        if (u < n_units && lane < 2 * kTileDim) {
+        if constexpr (CROSS) {
+            if (u < n_units && lane < 2 * kTileDim) {
+                // unit -> (row block, column block), column block major (CrossGrid); the team reads them from the
+                // control block's tile / p slots
+                const uint64_t row_blocks = (a.cross.rows + kTileDim - 1) / kTileDim;
+                uint64_t cb, rb;
+                if ((n_units >> 32) == 0) { const uint32_t c32 = (uint32_t)u / (uint32_t)row_blocks; cb = c32; rb = (uint32_t)u - c32 * (uint32_t)row_blocks; }
+                else { cb = u / row_blocks; rb = u - cb * row_blocks; }
+                if (lane == 0) { ctrl->tile[(flags >> 1) & 1u] = (uint32_t)rb; ctrl->p[(flags >> 1) & 1u] = (uint32_t)cb; }
+                const bool is_row = lane < kTileDim;
+                const uint64_t idx = is_row ? rb * kTileDim + lane : cb * kTileDim + (lane - kTileDim);
+                if (idx < (is_row ? a.cross.rows : a.cross.cols)) {
+                    const EnvView& v = is_row ? a.a : a.b;
+                    const uint64_t e = (is_row ? a.cross.a_first : a.cross.b_first) + idx;
+                    nx_off = __ldg(v.off + e);
+                    nx_M = __ldg(v.count + e);
+                    if (nx_M & 1u) nx_last = __ldg(v.key + nx_off + nx_M - 1);
+                    nx_present = true;
+                }
+            }
+        } else if (u < n_units && lane < 2 * kTileDim) {
             uint64_t tile, p;
             // unit -> (tile, anchor) in the sliced order (TileOrder, locohd_kernels.cuh); the team reads them from the
             // control block's slot of the unit's iteration (two slots: this fetch runs while the current unit is scored)
@@ -2329,10 +2351,14 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
         if (state == 2) break;
         if (loader) fetch();
         if (state == 1) continue;
-        const uint64_t out_first = __ldg(a.tiles[ctrl->tile[slot]].out_first + prow * kTileDim + pcol);
+        uint64_t out_first;   // cross: the score (row, column) itself; absent rows and columns were staged with size 0
+        if constexpr (CROSS)
+            out_first = ((uint64_t)ctrl->tile[slot] * kTileDim + prow) * a.cross.cols + (uint64_t)ctrl->p[slot] * kTileDim + pcol;
+        else
+            out_first = __ldg(a.tiles[ctrl->tile[slot]].out_first + prow * kTileDim + pcol);
         const uint32_t Ma = ctrl->M[prow], Mb = ctrl->M[kTileDim + pcol];
-        const uint32_t p = ctrl->p[slot];
-        const bool valid = out_first != kTileNone && Ma != 0 && Mb != 0;
+        const uint32_t p = CROSS ? 0u : ctrl->p[slot];
+        const bool valid = (CROSS || out_first != kTileNone) && Ma != 0 && Mb != 0;
         const uint64_t* kA = stage + (valid ? ctrl->start[prow] : 0u);
         const uint64_t* kB = stage + (valid ? ctrl->start[kTileDim + pcol] : 0u);
         mbar_wait(&ctrl->mbar, flags & 1u);
@@ -2503,6 +2529,79 @@ __global__ void job_means_kernel(const double* __restrict__ scores, const uint64
     for (uint64_t i = b + lane; i < e; i += 32) s += scores[i];
     for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(kFull, s, o);
     if (lane == 0) means[job] = (e > b) ? s / (double)(e - b) : 0.0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Cross matrices: the explicit pairs of a chunk (pair-kernel route) and the k nearest columns of every row
+
+__global__ void cross_pairs_kernel(uint64_t a_first, uint64_t b_first, uint64_t rows, uint64_t cols,
+                                   uint2* __restrict__ pairs) {
+    const uint64_t n = rows * cols;
+    for (uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (uint64_t)gridDim.x * blockDim.x) {
+        const uint64_t r = e / cols;
+        pairs[e] = make_uint2((uint32_t)(a_first + r), (uint32_t)(b_first + (e - r * cols)));
+    }
+}
+
+constexpr int kTopkWarps = 8;
+constexpr int kTopkMax = 32;
+
+// Total order of the k-nearest lists as an unsigned key: ascending doubles, -0.0 equal to +0.0, every NaN after
+// +inf and equal to every other NaN (ties are then broken by the column, as in a stable sort).
+__device__ __forceinline__ uint64_t topk_key(double x) {
+    if (x != x) return ~0ull;
+    const uint64_t b = x == 0.0 ? 0ull : (uint64_t)__double_as_longlong(x);
+    return (b >> 63) ? ~b : b | (1ull << 63);
+}
+
+// One warp per row.  Lane l keeps the k best of columns l, l + 32, ... in shared memory, sorted (it meets its columns
+// in increasing order, so an insertion goes behind the entries of an equal key); then k rounds of a butterfly
+// arg-min over the 32 list heads, ordered by (key, column), pick the row's k best.  Every step is fixed by the data:
+// the result is a deterministic function of the row.
+__global__ void __launch_bounds__(kTopkWarps * 32) row_topk_kernel(const double* __restrict__ scores, uint64_t rows,
+                                                                   uint64_t cols, int k, int64_t self_off,
+                                                                   double* __restrict__ knn_scores,
+                                                                   uint32_t* __restrict__ knn_index) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    uint64_t* keys = reinterpret_cast<uint64_t*>(smem_raw) + (size_t)wib * k * 32;          // [k][32]
+    uint32_t* cols_of = reinterpret_cast<uint32_t*>(reinterpret_cast<uint64_t*>(smem_raw) + (size_t)kTopkWarps * k * 32) +
+                        (size_t)wib * k * 32;                                                   // [k][32]
+    const uint64_t r = (uint64_t)blockIdx.x * kTopkWarps + wib;
+    if (r >= rows) return;
+    const double* row = scores + r * cols;
+    const uint64_t self = self_off == INT64_MIN ? ~0ull : (uint64_t)((int64_t)r + self_off);
+    int cnt = 0;
+    for (uint64_t j = lane; j < cols; j += 32) {
+        if (j == self) continue;
+        const uint64_t key = topk_key(__ldg(row + j));
+        int pos;
+        if (cnt < k) pos = cnt++;
+        else if (key < keys[(k - 1) * 32 + lane]) pos = k - 1;
+        else continue;
+        for (; pos > 0 && keys[(pos - 1) * 32 + lane] > key; --pos) {
+            keys[pos * 32 + lane] = keys[(pos - 1) * 32 + lane];
+            cols_of[pos * 32 + lane] = cols_of[(pos - 1) * 32 + lane];
+        }
+        keys[pos * 32 + lane] = key;
+        cols_of[pos * 32 + lane] = (uint32_t)j;
+    }
+    int head = 0;
+    for (int t = 0; t < k; ++t) {
+        uint64_t bk = head < cnt ? keys[head * 32 + lane] : ~0ull;
+        uint32_t bj = head < cnt ? cols_of[head * 32 + lane] : ~0u;   // columns are < 2^32 - 1: never a real one
+#pragma unroll
+        for (int o = 16; o; o >>= 1) {
+            const uint64_t ok = __shfl_xor_sync(kFull, bk, o);
+            const uint32_t oj = __shfl_xor_sync(kFull, bj, o);
+            if (ok < bk || (ok == bk && oj < bj)) { bk = ok; bj = oj; }
+        }
+        if ((int)(bj & 31u) == lane) ++head;   // the winner came from the lane that owns its column
+        if (lane == 0) {
+            if (knn_scores) knn_scores[r * k + t] = row[bj];
+            if (knn_index) knn_index[r * k + t] = bj;
+        }
+    }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2983,6 +3082,7 @@ LaunchOverrides read_launch_overrides() {
     if (const char* v = env("LOCOHD_TILE_SLICE")) { const long long s = std::atoll(v); o.tile_slice = s < 0 ? 0 : s; }
     if (const char* v = env("LOCOHD_TILE_SLICE_MB")) { const double mb = std::atof(v); if (mb > 0.0) o.tile_slice_mb = mb; }
     if (const char* v = env("LOCOHD_LEGACY_GATHER")) o.legacy_gather = v[0] && v[0] != '0';
+    if (const char* v = env("LOCOHD_CROSS_ROWS")) { const long long r = std::atoll(v); if (r > 0) o.cross_rows = (uint64_t)r; }
     return o;
 }
 
@@ -3028,8 +3128,9 @@ static uint64_t tile_slice(const ScoreArgs& a, double mean_a, double mean_b, con
     return s >= n ? 0 : s;
 }
 
+// cross: the cross matrix args.cross (score_tile_kernel<CP, REP, true>) instead of the job tiles args.tiles
 static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a, double mean_b,
-                        const LaunchOverrides& ov, cudaStream_t st) {
+                        const LaunchOverrides& ov, bool cross, cudaStream_t st) {
     ScoreArgs a = args;
     const TileGeometry g = tile_geometry(p, max_a, max_b, a.a.key_is_w, ov);
     const int teams = g.teams, team_bytes = g.team_bytes;
@@ -3042,27 +3143,56 @@ static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a,
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const uint64_t units = a.n_tiles * a.uniform_n;
+    const uint64_t units = cross ? cross_units(a.cross) : a.n_tiles * a.uniform_n;
+    if (!units) return 0;
     const uint64_t need = (units + teams - 1) / teams;
     const unsigned grid = (unsigned)(need < (uint64_t)sms ? need : (uint64_t)sms);   // persistent: teams claim units from the cursor
     cudaMemsetAsync(a.cursor, 0, sizeof(unsigned long long), st);
     const uint64_t per_team = units / ((uint64_t)grid * teams * 4);   // short launches: shorter runs even out the tail
     const uint64_t max_run = ov.tile_run ? ov.tile_run : kTileRun;
     a.run = (unsigned)(per_team < 1 ? 1 : (per_team > max_run ? max_run : per_team));
-    a.order = make_tile_order(a.n_tiles, a.uniform_n, tile_slice(a, mean_a, mean_b, ov));
+    if (!cross) a.order = make_tile_order(a.n_tiles, a.uniform_n, tile_slice(a, mean_a, mean_b, ov));
     auto go = [&](auto kernel) {
         cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         kernel<<<grid, teams * kTeamThreads, smem, st>>>(a, p, teams, team_bytes);
     };
-    if (g.cp == 8) { if (rep) go(score_tile_kernel<8, true>); else go(score_tile_kernel<8, false>); }
-    else go(score_tile_kernel<16, false>);
+    if (cross) {
+        if (g.cp == 8) { if (rep) go(score_tile_kernel<8, true, true>); else go(score_tile_kernel<8, false, true>); }
+        else go(score_tile_kernel<16, false, true>);
+    } else {
+        if (g.cp == 8) { if (rep) go(score_tile_kernel<8, true>); else go(score_tile_kernel<8, false>); }
+        else go(score_tile_kernel<16, false>);
+    }
+    return 1;
+}
+
+int launch_score_cross(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, const LaunchOverrides& ov,
+                       cudaStream_t st) {
+    return launch_tiles(args, p, max_a, max_b, 0.0, 0.0, ov, true, st);
+}
+
+int launch_cross_pairs(uint64_t a_first, uint64_t b_first, uint64_t rows, uint64_t cols, uint32_t* pairs, cudaStream_t st) {
+    if (!rows || !cols) return 0;
+    const uint64_t n = rows * cols;
+    const unsigned grid = (unsigned)std::min<uint64_t>((n + 255) / 256, 148ull * 32);
+    cross_pairs_kernel<<<grid, 256, 0, st>>>(a_first, b_first, rows, cols, reinterpret_cast<uint2*>(pairs));
+    return 1;
+}
+
+int launch_row_topk(const double* scores, uint64_t rows, uint64_t cols, int k, int64_t self_off, double* knn_scores,
+                    uint32_t* knn_index, cudaStream_t st) {
+    if (!rows || k < 1 || k > kTopkMax) return 0;
+    const int smem = kTopkWarps * k * 32 * (int)(sizeof(uint64_t) + sizeof(uint32_t));
+    cudaFuncSetAttribute(row_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    row_topk_kernel<<<(unsigned)((rows + kTopkWarps - 1) / kTopkWarps), kTopkWarps * 32, smem, st>>>(
+        scores, rows, cols, k, self_off, knn_scores, knn_index);
     return 1;
 }
 
 int launch_score(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a, double mean_b,
                  const LaunchOverrides& ov, cudaStream_t st) {
     if (!args.n_pairs) return 0;
-    if (args.tiles) return launch_tiles(args, p, max_a, max_b, mean_a, mean_b, ov, st);
+    if (args.tiles) return launch_tiles(args, p, max_a, max_b, mean_a, mean_b, ov, false, st);
     const unsigned pad_max = ((max_a + 1) & ~1u) + ((max_b + 1) & ~1u);
     const bool key_is_w = args.a.key_is_w != 0;
     const bool fast = p.hell2 && p.C <= 16;   // Hellinger-2 with or without category weights

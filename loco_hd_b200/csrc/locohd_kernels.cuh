@@ -178,6 +178,19 @@ __host__ __device__ inline void tile_unit(const TileOrder& o, T u, T* tile, T* p
     }
 }
 
+// Cross-matrix mode of score_tile_kernel: every environment a_first + r (r < rows) of env-set A against every
+// environment b_first + c (c < cols) of env-set B, score (r, c) at out[r * cols + c].  A unit is one block of 4 rows
+// x 4 columns; the tile of a unit follows from its index, so there is neither a job list nor a tile descriptor.
+// Unit order: column block major, u = column block * row blocks + row block - the 4 environments of a column block
+// are staged by consecutive units while the row blocks pass over them, and the rows of a chunk (a few hundred
+// environments) stay in L2 from one column block to the next, so every environment of B comes from DRAM once.
+struct CrossGrid {
+    uint64_t a_first, b_first;
+    uint64_t rows, cols;
+};
+static_assert(sizeof(CrossGrid) <= sizeof(TileOrder), "shares TileOrder's place in ScoreArgs: the layout is unchanged");
+__host__ __device__ inline uint64_t cross_units(const CrossGrid& g) { return ((g.rows + 3) / 4) * ((g.cols + 3) / 4); }
+
 struct ScoreArgs {
     const ScoreTile* tiles;        // tile mode (score_tile_kernel): jobs grouped by the host, uniform_n anchors each
     uint64_t n_tiles;
@@ -194,7 +207,10 @@ struct ScoreArgs {
     int only_unstaged;             // second pass: score only the pairs the fast kernel skipped
     int table_n;                   // sqrt / rsqrt table entries staged by the fast kernel
     int rep_n;                     // tile kernel: head entries of the count-indexed tables replicated per bank pair
-    TileOrder order;               // tile kernel: unit -> (tile, anchor), slice by slice (read from the parameter bank)
+    union {                        // tile kernel, read from the parameter bank:
+        TileOrder order;           //   job tiles: unit -> (tile, anchor), slice by slice
+        CrossGrid cross;           //   cross matrix (launch_score_cross): unit -> (row block, column block)
+    };
     unsigned long long* cursor;    // fast kernel: next unclaimed pair (zeroed before the launch); warps claim runs of
                                    // `run` consecutive pairs, so all resident warps work at one moving frontier
     unsigned run;                  // pairs per claim: kScoreRun for large launches, fewer when the launch has fewer
@@ -241,7 +257,8 @@ int launch_rows_copy(const double* values, const double* xyz, const uint8_t* cat
 // read_launch_overrides() once per API call, so that a process can change them between calls.  The defaults leave
 // every decision to the library.  No other code of the library reads the environment.
 struct LaunchOverrides {
-    bool no_tiles = false;        // LOCOHD_NO_TILES (non-zero integer): job lists never take score_tile_kernel
+    bool no_tiles = false;        // LOCOHD_NO_TILES (non-zero integer): job lists and cross matrices never take
+                                  // score_tile_kernel
     int tile_teams = 0;           // LOCOHD_TILE_TEAMS: lowers TileGeometry::teams when in [1, teams)
     int tile_rep = -1;            // LOCOHD_TILE_REP: lowers TileGeometry::rep_n when in [0, rep_n)
     unsigned tile_run = 0;        // LOCOHD_TILE_RUN (1 ... 4096): longest run of units a team claims (0: kTileRun)
@@ -250,10 +267,24 @@ struct LaunchOverrides {
     double tile_slice_mb = 0.0;   // LOCOHD_TILE_SLICE_MB (> 0): that L2 budget in MB (0: the default)
     bool legacy_gather = false;   // LOCOHD_LEGACY_GATHER (any value not starting with '0'): environments are built
                                   // with the multi-kernel gather
+    uint64_t cross_rows = 0;      // LOCOHD_CROSS_ROWS (> 0): lowers the rows of a cross-matrix chunk (rounded down to a
+                                  // multiple of 4, at least 4)
 };
 LaunchOverrides read_launch_overrides();
 int launch_score(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a, double mean_b,
                  const LaunchOverrides& ov, cudaStream_t st);
+// The cross matrix args.cross on the tile kernel (args.out, args.a / args.b, args.cursor are read; the caller has
+// checked that tile_geometry(...).teams >= 1).  Returns the number of launches, -1 when the tile kernel does not apply.
+int launch_score_cross(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, const LaunchOverrides& ov,
+                       cudaStream_t st);
+// Explicit pairs (a_first + row, b_first + column) of every entry of a rows x cols block, row-major, into pairs
+// [rows * cols][2]: the cross matrix on the pair kernel.
+int launch_cross_pairs(uint64_t a_first, uint64_t b_first, uint64_t rows, uint64_t cols, uint32_t* pairs, cudaStream_t st);
+// k nearest (1 <= k <= 32) of every row of scores [rows][cols]: ascending, equal scores by smaller column, NaN after
+// +inf (-0.0 and +0.0 are equal).  Column self_off + r of row r is left out (self_off = INT64_MIN: none is).  Row r
+// writes knn_scores / knn_index [r * k ...] (either may be nullptr); every row must have k eligible columns.
+int launch_row_topk(const double* scores, uint64_t rows, uint64_t cols, int k, int64_t self_off, double* knn_scores,
+                    uint32_t* knn_index, cudaStream_t st);
 // Launch geometry of score_tile_kernel for environments of at most max_a / max_b members (teams = 0: the kernel does
 // not apply; below 6 teams the pair kernel is the better one and job lists are not tiled).  The one place that decides
 // it: launch_tiles, the tile eligibility of locohd_score_jobs_stats and locohd_tile_geometry read it.
