@@ -249,6 +249,29 @@ int locohd_score_jobs_stats(locohd_ctx* ctx, const locohd_envset* a, const locoh
 int locohd_score_cross(locohd_ctx* ctx, const locohd_envset* a, uint64_t a_first, uint64_t n_a, const locohd_envset* b,
                        uint64_t b_first, uint64_t n_b, uint32_t wf_idx, int skip_self, double* out_scores, uint32_t k,
                        double* out_knn_scores, uint32_t* out_knn_index);
+/* Every unordered pair of one range once (an extension, for clustering within one env-set: scipy.cluster.hierarchy
+ * .linkage and scipy.spatial.distance.squareform take this vector).  For 0 <= i < j < n, out_scores[n i - i (i + 1) / 2
+ * + (j - i - 1)] is the score locohd_score_pairs gives for the pair (first + i, first + j) with weight function
+ * wf_idx: scipy's pdist order, n (n - 1) / 2 entries.  Each entry is bit-identical to M[i][j] of
+ * locohd_score_cross(s, first, n, s, first, n, ...), which scores both triangles: this call scores one, half the work
+ * and half the output.  Only symmetric statistical distances are accepted (Hellinger with any exponent,
+ * Kolmogorov-Smirnov); Kullback-Leibler and Renyi give LOCOHD_ERR_BAD_PARAM - use locohd_score_cross for them.
+ * Route as in locohd_score_cross (the tile kernel, counted by locohd_ctx_tile_launches, or explicit pairs on the pair
+ * kernel).  Rows are scored in chunks of whole blocks of 4 rows whose scores fit the 256 MB scratch (a device output
+ * takes the whole triangle in one launch of the tile kernel; LOCOHD_CROSS_ROWS in the environment lowers the rows per
+ * chunk); a chunk is one contiguous slice of out_scores, host or device memory.  Errors: a range outside the set
+ * LOCOHD_ERR_INDEX; an asymmetric distance, out_scores NULL with n >= 2, a bad wf_idx LOCOHD_ERR_BAD_PARAM; unknown
+ * categories and empty environments as in locohd_score_jobs.  n < 2 writes nothing. */
+int locohd_score_condensed(locohd_ctx* ctx, const locohd_envset* s, uint64_t first, uint64_t n, uint32_t wf_idx,
+                           double* out_scores);
+/* Planning query, no device needed: position `unit` of a launch of locohd_score_condensed on a range of n environments,
+ * for the chunk of row blocks [row_block0, row_block0 + row_blocks) (a row block: 4 rows; ceil(n / 4) blocks) -> the
+ * block of 4 x 4 pairs scored there, *out_row_block <= *out_col_block.  Units run column block major: first the
+ * column blocks of the chunk's own rows (a triangle, row blocks row_block0 .. column block), then every further column
+ * block with all row blocks of the chunk, row blocks ascending within a column block.  LOCOHD_ERR_BAD_PARAM for a
+ * chunk outside the blocks or a unit out of range. */
+int locohd_condensed_unit(uint64_t n, uint64_t row_block0, uint64_t row_blocks, uint64_t unit, uint64_t* out_row_block,
+                          uint64_t* out_col_block);
 /* Planning query, no device needed: how locohd_score_jobs[_stats] would group this job list for the tile kernel (jobs
  * that share runs of environments are scored tile by tile: up to 4 runs of A against up to 4 runs of B staged once per
  * anchor).  *out_tiles = tiles the list groups into (in list order if that tiles well, else regrouped by the ranks of

@@ -32,6 +32,7 @@ EXPORTED_SYMBOLS = [
     "locohd_envset_from_ragged_rows",
     "locohd_envset_from_coords", "locohd_envset_destroy", "locohd_envset_size", "locohd_envset_total_members",
     "locohd_envset_dump", "locohd_score_pairs", "locohd_score_jobs", "locohd_score_jobs_stats", "locohd_score_cross",
+    "locohd_score_condensed", "locohd_condensed_unit",
     "locohd_score_anchor_lists", "locohd_plan_job_tiles", "locohd_tile_unit", "locohd_tile_geometry",
     "locohd_from_primitives", "locohd_from_primitives_grad", "locohd_from_rows_grad", "locohd_from_coords_grad",
     "locohd_wf_integral_points", "locohd_wf_density_points", "locohd_sd_run",
@@ -123,6 +124,8 @@ def load_library() -> C.CDLL:
         "locohd_score_jobs": (C.c_int, [vp, vp, vp, u64, vp, vp, vp, vp]),
         "locohd_score_jobs_stats": (C.c_int, [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp]),
         "locohd_score_cross": (C.c_int, [vp, vp, u64, u64, vp, u64, u64, u32, C.c_int, vp, u32, vp, vp]),
+        "locohd_score_condensed": (C.c_int, [vp, vp, u64, u64, u32, vp]),
+        "locohd_condensed_unit": (C.c_int, [u64, u64, u64, u64, C.POINTER(u64), C.POINTER(u64)]),
         "locohd_score_anchor_lists": (C.c_int, [vp, vp, u64, vp, u64, vp, u64, vp, u64, u32, vp]),
         "locohd_plan_job_tiles": (C.c_int, [u64, vp, vp, vp, vp]),
         "locohd_tile_unit": (C.c_int, [u64, u64, u64, u64, C.POINTER(u64), C.POINTER(u64)]),
@@ -179,6 +182,16 @@ def tile_unit(n_tiles: int, n_anchors: int, slice_: int, unit: int):
     if st:
         raise LocoHDError(st, "locohd_tile_unit")
     return int(t.value), int(p.value)
+
+
+def condensed_unit(n: int, row_block0: int, row_blocks: int, unit: int):
+    """(row block, column block) at position `unit` of a condensed launch on n environments, for the chunk of row
+    blocks [row_block0, row_block0 + row_blocks) (locohd_condensed_unit; host-side, no device)."""
+    r, c = C.c_uint64(), C.c_uint64()
+    st = load_library().locohd_condensed_unit(n, row_block0, row_blocks, unit, C.byref(r), C.byref(c))
+    if st:
+        raise LocoHDError(st, "locohd_condensed_unit")
+    return int(r.value), int(c.value)
 
 
 def tile_geometry(n_categories: int, max_a: int, max_b: int) -> dict:
@@ -422,6 +435,16 @@ class Context:
         self._check(self.lib.locohd_score_cross(self.h, a.h, a_first, na, b.h, b_first, nb, wf_idx, int(skip_self),
                                                 _p(scores), k, _p(knn_scores), _p(knn_index)))
         return scores, knn_scores, knn_index
+
+    def score_condensed(self, env: "EnvSet", first: int = 0, n: Optional[int] = None, wf_idx: int = 0, out=None):
+        """locohd_score_condensed: the pairs (first + i, first + j), i < j < n, of one env-set in scipy's pdist order,
+        n (n - 1) / 2 scores; n defaults to the rest of the set.  `out`: None (a new host array), an output array or a
+        raw device pointer.  Returns `out`."""
+        n = len(env) - first if n is None else int(n)
+        if out is None:
+            out = np.empty(max(n * (n - 1) // 2, 0), np.float64)
+        self._check(self.lib.locohd_score_condensed(self.h, env.h, first, n, wf_idx, _p(out)))
+        return out
 
     def score_jobs(self, a: "EnvSet", b: "EnvSet", jobs, wf_idx=None, out=None, want_scores=True, want_means=False,
                    means_out=None):

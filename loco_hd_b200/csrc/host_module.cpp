@@ -1133,6 +1133,18 @@ struct LoCoHD {
         });
         return py::make_tuple(sc, ix);
     }
+
+    // the pairs i < j of one range, scipy's pdist order (locohd_score_condensed)
+    py::array_t<double> score_condensed(const std::shared_ptr<Environments>& env, const py::object& range,
+                                        int64_t wf_idx) {
+        check_pair(env, env);
+        const auto r = env_range(range, env->n_env, "env_range");
+        const uint32_t wf = wf_position(wf_idx);
+        py::array_t<double> out((py::ssize_t)(r.second * (r.second - (r.second > 0)) / 2));
+        double* o = out.mutable_data();
+        device_call(env->dev, [&](locohd_ctx* c) { return locohd_score_condensed(c, env->h, r.first, r.second, wf, o); });
+        return out;
+    }
 };
 
 }  // namespace
@@ -1240,7 +1252,13 @@ PYBIND11_MODULE(loco_hd, m) {
              "The k (1 ... 32) environments of b_range closest to every environment of a_range: (scores [n_a, k] "
              "ascending, columns [n_a, k] uint32 relative to the start of b_range).  Equal scores are ordered by column, "
              "NaN after inf.  exclude_self (env_b is env_a) leaves out each environment itself.  The score matrix "
-             "stays on the device.");
+             "stays on the device.")
+        .def("score_condensed", &LoCoHD::score_condensed, py::arg("env"), py::arg("env_range") = py::none(),
+             py::arg("wf_idx") = 0,
+             "Every pair i < j of env_range of env (a range (start, stop), None = the whole set) once, in the order of "
+             "scipy.spatial.distance.pdist: a float64 array [n (n - 1) / 2] that scipy.cluster.hierarchy.linkage and "
+             "squareform take.  Needs a symmetric statistical distance (Hellinger or Kolmogorov-Smirnov); "
+             "score_matrix gives both triangles of an asymmetric one.");
 
     py::class_<Structures, std::shared_ptr<Structures>>(m, "Structures")
         .def_readonly("n_structures", &Structures::n_structs)

@@ -1623,6 +1623,103 @@ int locohd_score_cross(locohd_ctx* ctx, const locohd_envset* a, uint64_t a_first
     API_END()
 }
 
+int locohd_score_condensed(locohd_ctx* ctx, const locohd_envset* s, uint64_t first, uint64_t n, uint32_t wf_idx,
+                           double* out_scores) {
+    API_BEGIN(ctx)
+    TRY_ST(need_params(ctx));
+    if (!s) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
+    if (first > s->n_env || n > s->n_env - first)
+        return fail(ctx, LOCOHD_ERR_INDEX, "condensed range beyond the env-set: [%llu, +%llu) of %llu",
+                    (unsigned long long)first, (unsigned long long)n, (unsigned long long)s->n_env);
+    // One triangle stands for the matrix only where the score is symmetric in its two environments.
+    if (ctx->kp.sd_kind != LOCOHD_SD_HELLINGER && ctx->kp.sd_kind != LOCOHD_SD_KOLMOGOROV_SMIRNOV)
+        return fail(ctx, LOCOHD_ERR_BAD_PARAM,
+                    "condensed scores need a symmetric statistical distance (Hellinger or Kolmogorov-Smirnov); "
+                    "locohd_score_cross gives both triangles of an asymmetric one");
+    if (n > 0xFFFFFFFEull) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "more than 2^32 - 2 environments");
+    TRY_ST(check_wf_indices(ctx, &wf_idx, 1));
+    if (n < 2) return 0;
+    if (!out_scores) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "no output");
+
+    // Route and weight function as in locohd_score_cross with the range on both sides.
+    const LaunchOverrides ov = read_launch_overrides();
+    const bool tiles = s->key_is_w && !ov.no_tiles && tile_geometry(ctx->kp, s->max_count, s->max_count, 1, ov).teams >= 6;
+    KParams kp = ctx->kp;
+    kp.wfs = ctx->d_wfs + wf_idx;
+    kp.n_wf = 1;
+    // Chunks of whole row blocks (4 rows from `first`): the scores of a chunk are one contiguous slice of the condensed
+    // vector.  A chunk takes row blocks while its scores fit the scratch budget, so the chunks further down, whose rows
+    // are shorter, take more of them; one row block may exceed the budget (rows of more than 8 M columns).
+    const bool direct = is_device_ptr(ctx, out_scores);   // scores go straight to the caller's vector
+    const uint64_t per_score = (direct ? 0 : 8) + (tiles ? 0 : 8);
+    const uint64_t budget = per_score ? kCrossScratchBytes / per_score : ~0ull;
+    const uint64_t nb = (n + 3) / 4, max_blocks = ov.cross_rows ? std::max<uint64_t>(ov.cross_rows / 4, 1) : nb;
+    auto row_base = [&](uint64_t i) { return n * i - triangle<uint64_t>(i); };   // condensed index of (i, i + 1)
+    auto scores_of = [&](uint64_t rb0, uint64_t rb1) { return row_base(std::min(4 * rb1, n)) - row_base(4 * rb0); };
+    const uint64_t scratch = per_score ? std::min(scores_of(0, nb), std::max(budget, scores_of(0, 1))) : 0;
+    double* d_chunk = nullptr;
+    uint32_t* d_pairs = nullptr;
+    auto cleanup = [&](int st) { dev_free(ctx, d_chunk); dev_free(ctx, d_pairs); return st; };
+    int st = 0;
+    if (!direct && (st = dev_alloc(ctx, &d_chunk, scratch))) return cleanup(st);
+    if (!tiles && (st = dev_alloc(ctx, &d_pairs, 2 * scratch))) return cleanup(st);
+    for (uint64_t rb0 = 0, rb1; rb0 < nb && !st; rb0 = rb1) {
+        rb1 = rb0 + 1;
+        while (rb1 < nb && rb1 - rb0 < max_blocks && scores_of(rb0, rb1 + 1) <= budget) ++rb1;
+        const uint64_t i0 = 4 * rb0, base = row_base(i0), count = scores_of(rb0, rb1);
+        if (!count) continue;   // the last row alone: it has no pair
+        double* scores = direct ? out_scores + base : d_chunk;
+        int launched = 0;
+        {
+            ProfScope ps(ctx, LOCOHD_PROF_SCORE);
+            ScoreArgs sa{};
+            sa.a = s->view(); sa.b = sa.a;
+            sa.out = scores;
+            sa.n_pairs = count;
+            sa.cursor = ctx->d_score_cursor; sa.run = 1;
+            if (tiles) {
+                sa.condensed = CondensedGrid{first, n, rb0, rb1 - rb0, base};
+                launched = launch_score_condensed(sa, kp, s->max_count, ov, ctx->stream);
+            } else {
+                ctx->launches += launch_condensed_pairs(first, n, i0, std::min(4 * rb1, n) - i0, d_pairs, ctx->stream);
+                sa.pairs = d_pairs;
+                const double mean = s->n_env ? (double)s->total / (double)s->n_env : 0.0;
+                launched = launch_score(sa, kp, s->max_count, s->max_count, mean, mean, ov, ctx->stream);
+            }
+        }
+        if (launched < 0) { st = fail(ctx, LOCOHD_ERR_UNSUPPORTED, "shared memory budget exceeded for %d categories", ctx->kp.C); break; }
+        ctx->launches += launched;
+        if (tiles) ctx->tile_launches += launched;
+        if (cudaGetLastError() != cudaSuccess) { st = fail(ctx, LOCOHD_ERR_CUDA, "condensed launch failed"); break; }
+        if (!direct && cudaMemcpyAsync(out_scores + base, d_chunk, count * sizeof(double), cudaMemcpyDeviceToHost,
+                                       ctx->stream) != cudaSuccess)
+            st = fail(ctx, LOCOHD_ERR_CUDA, "copy of a condensed chunk failed");
+    }
+    const int st2 = sync_and_check(ctx);
+    return cleanup(st ? st : st2);
+    API_END()
+}
+
+int locohd_condensed_unit(uint64_t n, uint64_t row_block0, uint64_t row_blocks, uint64_t unit, uint64_t* out_row_block,
+                          uint64_t* out_col_block) {
+    const uint64_t nb = n / 4 + (n % 4 != 0);
+    if (!out_row_block || !out_col_block || row_blocks == 0 || row_block0 > nb || row_blocks > nb - row_block0)
+        return LOCOHD_ERR_BAD_PARAM;
+    const unsigned __int128 R = row_blocks,
+                            units = R * (R + 1) / 2 + R * (unsigned __int128)(nb - row_block0 - row_blocks);
+    if ((units >> 64) != 0 || unit >= (uint64_t)units) return LOCOHD_ERR_BAD_PARAM;
+    uint64_t dr = 0, dc = 0;
+    condensed_unit<uint64_t>(row_blocks, unit, &dr, &dc);
+    if ((units >> 32) == 0) {   // the kernel's 32-bit path must agree
+        uint32_t r32 = 0, c32 = 0;
+        condensed_unit<uint32_t>((uint32_t)row_blocks, (uint32_t)unit, &r32, &c32);
+        if (r32 != dr || c32 != dc) return LOCOHD_ERR_CUDA;
+    }
+    *out_row_block = row_block0 + dr;
+    *out_col_block = row_block0 + dc;
+    return LOCOHD_OK;
+}
+
 int locohd_score_anchor_lists(locohd_ctx* ctx, const uint16_t* seq_a, uint64_t len_a, const double* dists_a,
                               uint64_t dlen_a, const uint16_t* seq_b, uint64_t len_b, const double* dists_b,
                               uint64_t dlen_b, uint32_t wf_idx, double* out_score) {

@@ -2184,11 +2184,16 @@ __device__ __forceinline__ void team_barrier(int team) {
     asm volatile("bar.sync %0, %1;" ::"r"(team + 1), "r"(kTeamThreads) : "memory");
 }
 
-// CROSS: the cross matrix a.cross (CrossGrid) instead of a job list in tiles - the loader derives the rows and
-// columns of a unit from its index, a unit has one anchor, and rows / columns past the matrix are absent.
-template <int CP, bool REP, bool CROSS = false>
+// What the units of a tile launch are: kJobs - a job list in tiles (a.tiles, a.order); kCross - the cross matrix
+// a.cross (CrossGrid); kCondensed - a chunk of the upper triangle of one range, a.condensed (CondensedGrid).  In the two
+// matrix modes the loader derives the rows and columns of a unit from its index, a unit has one anchor, and rows /
+// columns past the matrix are absent.
+enum class TileMode { kJobs, kCross, kCondensed };
+
+template <int CP, bool REP, TileMode MODE = TileMode::kJobs>
 __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_kernel(ScoreArgs a, KParams P, int teams,
                                                                                       int team_bytes) {
+    constexpr bool CROSS = MODE == TileMode::kCross, CONDENSED = MODE == TileMode::kCondensed;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int table_n = a.table_n;
@@ -2243,7 +2248,8 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
     constexpr int lstep = kTileDim;   // lane distance between consecutive chunks of a pair
     const int sub = lane >> 2;
     const int prow = row, pcol = lane & (kTileDim - 1);
-    const uint64_t n = a.uniform_n, n_units = CROSS ? cross_units(a.cross) : a.n_tiles * n;
+    const uint64_t n = a.uniform_n,
+                   n_units = CROSS ? cross_units(a.cross) : CONDENSED ? condensed_units(a.condensed) : a.n_tiles * n;
     const WfDev& wf = P.wfs[0];
 
     // Loader lanes 0..7 of warp 0 hold the descriptor of the NEXT unit: it is fetched one iteration ahead, right
@@ -2283,6 +2289,25 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
                     nx_off = __ldg(v.off + e);
                     nx_M = __ldg(v.count + e);
                     if (nx_M & 1u) nx_last = __ldg(v.key + nx_off + nx_M - 1);
+                    nx_present = true;
+                }
+            }
+        } else if constexpr (CONDENSED) {
+            if (u < n_units && lane < 2 * kTileDim) {
+                // unit -> (row block, column block >= row block), column block major (CondensedGrid); both sides are
+                // environments of the one range
+                const CondensedGrid& g = a.condensed;
+                uint64_t dr, dc;
+                if ((n_units >> 32) == 0) { uint32_t r32, c32; condensed_unit<uint32_t>((uint32_t)g.row_blocks, (uint32_t)u, &r32, &c32); dr = r32; dc = c32; }
+                else condensed_unit<uint64_t>(g.row_blocks, u, &dr, &dc);
+                const uint64_t rb = g.rb0 + dr, cb = g.rb0 + dc;
+                if (lane == 0) { ctrl->tile[(flags >> 1) & 1u] = (uint32_t)rb; ctrl->p[(flags >> 1) & 1u] = (uint32_t)cb; }
+                const uint64_t idx = (lane < kTileDim ? rb : cb) * kTileDim + (lane & (kTileDim - 1));
+                if (idx < g.n) {
+                    const uint64_t e = g.first + idx;
+                    nx_off = __ldg(a.a.off + e);
+                    nx_M = __ldg(a.a.count + e);
+                    if (nx_M & 1u) nx_last = __ldg(a.a.key + nx_off + nx_M - 1);
                     nx_present = true;
                 }
             }
@@ -2352,13 +2377,19 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
         if (loader) fetch();
         if (state == 1) continue;
         uint64_t out_first;   // cross: the score (row, column) itself; absent rows and columns were staged with size 0
-        if constexpr (CROSS)
+        bool upper = true;    // condensed: only pairs above the diagonal are scored, the others walk no event
+        if constexpr (CROSS) {
             out_first = ((uint64_t)ctrl->tile[slot] * kTileDim + prow) * a.cross.cols + (uint64_t)ctrl->p[slot] * kTileDim + pcol;
-        else
+        } else if constexpr (CONDENSED) {
+            const uint64_t i = (uint64_t)ctrl->tile[slot] * kTileDim + prow, j = (uint64_t)ctrl->p[slot] * kTileDim + pcol;
+            upper = j > i;
+            out_first = a.condensed.n * i - triangle<uint64_t>(i) + (j - i - 1) - a.condensed.base;
+        } else {
             out_first = __ldg(a.tiles[ctrl->tile[slot]].out_first + prow * kTileDim + pcol);
+        }
         const uint32_t Ma = ctrl->M[prow], Mb = ctrl->M[kTileDim + pcol];
-        const uint32_t p = CROSS ? 0u : ctrl->p[slot];
-        const bool valid = (CROSS || out_first != kTileNone) && Ma != 0 && Mb != 0;
+        const uint32_t p = MODE != TileMode::kJobs ? 0u : ctrl->p[slot];
+        const bool valid = (MODE != TileMode::kJobs || out_first != kTileNone) && upper && Ma != 0 && Mb != 0;
         const uint64_t* kA = stage + (valid ? ctrl->start[prow] : 0u);
         const uint64_t* kB = stage + (valid ? ctrl->start[kTileDim + pcol] : 0u);
         mbar_wait(&ctrl->mbar, flags & 1u);
@@ -2540,6 +2571,17 @@ __global__ void cross_pairs_kernel(uint64_t a_first, uint64_t b_first, uint64_t 
     for (uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (uint64_t)gridDim.x * blockDim.x) {
         const uint64_t r = e / cols;
         pairs[e] = make_uint2((uint32_t)(a_first + r), (uint32_t)(b_first + (e - r * cols)));
+    }
+}
+
+// One warp per row i of the chunk: its n - 1 - i pairs (i, j > i) at the row's condensed offset inside the chunk.
+__global__ void condensed_pairs_kernel(uint64_t first, uint64_t n, uint64_t i0, uint64_t rows, uint2* __restrict__ pairs) {
+    const int lane = threadIdx.x & 31;
+    const uint64_t warps = (uint64_t)gridDim.x * (blockDim.x >> 5);
+    for (uint64_t r = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < rows; r += warps) {
+        const uint64_t i = i0 + r;
+        uint2* row = pairs + (n * i - triangle<uint64_t>(i)) - (n * i0 - triangle<uint64_t>(i0));
+        for (uint64_t j = i + 1 + lane; j < n; j += 32) row[j - i - 1] = make_uint2((uint32_t)(first + i), (uint32_t)(first + j));
     }
 }
 
@@ -3128,9 +3170,9 @@ static uint64_t tile_slice(const ScoreArgs& a, double mean_a, double mean_b, con
     return s >= n ? 0 : s;
 }
 
-// cross: the cross matrix args.cross (score_tile_kernel<CP, REP, true>) instead of the job tiles args.tiles
+// mode: the job tiles args.tiles, the cross matrix args.cross or the condensed chunk args.condensed
 static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a, double mean_b,
-                        const LaunchOverrides& ov, bool cross, cudaStream_t st) {
+                        const LaunchOverrides& ov, TileMode mode, cudaStream_t st) {
     ScoreArgs a = args;
     const TileGeometry g = tile_geometry(p, max_a, max_b, a.a.key_is_w, ov);
     const int teams = g.teams, team_bytes = g.team_bytes;
@@ -3143,7 +3185,9 @@ static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a,
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const uint64_t units = cross ? cross_units(a.cross) : a.n_tiles * a.uniform_n;
+    const uint64_t units = mode == TileMode::kCross       ? cross_units(a.cross)
+                           : mode == TileMode::kCondensed ? condensed_units(a.condensed)
+                                                          : a.n_tiles * a.uniform_n;
     if (!units) return 0;
     const uint64_t need = (units + teams - 1) / teams;
     const unsigned grid = (unsigned)(need < (uint64_t)sms ? need : (uint64_t)sms);   // persistent: teams claim units from the cursor
@@ -3151,14 +3195,18 @@ static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a,
     const uint64_t per_team = units / ((uint64_t)grid * teams * 4);   // short launches: shorter runs even out the tail
     const uint64_t max_run = ov.tile_run ? ov.tile_run : kTileRun;
     a.run = (unsigned)(per_team < 1 ? 1 : (per_team > max_run ? max_run : per_team));
-    if (!cross) a.order = make_tile_order(a.n_tiles, a.uniform_n, tile_slice(a, mean_a, mean_b, ov));
+    if (mode == TileMode::kJobs) a.order = make_tile_order(a.n_tiles, a.uniform_n, tile_slice(a, mean_a, mean_b, ov));
     auto go = [&](auto kernel) {
         cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         kernel<<<grid, teams * kTeamThreads, smem, st>>>(a, p, teams, team_bytes);
     };
-    if (cross) {
-        if (g.cp == 8) { if (rep) go(score_tile_kernel<8, true, true>); else go(score_tile_kernel<8, false, true>); }
-        else go(score_tile_kernel<16, false, true>);
+    constexpr TileMode kCross = TileMode::kCross, kCondensed = TileMode::kCondensed;
+    if (mode == kCross) {
+        if (g.cp == 8) { if (rep) go(score_tile_kernel<8, true, kCross>); else go(score_tile_kernel<8, false, kCross>); }
+        else go(score_tile_kernel<16, false, kCross>);
+    } else if (mode == kCondensed) {
+        if (g.cp == 8) { if (rep) go(score_tile_kernel<8, true, kCondensed>); else go(score_tile_kernel<8, false, kCondensed>); }
+        else go(score_tile_kernel<16, false, kCondensed>);
     } else {
         if (g.cp == 8) { if (rep) go(score_tile_kernel<8, true>); else go(score_tile_kernel<8, false>); }
         else go(score_tile_kernel<16, false>);
@@ -3168,7 +3216,12 @@ static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a,
 
 int launch_score_cross(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, const LaunchOverrides& ov,
                        cudaStream_t st) {
-    return launch_tiles(args, p, max_a, max_b, 0.0, 0.0, ov, true, st);
+    return launch_tiles(args, p, max_a, max_b, 0.0, 0.0, ov, TileMode::kCross, st);
+}
+
+int launch_score_condensed(const ScoreArgs& args, const KParams& p, unsigned max_count, const LaunchOverrides& ov,
+                           cudaStream_t st) {
+    return launch_tiles(args, p, max_count, max_count, 0.0, 0.0, ov, TileMode::kCondensed, st);
 }
 
 int launch_cross_pairs(uint64_t a_first, uint64_t b_first, uint64_t rows, uint64_t cols, uint32_t* pairs, cudaStream_t st) {
@@ -3176,6 +3229,13 @@ int launch_cross_pairs(uint64_t a_first, uint64_t b_first, uint64_t rows, uint64
     const uint64_t n = rows * cols;
     const unsigned grid = (unsigned)std::min<uint64_t>((n + 255) / 256, 148ull * 32);
     cross_pairs_kernel<<<grid, 256, 0, st>>>(a_first, b_first, rows, cols, reinterpret_cast<uint2*>(pairs));
+    return 1;
+}
+
+int launch_condensed_pairs(uint64_t first, uint64_t n, uint64_t i0, uint64_t rows, uint32_t* pairs, cudaStream_t st) {
+    if (!rows) return 0;
+    const unsigned grid = (unsigned)std::min<uint64_t>((rows + 7) / 8, 148ull * 32);   // 8 rows (warps) per block
+    condensed_pairs_kernel<<<grid, 256, 0, st>>>(first, n, i0, rows, reinterpret_cast<uint2*>(pairs));
     return 1;
 }
 
@@ -3192,7 +3252,7 @@ int launch_row_topk(const double* scores, uint64_t rows, uint64_t cols, int k, i
 int launch_score(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a, double mean_b,
                  const LaunchOverrides& ov, cudaStream_t st) {
     if (!args.n_pairs) return 0;
-    if (args.tiles) return launch_tiles(args, p, max_a, max_b, mean_a, mean_b, ov, false, st);
+    if (args.tiles) return launch_tiles(args, p, max_a, max_b, mean_a, mean_b, ov, TileMode::kJobs, st);
     const unsigned pad_max = ((max_a + 1) & ~1u) + ((max_b + 1) & ~1u);
     const bool key_is_w = args.a.key_is_w != 0;
     const bool fast = p.hell2 && p.C <= 16;   // Hellinger-2 with or without category weights

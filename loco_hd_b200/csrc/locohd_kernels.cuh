@@ -191,6 +191,43 @@ struct CrossGrid {
 static_assert(sizeof(CrossGrid) <= sizeof(TileOrder), "shares TileOrder's place in ScoreArgs: the layout is unchanged");
 __host__ __device__ inline uint64_t cross_units(const CrossGrid& g) { return ((g.rows + 3) / 4) * ((g.cols + 3) / 4); }
 
+// Condensed mode of score_tile_kernel: the pairs i < j of one range, environments first + i and first + j (i, j < n)
+// of one env-set, score (i, j) at out[n i - i (i + 1) / 2 + (j - i - 1) - base] (scipy's pdist order; base: the
+// condensed index of the chunk's first score).  A chunk is the row blocks [rb0, rb0 + row_blocks) of the nb = ceil(n / 4)
+// blocks of 4 rows; its units are the blocks (rb, cb) with rb <= cb < nb, column block major as in cross mode, rows
+// ascending within a column block: a triangle of T(row_blocks) units for the column blocks of the chunk's own rows,
+// T(k) = k (k + 1) / 2, then a rectangle of row_blocks units per column block.
+struct CondensedGrid {
+    uint64_t first, n;
+    uint64_t rb0, row_blocks;
+    uint64_t base;
+};
+static_assert(sizeof(CondensedGrid) <= sizeof(TileOrder), "shares TileOrder's place in ScoreArgs: the layout is unchanged");
+template <class T>
+__host__ __device__ inline T triangle(T k) { return (k & 1) ? k * ((k + 1) >> 1) : (k >> 1) * (k + 1); }
+__host__ __device__ inline uint64_t condensed_units(const CondensedGrid& g) {
+    const uint64_t R = g.row_blocks, nb = (g.n + 3) / 4;
+    return triangle<uint64_t>(R) + R * (nb - g.rb0 - R);
+}
+// Unit u of a chunk of R row blocks -> (dr, dc): row block rb0 + dr, column block rb0 + dc.  Exact for every u below
+// the unit count as long as T(R) fits in T: the double square root may be one off, the integer steps correct it.
+template <class T>
+__host__ __device__ inline void condensed_unit(T R, T u, T* dr, T* dc) {
+    const T tri = triangle<T>(R);
+    if (u < tri) {   // column block k of the triangle holds its row blocks 0 .. k at units T(k) .. T(k + 1) - 1
+        T k = (T)((sqrt(8.0 * (double)u + 1.0) - 1.0) * 0.5);
+        if (k >= R) k = R - 1;
+        while (triangle<T>(k) > u) --k;
+        while (triangle<T>(k + 1) <= u) ++k;
+        *dc = k;
+        *dr = u - triangle<T>(k);
+    } else {
+        const T v = u - tri, q = v / R;
+        *dc = R + q;
+        *dr = v - q * R;
+    }
+}
+
 struct ScoreArgs {
     const ScoreTile* tiles;        // tile mode (score_tile_kernel): jobs grouped by the host, uniform_n anchors each
     uint64_t n_tiles;
@@ -210,6 +247,7 @@ struct ScoreArgs {
     union {                        // tile kernel, read from the parameter bank:
         TileOrder order;           //   job tiles: unit -> (tile, anchor), slice by slice
         CrossGrid cross;           //   cross matrix (launch_score_cross): unit -> (row block, column block)
+        CondensedGrid condensed;   //   upper triangle of one range (launch_score_condensed): the same, rb <= cb
     };
     unsigned long long* cursor;    // fast kernel: next unclaimed pair (zeroed before the launch); warps claim runs of
                                    // `run` consecutive pairs, so all resident warps work at one moving frontier
@@ -257,8 +295,8 @@ int launch_rows_copy(const double* values, const double* xyz, const uint8_t* cat
 // read_launch_overrides() once per API call, so that a process can change them between calls.  The defaults leave
 // every decision to the library.  No other code of the library reads the environment.
 struct LaunchOverrides {
-    bool no_tiles = false;        // LOCOHD_NO_TILES (non-zero integer): job lists and cross matrices never take
-                                  // score_tile_kernel
+    bool no_tiles = false;        // LOCOHD_NO_TILES (non-zero integer): job lists, cross matrices and condensed
+                                  // vectors never take score_tile_kernel
     int tile_teams = 0;           // LOCOHD_TILE_TEAMS: lowers TileGeometry::teams when in [1, teams)
     int tile_rep = -1;            // LOCOHD_TILE_REP: lowers TileGeometry::rep_n when in [0, rep_n)
     unsigned tile_run = 0;        // LOCOHD_TILE_RUN (1 ... 4096): longest run of units a team claims (0: kTileRun)
@@ -267,8 +305,8 @@ struct LaunchOverrides {
     double tile_slice_mb = 0.0;   // LOCOHD_TILE_SLICE_MB (> 0): that L2 budget in MB (0: the default)
     bool legacy_gather = false;   // LOCOHD_LEGACY_GATHER (any value not starting with '0'): environments are built
                                   // with the multi-kernel gather
-    uint64_t cross_rows = 0;      // LOCOHD_CROSS_ROWS (> 0): lowers the rows of a cross-matrix chunk (rounded down to a
-                                  // multiple of 4, at least 4)
+    uint64_t cross_rows = 0;      // LOCOHD_CROSS_ROWS (> 0): lowers the rows of a cross-matrix or condensed chunk
+                                  // (rounded down to a multiple of 4, at least 4)
 };
 LaunchOverrides read_launch_overrides();
 int launch_score(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a, double mean_b,
@@ -280,6 +318,13 @@ int launch_score_cross(const ScoreArgs& args, const KParams& p, unsigned max_a, 
 // Explicit pairs (a_first + row, b_first + column) of every entry of a rows x cols block, row-major, into pairs
 // [rows * cols][2]: the cross matrix on the pair kernel.
 int launch_cross_pairs(uint64_t a_first, uint64_t b_first, uint64_t rows, uint64_t cols, uint32_t* pairs, cudaStream_t st);
+// The chunk args.condensed of a condensed vector on the tile kernel (args.out, args.a, args.cursor are read; args.b is
+// args.a).  Returns the number of launches.
+int launch_score_condensed(const ScoreArgs& args, const KParams& p, unsigned max_count, const LaunchOverrides& ov,
+                           cudaStream_t st);
+// Explicit pairs (first + i, first + j), i < j < n, of the rows i0 <= i < i0 + rows in condensed order into
+// pairs [..][2]: a chunk of the condensed vector on the pair kernel.
+int launch_condensed_pairs(uint64_t first, uint64_t n, uint64_t i0, uint64_t rows, uint32_t* pairs, cudaStream_t st);
 // k nearest (1 <= k <= 32) of every row of scores [rows][cols]: ascending, equal scores by smaller column, NaN after
 // +inf (-0.0 and +0.0 are equal).  Column self_off + r of row r is left out (self_off = INT64_MIN: none is).  Row r
 // writes knn_scores / knn_index [r * k ...] (either may be nullptr); every row must have k eligible columns.

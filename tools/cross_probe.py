@@ -11,6 +11,10 @@ Shapes:
   * 5 000 x 100 000 k nearest (k = 16, matrix kept on the device) and the device memory that call takes at its peak
     (cudaMemGetInfo sampled every millisecond from a second thread while the call runs, above the value before
     the context's first scoring call).
+  * condensed vectors of one range (locohd_score_condensed) against score_cross of the range against itself, the two
+    calls alternated rep by rep: the first 20 000 environments into device and into host memory, the first 50 000
+    into device memory only (a 20 GB matrix), each on the tile route and the LOCOHD_NO_TILES=1 pair route; the
+    vector is checked bit for bit against the matrix's strict upper triangle on the device.
 Times are host clocks around whole calls (each ends in a device synchronisation): median of --reps after --warmup.
 The card's name and power limit are read in the same run.  Prints one JSON line per measurement, appends them to --out.
 --lib runs against another build of the library (the A/B of the kernel's unit order); --only restricts to names
@@ -167,8 +171,61 @@ def main():
     kj = blocked_jobs(0, 1, PER, 10_000)
     timed("score_batch_1x10000", 1e4, lambda: ctx.score_jobs_stats(env, env, kj, scores=True))
 
+    condensed(ctx, env)
     env.close()
     st.close()
+
+
+def alternated(name, a, b):
+    """a, b: (label, pairs, f).  The two calls alternate rep by rep, so drifts of the shared host and clocks hit both."""
+    if args.only not in name:
+        return
+    for _ in range(args.warmup):
+        a[2]()
+        b[2]()
+    t = {a[0]: [], b[0]: []}
+    for _ in range(args.reps):
+        for label, _, f in (a, b):
+            t0 = time.perf_counter()
+            f()
+            t[label].append(time.perf_counter() - t0)
+    med = {k: float(np.median(v)) for k, v in t.items()}
+    for label, pairs, _ in (a, b):
+        emit({"name": f"{name}_{label}", "pairs": int(pairs), "ms": round(1e3 * med[label], 3),
+              "ms_min": round(1e3 * min(t[label]), 3), "ms_max": round(1e3 * max(t[label]), 3),
+              "pairs_per_s": pairs / med[label]})
+    emit({"name": f"{name}_ratio", f"{a[0]}_over_{b[0]}": round(med[a[0]] / med[b[0]], 4)})
+
+
+def condensed(ctx, env):
+    for route in ("tiles", "pairs"):
+        if route == "pairs":
+            os.environ["LOCOHD_NO_TILES"] = "1"
+        for n, outs in ((20_000, ("device", "host")), (50_000, ("device",))):
+            name = f"condensed_{n}_{route}"
+            if args.only not in name:
+                continue
+            for where in outs:
+                if where == "device":
+                    vec = torch.empty(n * (n - 1) // 2, dtype=torch.float64, device="cuda")
+                    mat = torch.empty((n, n), dtype=torch.float64, device="cuda")
+                    kv, km = dict(out=vec.data_ptr()), dict(scores=mat.data_ptr())
+                else:
+                    kv, km = {}, {}
+                t0 = ctx.tile_launches
+                alternated(f"{name}_{where}",
+                           ("condensed", n * (n - 1) // 2, lambda: ctx.score_condensed(env, 0, n, **kv)),
+                           ("matrix", n * n, lambda: ctx.score_cross(env, env, 0, n, 0, n, **km)))
+                emit({"name": f"{name}_{where}_tile_launches", "tile_launches": ctx.tile_launches - t0})
+                if where == "device":
+                    iu = torch.triu_indices(n, n, 1, device="cuda")
+                    upper = mat[iu[0], iu[1]]
+                    del iu
+                    same = bool(torch.equal(upper.view(torch.int64), vec.view(torch.int64)))
+                    emit({"name": f"{name}_device_equals_matrix_upper_triangle", "bit_identical": same})
+                    del upper, vec, mat
+                    torch.cuda.empty_cache()
+    os.environ.pop("LOCOHD_NO_TILES", None)
 
 
 main()
