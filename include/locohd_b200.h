@@ -139,6 +139,10 @@ uint64_t locohd_ctx_launch_count(const locohd_ctx* ctx);
 /* How many of them were the tile scoring kernel (locohd_score_jobs[_stats] on job lists whose jobs share runs of
  * environments, e.g. the all-vs-all ensemble of compare_ensembles.py:250-296 listed in 4 x 4 blocks). */
 uint64_t locohd_ctx_tile_launches(const locohd_ctx* ctx);
+/* How many of those were the wide form, one CTA per 32 x 32 tile of jobs and one lane per anchor pair: taken when
+ * the list fills such tiles to at least 80 % and their stage fits shared memory, unless LOCOHD_WIDE_TILES=0 is set in
+ * the environment (the 4 x 4 tiles then score the list). */
+uint64_t locohd_ctx_wide_launches(const locohd_ctx* ctx);
 /* Per-kernel timing with CUDA events on the context stream (benchmark roofline accounting).  While enabled every
  * kernel group is bracketed by a pair of events; locohd_ctx_profile_read waits for the stream, adds the elapsed
  * times per group to ms[k] / launches[k] (k < LOCOHD_PROF_GROUPS, see locohd_prof_group) and clears the records. */

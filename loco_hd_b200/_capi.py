@@ -25,6 +25,7 @@ SD_KINDS = {"Hellinger": 0, "Kolmogorov-Smirnov": 1, "Kullback-Leibler": 2, "Ren
 EXPORTED_SYMBOLS = [
     "locohd_abi_version", "locohd_device_count", "locohd_ctx_create", "locohd_ctx_destroy", "locohd_last_error",
     "locohd_ctx_set_params", "locohd_ctx_stream", "locohd_ctx_synchronize", "locohd_ctx_launch_count", "locohd_ctx_tile_launches",
+    "locohd_ctx_wide_launches",
     "locohd_ctx_profile_enable", "locohd_ctx_profile_read", "locohd_measure_fp64_tflops",
     "locohd_host_alloc", "locohd_host_free", "locohd_structs_create", "locohd_structs_create_f32",
     "locohd_structs_destroy", "locohd_structs_update_xyz", "locohd_structs_update_xyz_f32",
@@ -100,6 +101,7 @@ def load_library() -> C.CDLL:
         "locohd_ctx_synchronize": (C.c_int, [vp]),
         "locohd_ctx_launch_count": (u64, [vp]),
         "locohd_ctx_tile_launches": (u64, [vp]),
+        "locohd_ctx_wide_launches": (u64, [vp]),
         "locohd_ctx_profile_enable": (C.c_int, [vp, C.c_int]),
         "locohd_ctx_profile_read": (C.c_int, [vp, vp, vp]),
         "locohd_measure_fp64_tflops": (C.c_int, [vp, C.POINTER(dbl)]),
@@ -257,6 +259,11 @@ class Context:
     @property
     def tile_launches(self) -> int:
         return int(self.lib.locohd_ctx_tile_launches(self.h))
+
+    @property
+    def wide_launches(self) -> int:
+        """The part of tile_launches that ran the wide (32 x 32) tile kernel."""
+        return int(self.lib.locohd_ctx_wide_launches(self.h))
 
     def synchronize(self):
         self._check(self.lib.locohd_ctx_synchronize(self.h))

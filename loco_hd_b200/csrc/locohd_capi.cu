@@ -23,10 +23,13 @@ namespace {
 std::mutex g_err_mutex;
 std::string g_global_err;
 
-// A job list grouped into tiles (plan_job_tiles) and whether score_tile_kernel pays for that grouping (tiles_pay)
+// A job list grouped into tiles (plan_job_tiles) and whether score_tile_kernel pays for that grouping (tiles_pay);
+// the same list in wide tiles and whether they are filled well enough for score_wide_kernel (wide_tiles_pay)
 struct TilePlan {
     std::vector<ScoreTile> tiles;
     bool pays = false;
+    std::vector<WideTile> wide;
+    bool wide_pays = false;
 };
 }
 
@@ -36,6 +39,7 @@ struct locohd_ctx {
     std::string err;
     uint64_t launches = 0;
     uint64_t tile_launches = 0;
+    uint64_t wide_launches = 0;   // the part of tile_launches that ran score_wide_kernel
     // tile plan of the last job list (a benchmark step, the next block of frames: the same list again)
     std::vector<locohd_job> tile_cache_jobs;
     TilePlan tile_cache_plan;
@@ -621,12 +625,15 @@ std::vector<ScoreTile> group_job_tiles(const std::vector<locohd_job>& jobs, cons
     return tiles;
 }
 
-// The same for job lists in any order (plain row-major (i, j) order of an ensemble, shuffled lists): the distinct A
-// runs and B runs are ranked, a job belongs to block (rank_a / 4, rank_b / 4) and sits in cell (rank_a % 4, rank_b % 4)
-// of it; blocks are scored in (block row, block column) order, which keeps the structures of a block row in L2.  A job
-// named twice opens a second tile of its block.  O(n log n) on the host, so it is only tried when the list order
-// itself does not tile.
-std::vector<ScoreTile> group_job_tiles_sorted(const std::vector<locohd_job>& jobs, const std::vector<uint64_t>& joff) {
+// The same for job lists in any order (plain row-major (i, j) order of an ensemble, shuffled lists) and for tiles of
+// any size DIM: the distinct A runs and B runs are ranked, a job belongs to block (rank_a / DIM, rank_b / DIM) and
+// sits in cell (rank_a % DIM, rank_b % DIM) of it; blocks are scored in (block row, block column) order, which keeps
+// the structures of a block row in L2.  A job named twice opens a second tile of its block.  O(n log n) on the host,
+// so at DIM = 4 it is only tried when the list order itself does not tile.  More than max_tiles tiles: stops and
+// returns no tiles (a list that cannot fill its tiles).
+template <int DIM>
+std::vector<TileDesc<DIM>> group_job_tiles_sorted(const std::vector<locohd_job>& jobs, const std::vector<uint64_t>& joff,
+                                                  size_t max_tiles = SIZE_MAX) {
     std::vector<uint64_t> av(jobs.size()), bv(jobs.size());
     for (size_t j = 0; j < jobs.size(); ++j) { av[j] = jobs[j].a_first; bv[j] = jobs[j].b_first; }
     std::sort(av.begin(), av.end()); av.erase(std::unique(av.begin(), av.end()), av.end());
@@ -636,10 +643,10 @@ std::vector<ScoreTile> group_job_tiles_sorted(const std::vector<locohd_job>& job
     for (size_t j = 0; j < jobs.size(); ++j) {
         const uint64_t ra = (uint64_t)(std::lower_bound(av.begin(), av.end(), jobs[j].a_first) - av.begin());
         const uint64_t rb = (uint64_t)(std::lower_bound(bv.begin(), bv.end(), jobs[j].b_first) - bv.begin());
-        items[j] = {((ra / kTileDim) << 32) | (rb / kTileDim), (uint32_t)((ra % kTileDim) * kTileDim + rb % kTileDim), (uint32_t)j};
+        items[j] = {((ra / DIM) << 32) | (rb / DIM), (uint32_t)((ra % DIM) * DIM + rb % DIM), (uint32_t)j};
     }
     std::stable_sort(items.begin(), items.end(), [](const Item& x, const Item& y) { return x.block < y.block; });
-    std::vector<ScoreTile> tiles;
+    std::vector<TileDesc<DIM>> tiles;
     size_t lo = 0;
     while (lo < items.size()) {
         size_t hi = lo;
@@ -647,14 +654,15 @@ std::vector<ScoreTile> group_job_tiles_sorted(const std::vector<locohd_job>& job
         size_t first_tile = tiles.size();
         for (size_t k = lo; k < hi; ++k) {
             const Item& it = items[k];
-            const int r = (int)(it.cell / kTileDim), c = (int)(it.cell % kTileDim);
+            const int r = (int)(it.cell / DIM), c = (int)(it.cell % DIM);
             size_t t = first_tile;   // first tile of this block whose cell is still free
             while (t < tiles.size() && tiles[t].out_first[it.cell] != kTileNone) ++t;
             if (t == tiles.size()) {
-                ScoreTile nt;
-                for (int q = 0; q < kTileDim; ++q) { nt.a_first[q] = kTileNone; nt.b_first[q] = kTileNone; }
-                for (int q = 0; q < kTileDim * kTileDim; ++q) nt.out_first[q] = kTileNone;
-                tiles.push_back(nt);
+                if (tiles.size() == max_tiles) return {};
+                tiles.emplace_back();
+                TileDesc<DIM>& nt = tiles.back();
+                for (int q = 0; q < DIM; ++q) { nt.a_first[q] = kTileNone; nt.b_first[q] = kTileNone; }
+                for (int q = 0; q < DIM * DIM; ++q) nt.out_first[q] = kTileNone;
             }
             tiles[t].a_first[r] = jobs[it.job].a_first;
             tiles[t].b_first[c] = jobs[it.job].b_first;
@@ -680,6 +688,12 @@ bool tiles_pay(const std::vector<ScoreTile>& tiles, uint64_t n_jobs) {
     return !tiles.empty() && n_jobs * 10 >= rows * kTileDim * 6 && rows >= 3 * tiles.size();
 }
 
+// A wide tile is one CTA of 1024 lanes, one per cell: it pays when at least 80 % of the cells hold a job.  Measured
+// against the 4 x 4 tiles (B200, profiles/r16a_wide_tiles.md): 1.20 x on the 1000-member ensemble in blocked order
+// (92 % filled), 0.98 x on 96 members (74 %); the 4 x 4 tiles, whose rows are one warp each, waste fewer lanes.
+constexpr uint64_t kWideFillPct = 80;
+size_t wide_tiles_max(uint64_t n_jobs) { return (size_t)(n_jobs * 100 / (kWideFillPct * kWideDim * kWideDim)); }
+
 // The list order itself (batch.py::blocked_pairs) when its tiles pay, else the sorted grouping (any other order).
 // Lists of fewer than 4 jobs, of unequal jobs or of empty jobs get no tiles.
 TilePlan plan_job_tiles(const std::vector<locohd_job>& jobs, const std::vector<uint64_t>& joff) {
@@ -690,8 +704,13 @@ TilePlan plan_job_tiles(const std::vector<locohd_job>& jobs, const std::vector<u
     plan.tiles = group_job_tiles(jobs, joff);
     plan.pays = tiles_pay(plan.tiles, jobs.size());
     if (!plan.pays) {
-        plan.tiles = group_job_tiles_sorted(jobs, joff);
+        plan.tiles = group_job_tiles_sorted<kTileDim>(jobs, joff);
         plan.pays = tiles_pay(plan.tiles, jobs.size());
+    }
+    const size_t wide_max = wide_tiles_max(jobs.size());
+    if (wide_max > 0) {
+        plan.wide = group_job_tiles_sorted<kWideDim>(jobs, joff, wide_max);
+        plan.wide_pays = !plan.wide.empty();
     }
     return plan;
 }
@@ -699,9 +718,10 @@ TilePlan plan_job_tiles(const std::vector<locohd_job>& jobs, const std::vector<u
 int run_score(locohd_ctx* ctx, const locohd_envset* a, const locohd_envset* b, uint64_t n_pairs,
               const uint32_t* d_pairs, const locohd_job* d_jobs, const uint64_t* d_job_off, uint64_t n_jobs,
               uint64_t uniform_n, const uint32_t* d_wf_idx, double* d_out, const LaunchOverrides& ov,
-              const ScoreTile* d_tiles = nullptr, uint64_t n_tiles = 0) {
+              const ScoreTile* d_tiles = nullptr, uint64_t n_tiles = 0, const WideTile* d_wide = nullptr) {
     ScoreArgs sa{};
     sa.tiles = d_tiles; sa.n_tiles = n_tiles;
+    if (d_wide) { sa.wide_tiles = d_wide; sa.wide = 1; }
     sa.a = a->view(); sa.b = b->view();
     sa.n_pairs = n_pairs; sa.pairs = d_pairs; sa.jobs = d_jobs; sa.job_pair_off = d_job_off; sa.n_jobs = n_jobs;
     sa.uniform_n = uniform_n; sa.wf_idx = d_wf_idx; sa.out = d_out; sa.stage_cap = 0; sa.only_unstaged = 0; sa.table_n = 0;
@@ -714,7 +734,8 @@ int run_score(locohd_ctx* ctx, const locohd_envset* a, const locohd_envset* b, u
       n = launch_score(sa, ctx->kp, a->max_count, b->max_count, mean_a, mean_b, ov, ctx->stream); }
     if (n < 0) return fail(ctx, LOCOHD_ERR_UNSUPPORTED, "shared memory budget exceeded for %d categories", ctx->kp.C);
     ctx->launches += n;
-    if (d_tiles) ctx->tile_launches += n;
+    if (d_tiles || d_wide) ctx->tile_launches += n;
+    if (d_wide) ctx->wide_launches += n;
     CU(ctx, cudaGetLastError());
     return 0;
 }
@@ -832,6 +853,7 @@ void* locohd_ctx_stream(locohd_ctx* ctx) { return ctx ? (void*)ctx->stream : nul
 
 uint64_t locohd_ctx_launch_count(const locohd_ctx* ctx) { return ctx ? ctx->launches : 0; }
 uint64_t locohd_ctx_tile_launches(const locohd_ctx* ctx) { return ctx ? ctx->tile_launches : 0; }
+uint64_t locohd_ctx_wide_launches(const locohd_ctx* ctx) { return ctx ? ctx->wide_launches : 0; }
 
 int locohd_ctx_synchronize(locohd_ctx* ctx) {
     API_BEGIN(ctx)
@@ -1485,9 +1507,12 @@ int locohd_score_jobs_stats(locohd_ctx* ctx, const locohd_envset* a, const locoh
     if (anchor_stats && (st = dev_alloc(ctx, &d_stat, 2 * n_per_job))) return cleanup(st);
     // Jobs that share runs of environments (an all-vs-all ensemble in 4 x 4 blocks) go to the tile kernel, which
     // stages every environment once per tile instead of once per pair.  It pays when the tiles are mostly full and
-    // at least 6 teams fit an SM: below that, one pair per warp with a stage of its own is the better kernel.
+    // at least 6 teams fit an SM: below that, one pair per warp with a stage of its own is the better kernel.  Lists
+    // that fill 32 x 32 tiles well go to the wide tile kernel when its stage fits (one lane per pair, no per-pair
+    // split: 1.2 x the rate of the 4 x 4 tiles on the 1000-member ensemble, profiles/r16a_wide_tiles.md).
     const LaunchOverrides ov = read_launch_overrides();
     InBuf<ScoreTile> dtiles;
+    InBuf<WideTile> dwide;
     TilePlan plan;   // alive until the call's final synchronisation
     if (!wf_idx && a->key_is_w && b->key_is_w && !ov.no_tiles &&
         tile_geometry(ctx->kp, a->max_count, b->max_count, 1, ov).teams >= 6) {
@@ -1501,11 +1526,18 @@ int locohd_score_jobs_stats(locohd_ctx* ctx, const locohd_envset* a, const locoh
                 ctx->tile_cache_plan = plan;
             }
         }
-        if (plan.pays && (st = dtiles.load(ctx, plan.tiles.data(), plan.tiles.size()))) return cleanup(st);
+        if (!(plan.wide_pays && ov.wide_tiles && wide_geometry(ctx->kp, a->max_count, b->max_count, 1, ov).fits))
+            plan.wide_pays = false;
+        if (plan.wide_pays) {
+            if ((st = dwide.load(ctx, plan.wide.data(), plan.wide.size()))) return cleanup(st);
+        } else if (plan.pays && (st = dtiles.load(ctx, plan.tiles.data(), plan.tiles.size()))) {
+            return cleanup(st);
+        }
     }
-    const uint64_t n_tiles = plan.pays ? plan.tiles.size() : 0;
+    const uint64_t n_tiles = plan.wide_pays ? plan.wide.size() : plan.pays ? plan.tiles.size() : 0;
     st = run_score(ctx, a, b, n_pairs, nullptr, dj.ptr, djoff.ptr, n_jobs, (uniform && hj[0].n) ? hj[0].n : 0,
-                   wf.ptr, d_scores, ov, n_tiles ? dtiles.ptr : nullptr, n_tiles);
+                   wf.ptr, d_scores, ov, (n_tiles && !plan.wide_pays) ? dtiles.ptr : nullptr, n_tiles,
+                   (n_tiles && plan.wide_pays) ? dwide.ptr : nullptr);
     if (!st && (means.ptr || anchor_stats)) {
         ProfScope ps(ctx, LOCOHD_PROF_OTHER);
         if (means.ptr) ctx->launches += launch_job_means(d_scores, djoff.ptr, n_jobs, means.ptr, ctx->stream);

@@ -17,6 +17,8 @@
 //   K2t  score_tile_kernel      job lists whose jobs share runs of environments (all-vs-all ensembles): a team of four
 //                               warps per (4 x 4 tile of structure pairs, anchor) stages the 8 environments once and
 //                               scores the 16 anchor pairs with 8 lanes each
+//   K2w  score_wide_kernel      the same on 32 x 32 tiles when they are well filled (the all-vs-all ensemble): one CTA
+//                               per (tile, anchor) stages the 64 environments once, one lane walks one anchor pair
 //   fallback gather (environments the fused kernel cannot take, rows of from_dmxs / from_coords):
 //   K1a  env_tile_kernel<false> one THREAD per anchor: FP32 prefilter over the candidate cells, counts the
 //                               survivors (upper bound of the environment size) -> scan -> store offsets
@@ -2550,6 +2552,269 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Wide tile kernel: the job tiles of score_tile_kernel at kWideDim x kWideDim, one lane per anchor pair.  A unit is
+// (wide tile, anchor) in the same sliced order (TileOrder); one CTA of 32 warps stages the <= 32 row and <= 32 column
+// environments of a unit (bulk copies on one mbarrier, fixed slots) and warp r, lane c scores pair (r, c): it starts
+// from the two anchors and walks all na + nb events of the merged list itself.  There is no merge-path split, no
+// per-chunk histogram, no prefix scan of counts and no reduction - the set-up score_tile_kernel needs because it
+// splits a pair over 8 lanes (~340 of its ~1 000 warp instructions and ~100 of its ~316 shared-memory wavefronts
+// per pair, DESIGN §3).  Staged environments per warp stay at 2, as in a team of four warps, so the
+// stage of the bench's largest environments (345 members) is the same ~178 KB and 32 warps still fit an SM.
+// The event arithmetic is that of score_tile_kernel (replicated head tables, count words of 8 count, 2 H, identical
+// compositions through m, the small-H^2 difference form); D and R are rebuilt from the counts at least every
+// kWideBlock events, so a walk keeps the bound of <= 128 roundings of either (~3e-14 relative, DESIGN §3).  The walk
+// is kept apart from score_tile_kernel's: sharing the event step would have to leave the nine instantiations of that
+// kernel instruction for instruction as they are (profiles/r16a_wide_tiles.md).
+constexpr int kWideThreads = kWideDim * 32;   // 1024: warp r = row r, lane c = column c
+constexpr int kWideBlock = 128;               // events between two rebuilds of D and R from the counts
+struct WideCtrl {
+    uint64_t mbar;
+    uint32_t tile[2];     // as TileCtrl: tile and anchor of the current unit and of the next one, slot = iteration & 1
+    uint32_t p[2];
+    uint32_t state;       // 0 = score, 1 = skip (an error was raised), 2 = no units left
+    uint32_t pad;
+    uint32_t M[2 * kWideDim];          // sizes of rows 0..31 and columns 0..31 of the current unit (0: absent)
+    // descriptor of the next unit: written by fetch() and read back by the loader warp only (lane l: row l, column l)
+    uint64_t nx_off[2 * kWideDim];
+    uint64_t nx_last[2 * kWideDim];    // an odd last member, stored by hand behind the bulk copy
+    uint32_t nx_M[2 * kWideDim];       // ~0u: absent
+};
+constexpr int kWideCtrlBytes = (int)((sizeof(WideCtrl) + 15) & ~size_t(15));
+
+template <int CP, bool REP>
+__global__ void __launch_bounds__(kWideThreads, 1) score_wide_kernel(ScoreArgs a, KParams P, int slot_a, int slot_b) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int lane = threadIdx.x & 31, row = threadIdx.x >> 5;
+    const int table_n = a.table_n;
+    const int rep_n = REP ? a.rep_n : 0;   // tables as in score_tile_kernel
+    const int mix_n = 15 * rep_n + table_n;
+    // count rows first: the row address of any category byte (cnt_lane + 128 byte) lies inside the allocation
+    // (wide_geometry), whatever the staged keys hold
+    uint32_t* cnt = reinterpret_cast<uint32_t*>(smem_raw) + row * CP * 32;   // [CP][32] per warp, as score_tile_kernel
+    WideCtrl* ctrl = reinterpret_cast<WideCtrl*>(smem_raw + CP * kWideThreads * 4);
+    double* s_ratio = reinterpret_cast<double*>(smem_raw + CP * kWideThreads * 4 + kWideCtrlBytes);
+    double* s_sqrt = s_ratio + table_n;
+    double* s_dsq = s_sqrt + mix_n;
+    uint64_t* stage_a = reinterpret_cast<uint64_t*>(s_dsq + mix_n);   // rows: slot_a keys each, then the columns
+    uint64_t* stage_b = stage_a + kWideDim * slot_a;
+    for (int x = threadIdx.x; x < table_n; x += blockDim.x) s_ratio[x] = sqrt((double)x / (double)(x + 1));
+    for (int x = threadIdx.x; x < mix_n; x += blockDim.x) {
+        const int e = x < 16 * rep_n ? x >> 4 : x - 15 * rep_n;
+        const double s0 = P.sqrt_tbl[e], s1 = P.sqrt_tbl[e + 1];
+        s_sqrt[x] = s0;
+        s_dsq[x] = s1 - s0;
+    }
+    // the loader is the last warp: on a diagonal tile its row has no pair above the diagonal, on a partial tile it is
+    // the first row to be absent
+    const bool loader = row == kWideDim - 1;
+    if (threadIdx.x == 0) { mbar_init(&ctrl->mbar, 1); fence_proxy_async(); }
+    const int C = P.C;
+    unsigned flags = 0;   // bit 0: parity of the mbarrier, bit 1: control-block slot of the NEXT fetch
+    const uint32_t sq_base = __shfl_sync(kFull, smem_u32(s_sqrt), lane);
+    const uint32_t dsq_base = __shfl_sync(kFull, smem_u32(s_dsq), lane);
+    const uint32_t ratio_base = __shfl_sync(kFull, smem_u32(s_ratio), lane);
+    const uint32_t cnt_lane = __shfl_sync(kFull, smem_u32(cnt + lane), lane);
+    const uint32_t copy8 = 8u * (lane & 15), cap8 = 120u * (uint32_t)rep_n;
+    const uint32_t sq_copy = __shfl_sync(kFull, sq_base + copy8, lane), sq_cap = __shfl_sync(kFull, sq_base + cap8, lane);
+    const uint32_t dsq_copy = __shfl_sync(kFull, dsq_base + copy8, lane), dsq_cap = __shfl_sync(kFull, dsq_base + cap8, lane);
+    auto sq_addr = [&](uint32_t e8) -> uint32_t { return REP ? min(16u * e8 + sq_copy, e8 + sq_cap) : sq_base + e8; };
+    auto dsq_addr = [&](uint32_t e8) -> uint32_t { return REP ? min(16u * e8 + dsq_copy, e8 + dsq_cap) : dsq_base + e8; };
+    const uint64_t n = a.uniform_n, n_units = a.n_tiles * n;
+    const WfDev& wf = P.wfs[0];
+
+    // The loader warp fetches the descriptor of the NEXT unit right after the CTA was released into the current one
+    // (lane l: row l and column l), claiming runs of units from a.cursor as score_tile_kernel does.
+    uint64_t run_pos = 0, run_end = 0, nx_unit = 0;   // loader warp, uniform
+    auto fetch = [&]() {
+        if (run_pos == run_end) {
+            unsigned long long got = 0;
+            if (lane == 0) got = atomicAdd(a.cursor, (unsigned long long)a.run);
+            got = __shfl_sync(kFull, got, 0);
+            run_pos = min((uint64_t)got, n_units);
+            run_end = min((uint64_t)got + a.run, n_units);
+        }
+        const uint64_t u = run_pos;
+        if (run_pos < run_end) ++run_pos;
+        nx_unit = u;
+        uint64_t off_a = 0, off_b = 0, last_a = 0, last_b = 0;
+        uint32_t m_a = ~0u, m_b = ~0u;
+        if (u < n_units) {
+            uint64_t tile, p;
+            if (((n_units | n) >> 32) == 0) { uint32_t t32, p32; tile_unit<uint32_t>(a.order, (uint32_t)u, &t32, &p32); tile = t32; p = p32; }
+            else tile_unit<uint64_t>(a.order, u, &tile, &p);
+            if (lane == 0) { ctrl->tile[(flags >> 1) & 1u] = (uint32_t)tile; ctrl->p[(flags >> 1) & 1u] = (uint32_t)p; }
+            const WideTile& T = a.wide_tiles[tile];
+            const uint64_t fa = __ldg(T.a_first + lane), fb = __ldg(T.b_first + lane);
+            if (fa != kTileNone) {
+                off_a = __ldg(a.a.off + fa + p);
+                m_a = __ldg(a.a.count + fa + p);
+                if (m_a & 1u) last_a = __ldg(a.a.key + off_a + m_a - 1);
+            }
+            if (fb != kTileNone) {
+                off_b = __ldg(a.b.off + fb + p);
+                m_b = __ldg(a.b.count + fb + p);
+                if (m_b & 1u) last_b = __ldg(a.b.key + off_b + m_b - 1);
+            }
+        }
+        ctrl->nx_off[lane] = off_a; ctrl->nx_last[lane] = last_a; ctrl->nx_M[lane] = m_a;
+        ctrl->nx_off[kWideDim + lane] = off_b; ctrl->nx_last[kWideDim + lane] = last_b; ctrl->nx_M[kWideDim + lane] = m_b;
+    };
+    __syncthreads();   // tables and the mbarrier
+    if (loader) fetch();
+
+    for (;;) {
+        const uint32_t slot = (flags >> 1) & 1u;   // where fetch() left this unit's tile and anchor
+        flags ^= 2u;
+        __syncthreads();   // every warp is done with the stage of the previous unit
+        if (loader) {
+            uint32_t state = 0;
+            if (nx_unit >= n_units) state = 2;
+            else {
+                uint32_t m_a = ctrl->nx_M[lane], m_b = ctrl->nx_M[kWideDim + lane];
+                const bool has_a = m_a != ~0u, has_b = m_b != ~0u;
+                if (__any_sync(kFull, (has_a && m_a == 0) || (has_b && m_b == 0))) { raise(P.err, LOCOHD_ERR_EMPTY_ENV); state = 1; }
+                if (!has_a || state) m_a = 0;
+                if (!has_b || state) m_b = 0;
+                // the even part of an environment comes as one bulk copy; an odd last member is stored by hand, so the
+                // sentinel behind it is never overwritten by the copy
+                const uint32_t bytes_a = (m_a & ~1u) * 8u, bytes_b = (m_b & ~1u) * 8u;
+                uint32_t total = bytes_a + bytes_b;
+#pragma unroll
+                for (int o = 16; o; o >>= 1) total += __shfl_xor_sync(kFull, total, o);
+                if (state == 0) {
+                    if (lane == 0) { fence_proxy_async(); mbar_expect_tx(&ctrl->mbar, total); }
+                    __syncwarp();
+                    uint64_t* sa = stage_a + lane * slot_a;
+                    uint64_t* sb = stage_b + lane * slot_b;
+                    if (m_a) {
+                        if (bytes_a) { fence_proxy_async(); bulk_g2s(sa, a.a.key + ctrl->nx_off[lane], bytes_a, &ctrl->mbar); }
+                        if (m_a & 1u) sa[m_a - 1] = ctrl->nx_last[lane];
+                        sa[m_a] = kSentinel;
+                    }
+                    if (m_b) {
+                        if (bytes_b) { fence_proxy_async(); bulk_g2s(sb, a.b.key + ctrl->nx_off[kWideDim + lane], bytes_b, &ctrl->mbar); }
+                        if (m_b & 1u) sb[m_b - 1] = ctrl->nx_last[kWideDim + lane];
+                        sb[m_b] = kSentinel;
+                    }
+                }
+                ctrl->M[lane] = m_a;
+                ctrl->M[kWideDim + lane] = m_b;
+            }
+            if (lane == 0) ctrl->state = state;
+        }
+        __syncthreads();   // descriptor, hand-copied members and sentinels are visible
+        const uint32_t state = ctrl->state;
+        if (state == 2) break;
+        if (loader) fetch();
+        if (state == 1) continue;
+        mbar_wait(&ctrl->mbar, flags & 1u);
+        flags ^= 1u;
+        // Unknown categories (pmf.rs:38-42): every member of the staged environments once, warp w reading row w and
+        // column w.  A staged environment belongs to at least one job of the tile, so this is what the walks meet.
+        {
+            const uint32_t m_a = ctrl->M[row], m_b = ctrl->M[kWideDim + row];
+            const uint8_t* ca = reinterpret_cast<const uint8_t*>(stage_a + row * slot_a);
+            const uint8_t* cb = reinterpret_cast<const uint8_t*>(stage_b + row * slot_b);
+            bool unknown = false;
+            for (uint32_t k = lane; k < m_a; k += 32) unknown |= ca[8 * k] >= (uint32_t)C;
+            for (uint32_t k = lane; k < m_b; k += 32) unknown |= cb[8 * k] >= (uint32_t)C;
+            if (__syncthreads_or(unknown)) {
+                if (threadIdx.x == 0) raise(P.err, LOCOHD_ERR_UNKNOWN_CATEGORY);
+                continue;
+            }
+        }
+        const uint64_t out_first = __ldg(a.wide_tiles[ctrl->tile[slot]].out_first + row * kWideDim + lane);
+        const uint32_t Ma = ctrl->M[row], Mb = ctrl->M[kWideDim + lane];
+        const bool valid = out_first != kTileNone && Ma != 0 && Mb != 0;   // absent cells walk no event
+        if (!__any_sync(kFull, valid)) continue;
+        const uint64_t* kA = stage_a + row * slot_a;
+        const uint64_t* kB = stage_b + lane * slot_b;
+        const uint64_t keyA0 = kA[0], keyB0 = kB[0];
+        const uint32_t catA0 = (uint32_t)(keyA0 & kCatMask), catB0 = (uint32_t)(keyB0 & kCatMask);
+        // start compositions: the two anchors alone (locohd.rs:82-84)
+#pragma unroll
+        for (int r = 0; r < CP; ++r) cnt[r * 32 + lane] = (r == (int)catA0 ? 8u : 0u) + (r == (int)catB0 ? 0x80000u : 0u);
+        uint32_t left_all = valid ? (Ma - 1u) + (Mb - 1u) : 0u;
+        double wprev = key_value(max(keyA0 & kWMask, keyB0 & kWMask));
+        uint32_t pa = smem_u32(kA + 1), pb = smem_u32(kB + 1);
+        // ratio-table entry of a side's total (members taken, anchor included) at p + d: the total is 1 at p = kX + 1
+        const uint32_t dA = ratio_base + 8u - pa, dB = ratio_base + 8u - pb;
+        uint64_t ra = lds_u64(pa), rb = lds_u64(pb);
+        double rA, rB, h, acc = 0.0;
+        // 4 H^2 in the difference form from the counts (small H^2 only)
+        auto exact_4h2 = [&]() -> double {
+            double s = 0.0;
+#pragma unroll
+            for (int r = 0; r < CP; ++r) {
+                const uint32_t word = cnt[r * 32 + lane];
+                const double u = __dmul_rn(lds_f64(sq_addr(word & 0xffffu)), rA) - __dmul_rn(lds_f64(sq_addr(word >> 16)), rB);
+                s = fma(u, u, s);
+            }
+            return 2.0 * s;
+        };
+        for (;;) {
+            // D, R, sum_r |a_r - b_r| and H from the counts: at the anchors, then every kWideBlock events
+            rA = __ldg(P.rsqrt_tbl + ((pa + dA - ratio_base) >> 3));
+            rB = __ldg(P.rsqrt_tbl + ((pb + dB - ratio_base) >> 3));
+            uint32_t l1 = 0;
+            double D = 0.0;
+#pragma unroll
+            for (int r = 0; r < CP; ++r) {
+                const uint32_t word = cnt[r * 32 + lane];
+                const uint32_t ka = word & 0xffffu, kb = word >> 16;
+                l1 += (ka > kb ? ka - kb : kb - ka) >> 3;
+                D = fma(lds_f64(sq_addr(ka)), lds_f64(sq_addr(kb)), D);
+            }
+            double R = __dmul_rn(rA, rB);
+            {
+                const double h2 = fma(-R, D, 1.0);
+                h = (l1 == 0) ? 0.0 : (h2 < kSmallH2 ? sqrt(exact_4h2()) : twice_sqrt_unit(h2));
+            }
+            const uint32_t nev = min(left_all, (uint32_t)kWideBlock);
+            left_all -= nev;
+            uint32_t m = l1 - 1u;   // identical compositions after the event taken with `left` to go: m + left == nev
+#pragma unroll 2
+            for (uint32_t left = nev; left != 0; --left) {
+                const bool takeA = ra <= (rb | kCatMask);   // == (ra & kWMask) <= (rb & kWMask)
+                const uint64_t raw = takeA ? ra : rb;
+                const double w = key_value(raw);
+                acc = fma(w - wprev, h, acc);
+                wprev = w;
+                uint32_t ca;   // cnt_lane + category * 128
+                asm("mad.lo.u32 %0, %1, 128, %2;" : "=r"(ca) : "r"((uint32_t)raw & 0xFFu), "r"(cnt_lane));
+                const uint32_t word = lds_u32_rmw(ca);
+                const uint32_t ka = word & 0xffffu, kb = word >> 16;
+                const uint32_t mine_k = takeA ? ka : kb, other_k = takeA ? kb : ka;
+                sts_u32_rmw(ca, word + (takeA ? 8u : 0x80000u));
+                asm("{\n\t.reg .pred p;\n\tsetp.ge.u32 p, %1, %2;\n\t@p add.u32 %0, %0, 2;\n\t}" : "+r"(m) : "r"(mine_k), "r"(other_k));
+                const uint32_t pk = takeA ? pa : pb;
+                D = fma(lds_f64(dsq_addr(mine_k)), lds_f64(sq_addr(other_k)), D);
+                R *= lds_f64(pk + (takeA ? dA : dB));
+                const uint64_t nxt = lds_u64(pk + 8u);
+                pa = takeA ? pk + 8u : pa;
+                pb = takeA ? pb : pk + 8u;
+                ra = takeA ? nxt : ra;
+                rb = takeA ? rb : nxt;
+                const double h2 = fma(-R, D, 1.0);
+                h = twice_sqrt_unit(h2);
+                if ((float)h2 < kSmallH2f) {   // h2 < 1e-8 (or negative): identical counts (exactly 0) or rare (difference form)
+                    if (m + left == nev) {
+                        h = 0.0;
+                    } else {
+                        rA = __ldg(P.rsqrt_tbl + ((pa + dA - ratio_base) >> 3));
+                        rB = __ldg(P.rsqrt_tbl + ((pb + dB - ratio_base) >> 3));
+                        h = sqrt(exact_4h2());
+                    }
+                }
+            }
+            if (left_all == 0) break;
+        }
+        acc = fma(wf.w_inf - wprev, h, acc);   // tail to infinity
+        if (valid) a.out[out_first + ctrl->p[slot]] = 0.5 * acc;
+    }
+}
+
 __global__ void job_means_kernel(const double* __restrict__ scores, const uint64_t* __restrict__ job_pair_off,
                                  uint64_t n_jobs, double* __restrict__ means) {
     const int lane = threadIdx.x & 31;
@@ -3125,6 +3390,7 @@ LaunchOverrides read_launch_overrides() {
     if (const char* v = env("LOCOHD_TILE_SLICE_MB")) { const double mb = std::atof(v); if (mb > 0.0) o.tile_slice_mb = mb; }
     if (const char* v = env("LOCOHD_LEGACY_GATHER")) o.legacy_gather = v[0] && v[0] != '0';
     if (const char* v = env("LOCOHD_CROSS_ROWS")) { const long long r = std::atoll(v); if (r > 0) o.cross_rows = (uint64_t)r; }
+    if (const char* v = env("LOCOHD_WIDE_TILES")) o.wide_tiles = std::atoi(v) != 0;
     return o;
 }
 
@@ -3149,6 +3415,33 @@ TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int
     if (ov.tile_rep >= 0 && ov.tile_rep < rep_n) rep_n = ov.tile_rep;
     g.teams = teams;
     g.rep_n = rep_n;
+    return g;
+}
+
+WideGeometry wide_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, const LaunchOverrides& ov) {
+    WideGeometry g{};
+    if (!(p.hell2 && p.unit_w && p.C >= 1 && p.C <= 16 && key_is_w)) return g;   // as tile_geometry
+    if (max_a < 1 || max_b < 1 || max_a > 4096u || max_b > 4096u) return g;
+    g.cp = p.C <= 8 ? 8 : 16;
+    g.slot_a = (int)((max_a + 2u) & ~1u);
+    g.slot_b = (int)((max_b + 2u) & ~1u);
+    const unsigned need = (max_a > max_b ? max_a : max_b) + 2u;
+    g.table_n = (int)((need + 63u) & ~63u);
+    // count rows of 1024 lanes, control block, the three tables and a stage of 32 + 32 environments
+    const int fixed = g.cp * kWideThreads * 4 + kWideCtrlBytes + 3 * g.table_n * 8 + kWideDim * (g.slot_a + g.slot_b) * 8;
+    const int budget = 227 * 1024;
+    if (fixed > budget) return g;
+    // what is left over replicates the head of the two count-indexed tables, as in tile_geometry
+    int rep_n = g.cp == 8 ? (budget - fixed) / 240 : 0;
+    if (rep_n > kTileRepMax) rep_n = kTileRepMax;
+    if (rep_n < 16) rep_n = 0;
+    if (ov.tile_rep >= 0 && ov.tile_rep < rep_n) rep_n = ov.tile_rep;
+    g.rep_n = rep_n;
+    g.smem = fixed + 240 * rep_n;
+    // the count-row address of a category byte (up to 255) of lane 31 of warp 31 stays inside the allocation
+    const int reach = ((kWideDim - 1) * g.cp + 256) * 128;
+    if (g.smem < reach) g.smem = reach;
+    g.fits = true;
     return g;
 }
 
@@ -3214,6 +3507,34 @@ static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a,
     return 1;
 }
 
+// the wide job tiles args.wide_tiles (args.n_tiles of them, args.uniform_n anchors each)
+static int launch_wide(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a,
+                       double mean_b, const LaunchOverrides& ov, cudaStream_t st) {
+    ScoreArgs a = args;
+    const WideGeometry g = wide_geometry(p, max_a, max_b, a.a.key_is_w, ov);
+    if (!g.fits) return -1;
+    a.table_n = g.table_n;
+    a.rep_n = g.rep_n;
+    const uint64_t units = a.n_tiles * a.uniform_n;
+    if (!units) return 0;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const unsigned grid = (unsigned)(units < (uint64_t)sms ? units : (uint64_t)sms);   // persistent, one CTA per SM
+    cudaMemsetAsync(a.cursor, 0, sizeof(unsigned long long), st);
+    const uint64_t per_cta = units / ((uint64_t)grid * 4);   // short launches: shorter runs even out the tail
+    const uint64_t max_run = ov.tile_run ? ov.tile_run : kTileRun;
+    a.run = (unsigned)(per_cta < 1 ? 1 : (per_cta > max_run ? max_run : per_cta));
+    a.order = make_tile_order(a.n_tiles, a.uniform_n, tile_slice(a, mean_a, mean_b, ov));
+    auto go = [&](auto kernel) {
+        cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem);
+        kernel<<<grid, kWideThreads, g.smem, st>>>(a, p, g.slot_a, g.slot_b);
+    };
+    if (g.cp == 8) { if (g.rep_n > 0) go(score_wide_kernel<8, true>); else go(score_wide_kernel<8, false>); }
+    else go(score_wide_kernel<16, false>);
+    return 1;
+}
+
 int launch_score_cross(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, const LaunchOverrides& ov,
                        cudaStream_t st) {
     return launch_tiles(args, p, max_a, max_b, 0.0, 0.0, ov, TileMode::kCross, st);
@@ -3252,6 +3573,7 @@ int launch_row_topk(const double* scores, uint64_t rows, uint64_t cols, int k, i
 int launch_score(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a, double mean_b,
                  const LaunchOverrides& ov, cudaStream_t st) {
     if (!args.n_pairs) return 0;
+    if (args.wide) return launch_wide(args, p, max_a, max_b, mean_a, mean_b, ov, st);
     if (args.tiles) return launch_tiles(args, p, max_a, max_b, mean_a, mean_b, ov, TileMode::kJobs, st);
     const unsigned pad_max = ((max_a + 1) & ~1u) + ((max_b + 1) & ~1u);
     const bool key_is_w = args.a.key_is_w != 0;

@@ -131,13 +131,18 @@ struct EnvBuild {
 // env-set B (columns), every job of the tile with the same number of anchors.  An all-vs-all ensemble listed in
 // 4 x 4 blocks (batch.py::blocked_pairs) is exactly a list of such tiles.  score_tile_kernel stages the <= 8
 // environments of (tile, anchor) once and scores the <= 16 anchor pairs they form.
+// score_wide_kernel takes the same kind of tile at kWideDim x kWideDim (one CTA, one lane per anchor pair).
 constexpr int kTileDim = 4;
+constexpr int kWideDim = 32;
 constexpr uint64_t kTileNone = ~0ull;
-struct __align__(16) ScoreTile {
-    uint64_t a_first[kTileDim];                 // first environment of row r in env-set A (kTileNone: no such row)
-    uint64_t b_first[kTileDim];                 // first environment of column c in env-set B
-    uint64_t out_first[kTileDim * kTileDim];    // index of the first score of job (r, c) in `out` (kTileNone: no job)
+template <int DIM>
+struct __align__(16) TileDesc {
+    uint64_t a_first[DIM];          // first environment of row r in env-set A (kTileNone: no such row)
+    uint64_t b_first[DIM];          // first environment of column c in env-set B
+    uint64_t out_first[DIM * DIM];  // index of the first score of job (r, c) in `out` (kTileNone: no job)
 };
+using ScoreTile = TileDesc<kTileDim>;
+using WideTile = TileDesc<kWideDim>;
 
 // Order of the units (tile, anchor) of a tile launch.  Tile-major order (all anchors of a tile, then the next tile)
 // re-reads an environment from DRAM for almost every tile it takes part in: the 8 structures of a tile hold 60 MB of
@@ -229,7 +234,10 @@ __host__ __device__ inline void condensed_unit(T R, T u, T* dr, T* dc) {
 }
 
 struct ScoreArgs {
-    const ScoreTile* tiles;        // tile mode (score_tile_kernel): jobs grouped by the host, uniform_n anchors each
+    union {
+        const ScoreTile* tiles;    // tile mode (score_tile_kernel): jobs grouped by the host, uniform_n anchors each
+        const WideTile* wide_tiles;   // wide tile mode (score_wide_kernel, `wide` set): the same at kWideDim
+    };
     uint64_t n_tiles;
     EnvView a, b;
     uint64_t n_pairs;
@@ -253,7 +261,9 @@ struct ScoreArgs {
                                    // `run` consecutive pairs, so all resident warps work at one moving frontier
     unsigned run;                  // pairs per claim: kScoreRun for large launches, fewer when the launch has fewer
                                    // pairs than 4 runs per resident warp (single structure pairs: latency)
+    unsigned wide;                 // != 0: the tiles are wide_tiles (in the padding behind `run`: the layout is unchanged)
 };
+static_assert(sizeof(ScoreArgs) == 232, "the parameter layout of the scoring kernels");
 
 // ---- launchers (all asynchronous on `st`; each returns the number of kernel launches it made) ----
 int launch_convert_categories(const uint16_t* in, uint8_t* out, uint64_t n, int C, cudaStream_t st);
@@ -307,6 +317,8 @@ struct LaunchOverrides {
                                   // with the multi-kernel gather
     uint64_t cross_rows = 0;      // LOCOHD_CROSS_ROWS (> 0): lowers the rows of a cross-matrix or condensed chunk
                                   // (rounded down to a multiple of 4, at least 4)
+    bool wide_tiles = true;       // LOCOHD_WIDE_TILES=0: job lists never take score_wide_kernel (the 4 x 4 tiles or
+                                  // the pair kernel score them)
 };
 LaunchOverrides read_launch_overrides();
 int launch_score(const ScoreArgs& args, const KParams& p, unsigned max_a, unsigned max_b, double mean_a, double mean_b,
@@ -343,6 +355,18 @@ struct TileGeometry {
     int team_bytes;   // shared memory per team
 };
 TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, const LaunchOverrides& ov);
+// Launch geometry of score_wide_kernel (fits = false: it does not apply).  One CTA of 1024 threads stages the <= 32
+// row and <= 32 column environments of a unit in fixed slots of slot_a / slot_b keys.  The one place that decides it:
+// launch_score and the route of locohd_score_jobs_stats read it.
+struct WideGeometry {
+    bool fits;
+    int cp;           // count rows per lane: 8 (C <= 8) or 16 (C <= 16), the instantiation score_wide_kernel<cp, ...>
+    int rep_n;        // replicated head of the count-indexed tables, as TileGeometry::rep_n
+    int table_n;      // entries of each table
+    int slot_a, slot_b;   // keys per staged row / column environment: members, sentinel, even
+    int smem;         // dynamic shared memory of the CTA
+};
+WideGeometry wide_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, const LaunchOverrides& ov);
 // One side of the pairs of a gradient call: environment `first` + p of `env` is that side of pair p.  The set was built
 // with keep_indices or from rows, so `dist` / `idx` hold the exact distances and the members' indices (inside their
 // structure, or the column inside their row).
