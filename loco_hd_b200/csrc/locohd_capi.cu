@@ -1456,6 +1456,13 @@ int locohd_tile_geometry(int n_categories, uint32_t max_a, uint32_t max_b, int* 
     return LOCOHD_OK;
 }
 
+// Pairs of environments of a and b take the tile kernels: W-keyed sets, the configuration the kernels have
+// (tile_geometry) and at least kTileMinTeams teams per SM.
+static bool tile_route(const locohd_ctx* ctx, const locohd_envset* a, const locohd_envset* b, const LaunchOverrides& ov) {
+    return a->key_is_w && b->key_is_w && !ov.no_tiles &&
+           tile_geometry(ctx->kp, a->max_count, b->max_count, 1, ov).teams >= kTileMinTeams;
+}
+
 int locohd_score_jobs(locohd_ctx* ctx, const locohd_envset* a, const locohd_envset* b, uint64_t n_jobs,
                       const locohd_job* jobs, const uint32_t* wf_idx, double* out_scores, double* out_job_means) {
     return locohd_score_jobs_stats(ctx, a, b, n_jobs, jobs, wf_idx, out_scores, out_job_means, nullptr, nullptr);
@@ -1514,8 +1521,7 @@ int locohd_score_jobs_stats(locohd_ctx* ctx, const locohd_envset* a, const locoh
     InBuf<ScoreTile> dtiles;
     InBuf<WideTile> dwide;
     TilePlan plan;   // alive until the call's final synchronisation
-    if (!wf_idx && a->key_is_w && b->key_is_w && !ov.no_tiles &&
-        tile_geometry(ctx->kp, a->max_count, b->max_count, 1, ov).teams >= 6) {
+    if (!wf_idx && tile_route(ctx, a, b, ov)) {
         if (!ctx->tile_cache_plan.tiles.empty() && ctx->tile_cache_jobs.size() == hj.size() &&
             std::memcmp(ctx->tile_cache_jobs.data(), hj.data(), hj.size() * sizeof(locohd_job)) == 0) {
             plan = ctx->tile_cache_plan;   // the list of the previous call: 2 ms instead of 25 for 500 000 jobs
@@ -1587,8 +1593,7 @@ int locohd_score_cross(locohd_ctx* ctx, const locohd_envset* a, uint64_t a_first
     // wf_idx is 0 -, Hellinger-2 with unit weights, C <= 16, >= 6 teams); else explicit pairs on the pair kernel, with
     // the chosen weight function as the kernels' function 0.
     const LaunchOverrides ov = read_launch_overrides();
-    const bool tiles = a->key_is_w && b->key_is_w && !ov.no_tiles &&
-                       tile_geometry(ctx->kp, a->max_count, b->max_count, 1, ov).teams >= 6;
+    const bool tiles = tile_route(ctx, a, b, ov);
     KParams kp = ctx->kp;
     kp.wfs = ctx->d_wfs + wf_idx;
     kp.n_wf = 1;
@@ -1675,7 +1680,7 @@ int locohd_score_condensed(locohd_ctx* ctx, const locohd_envset* s, uint64_t fir
 
     // Route and weight function as in locohd_score_cross with the range on both sides.
     const LaunchOverrides ov = read_launch_overrides();
-    const bool tiles = s->key_is_w && !ov.no_tiles && tile_geometry(ctx->kp, s->max_count, s->max_count, 1, ov).teams >= 6;
+    const bool tiles = tile_route(ctx, s, s, ov);
     KParams kp = ctx->kp;
     kp.wfs = ctx->d_wfs + wf_idx;
     kp.n_wf = 1;

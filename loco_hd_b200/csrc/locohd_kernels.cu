@@ -2186,6 +2186,171 @@ __device__ __forceinline__ void team_barrier(int team) {
     asm volatile("bar.sync %0, %1;" ::"r"(team + 1), "r"(kTeamThreads) : "memory");
 }
 
+// The tables of score_tile_kernel and score_wide_kernel, from `base` on: sqrt(k / (k + 1)) [table_n], indexed by a
+// side's total, then sqrt(k) and sqrt(k + 1) - sqrt(k) (exact: Sterbenz) [15 rep_n + table_n] each, indexed by a
+// count.  The two count-indexed ones are "mixed" when rep_n > 0: entries k < rep_n exist once per bank pair (entry k
+// of copy c at word 16 k + c; lane l reads copy l & 15, so these reads are conflict-free whatever the counts of the
+// 32 lanes are: 2 wavefronts per warp read instead of 3.8), the entries from rep_n on follow unreplicated.  Word index
+// of entry k for copy c: k + min(15 k + c, 15 rep_n) - one IMAD, one min and one add, no branch.  The host picks rep_n
+// from the shared memory the stage leaves over (tile_rep_n).
+struct TileTables {
+    int table_n, rep_n, mix_n;   // entries of ratio, replicated head, entries of sqrt and of dsq
+    double *ratio, *sqrt, *dsq;   // what follows the tables starts at dsq + mix_n
+    __device__ __forceinline__ TileTables(unsigned char* base, int n, int rep)
+        : table_n(n), rep_n(rep), mix_n(15 * rep + n) {
+        ratio = reinterpret_cast<double*>(base);
+        sqrt = ratio + table_n;
+        dsq = sqrt + mix_n;
+    }
+    __device__ __forceinline__ void fill(const KParams& P) const {
+        for (int x = threadIdx.x; x < table_n; x += blockDim.x) ratio[x] = ::sqrt((double)x / (double)(x + 1));
+        for (int x = threadIdx.x; x < mix_n; x += blockDim.x) {
+            const int e = x < 16 * rep_n ? x >> 4 : x - 15 * rep_n;
+            const double s0 = P.sqrt_tbl[e], s1 = P.sqrt_tbl[e + 1];
+            sqrt[x] = s0;
+            dsq[x] = s1 - s0;
+        }
+    }
+};
+
+// What a lane's walk carries from event to event: the shared-space addresses pa / pb of the next keys ra / rb of either
+// side (the ratio-table entry of a side's total is at p + dA / dB), D, R, 1 / sqrt of either total, h = 2 H, the weight
+// of the last event and the sum.  The walk carries h = 2 H (twice_sqrt_unit saves a multiply per event) and the sum is
+// halved at the end: scaling by 2 is exact, the sum is the one of H itself.
+struct TileWalk {
+    uint32_t pa, pb, dA, dB;
+    uint64_t ra, rb;
+    double D, R, rA, rB, h, wprev, acc;
+};
+
+// A lane's view of the tables and of its count words (cnt: the warp's count rows [CP][32], 8 count each).  The
+// shared-space addresses pass through an identity shuffle once so that ptxas keeps them in registers: left alone it
+// rematerialises them in every walk iteration.
+template <int CP, bool REP>
+struct TileLane {
+    const uint32_t* cnt;
+    int lane;
+    uint32_t sq_base, dsq_base, ratio_base, cnt_lane, sq_copy, sq_cap, dsq_copy, dsq_cap;
+    __device__ __forceinline__ TileLane(const TileTables& t, const uint32_t* cnt_rows, int lane_id)
+        : cnt(cnt_rows), lane(lane_id) {
+        sq_base = __shfl_sync(kFull, smem_u32(t.sqrt), lane);
+        dsq_base = __shfl_sync(kFull, smem_u32(t.dsq), lane);
+        ratio_base = __shfl_sync(kFull, smem_u32(t.ratio), lane);
+        cnt_lane = __shfl_sync(kFull, smem_u32(cnt + lane), lane);
+        const uint32_t copy8 = 8u * (lane & 15), cap8 = 120u * (uint32_t)t.rep_n;
+        sq_copy = __shfl_sync(kFull, sq_base + copy8, lane), sq_cap = __shfl_sync(kFull, sq_base + cap8, lane);
+        dsq_copy = __shfl_sync(kFull, dsq_base + copy8, lane), dsq_cap = __shfl_sync(kFull, dsq_base + cap8, lane);
+    }
+    // shared-space address of entry e of a count-indexed table, from e8 = 8 e (the count words hold 8 count):
+    // base + 8 e + min(120 e + 8 copy, 120 rep_n) = min(16 e8 + base + 8 copy, e8 + base + 120 rep_n) - one shift-add
+    // and one add-min (VIADDMNMX) per look-up
+    __device__ __forceinline__ uint32_t sq_addr(uint32_t e8) const { return REP ? min(16u * e8 + sq_copy, e8 + sq_cap) : sq_base + e8; }
+    __device__ __forceinline__ uint32_t dsq_addr(uint32_t e8) const { return REP ? min(16u * e8 + dsq_copy, e8 + dsq_cap) : dsq_base + e8; }
+    // 4 H^2 in the difference form from the counts (small H^2 only)
+    __device__ __forceinline__ double exact_4h2(double rA, double rB) const {
+        double s = 0.0;
+#pragma unroll
+        for (int r = 0; r < CP; ++r) {
+            const uint32_t word = cnt[r * 32 + lane];
+            const double u = __dmul_rn(lds_f64(sq_addr(word & 0xffffu)), rA) - __dmul_rn(lds_f64(sq_addr(word >> 16)), rB);
+            s = fma(u, u, s);
+        }
+        return 2.0 * s;
+    }
+    // h = 2 H where a walk starts, from w.R, w.D and the counts; l1 = sum_r |a_r - b_r| (0: identical compositions)
+    __device__ __forceinline__ double start_h(uint32_t l1, const TileWalk& w) const {
+        const double h2 = fma(-w.R, w.D, 1.0);
+        return (l1 == 0) ? 0.0 : (h2 < kSmallH2 ? sqrt(exact_4h2(w.rA, w.rB)) : twice_sqrt_unit(h2));
+    }
+};
+
+// nev events of a lane's walk over the merged keys of its pair, from the state w with sum_r |a_r - b_r| = l1: the event
+// of score_tile_kernel's header comment, kept short because the walk is bound by its instruction count.
+template <int CP, bool REP>
+__device__ __forceinline__ void walk_events(const TileLane<CP, REP>& L, const double* __restrict__ rsqrt_tbl, TileWalk& w,
+                                            uint32_t nev, uint32_t l1) {
+    // Identical compositions: an event moves sum_r |a_r - b_r| by +1 (my count of the category was >= the other
+    // side's) or -1, so after k events the sum is l1 - k + 2 #{events with mine >= other}.  The walk keeps
+    // m = l1 - 1 + 2 #{...} (one predicated add per event) and compares only where H^2 is tiny: there, after the
+    // event taken with `left` events to go (k = nev - left + 1), m + left == nev <=> identical <=> H = 0 exactly.
+    // Identical compositions are frequent in ensembles of near-copies; their h2 is a rounding residue below 1e-8,
+    // so they take the branch of the small-H^2 case instead of a test and a select on every event (6 -> 2
+    // instructions of bookkeeping per event against the count of differing categories).
+    uint32_t m = l1 - 1u;
+    // unrolled by 2: no register rotation of the carried key / weight and half the loop overhead, 130.8 -> 126.9 ms
+    // on the 200-structure ensemble (profiles/r6x); by 4: 128.7 ms (profiles/r6y)
+#pragma unroll 2
+    for (uint32_t left = nev; left != 0; --left) {
+        const bool takeA = w.ra <= (w.rb | kCatMask);   // == (ra & kWMask) <= (rb & kWMask)
+        const uint64_t raw = takeA ? w.ra : w.rb;
+        const double wk = key_value(raw);
+        w.acc = fma(wk - w.wprev, w.h, w.acc);
+        w.wprev = wk;
+        uint32_t ca;   // cnt_lane + category * 128
+        asm("mad.lo.u32 %0, %1, 128, %2;" : "=r"(ca) : "r"((uint32_t)raw & 0xFFu), "r"(L.cnt_lane));
+        const uint32_t word = lds_u32_rmw(ca);
+        const uint32_t ka = word & 0xffffu, kb = word >> 16;
+        const uint32_t mine_k = takeA ? ka : kb, other_k = takeA ? kb : ka;
+        sts_u32_rmw(ca, word + (takeA ? 8u : 0x80000u));
+        // a predicated add in place (left to itself, ptxas adds into a new register and selects: two instructions)
+        asm("{\n\t.reg .pred p;\n\tsetp.ge.u32 p, %1, %2;\n\t@p add.u32 %0, %0, 2;\n\t}" : "+r"(m) : "r"(mine_k), "r"(other_k));
+        const uint32_t pk = takeA ? w.pa : w.pb;
+        w.D = fma(lds_f64(L.dsq_addr(mine_k)), lds_f64(L.sq_addr(other_k)), w.D);
+        w.R *= lds_f64(pk + (takeA ? w.dA : w.dB));
+        const uint64_t nxt = lds_u64(pk + 8u);
+        w.pa = takeA ? pk + 8u : w.pa;
+        w.pb = takeA ? w.pb : pk + 8u;
+        w.ra = takeA ? nxt : w.ra;
+        w.rb = takeA ? w.rb : nxt;
+        const double h2 = fma(-w.R, w.D, 1.0);
+        w.h = twice_sqrt_unit(h2);
+        if ((float)h2 < kSmallH2f) {   // h2 < 1e-8 (or negative): identical counts (exactly 0) or rare (difference form)
+            if (m + left == nev) {
+                w.h = 0.0;
+            } else {
+                w.rA = __ldg(rsqrt_tbl + ((w.pa + w.dA - L.ratio_base) >> 3));
+                w.rB = __ldg(rsqrt_tbl + ((w.pb + w.dB - L.ratio_base) >> 3));
+                w.h = sqrt(L.exact_4h2(w.rA, w.rB));
+            }
+        }
+    }
+}
+
+// The next unit of a loader warp: units are claimed from a.cursor in runs of a.run consecutive ones with one
+// atomicAdd (run_pos / run_end: the claimed run, uniform over the warp).  n_units and beyond: no units left.
+__device__ __forceinline__ uint64_t claim_unit(const ScoreArgs& a, uint64_t n_units, uint64_t& run_pos, uint64_t& run_end,
+                                               int lane) {
+    if (run_pos == run_end) {
+        unsigned long long got = 0;
+        if (lane == 0) got = atomicAdd(a.cursor, (unsigned long long)a.run);
+        got = __shfl_sync(kFull, got, 0);
+        run_pos = min((uint64_t)got, n_units);
+        run_end = min((uint64_t)got + a.run, n_units);
+    }
+    const uint64_t u = run_pos;
+    if (run_pos < run_end) ++run_pos;
+    return u;
+}
+
+// Descriptor of environment first + p of v: its offset, its size and, when the size is odd, its last member (stage_env
+// stores it by hand; `last` is left as it is for an even size).
+__device__ __forceinline__ void load_env(const EnvView& v, uint64_t first, uint64_t p, uint64_t& off, uint32_t& M,
+                                         uint64_t& last) {
+    off = __ldg(v.off + first + p);
+    M = __ldg(v.count + first + p);
+    if (M & 1u) last = __ldg(v.key + off + M - 1);
+}
+
+// Stages the M >= 1 keys at `keys` into dst: the even part (bytes = 8 (M & ~1), which the caller has added to the
+// mbarrier's transaction count) as one bulk copy (16-byte granules) on mbar, an odd last member (loaded with the
+// descriptor) by hand, so the sentinel behind it is never overwritten by the copy.
+__device__ __forceinline__ void stage_env(uint64_t* dst, const uint64_t* keys, uint32_t bytes, uint32_t M, uint64_t last,
+                                          uint64_t* mbar) {
+    if (bytes) { fence_proxy_async(); bulk_g2s(dst, keys, bytes, mbar); }
+    if (M & 1u) dst[M - 1] = last;
+    dst[M] = kSentinel;
+}
+
 // What the units of a tile launch are: kJobs - a job list in tiles (a.tiles, a.order); kCross - the cross matrix
 // a.cross (CrossGrid); kCondensed - a chunk of the upper triangle of one range, a.condensed (CondensedGrid).  In the two
 // matrix modes the loader derives the rows and columns of a unit from its index, a unit has one anchor, and rows /
@@ -2198,29 +2363,14 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
     constexpr bool CROSS = MODE == TileMode::kCross, CONDENSED = MODE == TileMode::kCondensed;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    const int table_n = a.table_n;
-    // Tables.  The two count-indexed ones (sqrt(k), sqrt(k + 1) - sqrt(k)) are "mixed" when REP: entries k < rep_n
-    // exist once per bank pair (entry k of copy c at word 16 k + c; lane l reads copy l & 15, so these reads are
-    // conflict-free whatever the counts of the 32 lanes are: 2 wavefronts per warp read instead of 3.8), the entries
-    // from rep_n on follow unreplicated.  Word index of entry k for copy c: k + min(15 k + c, 15 rep_n) - one IMAD,
-    // one min and one add, no branch.  The host picks rep_n from the shared memory the teams leave over.
     const int rep_n = REP ? a.rep_n : 0;
-    const int mix_n = 15 * rep_n + table_n;
-    double* s_ratio = reinterpret_cast<double*>(smem_raw);   // sqrt(k / (k + 1)), indexed by a side's total
-    double* s_sqrt = s_ratio + table_n;                      // sqrt(k)
-    double* s_dsq = s_sqrt + mix_n;                          // sqrt(k + 1) - sqrt(k)   (exact: Sterbenz)
-    for (int x = threadIdx.x; x < table_n; x += blockDim.x) s_ratio[x] = sqrt((double)x / (double)(x + 1));
-    for (int x = threadIdx.x; x < mix_n; x += blockDim.x) {
-        const int e = x < 16 * rep_n ? x >> 4 : x - 15 * rep_n;
-        const double s0 = P.sqrt_tbl[e], s1 = P.sqrt_tbl[e + 1];
-        s_sqrt[x] = s0;
-        s_dsq[x] = s1 - s0;
-    }
+    const TileTables tables(smem_raw, a.table_n, rep_n);   // at the start of shared memory
+    tables.fill(P);
     __syncthreads();
     const int team = wib >> 2, row = wib & 3;
     if (team >= teams) return;
     const int C = P.C;
-    unsigned char* mine = smem_raw + (size_t)(table_n + 2 * mix_n) * 8 + (size_t)team * team_bytes;
+    unsigned char* mine = smem_raw + (size_t)(tables.table_n + 2 * tables.mix_n) * 8 + (size_t)team * team_bytes;
     uint32_t* cnt = reinterpret_cast<uint32_t*>(mine) + row * CP * 32;   // [CP][32] per warp: 8 A | 8 B << 16 (8 count:
                                                                          // the byte offset of the count's table entry)
     TileCtrl* ctrl = reinterpret_cast<TileCtrl*>(mine + CP * kTeamThreads * 4);
@@ -2228,18 +2378,7 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
     const bool loader = row == 0;
     if (loader && lane == 0) { mbar_init(&ctrl->mbar, 1); fence_proxy_async(); }
     unsigned flags = 0;   // bit 0: parity of the team's mbarrier, bit 1: control-block slot of the NEXT fetch
-    const uint32_t sq_base = __shfl_sync(kFull, smem_u32(s_sqrt), lane);
-    const uint32_t dsq_base = __shfl_sync(kFull, smem_u32(s_dsq), lane);
-    const uint32_t ratio_base = __shfl_sync(kFull, smem_u32(s_ratio), lane);
-    const uint32_t cnt_lane = __shfl_sync(kFull, smem_u32(cnt + lane), lane);
-    // shared-space address of entry e of a count-indexed table, from e8 = 8 e (the count words hold 8 count):
-    // base + 8 e + min(120 e + 8 copy, 120 rep_n) = min(16 e8 + base + 8 copy, e8 + base + 120 rep_n) - one shift-add
-    // and one add-min (VIADDMNMX) per look-up
-    const uint32_t copy8 = 8u * (lane & 15), cap8 = 120u * (uint32_t)rep_n;
-    const uint32_t sq_copy = __shfl_sync(kFull, sq_base + copy8, lane), sq_cap = __shfl_sync(kFull, sq_base + cap8, lane);
-    const uint32_t dsq_copy = __shfl_sync(kFull, dsq_base + copy8, lane), dsq_cap = __shfl_sync(kFull, dsq_base + cap8, lane);
-    auto sq_addr = [&](uint32_t e8) -> uint32_t { return REP ? min(16u * e8 + sq_copy, e8 + sq_cap) : sq_base + e8; };
-    auto dsq_addr = [&](uint32_t e8) -> uint32_t { return REP ? min(16u * e8 + dsq_copy, e8 + dsq_cap) : dsq_base + e8; };
+    const TileLane<CP, REP> L(tables, cnt, lane);
     // warp = row of the tile, 8 lanes per column.  (Measured and dropped, profiles/r6p: warp w scoring the pairs
     // (r, (r + w) mod 4) - a Latin square, equal event totals for the four warps, where ncu shows 19.6 % of the warp time
     // in the team barrier waiting for the row with the largest A_r - 134.9 -> 139.5 ms: the 32 lanes of a row share
@@ -2264,15 +2403,7 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
     uint32_t nx_M = 0;
     bool nx_present = false;
     auto fetch = [&]() {
-        if (run_pos == run_end) {
-            unsigned long long got = 0;
-            if (lane == 0) got = atomicAdd(a.cursor, (unsigned long long)a.run);
-            got = __shfl_sync(kFull, got, 0);
-            run_pos = min((uint64_t)got, n_units);
-            run_end = min((uint64_t)got + a.run, n_units);
-        }
-        const uint64_t u = run_pos;
-        if (run_pos < run_end) ++run_pos;
+        const uint64_t u = claim_unit(a, n_units, run_pos, run_end, lane);
         nx_unit = u; nx_off = 0; nx_M = 0; nx_last = 0; nx_present = false;
         if constexpr (CROSS) {
             if (u < n_units && lane < 2 * kTileDim) {
@@ -2286,11 +2417,7 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
                 const bool is_row = lane < kTileDim;
                 const uint64_t idx = is_row ? rb * kTileDim + lane : cb * kTileDim + (lane - kTileDim);
                 if (idx < (is_row ? a.cross.rows : a.cross.cols)) {
-                    const EnvView& v = is_row ? a.a : a.b;
-                    const uint64_t e = (is_row ? a.cross.a_first : a.cross.b_first) + idx;
-                    nx_off = __ldg(v.off + e);
-                    nx_M = __ldg(v.count + e);
-                    if (nx_M & 1u) nx_last = __ldg(v.key + nx_off + nx_M - 1);
+                    load_env(is_row ? a.a : a.b, (is_row ? a.cross.a_first : a.cross.b_first) + idx, 0, nx_off, nx_M, nx_last);
                     nx_present = true;
                 }
             }
@@ -2306,10 +2433,7 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
                 if (lane == 0) { ctrl->tile[(flags >> 1) & 1u] = (uint32_t)rb; ctrl->p[(flags >> 1) & 1u] = (uint32_t)cb; }
                 const uint64_t idx = (lane < kTileDim ? rb : cb) * kTileDim + (lane & (kTileDim - 1));
                 if (idx < g.n) {
-                    const uint64_t e = g.first + idx;
-                    nx_off = __ldg(a.a.off + e);
-                    nx_M = __ldg(a.a.count + e);
-                    if (nx_M & 1u) nx_last = __ldg(a.a.key + nx_off + nx_M - 1);
+                    load_env(a.a, g.first + idx, 0, nx_off, nx_M, nx_last);
                     nx_present = true;
                 }
             }
@@ -2323,10 +2447,7 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
             const ScoreTile& T = a.tiles[tile];
             const uint64_t first = lane < kTileDim ? __ldg(T.a_first + lane) : __ldg(T.b_first + (lane - kTileDim));
             if (first != kTileNone) {
-                const EnvView& v = lane < kTileDim ? a.a : a.b;
-                nx_off = __ldg(v.off + first + p);
-                nx_M = __ldg(v.count + first + p);
-                if (nx_M & 1u) nx_last = __ldg(v.key + nx_off + nx_M - 1);
+                load_env(lane < kTileDim ? a.a : a.b, first, p, nx_off, nx_M, nx_last);
                 nx_present = true;
             }
         }
@@ -2352,9 +2473,7 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
                     if (lane >= o) incl += t;
                 }
                 const uint32_t start = incl - slot;
-                // The even part of an environment comes as one bulk copy (16-byte granules); an odd last member was
-                // fetched with the descriptor and is stored by hand, so the sentinel behind it is never overwritten
-                // by the copy.
+                // the bulk copies of stage_env: the even part of every environment
                 const uint32_t bytes = (state == 0 && nx_present) ? (nx_M & ~1u) * 8u : 0u;
                 uint32_t total = bytes;
 #pragma unroll
@@ -2363,11 +2482,7 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
                     const EnvView& v = lane < kTileDim ? a.a : a.b;
                     if (lane == 0) { fence_proxy_async(); mbar_expect_tx(&ctrl->mbar, total); }
                     __syncwarp();
-                    if (lane < 2 * kTileDim && nx_present) {
-                        if (bytes) { fence_proxy_async(); bulk_g2s(stage + start, v.key + nx_off, bytes, &ctrl->mbar); }
-                        if (nx_M & 1u) stage[start + nx_M - 1] = nx_last;
-                        stage[start + nx_M] = kSentinel;
-                    }
+                    if (lane < 2 * kTileDim && nx_present) stage_env(stage + start, v.key + nx_off, bytes, nx_M, nx_last, &ctrl->mbar);
                 }
                 if (lane < 2 * kTileDim) { ctrl->start[lane] = start; ctrl->M[lane] = (state == 0 && nx_present) ? nx_M : 0u; }
             }
@@ -2451,7 +2566,8 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
         }
         if (__any_sync(kFull, unknown)) { raise(P.err, LOCOHD_ERR_UNKNOWN_CATEGORY); continue; }  // pmf.rs:38-42
         uint32_t l1 = 0;   // sum_r |a_r - b_r|: 0 <=> identical compositions
-        double D = 0.0;
+        TileWalk w;
+        w.D = 0.0;
 #pragma unroll
         for (int r = 0; r < CP; ++r) {
             const uint32_t v = (uint32_t)((hA[r >> 3] >> (8 * (r & 7))) & 0xFFu) |
@@ -2468,87 +2584,26 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
             cnt[r * 32 + lane] = 8u * ex;   // <= 1024 members a side (tile_geometry): 8 count fits 16 bits
             const uint32_t ka = ex & 0xffffu, kb = ex >> 16;
             l1 += ka > kb ? ka - kb : kb - ka;
-            D = fma(lds_f64(sq_addr(8u * ka)), lds_f64(sq_addr(8u * kb)), D);
+            w.D = fma(lds_f64(L.sq_addr(8u * ka)), lds_f64(L.sq_addr(8u * kb)), w.D);
         }
         const uint32_t totA = i + 1u, totB = j + 1u;   // members of either side before my chunk, anchors included
-        double rA = __ldg(P.rsqrt_tbl + totA), rB = __ldg(P.rsqrt_tbl + totB);
-        // 4 H^2 in the difference form from the counts (small H^2 only)
-        auto exact_4h2 = [&]() -> double {
-            double s = 0.0;
-#pragma unroll
-            for (int r = 0; r < CP; ++r) {
-                const uint32_t word = cnt[r * 32 + lane];
-                const double u = __dmul_rn(lds_f64(sq_addr(word & 0xffffu)), rA) - __dmul_rn(lds_f64(sq_addr(word >> 16)), rB);
-                s = fma(u, u, s);
-            }
-            return 2.0 * s;
-        };
+        w.rA = __ldg(P.rsqrt_tbl + totA), w.rB = __ldg(P.rsqrt_tbl + totB);
         uint64_t kprev = key0;
         if (i > 0) kprev = kA[i - 1] & kWMask;
         if (j > 0) kprev = max(kprev, kB[j - 1] & kWMask);
-        double wprev = key_value(kprev);
-        double R = __dmul_rn(rA, rB);
-        // The walk carries h = 2 H (twice_sqrt_unit saves a multiply per event) and halves the sum at the end: scaling
-        // by 2 is exact, the sum is the one of H itself.
-        double h;
-        {
-            const double h2 = fma(-R, D, 1.0);
-            h = (l1 == 0) ? 0.0 : (h2 < kSmallH2 ? sqrt(exact_4h2()) : twice_sqrt_unit(h2));
-        }
-        double acc = 0.0;
+        w.wprev = key_value(kprev);
+        w.R = __dmul_rn(w.rA, w.rB);
+        w.h = L.start_h(l1, w);
+        w.acc = 0.0;
         const uint32_t nev = (i1 - i) + (j1 - j);
-        uint32_t pa = smem_u32(kA + i), pb = smem_u32(kB + j);
-        const uint32_t dA = ratio_base + 8u * totA - pa, dB = ratio_base + 8u * totB - pb;
-        uint64_t ra = lds_u64(pa), rb = lds_u64(pb);
-        // Identical compositions: an event moves sum_r |a_r - b_r| by +1 (my count of the category was >= the other
-        // side's) or -1, so after k events the sum is l1 - k + 2 #{events with mine >= other}.  The walk keeps
-        // m = l1 - 1 + 2 #{...} (one predicated add per event) and compares only where H^2 is tiny: there, after the
-        // event taken with `left` events to go (k = nev - left + 1), m + left == nev <=> identical <=> H = 0 exactly.
-        // Identical compositions are frequent in ensembles of near-copies; their h2 is a rounding residue below 1e-8,
-        // so they take the branch of the small-H^2 case instead of a test and a select on every event (6 -> 2
-        // instructions of bookkeeping per event against the count of differing categories).
-        uint32_t m = l1 - 1u;
-        // unrolled by 2: no register rotation of the carried key / weight and half the loop overhead, 130.8 -> 126.9 ms
-        // on the 200-structure ensemble (profiles/r6x); by 4: 128.7 ms (profiles/r6y)
-#pragma unroll 2
-        for (uint32_t left = nev; left != 0; --left) {
-            const bool takeA = ra <= (rb | kCatMask);   // == (ra & kWMask) <= (rb & kWMask)
-            const uint64_t raw = takeA ? ra : rb;
-            const double w = key_value(raw);
-            acc = fma(w - wprev, h, acc);
-            wprev = w;
-            uint32_t ca;   // cnt_lane + category * 128
-            asm("mad.lo.u32 %0, %1, 128, %2;" : "=r"(ca) : "r"((uint32_t)raw & 0xFFu), "r"(cnt_lane));
-            const uint32_t word = lds_u32_rmw(ca);
-            const uint32_t ka = word & 0xffffu, kb = word >> 16;
-            const uint32_t mine_k = takeA ? ka : kb, other_k = takeA ? kb : ka;
-            sts_u32_rmw(ca, word + (takeA ? 8u : 0x80000u));
-            // a predicated add in place (left to itself, ptxas adds into a new register and selects: two instructions)
-            asm("{\n\t.reg .pred p;\n\tsetp.ge.u32 p, %1, %2;\n\t@p add.u32 %0, %0, 2;\n\t}" : "+r"(m) : "r"(mine_k), "r"(other_k));
-            const uint32_t pk = takeA ? pa : pb;
-            D = fma(lds_f64(dsq_addr(mine_k)), lds_f64(sq_addr(other_k)), D);
-            R *= lds_f64(pk + (takeA ? dA : dB));
-            const uint64_t nxt = lds_u64(pk + 8u);
-            pa = takeA ? pk + 8u : pa;
-            pb = takeA ? pb : pk + 8u;
-            ra = takeA ? nxt : ra;
-            rb = takeA ? rb : nxt;
-            const double h2 = fma(-R, D, 1.0);
-            h = twice_sqrt_unit(h2);
-            if ((float)h2 < kSmallH2f) {   // h2 < 1e-8 (or negative): identical counts (exactly 0) or rare (difference form)
-                if (m + left == nev) {
-                    h = 0.0;
-                } else {
-                    rA = __ldg(P.rsqrt_tbl + ((pa + dA - ratio_base) >> 3));
-                    rB = __ldg(P.rsqrt_tbl + ((pb + dB - ratio_base) >> 3));
-                    h = sqrt(exact_4h2());
-                }
-            }
-        }
-        if (sub == kTileLanes - 1) acc = fma(wf.w_inf - wprev, h, acc);   // tail to infinity: the last chunk's state is final
+        w.pa = smem_u32(kA + i), w.pb = smem_u32(kB + j);
+        w.dA = L.ratio_base + 8u * totA - w.pa, w.dB = L.ratio_base + 8u * totB - w.pb;
+        w.ra = lds_u64(w.pa), w.rb = lds_u64(w.pb);
+        walk_events(L, P.rsqrt_tbl, w, nev, l1);
+        if (sub == kTileLanes - 1) w.acc = fma(wf.w_inf - w.wprev, w.h, w.acc);   // tail to infinity: the last chunk's state is final
 #pragma unroll
-        for (int o = kTileLanes / 2; o; o >>= 1) acc += __shfl_xor_sync(kFull, acc, o * lstep);
-        if (sub == 0 && valid) a.out[out_first + p] = 0.5 * acc;
+        for (int o = kTileLanes / 2; o; o >>= 1) w.acc += __shfl_xor_sync(kFull, w.acc, o * lstep);
+        if (sub == 0 && valid) a.out[out_first + p] = 0.5 * w.acc;
     }
 }
 
@@ -2563,9 +2618,8 @@ __global__ void __launch_bounds__(kTileMaxTeams * kTeamThreads, 1) score_tile_ke
 // stage of the bench's largest environments (345 members) is the same ~178 KB and 32 warps still fit an SM.
 // The event arithmetic is that of score_tile_kernel (replicated head tables, count words of 8 count, 2 H, identical
 // compositions through m, the small-H^2 difference form); D and R are rebuilt from the counts at least every
-// kWideBlock events, so a walk keeps the bound of <= 128 roundings of either (~3e-14 relative, DESIGN §3).  The walk
-// is kept apart from score_tile_kernel's: sharing the event step would have to leave the nine instantiations of that
-// kernel instruction for instruction as they are (profiles/r16a_wide_tiles.md).
+// kWideBlock events, so a walk keeps the bound of <= 128 roundings of either (~3e-14 relative, DESIGN §3).  Tables,
+// lane view and event walk are those of score_tile_kernel (TileTables, TileLane, walk_events).
 constexpr int kWideThreads = kWideDim * 32;   // 1024: warp r = row r, lane c = column c
 constexpr int kWideBlock = 128;               // events between two rebuilds of D and R from the counts
 struct WideCtrl {
@@ -2586,40 +2640,22 @@ template <int CP, bool REP>
 __global__ void __launch_bounds__(kWideThreads, 1) score_wide_kernel(ScoreArgs a, KParams P, int slot_a, int slot_b) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, row = threadIdx.x >> 5;
-    const int table_n = a.table_n;
-    const int rep_n = REP ? a.rep_n : 0;   // tables as in score_tile_kernel
-    const int mix_n = 15 * rep_n + table_n;
-    // count rows first: the row address of any category byte (cnt_lane + 128 byte) lies inside the allocation
-    // (wide_geometry), whatever the staged keys hold
+    const int rep_n = REP ? a.rep_n : 0;
+    // count rows first, then the control block and the tables: the row address of any category byte (cnt_lane + 128
+    // byte) lies inside the allocation (wide_geometry), whatever the staged keys hold
     uint32_t* cnt = reinterpret_cast<uint32_t*>(smem_raw) + row * CP * 32;   // [CP][32] per warp, as score_tile_kernel
     WideCtrl* ctrl = reinterpret_cast<WideCtrl*>(smem_raw + CP * kWideThreads * 4);
-    double* s_ratio = reinterpret_cast<double*>(smem_raw + CP * kWideThreads * 4 + kWideCtrlBytes);
-    double* s_sqrt = s_ratio + table_n;
-    double* s_dsq = s_sqrt + mix_n;
-    uint64_t* stage_a = reinterpret_cast<uint64_t*>(s_dsq + mix_n);   // rows: slot_a keys each, then the columns
+    const TileTables tables(smem_raw + CP * kWideThreads * 4 + kWideCtrlBytes, a.table_n, rep_n);
+    uint64_t* stage_a = reinterpret_cast<uint64_t*>(tables.dsq + tables.mix_n);   // rows: slot_a keys each, then the columns
     uint64_t* stage_b = stage_a + kWideDim * slot_a;
-    for (int x = threadIdx.x; x < table_n; x += blockDim.x) s_ratio[x] = sqrt((double)x / (double)(x + 1));
-    for (int x = threadIdx.x; x < mix_n; x += blockDim.x) {
-        const int e = x < 16 * rep_n ? x >> 4 : x - 15 * rep_n;
-        const double s0 = P.sqrt_tbl[e], s1 = P.sqrt_tbl[e + 1];
-        s_sqrt[x] = s0;
-        s_dsq[x] = s1 - s0;
-    }
+    tables.fill(P);
     // the loader is the last warp: on a diagonal tile its row has no pair above the diagonal, on a partial tile it is
     // the first row to be absent
     const bool loader = row == kWideDim - 1;
     if (threadIdx.x == 0) { mbar_init(&ctrl->mbar, 1); fence_proxy_async(); }
     const int C = P.C;
     unsigned flags = 0;   // bit 0: parity of the mbarrier, bit 1: control-block slot of the NEXT fetch
-    const uint32_t sq_base = __shfl_sync(kFull, smem_u32(s_sqrt), lane);
-    const uint32_t dsq_base = __shfl_sync(kFull, smem_u32(s_dsq), lane);
-    const uint32_t ratio_base = __shfl_sync(kFull, smem_u32(s_ratio), lane);
-    const uint32_t cnt_lane = __shfl_sync(kFull, smem_u32(cnt + lane), lane);
-    const uint32_t copy8 = 8u * (lane & 15), cap8 = 120u * (uint32_t)rep_n;
-    const uint32_t sq_copy = __shfl_sync(kFull, sq_base + copy8, lane), sq_cap = __shfl_sync(kFull, sq_base + cap8, lane);
-    const uint32_t dsq_copy = __shfl_sync(kFull, dsq_base + copy8, lane), dsq_cap = __shfl_sync(kFull, dsq_base + cap8, lane);
-    auto sq_addr = [&](uint32_t e8) -> uint32_t { return REP ? min(16u * e8 + sq_copy, e8 + sq_cap) : sq_base + e8; };
-    auto dsq_addr = [&](uint32_t e8) -> uint32_t { return REP ? min(16u * e8 + dsq_copy, e8 + dsq_cap) : dsq_base + e8; };
+    const TileLane<CP, REP> L(tables, cnt, lane);
     const uint64_t n = a.uniform_n, n_units = a.n_tiles * n;
     const WfDev& wf = P.wfs[0];
 
@@ -2627,15 +2663,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) score_wide_kernel(ScoreArgs a
     // (lane l: row l and column l), claiming runs of units from a.cursor as score_tile_kernel does.
     uint64_t run_pos = 0, run_end = 0, nx_unit = 0;   // loader warp, uniform
     auto fetch = [&]() {
-        if (run_pos == run_end) {
-            unsigned long long got = 0;
-            if (lane == 0) got = atomicAdd(a.cursor, (unsigned long long)a.run);
-            got = __shfl_sync(kFull, got, 0);
-            run_pos = min((uint64_t)got, n_units);
-            run_end = min((uint64_t)got + a.run, n_units);
-        }
-        const uint64_t u = run_pos;
-        if (run_pos < run_end) ++run_pos;
+        const uint64_t u = claim_unit(a, n_units, run_pos, run_end, lane);
         nx_unit = u;
         uint64_t off_a = 0, off_b = 0, last_a = 0, last_b = 0;
         uint32_t m_a = ~0u, m_b = ~0u;
@@ -2646,16 +2674,8 @@ __global__ void __launch_bounds__(kWideThreads, 1) score_wide_kernel(ScoreArgs a
             if (lane == 0) { ctrl->tile[(flags >> 1) & 1u] = (uint32_t)tile; ctrl->p[(flags >> 1) & 1u] = (uint32_t)p; }
             const WideTile& T = a.wide_tiles[tile];
             const uint64_t fa = __ldg(T.a_first + lane), fb = __ldg(T.b_first + lane);
-            if (fa != kTileNone) {
-                off_a = __ldg(a.a.off + fa + p);
-                m_a = __ldg(a.a.count + fa + p);
-                if (m_a & 1u) last_a = __ldg(a.a.key + off_a + m_a - 1);
-            }
-            if (fb != kTileNone) {
-                off_b = __ldg(a.b.off + fb + p);
-                m_b = __ldg(a.b.count + fb + p);
-                if (m_b & 1u) last_b = __ldg(a.b.key + off_b + m_b - 1);
-            }
+            if (fa != kTileNone) load_env(a.a, fa, p, off_a, m_a, last_a);
+            if (fb != kTileNone) load_env(a.b, fb, p, off_b, m_b, last_b);
         }
         ctrl->nx_off[lane] = off_a; ctrl->nx_last[lane] = last_a; ctrl->nx_M[lane] = m_a;
         ctrl->nx_off[kWideDim + lane] = off_b; ctrl->nx_last[kWideDim + lane] = last_b; ctrl->nx_M[kWideDim + lane] = m_b;
@@ -2676,8 +2696,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) score_wide_kernel(ScoreArgs a
                 if (__any_sync(kFull, (has_a && m_a == 0) || (has_b && m_b == 0))) { raise(P.err, LOCOHD_ERR_EMPTY_ENV); state = 1; }
                 if (!has_a || state) m_a = 0;
                 if (!has_b || state) m_b = 0;
-                // the even part of an environment comes as one bulk copy; an odd last member is stored by hand, so the
-                // sentinel behind it is never overwritten by the copy
+                // the bulk copies of stage_env: the even part of every environment
                 const uint32_t bytes_a = (m_a & ~1u) * 8u, bytes_b = (m_b & ~1u) * 8u;
                 uint32_t total = bytes_a + bytes_b;
 #pragma unroll
@@ -2685,18 +2704,10 @@ __global__ void __launch_bounds__(kWideThreads, 1) score_wide_kernel(ScoreArgs a
                 if (state == 0) {
                     if (lane == 0) { fence_proxy_async(); mbar_expect_tx(&ctrl->mbar, total); }
                     __syncwarp();
-                    uint64_t* sa = stage_a + lane * slot_a;
-                    uint64_t* sb = stage_b + lane * slot_b;
-                    if (m_a) {
-                        if (bytes_a) { fence_proxy_async(); bulk_g2s(sa, a.a.key + ctrl->nx_off[lane], bytes_a, &ctrl->mbar); }
-                        if (m_a & 1u) sa[m_a - 1] = ctrl->nx_last[lane];
-                        sa[m_a] = kSentinel;
-                    }
-                    if (m_b) {
-                        if (bytes_b) { fence_proxy_async(); bulk_g2s(sb, a.b.key + ctrl->nx_off[kWideDim + lane], bytes_b, &ctrl->mbar); }
-                        if (m_b & 1u) sb[m_b - 1] = ctrl->nx_last[kWideDim + lane];
-                        sb[m_b] = kSentinel;
-                    }
+                    if (m_a) stage_env(stage_a + lane * slot_a, a.a.key + ctrl->nx_off[lane], bytes_a, m_a, ctrl->nx_last[lane], &ctrl->mbar);
+                    if (m_b)
+                        stage_env(stage_b + lane * slot_b, a.b.key + ctrl->nx_off[kWideDim + lane], bytes_b, m_b,
+                                  ctrl->nx_last[kWideDim + lane], &ctrl->mbar);
                 }
                 ctrl->M[lane] = m_a;
                 ctrl->M[kWideDim + lane] = m_b;
@@ -2736,82 +2747,35 @@ __global__ void __launch_bounds__(kWideThreads, 1) score_wide_kernel(ScoreArgs a
 #pragma unroll
         for (int r = 0; r < CP; ++r) cnt[r * 32 + lane] = (r == (int)catA0 ? 8u : 0u) + (r == (int)catB0 ? 0x80000u : 0u);
         uint32_t left_all = valid ? (Ma - 1u) + (Mb - 1u) : 0u;
-        double wprev = key_value(max(keyA0 & kWMask, keyB0 & kWMask));
-        uint32_t pa = smem_u32(kA + 1), pb = smem_u32(kB + 1);
+        TileWalk w;
+        w.wprev = key_value(max(keyA0 & kWMask, keyB0 & kWMask));
+        w.pa = smem_u32(kA + 1), w.pb = smem_u32(kB + 1);
         // ratio-table entry of a side's total (members taken, anchor included) at p + d: the total is 1 at p = kX + 1
-        const uint32_t dA = ratio_base + 8u - pa, dB = ratio_base + 8u - pb;
-        uint64_t ra = lds_u64(pa), rb = lds_u64(pb);
-        double rA, rB, h, acc = 0.0;
-        // 4 H^2 in the difference form from the counts (small H^2 only)
-        auto exact_4h2 = [&]() -> double {
-            double s = 0.0;
-#pragma unroll
-            for (int r = 0; r < CP; ++r) {
-                const uint32_t word = cnt[r * 32 + lane];
-                const double u = __dmul_rn(lds_f64(sq_addr(word & 0xffffu)), rA) - __dmul_rn(lds_f64(sq_addr(word >> 16)), rB);
-                s = fma(u, u, s);
-            }
-            return 2.0 * s;
-        };
+        w.dA = L.ratio_base + 8u - w.pa, w.dB = L.ratio_base + 8u - w.pb;
+        w.ra = lds_u64(w.pa), w.rb = lds_u64(w.pb);
+        w.acc = 0.0;
         for (;;) {
             // D, R, sum_r |a_r - b_r| and H from the counts: at the anchors, then every kWideBlock events
-            rA = __ldg(P.rsqrt_tbl + ((pa + dA - ratio_base) >> 3));
-            rB = __ldg(P.rsqrt_tbl + ((pb + dB - ratio_base) >> 3));
+            w.rA = __ldg(P.rsqrt_tbl + ((w.pa + w.dA - L.ratio_base) >> 3));
+            w.rB = __ldg(P.rsqrt_tbl + ((w.pb + w.dB - L.ratio_base) >> 3));
             uint32_t l1 = 0;
-            double D = 0.0;
+            w.D = 0.0;
 #pragma unroll
             for (int r = 0; r < CP; ++r) {
                 const uint32_t word = cnt[r * 32 + lane];
                 const uint32_t ka = word & 0xffffu, kb = word >> 16;
                 l1 += (ka > kb ? ka - kb : kb - ka) >> 3;
-                D = fma(lds_f64(sq_addr(ka)), lds_f64(sq_addr(kb)), D);
+                w.D = fma(lds_f64(L.sq_addr(ka)), lds_f64(L.sq_addr(kb)), w.D);
             }
-            double R = __dmul_rn(rA, rB);
-            {
-                const double h2 = fma(-R, D, 1.0);
-                h = (l1 == 0) ? 0.0 : (h2 < kSmallH2 ? sqrt(exact_4h2()) : twice_sqrt_unit(h2));
-            }
+            w.R = __dmul_rn(w.rA, w.rB);
+            w.h = L.start_h(l1, w);
             const uint32_t nev = min(left_all, (uint32_t)kWideBlock);
             left_all -= nev;
-            uint32_t m = l1 - 1u;   // identical compositions after the event taken with `left` to go: m + left == nev
-#pragma unroll 2
-            for (uint32_t left = nev; left != 0; --left) {
-                const bool takeA = ra <= (rb | kCatMask);   // == (ra & kWMask) <= (rb & kWMask)
-                const uint64_t raw = takeA ? ra : rb;
-                const double w = key_value(raw);
-                acc = fma(w - wprev, h, acc);
-                wprev = w;
-                uint32_t ca;   // cnt_lane + category * 128
-                asm("mad.lo.u32 %0, %1, 128, %2;" : "=r"(ca) : "r"((uint32_t)raw & 0xFFu), "r"(cnt_lane));
-                const uint32_t word = lds_u32_rmw(ca);
-                const uint32_t ka = word & 0xffffu, kb = word >> 16;
-                const uint32_t mine_k = takeA ? ka : kb, other_k = takeA ? kb : ka;
-                sts_u32_rmw(ca, word + (takeA ? 8u : 0x80000u));
-                asm("{\n\t.reg .pred p;\n\tsetp.ge.u32 p, %1, %2;\n\t@p add.u32 %0, %0, 2;\n\t}" : "+r"(m) : "r"(mine_k), "r"(other_k));
-                const uint32_t pk = takeA ? pa : pb;
-                D = fma(lds_f64(dsq_addr(mine_k)), lds_f64(sq_addr(other_k)), D);
-                R *= lds_f64(pk + (takeA ? dA : dB));
-                const uint64_t nxt = lds_u64(pk + 8u);
-                pa = takeA ? pk + 8u : pa;
-                pb = takeA ? pb : pk + 8u;
-                ra = takeA ? nxt : ra;
-                rb = takeA ? rb : nxt;
-                const double h2 = fma(-R, D, 1.0);
-                h = twice_sqrt_unit(h2);
-                if ((float)h2 < kSmallH2f) {   // h2 < 1e-8 (or negative): identical counts (exactly 0) or rare (difference form)
-                    if (m + left == nev) {
-                        h = 0.0;
-                    } else {
-                        rA = __ldg(P.rsqrt_tbl + ((pa + dA - ratio_base) >> 3));
-                        rB = __ldg(P.rsqrt_tbl + ((pb + dB - ratio_base) >> 3));
-                        h = sqrt(exact_4h2());
-                    }
-                }
-            }
+            walk_events(L, P.rsqrt_tbl, w, nev, l1);
             if (left_all == 0) break;
         }
-        acc = fma(wf.w_inf - wprev, h, acc);   // tail to infinity
-        if (valid) a.out[out_first + ctrl->p[slot]] = 0.5 * acc;
+        w.acc = fma(wf.w_inf - w.wprev, w.h, w.acc);   // tail to infinity
+        if (valid) a.out[out_first + ctrl->p[slot]] = 0.5 * w.acc;
     }
 }
 
@@ -3208,13 +3172,19 @@ static int fused_wfk(const KParams& p, const WfDev* host_wf, int key_is_w) {
     return 2;
 }
 
+static int sm_count() {
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    return sms;
+}
+
 template <int WFK, bool DEBUG, int CAP, bool LIST>
 static unsigned fused_grid_t(uint64_t n_env) {
     const int smem = FusedLayout<DEBUG, CAP>::kBytes * fused_warps(CAP, DEBUG);
     cudaFuncSetAttribute(env_fused_kernel<WFK, DEBUG, CAP, LIST>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    int dev = 0, sms = 148, occ = 1;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = sm_count();
+    int occ = 1;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, env_fused_kernel<WFK, DEBUG, CAP, LIST>, fused_warps(CAP, DEBUG) * 32, smem);
     if (occ < 1) occ = 1;
     const uint64_t need = (n_env + fused_warps(CAP, DEBUG) - 1) / fused_warps(CAP, DEBUG);
@@ -3325,9 +3295,8 @@ int launch_rows_copy(const double* values, const double* xyz, const uint8_t* cat
 
 template <class K>
 static unsigned persistent_grid(K kernel, int threads, int smem, uint64_t n_pairs, int warps) {
-    int dev = 0, sms = 148, occ = 1;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = sm_count();
+    int occ = 1;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, smem);
     if (occ < 1) occ = 1;
     const uint64_t need = (n_pairs + warps - 1) / warps;
@@ -3394,50 +3363,62 @@ LaunchOverrides read_launch_overrides() {
     return o;
 }
 
+// Whether the tile kernels apply - the configuration of score_fast_kernel<CP, true, false>, non-empty environments -
+// and, if so, their count rows per warp (cp) and the entries of each table (table_n) for environments of at most
+// max_a / max_b members.
+static bool tile_tables(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, int* cp, int* table_n) {
+    if (!(p.hell2 && p.unit_w && p.C >= 1 && p.C <= 16 && key_is_w) || max_a < 1 || max_b < 1) return false;
+    const unsigned need = (max_a > max_b ? max_a : max_b) + 2u;
+    *table_n = (int)((need + 63u) & ~63u);
+    *cp = p.C <= 8 ? 8 : 16;
+    return true;
+}
+
+// Entries of the replicated head of the two count-indexed tables (240 bytes each) in `spare` bytes of shared memory:
+// at most kTileRepMax, none below 16; LaunchOverrides::tile_rep lowers it.  Only the 8-row instantiations have the
+// replicated form.
+static int tile_rep_n(int cp, int spare, const LaunchOverrides& ov) {
+    int rep_n = cp == 8 ? spare / 240 : 0;
+    if (rep_n > kTileRepMax) rep_n = kTileRepMax;
+    if (rep_n < 16) rep_n = 0;
+    if (ov.tile_rep >= 0 && ov.tile_rep < rep_n) rep_n = ov.tile_rep;
+    return rep_n;
+}
+
+// Units a loader claims at once: a quarter of what each of `workers` (teams or CTAs) gets on average - short launches
+// take shorter runs, which even out the tail -, within 1 ... LaunchOverrides::tile_run (kTileRun by default).
+static unsigned claim_run(uint64_t units, uint64_t workers, const LaunchOverrides& ov) {
+    const uint64_t per_worker = units / (workers * 4);
+    const uint64_t max_run = ov.tile_run ? ov.tile_run : kTileRun;
+    return (unsigned)(per_worker < 1 ? 1 : (per_worker > max_run ? max_run : per_worker));
+}
+
 TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, const LaunchOverrides& ov) {
     TileGeometry g{};
-    if (!(p.hell2 && p.unit_w && p.C >= 1 && p.C <= 16 && key_is_w)) return g;   // the configuration of score_fast_kernel<CP, true, false>
-    if (max_a < 1 || max_b < 1 || max_a + max_b > 1024u) return g;   // chunks of at most 128 events per lane
-    const unsigned need = (max_a > max_b ? max_a : max_b) + 2u;
-    g.table_n = (int)((need + 63u) & ~63u);
-    g.cp = p.C <= 8 ? 8 : 16;
+    if (!tile_tables(p, max_a, max_b, key_is_w, &g.cp, &g.table_n) || max_a + max_b > 1024u)   // chunks of at most
+        return TileGeometry{};                                                                  // 128 events per lane
     g.stage_keys = kTileDim * (int)((max_a + 2u) & ~1u) + kTileDim * (int)((max_b + 2u) & ~1u);
     g.team_bytes = tile_team_bytes(g.cp, g.stage_keys);
     const int budget = 227 * 1024 - 3 * g.table_n * 8;
     int teams = budget / g.team_bytes;
     if (teams > kTileMaxTeams) teams = kTileMaxTeams;
     if (ov.tile_teams >= 1 && ov.tile_teams < teams) teams = ov.tile_teams;
-    // what the teams leave over replicates the head of the two count-indexed tables (240 bytes per entry); only the
-    // 8-row instantiation has the replicated form
-    int rep_n = teams > 0 && g.cp == 8 ? (budget - teams * g.team_bytes) / 240 : 0;
-    if (rep_n > kTileRepMax) rep_n = kTileRepMax;
-    if (rep_n < 16) rep_n = 0;
-    if (ov.tile_rep >= 0 && ov.tile_rep < rep_n) rep_n = ov.tile_rep;
     g.teams = teams;
-    g.rep_n = rep_n;
+    g.rep_n = teams > 0 ? tile_rep_n(g.cp, budget - teams * g.team_bytes, ov) : 0;   // what the teams leave over
     return g;
 }
 
 WideGeometry wide_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, const LaunchOverrides& ov) {
     WideGeometry g{};
-    if (!(p.hell2 && p.unit_w && p.C >= 1 && p.C <= 16 && key_is_w)) return g;   // as tile_geometry
-    if (max_a < 1 || max_b < 1 || max_a > 4096u || max_b > 4096u) return g;
-    g.cp = p.C <= 8 ? 8 : 16;
+    if (!tile_tables(p, max_a, max_b, key_is_w, &g.cp, &g.table_n) || max_a > 4096u || max_b > 4096u) return WideGeometry{};
     g.slot_a = (int)((max_a + 2u) & ~1u);
     g.slot_b = (int)((max_b + 2u) & ~1u);
-    const unsigned need = (max_a > max_b ? max_a : max_b) + 2u;
-    g.table_n = (int)((need + 63u) & ~63u);
     // count rows of 1024 lanes, control block, the three tables and a stage of 32 + 32 environments
     const int fixed = g.cp * kWideThreads * 4 + kWideCtrlBytes + 3 * g.table_n * 8 + kWideDim * (g.slot_a + g.slot_b) * 8;
     const int budget = 227 * 1024;
     if (fixed > budget) return g;
-    // what is left over replicates the head of the two count-indexed tables, as in tile_geometry
-    int rep_n = g.cp == 8 ? (budget - fixed) / 240 : 0;
-    if (rep_n > kTileRepMax) rep_n = kTileRepMax;
-    if (rep_n < 16) rep_n = 0;
-    if (ov.tile_rep >= 0 && ov.tile_rep < rep_n) rep_n = ov.tile_rep;
-    g.rep_n = rep_n;
-    g.smem = fixed + 240 * rep_n;
+    g.rep_n = tile_rep_n(g.cp, budget - fixed, ov);   // what is left over
+    g.smem = fixed + 240 * g.rep_n;
     // the count-row address of a category byte (up to 255) of lane 31 of warp 31 stays inside the allocation
     const int reach = ((kWideDim - 1) * g.cp + 256) * 128;
     if (g.smem < reach) g.smem = reach;
@@ -3475,19 +3456,15 @@ static int launch_tiles(const ScoreArgs& args, const KParams& p, unsigned max_a,
     a.rep_n = g.rep_n;
     const bool rep = a.rep_n > 0;
     const int smem = (g.table_n + 2 * (15 * a.rep_n + g.table_n)) * 8 + teams * team_bytes;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const uint64_t units = mode == TileMode::kCross       ? cross_units(a.cross)
                            : mode == TileMode::kCondensed ? condensed_units(a.condensed)
                                                           : a.n_tiles * a.uniform_n;
     if (!units) return 0;
     const uint64_t need = (units + teams - 1) / teams;
-    const unsigned grid = (unsigned)(need < (uint64_t)sms ? need : (uint64_t)sms);   // persistent: teams claim units from the cursor
+    const uint64_t sms = (uint64_t)sm_count();
+    const unsigned grid = (unsigned)(need < sms ? need : sms);   // persistent: teams claim units from the cursor
     cudaMemsetAsync(a.cursor, 0, sizeof(unsigned long long), st);
-    const uint64_t per_team = units / ((uint64_t)grid * teams * 4);   // short launches: shorter runs even out the tail
-    const uint64_t max_run = ov.tile_run ? ov.tile_run : kTileRun;
-    a.run = (unsigned)(per_team < 1 ? 1 : (per_team > max_run ? max_run : per_team));
+    a.run = claim_run(units, (uint64_t)grid * teams, ov);
     if (mode == TileMode::kJobs) a.order = make_tile_order(a.n_tiles, a.uniform_n, tile_slice(a, mean_a, mean_b, ov));
     auto go = [&](auto kernel) {
         cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
@@ -3517,14 +3494,10 @@ static int launch_wide(const ScoreArgs& args, const KParams& p, unsigned max_a, 
     a.rep_n = g.rep_n;
     const uint64_t units = a.n_tiles * a.uniform_n;
     if (!units) return 0;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const unsigned grid = (unsigned)(units < (uint64_t)sms ? units : (uint64_t)sms);   // persistent, one CTA per SM
+    const uint64_t sms = (uint64_t)sm_count();
+    const unsigned grid = (unsigned)(units < sms ? units : sms);   // persistent, one CTA per SM
     cudaMemsetAsync(a.cursor, 0, sizeof(unsigned long long), st);
-    const uint64_t per_cta = units / ((uint64_t)grid * 4);   // short launches: shorter runs even out the tail
-    const uint64_t max_run = ov.tile_run ? ov.tile_run : kTileRun;
-    a.run = (unsigned)(per_cta < 1 ? 1 : (per_cta > max_run ? max_run : per_cta));
+    a.run = claim_run(units, grid, ov);
     a.order = make_tile_order(a.n_tiles, a.uniform_n, tile_slice(a, mean_a, mean_b, ov));
     auto go = [&](auto kernel) {
         cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem);

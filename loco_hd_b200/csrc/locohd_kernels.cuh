@@ -343,8 +343,8 @@ int launch_condensed_pairs(uint64_t first, uint64_t n, uint64_t i0, uint64_t row
 int launch_row_topk(const double* scores, uint64_t rows, uint64_t cols, int k, int64_t self_off, double* knn_scores,
                     uint32_t* knn_index, cudaStream_t st);
 // Launch geometry of score_tile_kernel for environments of at most max_a / max_b members (teams = 0: the kernel does
-// not apply; below 6 teams the pair kernel is the better one and job lists are not tiled).  The one place that decides
-// it: launch_tiles, the tile eligibility of locohd_score_jobs_stats and locohd_tile_geometry read it.
+// not apply; below kTileMinTeams teams the pair kernel is the better one and pairs do not take the tile route).  The one
+// place that decides it: launch_tiles, the tile route of locohd_capi.cu and locohd_tile_geometry read it.
 struct TileGeometry {
     int teams;        // teams of four warps per CTA (LaunchOverrides::tile_teams lowers it)
     int cp;           // count rows per warp: 8 (C <= 8) or 16 (C <= 16), the instantiation score_tile_kernel<cp, ...>
@@ -355,6 +355,7 @@ struct TileGeometry {
     int team_bytes;   // shared memory per team
 };
 TileGeometry tile_geometry(const KParams& p, unsigned max_a, unsigned max_b, int key_is_w, const LaunchOverrides& ov);
+constexpr int kTileMinTeams = 6;   // with fewer teams per SM the pair kernel is the better one (the tile route is off)
 // Launch geometry of score_wide_kernel (fits = false: it does not apply).  One CTA of 1024 threads stages the <= 32
 // row and <= 32 column environments of a unit in fixed slots of slot_a / slot_b keys.  The one place that decides it:
 // launch_score and the route of locohd_score_jobs_stats read it.
