@@ -112,6 +112,7 @@ typedef enum locohd_prof_group {
 typedef struct locohd_ctx locohd_ctx;            /* one GPU + one stream + one LoCoHD parameter set */
 typedef struct locohd_structs locohd_structs;    /* device-resident set of primitive structures */
 typedef struct locohd_envset locohd_envset;      /* device-resident sorted environments of a list of anchors */
+typedef struct locohd_graph locohd_graph;        /* device-resident sparse result: pairs whose score is within a bound */
 
 /* A run of anchor pairs with identity pairing: pair p (0 <= p < n) scores environment
  * (a_first + p) of env-set A against environment (b_first + p) of env-set B. */
@@ -268,6 +269,31 @@ int locohd_score_cross(locohd_ctx* ctx, const locohd_envset* a, uint64_t a_first
  * categories and empty environments as in locohd_score_jobs.  n < 2 writes nothing. */
 int locohd_score_condensed(locohd_ctx* ctx, const locohd_envset* s, uint64_t first, uint64_t n, uint32_t wf_idx,
                            double* out_scores);
+/* Threshold graphs (an extension, for density clustering, connected components of similar sites and near-duplicate
+ * counts without the dense matrix): every pair whose score s satisfies s <= max_score, as a CSR graph that stays on
+ * the device until locohd_graph_copy.  NaN scores are never in the graph, +inf is when max_score is +inf, a NaN
+ * max_score is LOCOHD_ERR_BAD_PARAM.  Rows ascend, columns ascend within a row, and every stored score is
+ * bit-identical to the same entry of locohd_score_cross (locohd_score_within) or locohd_score_condensed
+ * (locohd_score_within_condensed) on the same range and route; the result is the same on every call.
+ * locohd_score_within: rows = n_a, row i holds the columns j (u32, relative to b_first) with M[i][j] <= max_score, M
+ * the matrix of locohd_score_cross; range, skip_self, wf_idx checks, route and chunks as there (LOCOHD_CROSS_ROWS
+ * lowers the rows per chunk).  locohd_score_within_condensed: rows = cols = n, row i holds only the columns j > i (the
+ * upper triangle) of the range against itself; symmetric distances only, as locohd_score_condensed.  Both score in
+ * chunks of the 256 MB scratch and read back one count per chunk; the graph storage grows geometrically and ends at
+ * 8 (rows + 1) + 12 nnz bytes.  Empty ranges give an empty graph of `rows` rows.  On any error *out is NULL; a failed
+ * allocation of the graph storage is LOCOHD_ERR_CUDA with the entries reached in the message.  The graph keeps its
+ * context's device memory until locohd_graph_destroy, which must come before locohd_ctx_destroy. */
+int locohd_score_within(locohd_ctx* ctx, const locohd_envset* a, uint64_t a_first, uint64_t n_a, const locohd_envset* b,
+                        uint64_t b_first, uint64_t n_b, uint32_t wf_idx, int skip_self, double max_score,
+                        locohd_graph** out);
+int locohd_score_within_condensed(locohd_ctx* ctx, const locohd_envset* s, uint64_t first, uint64_t n, uint32_t wf_idx,
+                                  double max_score, locohd_graph** out);
+/* rows, cols and stored entries of a graph (any output may be NULL) */
+int locohd_graph_shape(const locohd_graph* g, uint64_t* rows, uint64_t* cols, uint64_t* nnz);
+/* Copies indptr [rows + 1] (u64), indices [nnz] (u32) and scores [nnz] (f64) out of the graph: any may be NULL, each
+ * host or device memory; scipy.sparse.csr_matrix((scores, indices, indptr), shape=(rows, cols)) takes them. */
+int locohd_graph_copy(locohd_ctx* ctx, const locohd_graph* g, uint64_t* indptr, uint32_t* indices, double* scores);
+void locohd_graph_destroy(locohd_graph* g);
 /* Planning query, no device needed: position `unit` of a launch of locohd_score_condensed on a range of n environments,
  * for the chunk of row blocks [row_block0, row_block0 + row_blocks) (a row block: 4 rows; ceil(n / 4) blocks) -> the
  * block of 4 x 4 pairs scored there, *out_row_block <= *out_col_block.  Units run column block major: first the

@@ -33,7 +33,8 @@ EXPORTED_SYMBOLS = [
     "locohd_envset_from_ragged_rows",
     "locohd_envset_from_coords", "locohd_envset_destroy", "locohd_envset_size", "locohd_envset_total_members",
     "locohd_envset_dump", "locohd_score_pairs", "locohd_score_jobs", "locohd_score_jobs_stats", "locohd_score_cross",
-    "locohd_score_condensed", "locohd_condensed_unit",
+    "locohd_score_condensed", "locohd_condensed_unit", "locohd_score_within", "locohd_score_within_condensed",
+    "locohd_graph_shape", "locohd_graph_copy", "locohd_graph_destroy",
     "locohd_score_anchor_lists", "locohd_plan_job_tiles", "locohd_tile_unit", "locohd_tile_geometry",
     "locohd_from_primitives", "locohd_from_primitives_grad", "locohd_from_rows_grad", "locohd_from_coords_grad",
     "locohd_wf_integral_points", "locohd_wf_density_points", "locohd_sd_run",
@@ -128,6 +129,11 @@ def load_library() -> C.CDLL:
         "locohd_score_cross": (C.c_int, [vp, vp, u64, u64, vp, u64, u64, u32, C.c_int, vp, u32, vp, vp]),
         "locohd_score_condensed": (C.c_int, [vp, vp, u64, u64, u32, vp]),
         "locohd_condensed_unit": (C.c_int, [u64, u64, u64, u64, C.POINTER(u64), C.POINTER(u64)]),
+        "locohd_score_within": (C.c_int, [vp, vp, u64, u64, vp, u64, u64, u32, C.c_int, dbl, C.POINTER(vp)]),
+        "locohd_score_within_condensed": (C.c_int, [vp, vp, u64, u64, u32, dbl, C.POINTER(vp)]),
+        "locohd_graph_shape": (C.c_int, [vp, C.POINTER(u64), C.POINTER(u64), C.POINTER(u64)]),
+        "locohd_graph_copy": (C.c_int, [vp, vp, vp, vp, vp]),
+        "locohd_graph_destroy": (None, [vp]),
         "locohd_score_anchor_lists": (C.c_int, [vp, vp, u64, vp, u64, vp, u64, vp, u64, u32, vp]),
         "locohd_plan_job_tiles": (C.c_int, [u64, vp, vp, vp, vp]),
         "locohd_tile_unit": (C.c_int, [u64, u64, u64, u64, C.POINTER(u64), C.POINTER(u64)]),
@@ -453,6 +459,27 @@ class Context:
         self._check(self.lib.locohd_score_condensed(self.h, env.h, first, n, wf_idx, _p(out)))
         return out
 
+    def score_within(self, a: "EnvSet", b: "EnvSet", max_score: float, a_first: int = 0, n_a: Optional[int] = None,
+                     b_first: int = 0, n_b: Optional[int] = None, wf_idx: int = 0, skip_self: bool = False) -> "Graph":
+        """locohd_score_within: the entries M[i][j] <= max_score of the score_cross matrix of the same ranges, as a
+        device-resident CSR graph of n_a rows (columns relative to b_first); n_a / n_b default to the rest of the set."""
+        na = len(a) - a_first if n_a is None else int(n_a)
+        nb = len(b) - b_first if n_b is None else int(n_b)
+        h = C.c_void_p()
+        self._check(self.lib.locohd_score_within(self.h, a.h, a_first, na, b.h, b_first, nb, wf_idx, int(skip_self),
+                                                 float(max_score), C.byref(h)))
+        return Graph(self, h)
+
+    def score_within_condensed(self, env: "EnvSet", max_score: float, first: int = 0, n: Optional[int] = None,
+                               wf_idx: int = 0) -> "Graph":
+        """locohd_score_within_condensed: the pairs i < j of one range whose score is <= max_score, row i holding its
+        columns j > i (the upper triangle), as a device-resident CSR graph of n rows."""
+        n = len(env) - first if n is None else int(n)
+        h = C.c_void_p()
+        self._check(self.lib.locohd_score_within_condensed(self.h, env.h, first, n, wf_idx, float(max_score),
+                                                           C.byref(h)))
+        return Graph(self, h)
+
     def score_jobs(self, a: "EnvSet", b: "EnvSet", jobs, wf_idx=None, out=None, want_scores=True, want_means=False,
                    means_out=None):
         """`out` / `means_out`: numpy array (host) or raw device pointer; with `want_scores=False` and a `means_out`
@@ -659,6 +686,49 @@ class EnvSet:
     def close(self):
         if self.h and self.ctx.h:
             self.ctx.lib.locohd_envset_destroy(self.h)
+        self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class Graph:
+    """A threshold graph (locohd_graph) on the device: CSR rows of the pairs whose score is within the bound."""
+
+    def __init__(self, ctx: Context, h):
+        self.ctx, self.h = ctx, h
+
+    def _shape(self):
+        rows, cols, nnz = C.c_uint64(), C.c_uint64(), C.c_uint64()
+        self.ctx._check(self.ctx.lib.locohd_graph_shape(self.h, C.byref(rows), C.byref(cols), C.byref(nnz)))
+        return int(rows.value), int(cols.value), int(nnz.value)
+
+    @property
+    def shape(self) -> Tuple[int, int]:
+        return self._shape()[:2]
+
+    @property
+    def nnz(self) -> int:
+        return self._shape()[2]
+
+    def copy(self, indptr=None, indices=None, scores=None):
+        """-> (indptr [rows + 1] uint64, indices [nnz] uint32, scores [nnz] float64).  Each argument: None (a new host
+        array), False (not copied, None returned), an output array or a raw device pointer."""
+        rows, _, nnz = self._shape()
+
+        def buf(x, n, dtype):
+            return np.empty(n, dtype) if x is None else (None if x is False else x)
+
+        ip, ix, sc = buf(indptr, rows + 1, np.uint64), buf(indices, nnz, np.uint32), buf(scores, nnz, np.float64)
+        self.ctx._check(self.ctx.lib.locohd_graph_copy(self.ctx.h, self.h, _p(ip), _p(ix), _p(sc)))
+        return ip, ix, sc
+
+    def close(self):
+        if self.h and self.ctx.h:
+            self.ctx.lib.locohd_graph_destroy(self.h)
         self.h = None
 
     def __del__(self):

@@ -1145,6 +1145,54 @@ struct LoCoHD {
         device_call(env->dev, [&](locohd_ctx* c) { return locohd_score_condensed(c, env->h, r.first, r.second, wf, o); });
         return out;
     }
+
+    // threshold graphs (locohd_score_within[_condensed]) -> host CSR arrays (indptr, indices, scores)
+    static double graph_bound(double max_score) {
+        if (std::isnan(max_score)) throw py::value_error("max_score is NaN");
+        return max_score;
+    }
+    static py::tuple graph_arrays(const std::shared_ptr<Dev>& dev, locohd_graph* g) {
+        std::unique_ptr<locohd_graph, void (*)(locohd_graph*)> hold(g, locohd_graph_destroy);
+        uint64_t rows = 0, cols = 0, nnz = 0;
+        locohd_graph_shape(g, &rows, &cols, &nnz);
+        py::array_t<int64_t> indptr((py::ssize_t)(rows + 1));
+        py::array_t<uint32_t> indices((py::ssize_t)nnz);
+        py::array_t<double> scores((py::ssize_t)nnz);
+        uint64_t* pi = reinterpret_cast<uint64_t*>(indptr.mutable_data());
+        uint32_t* px = indices.mutable_data();
+        double* ps = scores.mutable_data();
+        device_call(dev, [&](locohd_ctx* c) { return locohd_graph_copy(c, g, pi, px, ps); });
+        return py::make_tuple(indptr, indices, scores);
+    }
+
+    py::tuple environments_within(const std::shared_ptr<Environments>& ea, const std::shared_ptr<Environments>& eb,
+                                  double max_score, const py::object& a_range, const py::object& b_range,
+                                  bool exclude_self, int64_t wf_idx) {
+        check_pair(ea, eb);
+        const auto ra = env_range(a_range, ea->n_env, "a_range"), rb = env_range(b_range, eb->n_env, "b_range");
+        const uint32_t wf = wf_position(wf_idx);
+        if (exclude_self && ea != eb) throw py::value_error("exclude_self needs env_b to be env_a");
+        const double bound = graph_bound(max_score);
+        locohd_graph* g = nullptr;
+        device_call(ea->dev, [&](locohd_ctx* c) {
+            return locohd_score_within(c, ea->h, ra.first, ra.second, eb->h, rb.first, rb.second, wf, exclude_self ? 1 : 0,
+                                       bound, &g);
+        });
+        return graph_arrays(ea->dev, g);
+    }
+
+    py::tuple environments_within_condensed(const std::shared_ptr<Environments>& env, double max_score,
+                                            const py::object& range, int64_t wf_idx) {
+        check_pair(env, env);
+        const auto r = env_range(range, env->n_env, "env_range");
+        const uint32_t wf = wf_position(wf_idx);
+        const double bound = graph_bound(max_score);
+        locohd_graph* g = nullptr;
+        device_call(env->dev, [&](locohd_ctx* c) {
+            return locohd_score_within_condensed(c, env->h, r.first, r.second, wf, bound, &g);
+        });
+        return graph_arrays(env->dev, g);
+    }
 };
 
 }  // namespace
@@ -1258,7 +1306,19 @@ PYBIND11_MODULE(loco_hd, m) {
              "Every pair i < j of env_range of env (a range (start, stop), None = the whole set) once, in the order of "
              "scipy.spatial.distance.pdist: a float64 array [n (n - 1) / 2] that scipy.cluster.hierarchy.linkage and "
              "squareform take.  Needs a symmetric statistical distance (Hellinger or Kolmogorov-Smirnov); "
-             "score_matrix gives both triangles of an asymmetric one.");
+             "score_matrix gives both triangles of an asymmetric one.")
+        .def("environments_within", &LoCoHD::environments_within, py::arg("env_a"), py::arg("env_b"),
+             py::arg("max_score"), py::arg("a_range") = py::none(), py::arg("b_range") = py::none(),
+             py::arg("exclude_self") = false, py::arg("wf_idx") = 0,
+             "Every pair of a_range of env_a and b_range of env_b whose score_matrix entry is <= max_score, as CSR "
+             "arrays (indptr int64 [n_a + 1], columns uint32 [nnz] relative to the start of b_range, scores float64 "
+             "[nnz]) that scipy.sparse.csr_matrix((scores, columns, indptr), shape=(n_a, n_b)) takes.  Rows and the "
+             "columns within a row ascend; NaN scores are never in it.  The matrix stays on the device.")
+        .def("environments_within_condensed", &LoCoHD::environments_within_condensed, py::arg("env"),
+             py::arg("max_score"), py::arg("env_range") = py::none(), py::arg("wf_idx") = 0,
+             "The pairs i < j of env_range of env whose score is <= max_score: CSR arrays as environments_within with "
+             "n rows, row i holding only columns j > i (the upper triangle).  Needs a symmetric statistical distance, "
+             "as score_condensed.");
 
     py::class_<Structures, std::shared_ptr<Structures>>(m, "Structures")
         .def_readonly("n_structures", &Structures::n_structs)

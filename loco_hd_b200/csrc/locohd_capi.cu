@@ -55,13 +55,14 @@ struct locohd_ctx {
     double* d_sqrt_tbl = nullptr;
     double* d_rsqrt_tbl = nullptr;
     int* d_err = nullptr;
-    ScanStats* d_scan = nullptr;   // two slots: [0] anchor order, [1] environment sizes
+    ScanStats* d_scan = nullptr;   // three slots: [0] anchor order, [1] environment sizes, [2] a chunk of a graph
     FusedStats* d_fstats = nullptr;  // fused gather: store cursor, sample sum, largest environment, overflow word
     unsigned long long* d_score_cursor = nullptr;   // scoring kernel: next unclaimed pair
     // pinned host mirrors: the error word and the gather statistics come back with asynchronous copies queued before
     // the stream synchronisation (no separate blocking cudaMemcpy per synchronisation point)
     int* h_err = nullptr;
     FusedStats* h_fstats = nullptr;   // two slots: [0] sizing sample, [1] result of the fused gather
+    ScanStats* h_scan = nullptr;      // d_scan[2]: the entries of a chunk of a graph (locohd_score_within[_condensed])
     // pinned staging area of the one-call entry point (small calls: all inputs travel in one copy)
     unsigned char* h_stage = nullptr;
     size_t h_stage_bytes = 0;
@@ -144,6 +145,16 @@ struct locohd_envset {
         v.n_env = n_env; v.off = d_off; v.count = d_count; v.key = d_key; v.key_is_w = key_is_w ? 1 : 0;
         return v;
     }
+};
+
+// A threshold graph in CSR form (locohd_score_within[_condensed]): row r holds the columns indices[indptr[r] ..
+// indptr[r + 1]) with their scores.
+struct locohd_graph {
+    locohd_ctx* ctx = nullptr;
+    uint64_t rows = 0, cols = 0, nnz = 0;
+    uint64_t* d_indptr = nullptr;    // [rows + 1]
+    uint32_t* d_indices = nullptr;   // [nnz]
+    double* d_scores = nullptr;      // [nnz]
 };
 
 namespace {
@@ -815,11 +826,12 @@ int locohd_ctx_create(int device, locohd_ctx** out) {
     }
     if ((ce = cudaMalloc(&ctx->d_err, sizeof(int))) != cudaSuccess) return bail(ce);
     if ((ce = cudaMemset(ctx->d_err, 0, sizeof(int))) != cudaSuccess) return bail(ce);
-    if ((ce = cudaMalloc(&ctx->d_scan, 2 * sizeof(ScanStats))) != cudaSuccess) return bail(ce);
+    if ((ce = cudaMalloc(&ctx->d_scan, 3 * sizeof(ScanStats))) != cudaSuccess) return bail(ce);
     if ((ce = cudaMalloc(&ctx->d_fstats, sizeof(FusedStats))) != cudaSuccess) return bail(ce);
     if ((ce = cudaMalloc(&ctx->d_score_cursor, sizeof(unsigned long long))) != cudaSuccess) return bail(ce);
     if ((ce = cudaHostAlloc((void**)&ctx->h_err, sizeof(int), cudaHostAllocDefault)) != cudaSuccess) return bail(ce);
     if ((ce = cudaHostAlloc((void**)&ctx->h_fstats, 2 * sizeof(FusedStats), cudaHostAllocDefault)) != cudaSuccess) return bail(ce);
+    if ((ce = cudaHostAlloc((void**)&ctx->h_scan, sizeof(ScanStats), cudaHostAllocDefault)) != cudaSuccess) return bail(ce);
     *ctx->h_err = 0;
     if ((ce = cudaMalloc(&ctx->d_sqrt_tbl, kSqrtTableSize * sizeof(double))) != cudaSuccess) return bail(ce);
     if ((ce = cudaMalloc(&ctx->d_rsqrt_tbl, kSqrtTableSize * sizeof(double))) != cudaSuccess) return bail(ce);
@@ -844,7 +856,7 @@ void locohd_ctx_destroy(locohd_ctx* ctx) {
     cudaFree(ctx->d_cat_w); cudaFree(ctx->d_cat_sw); cudaFree(ctx->d_wfs); cudaFree(ctx->d_tag_pairs);
     cudaFree(ctx->d_sqrt_tbl); cudaFree(ctx->d_rsqrt_tbl); cudaFree(ctx->d_err); cudaFree(ctx->d_scan);
     cudaFree(ctx->d_fstats); cudaFree(ctx->d_score_cursor);
-    cudaFreeHost(ctx->h_err); cudaFreeHost(ctx->h_fstats); cudaFreeHost(ctx->h_stage);
+    cudaFreeHost(ctx->h_err); cudaFreeHost(ctx->h_fstats); cudaFreeHost(ctx->h_scan); cudaFreeHost(ctx->h_stage);
     cudaStreamDestroy(ctx->stream);
     delete ctx;
 }
@@ -1565,6 +1577,114 @@ int locohd_score_jobs_stats(locohd_ctx* ctx, const locohd_envset* a, const locoh
 // than one launch needs to fill the GPU), and the rows of a chunk stay in L2 while the column blocks pass.
 constexpr uint64_t kCrossScratchBytes = 256ull << 20;
 
+// Route and weight function of the pairs of two ranges (locohd_score_cross, locohd_score_condensed and their graph
+// forms): the tile kernel under the condition of locohd_score_jobs_stats (W-keyed sets - one weight function, so
+// wf_idx is 0 -, Hellinger-2 with unit weights, C <= 16, >= 6 teams); else explicit pairs on the pair kernel, with the
+// chosen weight function as the kernels' function 0.
+struct PairRoute {
+    LaunchOverrides ov;
+    bool tiles;
+    KParams kp;
+};
+
+static PairRoute pair_route(const locohd_ctx* ctx, const locohd_envset* a, const locohd_envset* b, uint32_t wf_idx) {
+    PairRoute r;
+    r.ov = read_launch_overrides();
+    r.tiles = tile_route(ctx, a, b, r.ov);
+    r.kp = ctx->kp;
+    r.kp.wfs = ctx->d_wfs + wf_idx;
+    r.kp.n_wf = 1;
+    return r;
+}
+
+// Rows per chunk of an n_a x n_b cross matrix whose entries take per_entry bytes of scratch (0: none, one chunk).
+// Chunks of R whole rows (R a multiple of 4): a chunk of the dense output is one contiguous block, and the k nearest
+// of a row are found in one pass over it.
+static uint64_t cross_chunk_rows(uint64_t n_a, uint64_t n_b, uint64_t per_entry, const LaunchOverrides& ov) {
+    uint64_t R = per_entry ? kCrossScratchBytes / (per_entry * n_b) : n_a;
+    if (ov.cross_rows && ov.cross_rows < R) R = ov.cross_rows;
+    R = std::max<uint64_t>(R / 4 * 4, 4);
+    return std::min<uint64_t>(R, (n_a + 3) / 4 * 4);
+}
+
+// Scores environments a_first + i (i < rows) of a against b_first + j (j < cols) of b into scores[i * cols + j] on
+// the route's kernel; d_pairs: room for the 2 rows cols pair entries of the pair route.
+static int score_cross_chunk(locohd_ctx* ctx, const PairRoute& r, const locohd_envset* a, uint64_t a_first,
+                             const locohd_envset* b, uint64_t b_first, uint64_t rows, uint64_t cols, double* scores,
+                             uint32_t* d_pairs) {
+    int n = 0;
+    {
+        ProfScope ps(ctx, LOCOHD_PROF_SCORE);
+        ScoreArgs sa{};
+        sa.a = a->view(); sa.b = b->view();
+        sa.out = scores;
+        sa.cursor = ctx->d_score_cursor; sa.run = 1;
+        sa.n_pairs = rows * cols;
+        if (r.tiles) {
+            sa.cross = CrossGrid{a_first, b_first, rows, cols};
+            n = launch_score_cross(sa, r.kp, a->max_count, b->max_count, r.ov, ctx->stream);
+        } else {
+            ctx->launches += launch_cross_pairs(a_first, b_first, rows, cols, d_pairs, ctx->stream);
+            sa.pairs = d_pairs;
+            const double mean_a = a->n_env ? (double)a->total / (double)a->n_env : 0.0;
+            const double mean_b = b->n_env ? (double)b->total / (double)b->n_env : 0.0;
+            n = launch_score(sa, r.kp, a->max_count, b->max_count, mean_a, mean_b, r.ov, ctx->stream);
+        }
+    }
+    if (n < 0) return fail(ctx, LOCOHD_ERR_UNSUPPORTED, "shared memory budget exceeded for %d categories", ctx->kp.C);
+    ctx->launches += n;
+    if (r.tiles) ctx->tile_launches += n;
+    return 0;
+}
+
+// Chunks of whole row blocks (4 rows from `first`) of the condensed vector of n environments: the scores of a chunk
+// are one contiguous slice of the vector.  A chunk takes row blocks while its scores fit the scratch budget (entries
+// of per_score bytes; 0: no scratch, one chunk), so the chunks further down, whose rows are shorter, take more of
+// them; one row block may exceed the budget (rows of more than 8 M columns).
+struct CondensedChunks {
+    uint64_t n, nb, max_blocks, budget;
+    CondensedChunks(uint64_t n_, uint64_t per_score, const LaunchOverrides& ov)
+        : n(n_), nb((n_ + 3) / 4), max_blocks(ov.cross_rows ? std::max<uint64_t>(ov.cross_rows / 4, 1) : (n_ + 3) / 4),
+          budget(per_score ? kCrossScratchBytes / per_score : ~0ull) {}
+    uint64_t row_base(uint64_t i) const { return n * i - triangle<uint64_t>(i); }   // condensed index of (i, i + 1)
+    uint64_t scores_of(uint64_t rb0, uint64_t rb1) const { return row_base(std::min(4 * rb1, n)) - row_base(4 * rb0); }
+    uint64_t end(uint64_t rb0) const {   // the row block after the chunk that starts at rb0
+        uint64_t rb1 = rb0 + 1;
+        while (rb1 < nb && rb1 - rb0 < max_blocks && scores_of(rb0, rb1 + 1) <= budget) ++rb1;
+        return rb1;
+    }
+    uint64_t scratch() const { return std::min(scores_of(0, nb), std::max(budget, scores_of(0, 1))); }   // largest chunk
+};
+
+// Scores the chunk of row blocks [rb0, rb1) of the condensed vector into `scores` (its slice) on the route's kernel;
+// d_pairs: room for the chunk's pair entries on the pair route.
+static int score_condensed_chunk(locohd_ctx* ctx, const PairRoute& r, const locohd_envset* s, uint64_t first,
+                                 const CondensedChunks& c, uint64_t rb0, uint64_t rb1, double* scores, uint32_t* d_pairs) {
+    const uint64_t i0 = 4 * rb0;
+    int launched = 0;
+    {
+        ProfScope ps(ctx, LOCOHD_PROF_SCORE);
+        ScoreArgs sa{};
+        sa.a = s->view(); sa.b = sa.a;
+        sa.out = scores;
+        sa.n_pairs = c.scores_of(rb0, rb1);
+        sa.cursor = ctx->d_score_cursor; sa.run = 1;
+        if (r.tiles) {
+            sa.condensed = CondensedGrid{first, c.n, rb0, rb1 - rb0, c.row_base(i0)};
+            launched = launch_score_condensed(sa, r.kp, s->max_count, r.ov, ctx->stream);
+        } else {
+            ctx->launches += launch_condensed_pairs(first, c.n, i0, std::min(4 * rb1, c.n) - i0, d_pairs, ctx->stream);
+            sa.pairs = d_pairs;
+            const double mean = s->n_env ? (double)s->total / (double)s->n_env : 0.0;
+            launched = launch_score(sa, r.kp, s->max_count, s->max_count, mean, mean, r.ov, ctx->stream);
+        }
+    }
+    if (launched < 0) return fail(ctx, LOCOHD_ERR_UNSUPPORTED, "shared memory budget exceeded for %d categories", ctx->kp.C);
+    ctx->launches += launched;
+    if (r.tiles) ctx->tile_launches += launched;
+    return 0;
+}
+
 int locohd_score_cross(locohd_ctx* ctx, const locohd_envset* a, uint64_t a_first, uint64_t n_a, const locohd_envset* b,
                        uint64_t b_first, uint64_t n_b, uint32_t wf_idx, int skip_self, double* out_scores, uint32_t k,
                        double* out_knn_scores, uint32_t* out_knn_index) {
@@ -1589,22 +1709,9 @@ int locohd_score_cross(locohd_ctx* ctx, const locohd_envset* a, uint64_t a_first
     if (a->key_is_w != b->key_is_w) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "environment sets were built with different weight-function modes");
     if (!n_a || !n_b) return 0;
 
-    // Route: the tile kernel under the condition of locohd_score_jobs_stats (W-keyed sets - one weight function, so
-    // wf_idx is 0 -, Hellinger-2 with unit weights, C <= 16, >= 6 teams); else explicit pairs on the pair kernel, with
-    // the chosen weight function as the kernels' function 0.
-    const LaunchOverrides ov = read_launch_overrides();
-    const bool tiles = tile_route(ctx, a, b, ov);
-    KParams kp = ctx->kp;
-    kp.wfs = ctx->d_wfs + wf_idx;
-    kp.n_wf = 1;
-    // Chunks of R whole rows (R a multiple of 4): a chunk of the dense output is one contiguous block, and the k nearest
-    // of a row are found in one pass over it.
+    const PairRoute route = pair_route(ctx, a, b, wf_idx);
     const bool direct = out_scores && is_device_ptr(ctx, out_scores);   // scores go straight to the caller's matrix
-    const uint64_t per_entry = (direct ? 0 : 8) + (tiles ? 0 : 8);
-    uint64_t R = per_entry ? kCrossScratchBytes / (per_entry * n_b) : n_a;
-    if (ov.cross_rows && ov.cross_rows < R) R = ov.cross_rows;
-    R = std::max<uint64_t>(R / 4 * 4, 4);
-    R = std::min<uint64_t>(R, (n_a + 3) / 4 * 4);
+    const uint64_t R = cross_chunk_rows(n_a, n_b, (direct ? 0 : 8) + (route.tiles ? 0 : 8), route.ov);
     OutBuf<double> kscores;
     OutBuf<uint32_t> kindex;
     TRY_ST(kscores.prepare(ctx, out_knn_scores, knn ? n_a * k : 0));
@@ -1614,33 +1721,12 @@ int locohd_score_cross(locohd_ctx* ctx, const locohd_envset* a, uint64_t a_first
     auto cleanup = [&](int st) { dev_free(ctx, d_chunk); dev_free(ctx, d_pairs); return st; };
     int st = 0;
     if (!direct && (st = dev_alloc(ctx, &d_chunk, R * n_b))) return cleanup(st);
-    if (!tiles && (st = dev_alloc(ctx, &d_pairs, 2 * R * n_b))) return cleanup(st);
+    if (!route.tiles && (st = dev_alloc(ctx, &d_pairs, 2 * R * n_b))) return cleanup(st);
     const int64_t self_off = skip_self ? (int64_t)a_first - (int64_t)b_first : INT64_MIN;
     for (uint64_t row0 = 0; row0 < n_a && !st; row0 += R) {
         const uint64_t rows = std::min(R, n_a - row0);
         double* scores = direct ? out_scores + row0 * n_b : d_chunk;
-        int n = 0;
-        {
-            ProfScope ps(ctx, LOCOHD_PROF_SCORE);
-            ScoreArgs sa{};
-            sa.a = a->view(); sa.b = b->view();
-            sa.out = scores;
-            sa.cursor = ctx->d_score_cursor; sa.run = 1;
-            if (tiles) {
-                sa.n_pairs = rows * n_b;
-                sa.cross = CrossGrid{a_first + row0, b_first, rows, n_b};
-                n = launch_score_cross(sa, kp, a->max_count, b->max_count, ov, ctx->stream);
-            } else {
-                ctx->launches += launch_cross_pairs(a_first + row0, b_first, rows, n_b, d_pairs, ctx->stream);
-                sa.n_pairs = rows * n_b; sa.pairs = d_pairs;
-                const double mean_a = a->n_env ? (double)a->total / (double)a->n_env : 0.0;
-                const double mean_b = b->n_env ? (double)b->total / (double)b->n_env : 0.0;
-                n = launch_score(sa, kp, a->max_count, b->max_count, mean_a, mean_b, ov, ctx->stream);
-            }
-        }
-        if (n < 0) { st = fail(ctx, LOCOHD_ERR_UNSUPPORTED, "shared memory budget exceeded for %d categories", ctx->kp.C); break; }
-        ctx->launches += n;
-        if (tiles) ctx->tile_launches += n;
+        if ((st = score_cross_chunk(ctx, route, a, a_first + row0, b, b_first, rows, n_b, scores, d_pairs))) break;
         if (knn) {
             ProfScope ps(ctx, LOCOHD_PROF_OTHER);
             ctx->launches += launch_row_topk(scores, rows, n_b, (int)k, skip_self ? self_off + (int64_t)row0 : INT64_MIN,
@@ -1679,54 +1765,23 @@ int locohd_score_condensed(locohd_ctx* ctx, const locohd_envset* s, uint64_t fir
     if (!out_scores) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "no output");
 
     // Route and weight function as in locohd_score_cross with the range on both sides.
-    const LaunchOverrides ov = read_launch_overrides();
-    const bool tiles = tile_route(ctx, s, s, ov);
-    KParams kp = ctx->kp;
-    kp.wfs = ctx->d_wfs + wf_idx;
-    kp.n_wf = 1;
-    // Chunks of whole row blocks (4 rows from `first`): the scores of a chunk are one contiguous slice of the condensed
-    // vector.  A chunk takes row blocks while its scores fit the scratch budget, so the chunks further down, whose rows
-    // are shorter, take more of them; one row block may exceed the budget (rows of more than 8 M columns).
+    const PairRoute route = pair_route(ctx, s, s, wf_idx);
     const bool direct = is_device_ptr(ctx, out_scores);   // scores go straight to the caller's vector
-    const uint64_t per_score = (direct ? 0 : 8) + (tiles ? 0 : 8);
-    const uint64_t budget = per_score ? kCrossScratchBytes / per_score : ~0ull;
-    const uint64_t nb = (n + 3) / 4, max_blocks = ov.cross_rows ? std::max<uint64_t>(ov.cross_rows / 4, 1) : nb;
-    auto row_base = [&](uint64_t i) { return n * i - triangle<uint64_t>(i); };   // condensed index of (i, i + 1)
-    auto scores_of = [&](uint64_t rb0, uint64_t rb1) { return row_base(std::min(4 * rb1, n)) - row_base(4 * rb0); };
-    const uint64_t scratch = per_score ? std::min(scores_of(0, nb), std::max(budget, scores_of(0, 1))) : 0;
+    const uint64_t per_score = (direct ? 0 : 8) + (route.tiles ? 0 : 8);
+    const CondensedChunks chunks(n, per_score, route.ov);
+    const uint64_t scratch = per_score ? chunks.scratch() : 0;
     double* d_chunk = nullptr;
     uint32_t* d_pairs = nullptr;
     auto cleanup = [&](int st) { dev_free(ctx, d_chunk); dev_free(ctx, d_pairs); return st; };
     int st = 0;
     if (!direct && (st = dev_alloc(ctx, &d_chunk, scratch))) return cleanup(st);
-    if (!tiles && (st = dev_alloc(ctx, &d_pairs, 2 * scratch))) return cleanup(st);
-    for (uint64_t rb0 = 0, rb1; rb0 < nb && !st; rb0 = rb1) {
-        rb1 = rb0 + 1;
-        while (rb1 < nb && rb1 - rb0 < max_blocks && scores_of(rb0, rb1 + 1) <= budget) ++rb1;
-        const uint64_t i0 = 4 * rb0, base = row_base(i0), count = scores_of(rb0, rb1);
+    if (!route.tiles && (st = dev_alloc(ctx, &d_pairs, 2 * scratch))) return cleanup(st);
+    for (uint64_t rb0 = 0, rb1; rb0 < chunks.nb && !st; rb0 = rb1) {
+        rb1 = chunks.end(rb0);
+        const uint64_t base = chunks.row_base(4 * rb0), count = chunks.scores_of(rb0, rb1);
         if (!count) continue;   // the last row alone: it has no pair
         double* scores = direct ? out_scores + base : d_chunk;
-        int launched = 0;
-        {
-            ProfScope ps(ctx, LOCOHD_PROF_SCORE);
-            ScoreArgs sa{};
-            sa.a = s->view(); sa.b = sa.a;
-            sa.out = scores;
-            sa.n_pairs = count;
-            sa.cursor = ctx->d_score_cursor; sa.run = 1;
-            if (tiles) {
-                sa.condensed = CondensedGrid{first, n, rb0, rb1 - rb0, base};
-                launched = launch_score_condensed(sa, kp, s->max_count, ov, ctx->stream);
-            } else {
-                ctx->launches += launch_condensed_pairs(first, n, i0, std::min(4 * rb1, n) - i0, d_pairs, ctx->stream);
-                sa.pairs = d_pairs;
-                const double mean = s->n_env ? (double)s->total / (double)s->n_env : 0.0;
-                launched = launch_score(sa, kp, s->max_count, s->max_count, mean, mean, ov, ctx->stream);
-            }
-        }
-        if (launched < 0) { st = fail(ctx, LOCOHD_ERR_UNSUPPORTED, "shared memory budget exceeded for %d categories", ctx->kp.C); break; }
-        ctx->launches += launched;
-        if (tiles) ctx->tile_launches += launched;
+        if ((st = score_condensed_chunk(ctx, route, s, first, chunks, rb0, rb1, scores, d_pairs))) break;
         if (cudaGetLastError() != cudaSuccess) { st = fail(ctx, LOCOHD_ERR_CUDA, "condensed launch failed"); break; }
         if (!direct && cudaMemcpyAsync(out_scores + base, d_chunk, count * sizeof(double), cudaMemcpyDeviceToHost,
                                        ctx->stream) != cudaSuccess)
@@ -1736,6 +1791,192 @@ int locohd_score_condensed(locohd_ctx* ctx, const locohd_envset* s, uint64_t fir
     return cleanup(st ? st : st2);
     API_END()
 }
+
+// One call of locohd_score_within[_condensed]: the graph grows chunk by chunk.  Per chunk the rows' entries are
+// counted, scanned and the total read back (one synchronisation), the storage grows to hold them, and the fill kernel
+// writes them behind the entries of the earlier chunks.  Everything is freed unless finish() hands the graph out.
+struct GraphBuild {
+    locohd_ctx* ctx;
+    locohd_graph* g = nullptr;
+    uint64_t cap = 0;                    // entries the storage of g holds room for
+    double* d_chunk = nullptr;           // scores of a chunk
+    uint32_t* d_pairs = nullptr;         // pair list of a chunk (pair route)
+    uint32_t* d_counts = nullptr;        // entries per row of a chunk
+    uint64_t* d_off = nullptr;           // their exclusive scan [rows + 1]
+    uint64_t* d_scan_scratch = nullptr;
+
+    explicit GraphBuild(locohd_ctx* c) : ctx(c) {}
+    ~GraphBuild() {
+        dev_free(ctx, d_chunk); dev_free(ctx, d_pairs); dev_free(ctx, d_counts); dev_free(ctx, d_off);
+        dev_free(ctx, d_scan_scratch);
+        destroy_graph(g);
+    }
+    // An empty graph of rows x cols, and scratch for chunks of at most chunk_rows rows and chunk_scores scores.
+    int start(uint64_t rows, uint64_t cols, uint64_t chunk_rows, uint64_t chunk_scores, bool pair_route) {
+        g = new locohd_graph();
+        g->ctx = ctx; g->rows = rows; g->cols = cols;
+        TRY_ST(dev_alloc(ctx, &g->d_indptr, rows + 1));
+        CU(ctx, cudaMemsetAsync(g->d_indptr, 0, (rows + 1) * sizeof(uint64_t), ctx->stream));
+        if (!chunk_rows) return 0;
+        TRY_ST(dev_alloc(ctx, &d_chunk, chunk_scores));
+        if (pair_route) TRY_ST(dev_alloc(ctx, &d_pairs, 2 * chunk_scores));
+        TRY_ST(dev_alloc(ctx, &d_counts, chunk_rows));
+        TRY_ST(dev_alloc(ctx, &d_off, chunk_rows + 1));
+        return dev_alloc(ctx, &d_scan_scratch, scan_scratch_entries(chunk_rows));
+    }
+    // Moves the entries to storage for exactly nc >= nnz entries.
+    int resize(uint64_t nc) {
+        uint32_t* ni = nullptr;
+        double* ns = nullptr;
+        if (nc && (dev_alloc(ctx, &ni, nc) || dev_alloc(ctx, &ns, nc))) {
+            cudaGetLastError();
+            dev_free(ctx, ni); dev_free(ctx, ns);
+            return fail(ctx, LOCOHD_ERR_CUDA, "no device memory for a graph of %llu entries (%llu entries reached)",
+                        (unsigned long long)nc, (unsigned long long)g->nnz);
+        }
+        if (g->nnz) {
+            CU(ctx, cudaMemcpyAsync(ni, g->d_indices, g->nnz * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ctx->stream));
+            CU(ctx, cudaMemcpyAsync(ns, g->d_scores, g->nnz * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+        }
+        dev_free(ctx, g->d_indices); dev_free(ctx, g->d_scores);
+        g->d_indices = ni; g->d_scores = ns;
+        cap = nc;
+        return 0;
+    }
+    // Geometric growth: the storage never holds room for more than twice the entries reached.
+    int reserve(uint64_t need) { return need <= cap ? 0 : resize(std::max(need, 2 * cap)); }
+    // The entries of one chunk, scored into d_chunk.
+    int add(const GraphChunk& c, bool within) {
+        {
+            ProfScope ps(ctx, LOCOHD_PROF_OTHER);
+            ctx->launches += launch_graph_count(c, within, d_counts, ctx->stream);
+            ctx->launches += launch_scan(d_counts, c.rows, 0, d_off, d_scan_scratch, ctx->d_scan + 2, ctx->stream);
+        }
+        CU(ctx, cudaGetLastError());
+        CU(ctx, cudaMemcpyAsync(ctx->h_scan, ctx->d_scan + 2, sizeof(ScanStats), cudaMemcpyDeviceToHost, ctx->stream));
+        TRY_ST(sync_and_check(ctx));   // also surfaces the scoring kernel's errors of this chunk
+        const uint64_t entries = ctx->h_scan->total;
+        TRY_ST(reserve(g->nnz + entries));
+        {
+            ProfScope ps(ctx, LOCOHD_PROF_OTHER);
+            ctx->launches += launch_graph_fill(c, within, d_off, g->nnz, g->d_indptr, g->d_indices, g->d_scores,
+                                               ctx->stream);
+        }
+        CU(ctx, cudaGetLastError());
+        g->nnz += entries;
+        return 0;
+    }
+    // Closes the last row (the chunk of the condensed vector's last row alone is never launched), trims the storage to
+    // the entries and hands the graph out.
+    int finish(locohd_graph** out) {
+        CU(ctx, cudaMemcpyAsync(g->d_indptr + g->rows, &g->nnz, sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
+        if (cap > g->nnz) TRY_ST(resize(g->nnz));
+        TRY_ST(sync_and_check(ctx));
+        *out = g;
+        g = nullptr;
+        return 0;
+    }
+    static void destroy_graph(locohd_graph* gr) {
+        if (!gr) return;
+        locohd_ctx* c = gr->ctx;
+        DeviceGuard dg(c->device);
+        dev_free(c, gr->d_indptr); dev_free(c, gr->d_indices); dev_free(c, gr->d_scores);
+        delete gr;
+    }
+};
+
+int locohd_score_within(locohd_ctx* ctx, const locohd_envset* a, uint64_t a_first, uint64_t n_a, const locohd_envset* b,
+                        uint64_t b_first, uint64_t n_b, uint32_t wf_idx, int skip_self, double max_score,
+                        locohd_graph** out) {
+    API_BEGIN(ctx)
+    if (out) *out = nullptr;
+    TRY_ST(need_params(ctx));
+    if (!a || !b || !out) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
+    if (a_first > a->n_env || n_a > a->n_env - a_first || b_first > b->n_env || n_b > b->n_env - b_first)
+        return fail(ctx, LOCOHD_ERR_INDEX, "graph range beyond the env-set: A [%llu, +%llu) of %llu, B [%llu, +%llu) of %llu",
+                    (unsigned long long)a_first, (unsigned long long)n_a, (unsigned long long)a->n_env,
+                    (unsigned long long)b_first, (unsigned long long)n_b, (unsigned long long)b->n_env);
+    if (skip_self && a != b) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "skip_self needs the same env-set on both sides");
+    if (n_b > 0xFFFFFFFEull) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "more than 2^32 - 2 columns");
+    if (std::isnan(max_score)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "max_score is NaN");
+    TRY_ST(check_wf_indices(ctx, &wf_idx, 1));
+    if (a->key_is_w != b->key_is_w) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "environment sets were built with different weight-function modes");
+
+    // Route and chunks as in locohd_score_cross; the scores of a chunk always go to the scratch.
+    const PairRoute route = pair_route(ctx, a, b, wf_idx);
+    const uint64_t R = n_a && n_b ? cross_chunk_rows(n_a, n_b, route.tiles ? 8 : 16, route.ov) : 0;
+    GraphBuild gb(ctx);
+    int st = gb.start(n_a, n_b, R, R * n_b, !route.tiles);
+    const int64_t self_off = skip_self ? (int64_t)a_first - (int64_t)b_first : INT64_MIN;
+    for (uint64_t row0 = 0; R && row0 < n_a && !st; row0 += R) {
+        const uint64_t rows = std::min(R, n_a - row0);
+        if ((st = score_cross_chunk(ctx, route, a, a_first + row0, b, b_first, rows, n_b, gb.d_chunk, gb.d_pairs))) break;
+        if (cudaGetLastError() != cudaSuccess) { st = fail(ctx, LOCOHD_ERR_CUDA, "graph launch failed"); break; }
+        st = gb.add(GraphChunk{gb.d_chunk, rows, n_b, row0, skip_self ? self_off + (int64_t)row0 : INT64_MIN, max_score},
+                    false);
+    }
+    if (!st) st = gb.finish(out);
+    const int st2 = sync_and_check(ctx);
+    return st ? st : st2;
+    API_END()
+}
+
+int locohd_score_within_condensed(locohd_ctx* ctx, const locohd_envset* s, uint64_t first, uint64_t n, uint32_t wf_idx,
+                                  double max_score, locohd_graph** out) {
+    API_BEGIN(ctx)
+    if (out) *out = nullptr;
+    TRY_ST(need_params(ctx));
+    if (!s || !out) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null argument");
+    if (first > s->n_env || n > s->n_env - first)
+        return fail(ctx, LOCOHD_ERR_INDEX, "graph range beyond the env-set: [%llu, +%llu) of %llu",
+                    (unsigned long long)first, (unsigned long long)n, (unsigned long long)s->n_env);
+    if (ctx->kp.sd_kind != LOCOHD_SD_HELLINGER && ctx->kp.sd_kind != LOCOHD_SD_KOLMOGOROV_SMIRNOV)
+        return fail(ctx, LOCOHD_ERR_BAD_PARAM,
+                    "an upper-triangle graph needs a symmetric statistical distance (Hellinger or Kolmogorov-Smirnov); "
+                    "locohd_score_within gives both triangles of an asymmetric one");
+    if (n > 0xFFFFFFFEull) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "more than 2^32 - 2 environments");
+    if (std::isnan(max_score)) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "max_score is NaN");
+    TRY_ST(check_wf_indices(ctx, &wf_idx, 1));
+
+    // Route and chunks as in locohd_score_condensed; the scores of a chunk always go to the scratch.
+    const PairRoute route = pair_route(ctx, s, s, wf_idx);
+    const CondensedChunks chunks(n, route.tiles ? 8 : 16, route.ov);
+    GraphBuild gb(ctx);
+    int st = gb.start(n, n, n < 2 ? 0 : n, n < 2 ? 0 : chunks.scratch(), !route.tiles);
+    for (uint64_t rb0 = 0, rb1; n >= 2 && rb0 < chunks.nb && !st; rb0 = rb1) {
+        rb1 = chunks.end(rb0);
+        if (!chunks.scores_of(rb0, rb1)) continue;   // the last row alone: finish() closes it
+        if ((st = score_condensed_chunk(ctx, route, s, first, chunks, rb0, rb1, gb.d_chunk, gb.d_pairs))) break;
+        if (cudaGetLastError() != cudaSuccess) { st = fail(ctx, LOCOHD_ERR_CUDA, "graph launch failed"); break; }
+        const uint64_t i0 = 4 * rb0;
+        st = gb.add(GraphChunk{gb.d_chunk, std::min(4 * rb1, n) - i0, n, i0, INT64_MIN, max_score}, true);
+    }
+    if (!st) st = gb.finish(out);
+    const int st2 = sync_and_check(ctx);
+    return st ? st : st2;
+    API_END()
+}
+
+int locohd_graph_shape(const locohd_graph* g, uint64_t* rows, uint64_t* cols, uint64_t* nnz) {
+    if (!g) return fail(nullptr, LOCOHD_ERR_BAD_PARAM, "null graph");
+    if (rows) *rows = g->rows;
+    if (cols) *cols = g->cols;
+    if (nnz) *nnz = g->nnz;
+    return 0;
+}
+
+int locohd_graph_copy(locohd_ctx* ctx, const locohd_graph* g, uint64_t* indptr, uint32_t* indices, double* scores) {
+    API_BEGIN(ctx)
+    if (!g) return fail(ctx, LOCOHD_ERR_BAD_PARAM, "null graph");
+    if (indptr) CU(ctx, cudaMemcpyAsync(indptr, g->d_indptr, (g->rows + 1) * sizeof(uint64_t), cudaMemcpyDefault, ctx->stream));
+    if (indices && g->nnz)
+        CU(ctx, cudaMemcpyAsync(indices, g->d_indices, g->nnz * sizeof(uint32_t), cudaMemcpyDefault, ctx->stream));
+    if (scores && g->nnz) CU(ctx, cudaMemcpyAsync(scores, g->d_scores, g->nnz * sizeof(double), cudaMemcpyDefault, ctx->stream));
+    return sync_and_check(ctx);
+    API_END()
+}
+
+void locohd_graph_destroy(locohd_graph* g) { GraphBuild::destroy_graph(g); }
 
 int locohd_condensed_unit(uint64_t n, uint64_t row_block0, uint64_t row_blocks, uint64_t unit, uint64_t* out_row_block,
                           uint64_t* out_col_block) {

@@ -2875,6 +2875,73 @@ __global__ void __launch_bounds__(kTopkWarps * 32) row_topk_kernel(const double*
     }
 }
 
+// Threshold graphs: the entries s <= max_score of a chunk of scores as CSR rows.  One warp per row; a ballot per tile
+// of 32 columns gives every lane its slot (the entries below it in the tile plus the row's running count), so the
+// columns come out ascending and the result is a function of the scores alone.  NaN never passes the comparison.
+constexpr int kGraphWarps = 8;
+
+template <bool WITHIN>
+__device__ __forceinline__ void graph_row(const GraphChunk& g, uint64_t r, const double** row, uint64_t* len,
+                                          uint64_t* col0, uint64_t* skip) {
+    if (WITHIN) {   // row i of the condensed slice that starts at (row0, row0 + 1)
+        const uint64_t i = g.row0 + r, n = g.cols;
+        *row = g.scores + ((n * i - triangle<uint64_t>(i)) - (n * g.row0 - triangle<uint64_t>(g.row0)));
+        *len = n - 1 - i;
+        *col0 = i + 1;
+        *skip = ~0ull;
+    } else {
+        *row = g.scores + r * g.cols;
+        *len = g.cols;
+        *col0 = 0;
+        *skip = g.self_off == INT64_MIN ? ~0ull : (uint64_t)((int64_t)r + g.self_off);
+    }
+}
+
+template <bool WITHIN>
+__global__ void __launch_bounds__(kGraphWarps * 32) graph_count_kernel(const GraphChunk g, uint32_t* __restrict__ counts) {
+    const int lane = threadIdx.x & 31;
+    const uint64_t r = (uint64_t)blockIdx.x * kGraphWarps + (threadIdx.x >> 5);
+    if (r >= g.rows) return;
+    const double* row;
+    uint64_t len, col0, skip;
+    graph_row<WITHIN>(g, r, &row, &len, &col0, &skip);
+    uint32_t c = 0;
+    for (uint64_t j0 = 0; j0 < len; j0 += 32) {
+        const uint64_t j = j0 + lane;
+        c += __popc(__ballot_sync(kFull, j < len && j != skip && __ldg(row + j) <= g.max_score));
+    }
+    if (lane == 0) counts[r] = c;
+}
+
+template <bool WITHIN>
+__global__ void __launch_bounds__(kGraphWarps * 32) graph_fill_kernel(const GraphChunk g, const uint64_t* __restrict__ off,
+                                                                      uint64_t nnz0, uint64_t* __restrict__ indptr,
+                                                                      uint32_t* __restrict__ indices,
+                                                                      double* __restrict__ values) {
+    const int lane = threadIdx.x & 31;
+    const uint64_t r = (uint64_t)blockIdx.x * kGraphWarps + (threadIdx.x >> 5);
+    if (r >= g.rows) return;
+    const double* row;
+    uint64_t len, col0, skip;
+    graph_row<WITHIN>(g, r, &row, &len, &col0, &skip);
+    const unsigned below = (1u << lane) - 1u;
+    uint64_t at = nnz0 + off[r];
+#pragma unroll 1   // unrolled, the within-mode instantiation spills at the 32 registers ptxas gives it
+    for (uint64_t j0 = 0; j0 < len; j0 += 32) {
+        const uint64_t j = j0 + lane;
+        const double s = j < len ? __ldg(row + j) : 0.0;
+        const bool in = j < len && j != skip && s <= g.max_score;
+        const unsigned b = __ballot_sync(kFull, in);
+        if (in) {
+            const uint64_t k = at + __popc(b & below);
+            indices[k] = (uint32_t)(col0 + j);
+            values[k] = s;
+        }
+        at += __popc(b);
+    }
+    if (lane == 0) indptr[g.row0 + r + 1] = at;
+}
+
 // ------------------------------------------------------------------------------------------------
 // f32 wire format, per-frame centroids, weight-function index check, per-anchor statistics over jobs
 // ------------------------------------------------------------------------------------------------
@@ -3540,6 +3607,23 @@ int launch_row_topk(const double* scores, uint64_t rows, uint64_t cols, int k, i
     cudaFuncSetAttribute(row_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     row_topk_kernel<<<(unsigned)((rows + kTopkWarps - 1) / kTopkWarps), kTopkWarps * 32, smem, st>>>(
         scores, rows, cols, k, self_off, knn_scores, knn_index);
+    return 1;
+}
+
+int launch_graph_count(const GraphChunk& g, bool within, uint32_t* counts, cudaStream_t st) {
+    if (!g.rows) return 0;
+    const unsigned grid = blocks_for(g.rows, kGraphWarps);
+    if (within) graph_count_kernel<true><<<grid, kGraphWarps * 32, 0, st>>>(g, counts);
+    else graph_count_kernel<false><<<grid, kGraphWarps * 32, 0, st>>>(g, counts);
+    return 1;
+}
+
+int launch_graph_fill(const GraphChunk& g, bool within, const uint64_t* off, uint64_t nnz0, uint64_t* indptr,
+                      uint32_t* indices, double* values, cudaStream_t st) {
+    if (!g.rows) return 0;
+    const unsigned grid = blocks_for(g.rows, kGraphWarps);
+    if (within) graph_fill_kernel<true><<<grid, kGraphWarps * 32, 0, st>>>(g, off, nnz0, indptr, indices, values);
+    else graph_fill_kernel<false><<<grid, kGraphWarps * 32, 0, st>>>(g, off, nnz0, indptr, indices, values);
     return 1;
 }
 

@@ -342,6 +342,22 @@ int launch_condensed_pairs(uint64_t first, uint64_t n, uint64_t i0, uint64_t row
 // writes knn_scores / knn_index [r * k ...] (either may be nullptr); every row must have k eligible columns.
 int launch_row_topk(const double* scores, uint64_t rows, uint64_t cols, int k, int64_t self_off, double* knn_scores,
                     uint32_t* knn_index, cudaStream_t st);
+// A chunk of scores as rows of a threshold graph (entries s <= max_score).  Between mode: row r (< rows) holds the
+// `cols` scores at scores[r * cols], column j relative to the column range; column self_off + r is left out (self_off
+// = INT64_MIN: none is).  Within mode: row r is row i = row0 + r of the condensed vector of cols = n environments,
+// scores[0] its entry (row0, row0 + 1); the row holds the n - 1 - i columns j > i.  Row r is row row0 + r of the graph.
+struct GraphChunk {
+    const double* scores;
+    uint64_t rows, cols, row0;
+    int64_t self_off;
+    double max_score;
+};
+// counts[r] = the entries of row r
+int launch_graph_count(const GraphChunk& g, bool within, uint32_t* counts, cudaStream_t st);
+// off: exclusive scan of the counts [rows + 1].  Entry k of row r (columns ascending) goes to indices / values
+// [nnz0 + off[r] + k]; indptr[row0 + r + 1] = nnz0 + off[r + 1].
+int launch_graph_fill(const GraphChunk& g, bool within, const uint64_t* off, uint64_t nnz0, uint64_t* indptr,
+                      uint32_t* indices, double* values, cudaStream_t st);
 // Launch geometry of score_tile_kernel for environments of at most max_a / max_b members (teams = 0: the kernel does
 // not apply; below kTileMinTeams teams the pair kernel is the better one and pairs do not take the tile route).  The one
 // place that decides it: launch_tiles, the tile route of locohd_capi.cu and locohd_tile_geometry read it.

@@ -15,6 +15,12 @@ Shapes:
     calls alternated rep by rep: the first 20 000 environments into device and into host memory, the first 50 000
     into device memory only (a 20 GB matrix), each on the tile route and the LOCOHD_NO_TILES=1 pair route; the
     vector is checked bit for bit against the matrix's strict upper triangle on the device.
+  * threshold graphs (locohd_score_within[_condensed], names starting with "within"), alternated with the dense calls
+    they replace: 2 000 x 50 000 on both routes at max_score = the 0.1 %, 10 % and 100 % quantiles of that matrix,
+    the graph kept on the device against score_cross into a device matrix, and the graph copied to host arrays (what
+    LoCoHD.environments_within returns) against score_cross into host memory (score_matrix); the first 20 000
+    environments in within mode against score_condensed into device and host memory.  Every graph is checked bit for
+    bit against the thresholded dense result.
 Times are host clocks around whole calls (each ends in a device synchronisation): median of --reps after --warmup.
 The card's name and power limit are read in the same run.  Prints one JSON line per measurement, appends them to --out.
 --lib runs against another build of the library (the A/B of the kernel's unit order); --only restricts to names
@@ -171,6 +177,7 @@ def main():
     kj = blocked_jobs(0, 1, PER, 10_000)
     timed("score_batch_1x10000", 1e4, lambda: ctx.score_jobs_stats(env, env, kj, scores=True))
 
+    within(ctx, env)
     condensed(ctx, env)
     env.close()
     st.close()
@@ -195,6 +202,82 @@ def alternated(name, a, b):
               "ms_min": round(1e3 * min(t[label]), 3), "ms_max": round(1e3 * max(t[label]), 3),
               "pairs_per_s": pairs / med[label]})
     emit({"name": f"{name}_ratio", f"{a[0]}_over_{b[0]}": round(med[a[0]] / med[b[0]], 4)})
+
+
+def graph_equals(g, indptr, indices, scores):
+    ip, ix, sc = g.copy()
+    return bool(np.array_equal(ip, indptr) and np.array_equal(ix, indices) and
+                np.array_equal(sc.view(np.uint64), scores.view(np.uint64)))
+
+
+def within(ctx, env):
+    n_a, n_b = 2000, 50_000
+    for route in ("tiles", "pairs"):
+        name = f"within_2000x50000_{route}"
+        if args.only not in name:
+            continue
+        if route == "pairs":
+            os.environ["LOCOHD_NO_TILES"] = "1"
+        M = ctx.score_cross(env, env, 0, n_a, PER, n_b)[0]
+        dev = torch.empty((n_a, n_b), dtype=torch.float64, device="cuda")
+        for q, bound in zip((0.001, 0.1, 1.0), np.quantile(M, (0.001, 0.1, 1.0))):
+            bound = float(bound)
+            t0 = ctx.tile_launches
+            g = ctx.score_within(env, env, bound, 0, n_a, PER, n_b)
+            keep = M <= bound
+            r, c = np.nonzero(keep)
+            indptr = np.concatenate([[0], np.cumsum(keep.sum(axis=1))]).astype(np.uint64)
+            emit({"name": f"{name}_q{q}", "max_score": bound, "nnz": g.nnz, "density": g.nnz / (n_a * n_b),
+                  "tile_launches": ctx.tile_launches - t0,
+                  "bit_identical_to_thresholded_matrix": graph_equals(g, indptr, c.astype(np.uint32), M[r, c])})
+            g.close()
+            del keep, r, c
+            alternated(f"{name}_q{q}_device",
+                       ("graph", n_a * n_b, lambda: ctx.score_within(env, env, bound, 0, n_a, PER, n_b).close()),
+                       ("matrix", n_a * n_b, lambda: ctx.score_cross(env, env, 0, n_a, PER, n_b, scores=dev.data_ptr())))
+
+            def to_host():
+                g = ctx.score_within(env, env, bound, 0, n_a, PER, n_b)
+                g.copy()
+                g.close()
+
+            alternated(f"{name}_q{q}_host", ("graph", n_a * n_b, to_host),
+                       ("matrix", n_a * n_b, lambda: ctx.score_cross(env, env, 0, n_a, PER, n_b)))
+        del M, dev
+        torch.cuda.empty_cache()
+    os.environ.pop("LOCOHD_NO_TILES", None)
+    n = 20_000
+    name = f"within_condensed_{n}_tiles"
+    if args.only not in name:
+        return
+    c = ctx.score_condensed(env, 0, n)
+    k = [int(q * (len(c) - 1)) for q in (0.001, 0.1)]
+    part = np.partition(c, k)
+    vec = torch.empty(len(c), dtype=torch.float64, device="cuda")
+    for q, bound in ((0.001, part[k[0]]), (0.1, part[k[1]]), (1.0, c.max())):
+        bound = float(bound)
+        g = ctx.score_within_condensed(env, bound, 0, n)
+        iu, ju = np.triu_indices(n, 1)
+        keep = c <= bound
+        indptr = np.zeros(n + 1, np.uint64)
+        indptr[1:] = np.cumsum(np.bincount(iu[keep], minlength=n))
+        emit({"name": f"{name}_q{q}", "max_score": bound, "nnz": g.nnz, "density": g.nnz / len(c),
+              "bit_identical_to_thresholded_condensed": graph_equals(g, indptr, ju[keep].astype(np.uint32), c[keep])})
+        g.close()
+        del iu, ju, keep
+        alternated(f"{name}_q{q}_device",
+                   ("graph", len(c), lambda: ctx.score_within_condensed(env, bound, 0, n).close()),
+                   ("condensed", len(c), lambda: ctx.score_condensed(env, 0, n, out=vec.data_ptr())))
+
+        def to_host():
+            g = ctx.score_within_condensed(env, bound, 0, n)
+            g.copy()
+            g.close()
+
+        alternated(f"{name}_q{q}_host", ("graph", len(c), to_host),
+                   ("condensed", len(c), lambda: ctx.score_condensed(env, 0, n)))
+    del c, part, vec
+    torch.cuda.empty_cache()
 
 
 def condensed(ctx, env):
